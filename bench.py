@@ -25,8 +25,11 @@ One "step" = one vector env step (B env-steps per GPU).
              "port-implicit" = the oracle's right-hand side under an adaptive variable-order BDF at rtol = atol = 1e-6 (the
              class of solver the reference uses, CasADi CVODES, which is not installable here) -- the faster one is `value`.
   --impl reference  times that faster CPU arm alone (rank 0), sample sized for >= 10 s whatever --steps is.
+  --dump-outputs DIR  after the timed steps, writes what the headline's last timed step returned (rank 0's envs) as .npy files, so
+             that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs B] [--integrator graded|fixed]
+                    [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...      (one rank per GPU)
 """
 import argparse
@@ -56,6 +59,25 @@ def flop_per_env_step(rk4_steps):
 def algorithmic_bytes_per_env_step(obs_dim):
     # SURVEY.md 8d: read x,u,action,scalars ; write x,u,obs,reward,done,info (+ per-CTA weather tile, amortised)
     return (224 + 48 + 24 + 16) + (224 + 48 + obs_dim * 4 + 8 + 1 + 88) + 16
+
+
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much, all files together
+
+
+def dump_outputs(path, obs, reward, done):
+    """Writes one step's outputs to `path`: obs.npy [n, obs_dim] f32, reward.npy [n] f64, done.npy [n] f32 (0 / 1) and
+    env_index.npy [n] f64, the env each row belongs to.  All rows if they fit in DUMP_BYTES, else a sample of rows drawn with a
+    fixed seed, so that the same batch size always selects the same envs."""
+    B = obs.shape[0]
+    row_bytes = obs.shape[1] * 4 + 8 + 4 + 8
+    idx = np.arange(B)
+    if B * row_bytes > DUMP_BYTES - 4096:  # 4096: room for the four .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(B, (DUMP_BYTES - 4096) // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    out = {"obs": obs[idx].astype(np.float32), "reward": reward[idx].astype(np.float64), "done": done[idx].astype(np.float32),
+           "env_index": idx.astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def csrc_hash():
@@ -305,6 +327,8 @@ def run_ours(args, rank, world, local):
     total_ms, kernel_ms, micro, launches = time_steps(env, actions, K, Wm, flush, barrier, dev, world)
     value = world * B * K / (total_ms * 1e-3)
     finite = bool(torch.isfinite(env.state_t).all().item())
+    # what step_tensor returned in the last timed step (device views the next step overwrites): host copies, written at the end
+    last_step = (env.obs_t.cpu().numpy(), env.reward_t.cpu().numpy(), env.done_t.cpu().numpy()) if args.dump_outputs and rank == 0 else None
 
     # ---- end to end through the numpy VecEnv API (host buffers, copies inside the timed region)
     a_host = actions[Wm:].cpu().numpy()
@@ -383,8 +407,8 @@ def run_ours(args, rank, world, local):
         stats_allreduce = {"error": str(exc)[:300]}
     env.close()
 
-    # ---- further workloads inside the same run
-    Kx, Wx = max(3, min(K, 6)), 3
+    # ---- further workloads inside the same run, K timed steps each like the headline
+    Wx = 3
     configs = {}
     other = "fixed" if args.integrator == "graded" else "graded"
     configs[f"config2_{other}"] = extra_config(
@@ -393,7 +417,7 @@ def run_ours(args, rank, world, local):
         dict(integrator=other, precision="fp64"), B, K, Wm, flush, barrier, dev, world, rank, local, peak64)
     configs["saturated_fp64"] = extra_config(
         "saturated_fp64", "262 144 envs per GPU, fp64 parity mode, nominal parameters, one weather table (the regime the one-CTA-per-32-envs "
-        "design is built for; BASELINE configs[4] sweep point)", dict(integrator=args.integrator, precision="fp64"), 262144, Kx, Wx, flush,
+        "design is built for; BASELINE configs[4] sweep point)", dict(integrator=args.integrator, precision="fp64"), 262144, K, Wx, flush,
         barrier, dev, world, rank, local, peak64)
     configs["config3_fp32_uncertainty"] = extra_config(
         "config3_fp32_uncertainty", "BASELINE configs[2]: 262 144 envs per GPU, fp32 throughput mode (flux units fp32, RK4 state fp64), "
@@ -402,11 +426,11 @@ def run_ours(args, rank, world, local):
         "leaf mass) and their CTAs run twice the RK4 steps (27.5 ms per step; 20.5 after 12 steps); a whole season averages 18.2 ms per "
         "step (profiles/r2_season_throughput.txt)",
         dict(integrator=args.integrator, precision="fp32", uncertainty_scale=0.3, base_env_params=dict(start_train_day=0, end_train_day=18)),
-        262144, Kx, 24, flush, barrier, dev, world, rank, local, peak32)
+        262144, K, 24, flush, barrier, dev, world, rank, local, peak32)
     if world >= 8:
         configs["config4_65536_per_gpu"] = extra_config(
             "config4_65536_per_gpu", "BASELINE configs[3] shape: 65 536 envs per GPU x 8 GPUs, fp64, U(-1,1) actions resident on the device",
-            dict(integrator=args.integrator, precision="fp64"), 65536, Kx, Wx, flush, barrier, dev, world, rank, local, peak64)
+            dict(integrator=args.integrator, precision="fp64"), 65536, K, Wx, flush, barrier, dev, world, rank, local, peak64)
 
     if rank == 0:
         peak = peak64 if args.precision == "fp64" else peak32
@@ -471,6 +495,8 @@ def run_ours(args, rank, world, local):
                                  note="value = the faster CPU arm; 'port' runs the GPU arm's RK4 contract, 'port-implicit' an adaptive BDF at the "
                                       "reference solver's tolerances (rtol = atol = 1e-6) on the same right-hand side"),
         }
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, *last_step)
         emit(line)
 
 
@@ -486,7 +512,11 @@ def main():
     ap.add_argument("--role-warps", type=int, default=0)
     ap.add_argument("--precision", default="fp64", choices=["fp64", "fp32"],
                     help="fp64 = parity mode (the BASELINE metric); fp32 = throughput mode (flux groups in fp32, RK4 state in fp64)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's last timed step (observations, rewards, dones of rank 0's envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the CPU arm's sample size follows its measured speed, so its inputs vary")
     if args.integrator is None:
         args.integrator = "graded"  # == glgym.vec_env.DEFAULT_INTEGRATOR (not imported here: --impl reference must not need torch)
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))

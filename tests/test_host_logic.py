@@ -250,3 +250,29 @@ def test_bench_contract_helpers():
     prof = json.load(open(os.path.join(ROOT, "profiles", "r2_traffic.json")))
     assert {"csrc_sha16", "graded_fp64_B4096", "fixed_fp64_B4096", "graded_fp64_B262144"} <= set(prof)
     assert prof["csrc_sha16"] == open(os.path.join(ROOT, "profiles", "r2_csrc_sha16.txt")).read().strip()
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every row while the files fit the byte limit, above it a fixed seeded sample of rows that stays
+    under the limit; float32 / float64 files only."""
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(0)
+    B, D = 300, 263
+    obs, rew, done = rng.random((B, D), dtype=np.float32), rng.random(B), (rng.random(B) < 0.1).astype(np.uint8)
+    bench.dump_outputs(str(tmp_path / "all"), obs, rew, done)
+    z = {n: np.load(tmp_path / "all" / f"{n}.npy") for n in ("obs", "reward", "done", "env_index")}
+    assert {a.dtype for a in z.values()} <= {np.dtype(np.float32), np.dtype(np.float64)}
+    assert np.array_equal(z["obs"], obs) and np.array_equal(z["reward"], rew) and np.array_equal(z["done"], done)
+    assert np.array_equal(z["env_index"], np.arange(B))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 100 * (D * 4 + 20))
+    samples = []
+    for tag in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / tag), obs, rew, done)
+        assert sum(f.stat().st_size for f in (tmp_path / tag).iterdir()) <= bench.DUMP_BYTES
+        samples.append({n: np.load(tmp_path / tag / f"{n}.npy") for n in ("obs", "reward", "done", "env_index")})
+    idx = samples[0]["env_index"].astype(np.int64)
+    assert len(idx) == 100 and np.all(np.diff(idx) > 0)
+    assert all(np.array_equal(samples[0][n], samples[1][n]) for n in samples[0])
+    assert np.array_equal(samples[0]["obs"], obs[idx]) and np.array_equal(samples[0]["reward"], rew[idx])

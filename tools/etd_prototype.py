@@ -5,8 +5,9 @@ work.  Error against the Radau(1e-12) truth fixtures, WITHOUT the transient-stif
 top-compartment mode exceeds the step's stability limit therefore diverge at the coarse grids).  Result recorded in DESIGN.md
 "Known limits": 215 steps (n_sub 180) stay within 3.5e-7 on the random-action set, 192 steps within 6.8e-7 -- 1.4-1.5x fewer steps
 than the shipped 300 at a 2-3x margin to the 1e-6 gate instead of 19x.      python tools/etd_prototype.py"""
-import sys, numpy as np, time
-sys.path.insert(0,'/root/repo/tests'); sys.path.insert(0,'/root/repo/greenlight-gym2_b200')
+import os, sys, numpy as np, time
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, os.path.join(ROOT, "greenlight-gym2_b200"))
 import oracle_binding as ob
 def phis(z):
     # phi1..phi3 at z (z <= 0), series for small |z|
@@ -57,7 +58,8 @@ def integrate(x, u, d, p, n_sub, sched, etd=True):
     return x, steps
 if __name__ == "__main__":
     rel=lambda a,b: float(np.max(np.abs(a-b)/np.maximum(np.abs(b),1e-3)))
-    zr=np.load('/root/repo/tests/golden/truth_random_actions.npz'); zb=np.load('/root/repo/tests/golden/truth_rule_based.npz')
+    gold = os.path.join(ROOT, "tests", "golden")
+    zr=np.load(os.path.join(gold, "truth_random_actions.npz")); zb=np.load(os.path.join(gold, "truth_rule_based.npz"))
     sets={"random":(zr, range(0,120,4)), "rule-based":(zb, range(0,249,6))}
     for n_sub, sched in ((260,[16,8,4,4,4,4,2,2,2,2,2,2]), (180,[16,8,4,4,4,2,2,2,2]), (150,[16,8,8,4,4,4,2,2,2,2]), (120,[32,16,8,4,4,4,2,2,2,2]), (100,[32,16,8,4,4,4,2,2,2,2])):
         for name,(z,idx) in sets.items():
