@@ -23,6 +23,7 @@
 #include "glg_kernels.cuh"
 #include "glg_roles.cuh"
 #include "glg_rollout.cuh"
+#include "glg_replay.cuh"
 
 
 static thread_local std::string g_create_error = "";
@@ -42,6 +43,7 @@ struct glg_handle {
     double *weather = nullptr, *start_day = nullptr;
     int *reset_tables = nullptr;
     int n_tables = 0, rows = 0, n_reset_tables = 0;
+    unsigned long long weather_gen = 0;  // bumped by every glg_set_weather: replay buffers hold keys into the bank
     // pinned host staging for glg_step_host
     float *h_actions = nullptr, *h_obs = nullptr;
     double *h_reward = nullptr;
@@ -312,6 +314,7 @@ extern "C" int glg_set_weather(glg_handle *h, const double *tables_host, int32_t
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaFree(h->weather); cudaFree(h->start_day); cudaFree(h->reset_tables);
     h->weather = nullptr; h->start_day = nullptr; h->reset_tables = nullptr;
+    ++h->weather_gen;
     const size_t n = (size_t)n_tables * rows * GLG_ND;
     GLG_CUDA(h, cudaMalloc((void **)&h->weather, n * sizeof(double)));
     GLG_CUDA(h, cudaMemcpy(h->weather, tables_host, n * sizeof(double), cudaMemcpyHostToDevice));
@@ -986,6 +989,215 @@ extern "C" float *glg_rollout_starts_dev(glg_handle *h) { return h ? h->roll_sta
 extern "C" float *glg_rollout_advantages_dev(glg_handle *h) { return h ? h->roll_adv : nullptr; }
 extern "C" float *glg_rollout_returns_dev(glg_handle *h) { return h ? h->roll_ret : nullptr; }
 extern "C" double *glg_rollout_stats_dev(glg_handle *h) { return h ? h->roll_stat : nullptr; }
+
+// ---- device replay buffer (glg_replay.cuh): its own object, so several can share an env and none dangles from the handle ----
+struct glg_replay {
+    glg_handle *h = nullptr;
+    int device = 0;
+    glg_replay_config cfg = {};
+    unsigned long long weather_gen = 0;  // bank generation the keys refer to
+    long long cap = 0, pos = 0;
+    bool full = false, is_reset = false;
+    uint32_t calls = 0;  // sample calls so far (Philox counter)
+    int blocks = 0, n_head = 0, nf = 0;
+    size_t bytes = 0;
+    float *obs_norm = nullptr, *last_head = nullptr, *head_obs = nullptr, *head_next = nullptr, *act = nullptr, *rew = nullptr;
+    int *key_obs = nullptr, *key_next = nullptr, *anchor_t = nullptr, *anchor_tbl = nullptr;
+    unsigned char *dn = nullptr;
+    double *stat = nullptr, *partial = nullptr, *norm64 = nullptr, *ret = nullptr;
+};
+
+extern "C" void glg_replay_destroy(glg_replay *r) {
+    if (!r) return;
+    cudaSetDevice(r->device);  // the handle may already be gone: nothing here reads it
+    cudaFree(r->obs_norm); cudaFree(r->last_head); cudaFree(r->head_obs); cudaFree(r->head_next); cudaFree(r->act); cudaFree(r->rew);
+    cudaFree(r->key_obs); cudaFree(r->key_next); cudaFree(r->anchor_t); cudaFree(r->anchor_tbl); cudaFree(r->dn);
+    cudaFree(r->stat); cudaFree(r->partial); cudaFree(r->norm64); cudaFree(r->ret);
+    delete r;
+}
+
+template <typename T>
+static cudaError_t replay_alloc(glg_replay *r, T **p, size_t n) {
+    r->bytes += n * sizeof(T);
+    return dev_alloc(p, n);
+}
+
+extern "C" int glg_replay_create(glg_handle *h, const glg_replay_config *cfg, glg_replay **out) {
+    if (!h || !cfg || !out) {
+        g_create_error = "glg_replay_create: null argument";
+        return GLG_ERR_ARG;
+    }
+    *out = nullptr;
+    if (cfg->buffer_size < 1 || !(cfg->gamma >= 0.0 && cfg->gamma <= 1.0) || !(cfg->clip_obs > 0) || !(cfg->clip_reward > 0) ||
+        !(cfg->epsilon > 0))
+        return fail(h, GLG_ERR_ARG, "glg_replay_create: invalid buffer_size / gamma / clip / epsilon");
+    if (!h->have_weather) return fail(h, GLG_ERR_STATE, "glg_replay_create: weather bank not set (glg_set_weather)");
+    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim;
+    const long long cap = cfg->buffer_size / h->B > 1 ? cfg->buffer_size / h->B : 1;  // ReplayBuffer: max(buffer_size // n_envs, 1)
+    if (cap > INT32_MAX) return fail(h, GLG_ERR_ARG, "glg_replay_create: more than 2^31 - 1 slots per env");
+    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+    glg_replay *r = new (std::nothrow) glg_replay();
+    if (!r) return fail(h, GLG_ERR_ALLOC, "glg_replay_create: out of host memory");
+    r->h = h;
+    r->device = h->cfg.device;
+    r->cfg = *cfg;
+    r->weather_gen = h->weather_gen;
+    r->cap = cap;
+    r->blocks = (int)((B + GLG_ROLL_ROWS - 1) / GLG_ROLL_ROWS);
+    r->nf = h->fc_off >= 0 ? 5 * h->cfg.Np : 0;
+    r->n_head = h->obs_dim - r->nf;
+    const size_t CB = (size_t)cap * B, H = (size_t)r->n_head;
+    cudaError_t e = replay_alloc(r, &r->head_obs, CB * H);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->head_next, CB * H);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->key_obs, CB);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->key_next, CB);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->act, CB * GLG_NU);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->rew, CB);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->dn, CB);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->obs_norm, B * D);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->last_head, B * H);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->anchor_t, B);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->anchor_tbl, B);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->ret, B);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->stat, (D + 1) * 3);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->partial, (size_t)r->blocks * (D + 1) * 2);
+    if (e == cudaSuccess) e = replay_alloc(r, &r->norm64, (D + 1) * 2);
+    if (e == cudaSuccess) {
+        std::vector<double> st((D + 1) * 3);
+        for (size_t c = 0; c <= D; ++c) {  // RunningMeanStd: mean 0, var 1, count 1e-4
+            st[3 * c] = 0.0;
+            st[3 * c + 1] = 1.0;
+            st[3 * c + 2] = 1e-4;
+        }
+        e = cudaMemcpy(r->stat, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) {
+        glg_replay_destroy(r);
+        return fail(h, GLG_ERR_CUDA, (std::string("glg_replay_create: ") + cudaGetErrorString(e)).c_str());
+    }
+    *out = r;
+    return GLG_OK;
+}
+
+static int replay_check(glg_replay *r, const char *what) {
+    glg_handle *h = r->h;
+    if (r->weather_gen != h->weather_gen) {
+        h->err = std::string(what) + ": the weather bank was replaced (glg_set_weather) after this replay buffer was created; "
+                                     "its stored forecast keys no longer refer to it";
+        return GLG_ERR_STATE;
+    }
+    return GLG_OK;
+}
+
+// the VecNormalize part of a store / reset: glg_rollout.cuh's kernels on the buffer's own statistics
+static void replay_normalize(glg_replay *r, bool after_step, cudaStream_t s) {
+    glg_handle *h = r->h;
+    GlgRollArgs a;
+    memset(&a, 0, sizeof a);
+    a.B = h->B; a.obs_dim = h->obs_dim; a.n_blocks = r->blocks;
+    a.training = r->cfg.training; a.norm_obs = r->cfg.norm_obs; a.norm_reward = r->cfg.norm_reward;
+    a.gamma = r->cfg.gamma; a.clip_obs = r->cfg.clip_obs; a.clip_reward = r->cfg.clip_reward; a.epsilon = r->cfg.epsilon;
+    a.obs = h->obs;
+    a.reward = after_step ? h->reward : nullptr;
+    a.done = after_step ? h->done : nullptr;
+    a.ret = r->ret; a.stat = r->stat; a.partial = r->partial; a.norm64 = r->norm64;
+    a.obs_out = r->obs_norm;
+    glg_roll_moments_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(a);
+    glg_roll_finish_kernel<<<(h->obs_dim + 1 + GLG_ROLL_NT / 32 - 1) / (GLG_ROLL_NT / 32), GLG_ROLL_NT, 0, s>>>(a);
+    glg_roll_apply_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(a);
+    h->launches += 3;
+}
+
+static void replay_write_args(const glg_replay *r, GlgReplayArgs *w) {
+    const glg_handle *h = r->h;
+    memset(w, 0, sizeof *w);
+    w->B = h->B; w->obs_dim = h->obs_dim; w->n_head = r->n_head; w->nf = r->nf; w->fc_off = h->fc_off; w->Np = h->cfg.Np;
+    w->rows = h->rows; w->auto_reset = h->cfg.auto_reset;
+    w->obs = h->obs; w->term_obs = h->term_obs; w->reward = h->reward; w->done = h->done; w->timestep = h->timestep; w->table = h->table;
+    w->last_head = r->last_head; w->anchor_t = r->anchor_t; w->anchor_tbl = r->anchor_tbl;
+    w->head_obs = r->head_obs; w->head_next = r->head_next; w->key_obs = r->key_obs; w->key_next = r->key_next;
+    w->act = r->act; w->rew = r->rew; w->dn = r->dn;
+}
+
+extern "C" int glg_replay_reset(glg_replay *r, void *stream) {
+    if (!r) return GLG_ERR_ARG;
+    glg_handle *h = r->h;
+    int rc = replay_check(r, "glg_replay_reset");
+    if (rc) return rc;
+    if (!h->is_reset) return fail(h, GLG_ERR_STATE, "glg_replay_reset: the env has not been reset (glg_reset)");
+    GLG_CUDA(h, cudaSetDevice(r->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    replay_normalize(r, false, s);
+    GlgReplayArgs w;
+    replay_write_args(r, &w);
+    w.store = 0;
+    glg_replay_write_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(w);
+    h->launches += 1;
+    GLG_CUDA(h, cudaGetLastError());
+    r->is_reset = true;
+    return GLG_OK;
+}
+
+extern "C" int glg_replay_store(glg_replay *r, const float *actions_dev, void *stream) {
+    if (!r) return GLG_ERR_ARG;
+    glg_handle *h = r->h;
+    if (!actions_dev) return fail(h, GLG_ERR_ARG, "glg_replay_store: actions_dev is NULL");
+    int rc = replay_check(r, "glg_replay_store");
+    if (rc) return rc;
+    if (!r->is_reset) return fail(h, GLG_ERR_STATE, "glg_replay_store: store before glg_replay_reset");
+    GLG_CUDA(h, cudaSetDevice(r->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    replay_normalize(r, true, s);
+    GlgReplayArgs w;
+    replay_write_args(r, &w);
+    w.store = 1;
+    w.slot = (size_t)r->pos;
+    w.actions = actions_dev;
+    glg_replay_write_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(w);
+    h->launches += 1;
+    GLG_CUDA(h, cudaGetLastError());
+    if (++r->pos == r->cap) {
+        r->full = true;
+        r->pos = 0;
+    }
+    return GLG_OK;
+}
+
+extern "C" int glg_replay_sample(glg_replay *r, int32_t n, float *obs_dev, float *next_obs_dev, float *actions_dev,
+                                 float *rewards_dev, float *dones_dev, int32_t *index_dev, void *stream) {
+    if (!r) return GLG_ERR_ARG;
+    glg_handle *h = r->h;
+    if (n < 1 || !obs_dev || !next_obs_dev || !actions_dev || !rewards_dev || !dones_dev)
+        return fail(h, GLG_ERR_ARG, "glg_replay_sample: n < 1 or a NULL output");
+    int rc = replay_check(r, "glg_replay_sample");
+    if (rc) return rc;
+    const long long upper = r->full ? r->cap : r->pos;
+    if (upper == 0) return fail(h, GLG_ERR_STATE, "glg_replay_sample: the replay buffer is empty (no glg_replay_store yet)");
+    GLG_CUDA(h, cudaSetDevice(r->device));
+    GlgReplaySampleArgs S;
+    memset(&S, 0, sizeof S);
+    S.n = n; S.B = h->B; S.obs_dim = h->obs_dim; S.n_head = r->n_head; S.nf = r->nf; S.fc_off = h->fc_off;
+    S.norm_obs = r->cfg.norm_obs; S.norm_reward = r->cfg.norm_reward;
+    S.upper = (uint32_t)upper; S.call = r->calls; S.seed = r->cfg.seed;
+    S.clip_obs = r->cfg.clip_obs; S.clip_reward = r->cfg.clip_reward;
+    S.norm64 = r->norm64;
+    S.weather = h->weather;  // read on every call: glg_set_weather reallocates the bank
+    S.head_obs = r->head_obs; S.head_next = r->head_next; S.key_obs = r->key_obs; S.key_next = r->key_next;
+    S.act = r->act; S.rew = r->rew; S.dn = r->dn;
+    S.obs_out = obs_dev; S.next_out = next_obs_dev; S.act_out = actions_dev; S.rew_out = rewards_dev; S.done_out = dones_dev;
+    S.idx_out = index_dev;
+    constexpr int per_cta = GLG_REPLAY_NT / 32;
+    glg_replay_sample_kernel<<<(n + per_cta - 1) / per_cta, GLG_REPLAY_NT, 0, (cudaStream_t)stream>>>(S);
+    h->launches += 1;
+    GLG_CUDA(h, cudaGetLastError());
+    ++r->calls;
+    return GLG_OK;
+}
+
+extern "C" int64_t glg_replay_size(const glg_replay *r) { return r ? (r->full ? r->cap : r->pos) : 0; }
+extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)r->bytes : 0; }
+extern "C" float *glg_replay_obs_dev(glg_replay *r) { return r ? r->obs_norm : nullptr; }
+extern "C" double *glg_replay_stats_dev(glg_replay *r) { return r ? r->stat : nullptr; }
 
 // ---- episode-statistics all-reduce over NCCL (run-time binding: nccl_api above)
 extern "C" int glg_nccl_unique_id(uint8_t id_out[128]) {

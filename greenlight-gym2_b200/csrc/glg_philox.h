@@ -51,3 +51,11 @@ GLG_HD uint32_t glg_rand_below(uint64_t seed, uint64_t env_id, uint32_t step_ctr
                                      (uint32_t)(seed >> 32));
     return (uint32_t)(((uint64_t)r.v[0] * (uint64_t)n) >> 32);
 }
+
+// replay-buffer index of sample i of sample call `call` (draw block 65, counter (65, call, i, 0), key = the buffer's seed):
+// slot uniform in [0, upper), env uniform in [0, B)  -- ReplayBuffer.sample's two randint draws
+GLG_HD void glg_replay_draw(uint64_t seed, uint32_t call, uint32_t i, uint32_t upper, uint32_t B, uint32_t *slot, uint32_t *env) {
+    GlgPhilox4 r = glg_philox4x32_10(65u, call, i, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
+    *slot = (uint32_t)(((uint64_t)r.v[0] * (uint64_t)upper) >> 32);
+    *env = (uint32_t)(((uint64_t)r.v[1] * (uint64_t)B) >> 32);
+}

@@ -10,6 +10,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch/CUD
     if name == "TomatoEnv":
         from .tomato_env import TomatoEnv
         return TomatoEnv
+    if name == "DeviceReplayBuffer":
+        from .replay import DeviceReplayBuffer
+        return DeviceReplayBuffer
     if name == "GreenLight":
         from .model import GreenLight
         return GreenLight

@@ -38,6 +38,13 @@ class GlgRolloutConfig(C.Structure):
                 ("epsilon", C.c_double)]
 
 
+class GlgReplayConfig(C.Structure):
+    """struct glg_replay_config (include/glgym.h)."""
+    _fields_ = [("buffer_size", C.c_int64), ("training", C.c_int32), ("norm_obs", C.c_int32), ("norm_reward", C.c_int32),
+                ("reserved", C.c_int32), ("gamma", C.c_double), ("clip_obs", C.c_double), ("clip_reward", C.c_double),
+                ("epsilon", C.c_double), ("seed", C.c_uint64)]
+
+
 class GlgEnvState(C.Structure):
     """struct glg_env_state (include/glgym.h): host pointers, NULL = skip."""
     _fields_ = [("x", C.c_void_p), ("u", C.c_void_p), ("timestep", C.c_void_p), ("table", C.c_void_p), ("time", C.c_void_p),
@@ -92,6 +99,15 @@ SIGNATURES = {
     "glg_rollout_advantages_dev": (C.c_void_p, [C.c_void_p]),
     "glg_rollout_returns_dev": (C.c_void_p, [C.c_void_p]),
     "glg_rollout_stats_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_replay_create": (C.c_int, [C.c_void_p, C.POINTER(GlgReplayConfig), C.POINTER(C.c_void_p)]),
+    "glg_replay_destroy": (None, [C.c_void_p]),
+    "glg_replay_reset": (C.c_int, [C.c_void_p, _VP]),
+    "glg_replay_store": (C.c_int, [C.c_void_p, _FP, _VP]),
+    "glg_replay_sample": (C.c_int, [C.c_void_p, C.c_int32, _FP, _FP, _FP, _FP, _FP, _IP, _VP]),
+    "glg_replay_size": (C.c_int64, [C.c_void_p]),
+    "glg_replay_bytes": (C.c_int64, [C.c_void_p]),
+    "glg_replay_obs_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_replay_stats_dev": (C.c_void_p, [C.c_void_p]),
     "glg_nccl_unique_id": (C.c_int, [C.c_void_p]),
     "glg_nccl_init": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "glg_allreduce_stats": (C.c_int, [C.c_void_p, _VP]),

@@ -231,6 +231,46 @@ float *glg_rollout_advantages_dev(glg_handle *h);
 float *glg_rollout_returns_dev(glg_handle *h);
 double *glg_rollout_stats_dev(glg_handle *h);
 
+/* ---- device replay buffer for off-policy agents (SAC) ------------------------------------------------------------------------
+ * SB3 2.6.0's ReplayBuffer (optimize_memory_usage False, handle_timeout_termination True) filled the way
+ * OffPolicyAlgorithm._store_transition fills it behind VecNormalize (RL/utils.py:60-67), as kernels on the handle's outputs
+ * (csrc/glg_replay.cuh).  Its own object: several buffers may share one env handle; destroy each before glg_destroy of the handle.
+ * Capacity max(buffer_size / B, 1) slots per env, a ring indexed by pos with a `full` flag.  Each slot holds, per env, the raw
+ * observation the transition started from, the raw next observation (the terminal observation of an env that finished under
+ * auto_reset), the action, the raw reward (float32) and done.  Observations are stored without their WeatherForecastObservations
+ * block plus the bank row that block is read from (221 B per transition at the default stack instead of 2140 B); the sample
+ * kernel rebuilds the block from the weather bank bit for bit.  So glg_set_weather invalidates every replay buffer of the handle:
+ * their store and sample then fail with GLG_ERR_STATE.  Errors are reported through glg_last_error of the handle. */
+typedef struct glg_replay_config {
+    int64_t buffer_size;  /* transitions over all envs (SB3 buffer_size) */
+    int32_t training;     /* 1: update the running statistics (VecNormalize.training) */
+    int32_t norm_obs, norm_reward, reserved;
+    double gamma, clip_obs, clip_reward, epsilon; /* VecNormalize's; 0.99 / 10 / 10 / 1e-8 by default */
+    uint64_t seed;        /* Philox key of the sample indices */
+} glg_replay_config;
+typedef struct glg_replay glg_replay;
+int glg_replay_create(glg_handle *h, const glg_replay_config *cfg, glg_replay **out);
+void glg_replay_destroy(glg_replay *r);
+/* After glg_reset: the observation statistics are fed with the new observations, which are normalised into glg_replay_obs_dev,
+ * the discounted returns are zeroed and every env's next transition starts from its current observation (VecNormalize.reset).
+ * Stored transitions are kept.  Four launches on `stream`. */
+int glg_replay_reset(glg_replay *r, void *stream);
+/* After any glg_step* of the handle: VecNormalize.step_wait on the new observations and rewards (statistics, normalised current
+ * observation, returns) and the transition into slot pos.  actions_dev float32 [B][6]: the action to store (SB3 stores the
+ * policy's scaled action).  Four launches on `stream`. */
+int glg_replay_store(glg_replay *r, const float *actions_dev, void *stream);
+/* ReplayBuffer.sample(n) with VecNormalize: n transitions drawn with replacement, slot = Philox-uniform in [0, glg_replay_size),
+ * env uniform in [0, B) (glg_replay_draw in csrc/glg_philox.h: draw block 65, counter (65, sample-call number, i, 0), key = seed).
+ * obs_dev / next_obs_dev float32 [n][obs_dim] normalised with the current statistics and clipped, actions_dev float32 [n][6],
+ * rewards_dev float32 [n] normalised by the return statistics and clipped, dones_dev float32 [n]; index_dev int32 [n][2]
+ * receives the drawn (slot, env) pairs, or NULL.  GLG_ERR_STATE on an empty buffer.  One launch on `stream`. */
+int glg_replay_sample(glg_replay *r, int32_t n, float *obs_dev, float *next_obs_dev, float *actions_dev, float *rewards_dev,
+                      float *dones_dev, int32_t *index_dev, void *stream);
+int64_t glg_replay_size(const glg_replay *r);   /* valid slots per env: pos, or the capacity once the ring is full */
+int64_t glg_replay_bytes(const glg_replay *r);  /* device bytes the buffer holds */
+float *glg_replay_obs_dev(glg_replay *r);       /* float32 [B][obs_dim]: normalised current observation */
+double *glg_replay_stats_dev(glg_replay *r);    /* double [obs_dim + 1][3]: running (mean, var, count); last row = returns */
+
 /* Multi-GPU episode statistics (SURVEY 8e): the step path has no collective; the one exchange is a sum of the 16-entry
  * statistics vector over the ranks' handles, once per logging interval -- ncclAllReduce on the handle's device buffer.
  * NCCL is bound at run time (dlopen of libnccl.so.2, the copy torch already loaded when there is one), so libglgym.so has no
