@@ -24,6 +24,7 @@
 #include "glg_roles.cuh"
 #include "glg_rollout.cuh"
 #include "glg_replay.cuh"
+#include "glg_plan.cuh"
 
 
 static thread_local std::string g_create_error = "";
@@ -1198,6 +1199,206 @@ extern "C" int64_t glg_replay_size(const glg_replay *r) { return r ? (r->full ? 
 extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)r->bytes : 0; }
 extern "C" float *glg_replay_obs_dev(glg_replay *r) { return r ? r->obs_norm : nullptr; }
 extern "C" double *glg_replay_stats_dev(glg_replay *r) { return r ? r->stat : nullptr; }
+
+// ---- receding-horizon planner (glg_plan.cuh): its own object holding a second, internal handle of B K planning envs that the
+// unchanged step kernels advance; the env handle is only read ----
+struct glg_plan {
+    glg_handle *h = nullptr;   // the env whose states are planned from (read only)
+    glg_handle *hp = nullptr;  // planning envs: B K, no auto-reset, nominal model; shares h's weather bank (see plan_sync)
+    int device = 0, B = 0, BK = 0;
+    glg_plan_config cfg = {};
+    unsigned long long weather_gen = 0;  // bank generation hp's pointers refer to
+    uint32_t calls = 0;                  // glg_plan_run calls so far (Philox counter word 1)
+    float *mean = nullptr, *std = nullptr, *cand = nullptr;
+    double *ret = nullptr;
+    unsigned char *alive = nullptr;
+};
+
+static constexpr long long kPlanMaxBatch = 4194304;  // B K: the largest batch the step kernels were run at (profiles/r2_config_sweep.txt)
+
+extern "C" void glg_plan_destroy(glg_plan *p) {
+    if (!p) return;
+    cudaSetDevice(p->device);  // the env handle may already be gone: nothing here reads it
+    if (p->hp) {
+        p->hp->weather = nullptr; p->hp->start_day = nullptr; p->hp->reset_tables = nullptr;  // the env's, not hp's
+        glg_destroy(p->hp);
+    }
+    cudaFree(p->mean); cudaFree(p->std); cudaFree(p->cand); cudaFree(p->ret); cudaFree(p->alive);
+    delete p;
+}
+
+extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_plan **out) {
+    if (!h || !cfg || !out) {
+        g_create_error = "glg_plan_create: null argument";
+        return GLG_ERR_ARG;
+    }
+    *out = nullptr;
+    const glg_plan_config &c = *cfg;
+    if (c.horizon < 1 || c.n_candidates < 1 || c.n_elites < 1 || c.n_elites > c.n_candidates || c.n_candidates > GLG_PLAN_MAXK ||
+        c.n_iterations < 1)
+        return fail(h, GLG_ERR_ARG, "glg_plan_create: need horizon >= 1, 1 <= n_elites <= n_candidates <= 4096, n_iterations >= 1");
+    if (!(c.gamma > 0.0 && c.gamma <= 1.0) || !(c.init_std > 0.0 && c.init_std < 3.4e38))  // std is stored as float
+        return fail(h, GLG_ERR_ARG, "glg_plan_create: need 0 < gamma <= 1 and a finite init_std > 0");
+    if ((long long)h->B * c.n_candidates > kPlanMaxBatch)
+        return fail(h, GLG_ERR_ARG, "glg_plan_create: num_envs * n_candidates > 4194304 planning envs");
+    if ((uint64_t)c.n_iterations * (uint64_t)c.horizon * 3u > UINT32_MAX)
+        return fail(h, GLG_ERR_ARG, "glg_plan_create: n_iterations * horizon * 3 must fit the 32-bit Philox counter word");
+    if (!h->have_params || !h->have_weather)
+        return fail(h, GLG_ERR_STATE, "glg_plan_create: set the env's parameters and weather bank first");
+    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+    glg_plan *p = new (std::nothrow) glg_plan();
+    if (!p) return fail(h, GLG_ERR_ALLOC, "glg_plan_create: out of host memory");
+    p->h = h;
+    p->device = h->cfg.device;
+    p->cfg = c;
+    p->B = h->B;
+    p->BK = h->B * c.n_candidates;
+    glg_config pc = h->cfg;  // precision, integrator, n_sub, N, Np, prices, constraints and the observation stack stay the env's
+    pc.num_envs = p->BK;
+    pc.auto_reset = 0;
+    pc.uncertainty_scale = 0.0;
+    pc.env_id_offset = 0;
+    pc.role_warps = 0;
+    pc.role_lanes = 0;
+    int rc = glg_create(&pc, &p->hp);
+    if (rc != GLG_OK) {
+        h->err = std::string("glg_plan_create: planning handle: ") + g_create_error;
+        glg_plan_destroy(p);
+        return rc;
+    }
+    p->hp->is_reset = true;  // every run / evaluate loads its states (fan-out) before stepping
+    const size_t HB6 = (size_t)c.horizon * p->B * GLG_NU, HBK6 = (size_t)c.horizon * p->BK * GLG_NU;
+    cudaError_t e = dev_alloc(&p->mean, HB6);
+    if (e == cudaSuccess) e = dev_alloc(&p->std, HB6);
+    if (e == cudaSuccess) e = dev_alloc(&p->cand, HBK6);
+    if (e == cudaSuccess) e = dev_alloc(&p->ret, (size_t)p->BK);
+    if (e == cudaSuccess) e = dev_alloc(&p->alive, (size_t)p->BK);
+    if (e == cudaSuccess) {
+        std::vector<float> s0(HB6, (float)c.init_std);
+        e = cudaMemcpy(p->std, s0.data(), HB6 * sizeof(float), cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) {
+        glg_plan_destroy(p);
+        return fail(h, GLG_ERR_CUDA, (std::string("glg_plan_create: ") + cudaGetErrorString(e)).c_str());
+    }
+    p->weather_gen = h->weather_gen;
+    *out = p;
+    return GLG_OK;
+}
+
+// Before every run / evaluate: the env must be reset and still hold the bank the planner was created under; its parameters
+// (glg_set_params may have been called since) and bank pointers are copied into the planning handle.  Host fields only.
+static int plan_sync(glg_plan *p, const char *what) {
+    glg_handle *h = p->h, *hp = p->hp;
+    if (p->weather_gen != h->weather_gen) {
+        h->err = std::string(what) + ": the weather bank was replaced (glg_set_weather) after this planner was created";
+        return GLG_ERR_STATE;
+    }
+    if (!h->is_reset) {
+        h->err = std::string(what) + ": the env has not been reset (glg_reset)";
+        return GLG_ERR_STATE;
+    }
+    hp->uni = h->uni;
+    hp->general = h->general;
+    hp->have_params = true;
+    hp->weather = h->weather; hp->start_day = h->start_day; hp->reset_tables = h->reset_tables;
+    hp->n_tables = h->n_tables; hp->rows = h->rows; hp->n_reset_tables = h->n_reset_tables;
+    hp->have_weather = true;
+    return GLG_OK;
+}
+
+static int plan_fanout(glg_plan *p, cudaStream_t s) {
+    glg_handle *h = p->h, *hp = p->hp;
+    GlgPlanFanArgs A;
+    memset(&A, 0, sizeof A);
+    A.B = p->B; A.K = p->cfg.n_candidates;
+    A.x = h->x; A.u = h->u; A.time = h->time; A.timestep = h->timestep; A.table = h->table; A.step_ctr = h->step_ctr;
+    A.px = hp->x; A.pu = hp->u; A.ptime = hp->time; A.pep_return = hp->ep_return; A.pep_info = hp->ep_info;
+    A.ptimestep = hp->timestep; A.ptable = hp->table; A.pep_len = hp->ep_len; A.pstep_ctr = hp->step_ctr; A.pdone = hp->done;
+    A.ret = p->ret; A.alive = p->alive;
+    glg_plan_fanout_kernel<<<(p->BK + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, s>>>(A);
+    GLG_CUDA(h, cudaGetLastError());
+    return GLG_OK;
+}
+
+// H steps of the planning envs with the actions seq[t] ([B K][6] each), discounted returns accumulated into p->ret
+static int plan_rollout(glg_plan *p, const float *seq, cudaStream_t s) {
+    glg_handle *h = p->h, *hp = p->hp;
+    const size_t step_stride = (size_t)p->BK * GLG_NU;
+    double d = 1.0;
+    for (int t = 0; t < p->cfg.horizon; ++t) {
+        const int rc = glg_step(hp, seq + (size_t)t * step_stride, nullptr, s);
+        if (rc != GLG_OK) {
+            h->err = "planning step: " + hp->err;
+            return rc;
+        }
+        glg_plan_accum_kernel<<<(p->BK + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, s>>>(p->BK, d, hp->reward, hp->done, p->ret,
+                                                                                            p->alive);
+        GLG_CUDA(h, cudaGetLastError());
+        d *= p->cfg.gamma;
+    }
+    return GLG_OK;
+}
+
+extern "C" int glg_plan_run(glg_plan *p, float *actions_dev, void *stream) {
+    if (!p) return GLG_ERR_ARG;
+    glg_handle *h = p->h;
+    if (!actions_dev) return fail(h, GLG_ERR_ARG, "glg_plan_run: actions_dev is NULL");
+    int rc = plan_sync(p, "glg_plan_run");
+    if (rc) return rc;
+    GLG_CUDA(h, cudaSetDevice(p->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const glg_plan_config &c = p->cfg;
+    for (int it = 0; it < c.n_iterations; ++it) {
+        if ((rc = plan_fanout(p, s))) return rc;
+        GlgPlanSampleArgs S;
+        memset(&S, 0, sizeof S);
+        S.B = p->B; S.K = c.n_candidates; S.H = c.horizon; S.it = (uint32_t)it; S.call = p->calls; S.seed = c.seed;
+        S.mean = p->mean; S.std = p->std; S.cand = p->cand;
+        glg_plan_sample_kernel<<<(p->BK + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, s>>>(S);
+        GLG_CUDA(h, cudaGetLastError());
+        if ((rc = plan_rollout(p, p->cand, s))) return rc;
+        GlgPlanUpdateArgs U;
+        memset(&U, 0, sizeof U);
+        U.B = p->B; U.K = c.n_candidates; U.E = c.n_elites; U.H = c.horizon;
+        U.ret = p->ret; U.cand = p->cand; U.mean = p->mean; U.std = p->std;
+        U.actions = it + 1 == c.n_iterations ? actions_dev : nullptr;
+        glg_plan_update_kernel<<<p->B, GLG_PLAN_NT, 0, s>>>(U);
+        GLG_CUDA(h, cudaGetLastError());
+    }
+    ++p->calls;
+    return GLG_OK;
+}
+
+extern "C" int glg_plan_evaluate(glg_plan *p, const float *seq_dev, double *returns_dev, void *stream) {
+    if (!p) return GLG_ERR_ARG;
+    glg_handle *h = p->h;
+    if (!seq_dev || !returns_dev) return fail(h, GLG_ERR_ARG, "glg_plan_evaluate: seq_dev or returns_dev is NULL");
+    int rc = plan_sync(p, "glg_plan_evaluate");
+    if (rc) return rc;
+    GLG_CUDA(h, cudaSetDevice(p->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = plan_fanout(p, s))) return rc;
+    if ((rc = plan_rollout(p, seq_dev, s))) return rc;
+    if (returns_dev != p->ret)
+        GLG_CUDA(h, cudaMemcpyAsync(returns_dev, p->ret, (size_t)p->BK * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    return GLG_OK;
+}
+
+extern "C" int glg_plan_shift(glg_plan *p, void *stream) {
+    if (!p) return GLG_ERR_ARG;
+    glg_handle *h = p->h;
+    GLG_CUDA(h, cudaSetDevice(p->device));
+    glg_plan_shift_kernel<<<(p->B * GLG_NU + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, (cudaStream_t)stream>>>(
+        p->B, p->cfg.horizon, (float)p->cfg.init_std, p->mean, p->std);
+    GLG_CUDA(h, cudaGetLastError());
+    return GLG_OK;
+}
+
+extern "C" float *glg_plan_mean_dev(glg_plan *p) { return p ? p->mean : nullptr; }
+extern "C" float *glg_plan_std_dev(glg_plan *p) { return p ? p->std : nullptr; }
+extern "C" float *glg_plan_candidates_dev(glg_plan *p) { return p ? p->cand : nullptr; }
+extern "C" double *glg_plan_returns_dev(glg_plan *p) { return p ? p->ret : nullptr; }
 
 // ---- episode-statistics all-reduce over NCCL (run-time binding: nccl_api above)
 extern "C" int glg_nccl_unique_id(uint8_t id_out[128]) {

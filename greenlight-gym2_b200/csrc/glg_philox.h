@@ -59,3 +59,13 @@ GLG_HD void glg_replay_draw(uint64_t seed, uint32_t call, uint32_t i, uint32_t u
     *slot = (uint32_t)(((uint64_t)r.v[0] * (uint64_t)upper) >> 32);
     *env = (uint32_t)(((uint64_t)r.v[1] * (uint64_t)B) >> 32);
 }
+
+// planner sampling noise of candidate c (draw block 66, counter (66, call, draw, c), key = the planner's seed; draw = (it H + t) 3 + p
+// for component pair p of step t in CEM iteration it): two standard normals by Box-Muller, u1 = 1 - U in (0, 1], u2 = U'
+GLG_HD void glg_plan_normal2(uint64_t seed, uint32_t call, uint32_t draw, uint32_t c, double *z0, double *z1) {
+    GlgPhilox4 r = glg_philox4x32_10(66u, call, draw, c, (uint32_t)seed, (uint32_t)(seed >> 32));
+    const double u1 = 1.0 - glg_u01(r.v[0], r.v[1]), u2 = glg_u01(r.v[2], r.v[3]);
+    const double rad = sqrt(-2.0 * log(u1)), ang = 6.283185307179586 * u2;
+    *z0 = rad * cos(ang);
+    *z1 = rad * sin(ang);
+}

@@ -13,6 +13,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch/CUD
     if name == "DeviceReplayBuffer":
         from .replay import DeviceReplayBuffer
         return DeviceReplayBuffer
+    if name == "DevicePlanner":
+        from .planning import DevicePlanner
+        return DevicePlanner
     if name == "GreenLight":
         from .model import GreenLight
         return GreenLight

@@ -45,6 +45,12 @@ class GlgReplayConfig(C.Structure):
                 ("epsilon", C.c_double), ("seed", C.c_uint64)]
 
 
+class GlgPlanConfig(C.Structure):
+    """struct glg_plan_config (include/glgym.h)."""
+    _fields_ = [("horizon", C.c_int32), ("n_candidates", C.c_int32), ("n_elites", C.c_int32), ("n_iterations", C.c_int32),
+                ("gamma", C.c_double), ("init_std", C.c_double), ("seed", C.c_uint64)]
+
+
 class GlgEnvState(C.Structure):
     """struct glg_env_state (include/glgym.h): host pointers, NULL = skip."""
     _fields_ = [("x", C.c_void_p), ("u", C.c_void_p), ("timestep", C.c_void_p), ("table", C.c_void_p), ("time", C.c_void_p),
@@ -108,6 +114,15 @@ SIGNATURES = {
     "glg_replay_bytes": (C.c_int64, [C.c_void_p]),
     "glg_replay_obs_dev": (C.c_void_p, [C.c_void_p]),
     "glg_replay_stats_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_plan_create": (C.c_int, [C.c_void_p, C.POINTER(GlgPlanConfig), C.POINTER(C.c_void_p)]),
+    "glg_plan_destroy": (None, [C.c_void_p]),
+    "glg_plan_run": (C.c_int, [C.c_void_p, _FP, _VP]),
+    "glg_plan_evaluate": (C.c_int, [C.c_void_p, _FP, _DP, _VP]),
+    "glg_plan_shift": (C.c_int, [C.c_void_p, _VP]),
+    "glg_plan_mean_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_plan_std_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_plan_candidates_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_plan_returns_dev": (C.c_void_p, [C.c_void_p]),
     "glg_nccl_unique_id": (C.c_int, [C.c_void_p]),
     "glg_nccl_init": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "glg_allreduce_stats": (C.c_int, [C.c_void_p, _VP]),

@@ -271,6 +271,50 @@ int64_t glg_replay_bytes(const glg_replay *r);  /* device bytes the buffer holds
 float *glg_replay_obs_dev(glg_replay *r);       /* float32 [B][obs_dim]: normalised current observation */
 double *glg_replay_stats_dev(glg_replay *r);    /* double [obs_dim + 1][3]: running (mean, var, count); last row = returns */
 
+/* ---- receding-horizon planner: model-predictive control by the cross-entropy method (CEM) ------------------------------------
+ * Scores candidate action sequences from the envs' CURRENT states with the step kernels (csrc/glg_plan.cuh) on the same reward as
+ * the env.  A planner belongs to one env handle of B envs; it owns a second, internal handle of B K planning envs (planning env
+ * c = b K + k starts from env b) created with the env's configuration except auto_reset 0, uncertainty_scale 0 (nominal model),
+ * env_id_offset 0 and automatic kernel selection.  The env handle is only read.  Per env it keeps a sampling distribution over
+ * sequences, mean and std float32 [H][B][6] in the action space (initially 0 and init_std), plus a seed and a call counter.
+ * glg_plan_run, each of n_iterations CEM iterations:
+ *   1. fan-out: x, u, timestep, table, clock and step_ctr of env b are copied into its K planning envs (device to device);
+ *      their episode accumulators and done are zeroed.
+ *   2. sample: candidate k = 0 is the mean; k >= 1: a = (float) clamp(mean + std z, -1, 1) in fp64, z standard normal by
+ *      Box-Muller from Philox4x32-10 with counter (66, call, (it H + t) 3 + p, c) and key seed (glg_plan_normal2 in
+ *      csrc/glg_philox.h; call = earlier glg_plan_run calls, p = component pair), laid out [H][B K][6].
+ *   3. roll out: H glg_step of the planning envs; R_c = sum_t gamma^t reward_t over the steps up to and including the one that
+ *      ends the episode (done); nothing after it counts.
+ *   4. update: the n_elites largest returns of each env (ties to the lower k; non-finite returns rank last) give the new mean and
+ *      population standard deviation per (t, component), summed in fp64 in ascending k, stored float32.  Deterministic.
+ * The action returned for env b is the final mean[0][b].  Parameters (glg_set_params) are taken from the env at every call;
+ * glg_set_weather on the env invalidates the planner (GLG_ERR_STATE).  Destroy the planner before its env handle.  Errors are
+ * reported through glg_last_error of the env handle. */
+typedef struct glg_plan_config {
+    int32_t horizon;       /* H >= 1 steps */
+    int32_t n_candidates;  /* K sequences per env, 1 .. 4096; num_envs * K <= 4194304 */
+    int32_t n_elites;      /* E, 1 .. K */
+    int32_t n_iterations;  /* I >= 1 CEM iterations per glg_plan_run */
+    double gamma;          /* discount in (0, 1] */
+    double init_std;       /* > 0: std after create and glg_plan_shift */
+    uint64_t seed;         /* Philox key of the samples */
+} glg_plan_config;
+typedef struct glg_plan glg_plan;
+int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_plan **out);
+void glg_plan_destroy(glg_plan *p);
+/* One decision: n_iterations CEM iterations from the env's current states; actions_dev float32 [B][6] <- mean[0].  GLG_ERR_STATE
+ * before the env's first glg_reset.  Enqueued on `stream` (n_iterations (3 + 2 H) launches). */
+int glg_plan_run(glg_plan *p, float *actions_dev, void *stream);
+/* Fan-out and roll-out alone, for caller-supplied sequences: seq_dev float32 [H][B K][6], returns_dev double [B K] (may be
+ * glg_plan_returns_dev). */
+int glg_plan_evaluate(glg_plan *p, const float *seq_dev, double *returns_dev, void *stream);
+/* Receding horizon: mean[t] <- mean[t + 1], mean[H - 1] <- 0 (hold the current controls), std <- init_std. */
+int glg_plan_shift(glg_plan *p, void *stream);
+float *glg_plan_mean_dev(glg_plan *p);        /* float32 [H][B][6]; writeable (re-initialise the distribution) */
+float *glg_plan_std_dev(glg_plan *p);         /* float32 [H][B][6]; writeable */
+float *glg_plan_candidates_dev(glg_plan *p);  /* float32 [H][B K][6]: the last iteration's samples */
+double *glg_plan_returns_dev(glg_plan *p);    /* double [B K]: the last roll-out's returns */
+
 /* Multi-GPU episode statistics (SURVEY 8e): the step path has no collective; the one exchange is a sum of the 16-entry
  * statistics vector over the ranks' handles, once per logging interval -- ncclAllReduce on the handle's device buffer.
  * NCCL is bound at run time (dlopen of libnccl.so.2, the copy torch already loaded when there is one), so libglgym.so has no
