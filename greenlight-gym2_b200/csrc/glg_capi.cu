@@ -63,12 +63,6 @@ struct glg_handle {
     double ctrl[GLG_NCTRL];  // rule-based controller settings (defaults: configs/agents/rule_based.yml)
     int obs_nmod = 0, obs_mod[GLG_MAXOBSMOD] = {}, obs_off[GLG_MAXOBSMOD] = {}, fc_off = -1;
     void *nccl_comm = nullptr;  // ncclComm_t (glg_nccl_init)
-    // device rollout (glg_rollout_create)
-    glg_rollout_config roll = {};
-    bool have_roll = false;
-    int roll_blocks = 0;
-    float *roll_obs = nullptr, *roll_rew = nullptr, *roll_starts = nullptr, *roll_adv = nullptr, *roll_ret = nullptr;
-    double *roll_stat = nullptr, *roll_partial = nullptr, *roll_norm = nullptr, *roll_acc = nullptr;
     std::string err;
 };
 static const double kDefaultCtrl[GLG_NCTRL] = {0, 18, -1, 366, 400, 10, 19.5, 16.5, 0, 5, 800, 4, 85, 2, 5, 1, -1, 5, 10, -1, 4, -2,
@@ -182,8 +176,6 @@ extern "C" void glg_destroy(glg_handle *h) {
     if (h->h_head) cudaFreeHost(h->h_head);
     if (h->h_res) cudaFreeHost(h->h_res);
     if (h->order_event) cudaEventDestroy(h->order_event);
-    cudaFree(h->roll_obs); cudaFree(h->roll_rew); cudaFree(h->roll_starts); cudaFree(h->roll_adv); cudaFree(h->roll_ret);
-    cudaFree(h->roll_stat); cudaFree(h->roll_partial); cudaFree(h->roll_norm); cudaFree(h->roll_acc);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     if (h->nccl_comm) {
         std::string e;
@@ -905,107 +897,152 @@ static int state_ex(glg_handle *h, const glg_env_state *s, bool to_dev) {
 extern "C" int glg_get_state_ex(glg_handle *h, const glg_env_state *out_host) { return state_ex(h, out_host, false); }
 extern "C" int glg_set_state_ex(glg_handle *h, const glg_env_state *in_host) { return state_ex(h, in_host, true); }
 
-// ---- device rollout: VecNormalize + rollout buffer + GAE (glg_rollout.cuh) -------------------------------------
-extern "C" int glg_rollout_create(glg_handle *h, const glg_rollout_config *cfg) {
-    if (!h || !cfg) return GLG_ERR_ARG;
+// ---- VecNormalize state of a rollout or replay buffer, updated by the glg_roll_* kernels (glg_rollout.cuh) ----
+struct GlgNorm {
+    int training = 0, norm_obs = 0, norm_reward = 0, blocks = 0;
+    double gamma = 0.0, clip_obs = 0.0, clip_reward = 0.0, epsilon = 0.0;
+    size_t bytes = 0;  // device bytes of the arrays below
+    double *ret = nullptr, *stat = nullptr, *partial = nullptr, *norm64 = nullptr;
+};
+
+template <typename T>
+static cudaError_t counted_alloc(size_t *bytes, T **p, size_t n) {
+    *bytes += n * sizeof(T);
+    return dev_alloc(p, n);
+}
+
+// c: glg_rollout_config or glg_replay_config, which share the VecNormalize fields.  Arrays for the handle's batch.
+template <class Cfg>
+static cudaError_t norm_create(GlgNorm *n, const glg_handle *h, const Cfg &c) {
+    n->training = c.training; n->norm_obs = c.norm_obs; n->norm_reward = c.norm_reward;
+    n->gamma = c.gamma; n->clip_obs = c.clip_obs; n->clip_reward = c.clip_reward; n->epsilon = c.epsilon;
+    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim;
+    n->blocks = (int)((B + GLG_ROLL_ROWS - 1) / GLG_ROLL_ROWS);
+    cudaError_t e = counted_alloc(&n->bytes, &n->ret, B);
+    if (e == cudaSuccess) e = counted_alloc(&n->bytes, &n->stat, (D + 1) * 3);
+    if (e == cudaSuccess) e = counted_alloc(&n->bytes, &n->partial, (size_t)n->blocks * (D + 1) * 2);
+    if (e == cudaSuccess) e = counted_alloc(&n->bytes, &n->norm64, (D + 1) * 2);
+    if (e != cudaSuccess) return e;
+    std::vector<double> st;
+    for (size_t c = 0; c <= D; ++c) st.insert(st.end(), {0.0, 1.0, 1e-4});  // RunningMeanStd: mean 0, var 1, count 1e-4
+    return cudaMemcpy(n->stat, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice);
+}
+
+static void norm_free(GlgNorm *n) { cudaFree(n->ret); cudaFree(n->stat); cudaFree(n->partial); cudaFree(n->norm64); }
+
+// VecNormalize.step_wait (after_step) or .reset on the handle's current outputs: statistics updated, normalised observations into
+// obs_out, normalised rewards into reward_out and episode starts into starts_out (either may be NULL).  Three launches on s.
+static void norm_update(const GlgNorm &n, glg_handle *h, bool after_step, float *obs_out, float *reward_out, float *starts_out,
+                        cudaStream_t s) {
+    GlgRollArgs a;
+    memset(&a, 0, sizeof a);
+    a.B = h->B; a.obs_dim = h->obs_dim; a.n_blocks = n.blocks;
+    a.training = n.training; a.norm_obs = n.norm_obs; a.norm_reward = n.norm_reward;
+    a.gamma = n.gamma; a.clip_obs = n.clip_obs; a.clip_reward = n.clip_reward; a.epsilon = n.epsilon;
+    a.obs = h->obs;
+    a.reward = after_step ? h->reward : nullptr;
+    a.done = after_step ? h->done : nullptr;
+    a.ret = n.ret; a.stat = n.stat; a.partial = n.partial; a.norm64 = n.norm64;
+    a.obs_out = obs_out; a.reward_out = reward_out; a.starts_out = starts_out;
+    glg_roll_moments_kernel<<<n.blocks, GLG_ROLL_NT, 0, s>>>(a);
+    glg_roll_finish_kernel<<<(h->obs_dim + 1 + GLG_ROLL_NT / 32 - 1) / (GLG_ROLL_NT / 32), GLG_ROLL_NT, 0, s>>>(a);
+    glg_roll_apply_kernel<<<n.blocks, GLG_ROLL_NT, 0, s>>>(a);
+    h->launches += 3;
+}
+
+// ---- device rollout: VecNormalize + rollout buffer + GAE (glg_rollout.cuh); its own object, like the replay buffer ----------
+struct glg_rollout {
+    glg_handle *h = nullptr;
+    int device = 0, n_steps = 0;
+    double gae_lambda = 0.0;
+    GlgNorm norm;
+    float *obs = nullptr, *rew = nullptr, *starts = nullptr, *adv = nullptr, *ret = nullptr;
+};
+
+extern "C" void glg_rollout_destroy(glg_rollout *r) {
+    if (!r) return;
+    cudaSetDevice(r->device);  // the handle may already be gone: nothing here reads it
+    cudaFree(r->obs); cudaFree(r->rew); cudaFree(r->starts); cudaFree(r->adv); cudaFree(r->ret);
+    norm_free(&r->norm);
+    delete r;
+}
+
+extern "C" int glg_rollout_create(glg_handle *h, const glg_rollout_config *cfg, glg_rollout **out) {
+    if (!h || !cfg || !out) return GLG_ERR_ARG;
+    *out = nullptr;
     if (cfg->n_steps < 1 || !(cfg->gamma >= 0.0 && cfg->gamma <= 1.0) || !(cfg->gae_lambda >= 0.0 && cfg->gae_lambda <= 1.0) ||
         !(cfg->clip_obs > 0) || !(cfg->clip_reward > 0) || !(cfg->epsilon > 0))
         return fail(h, GLG_ERR_ARG, "glg_rollout_create: invalid n_steps / gamma / gae_lambda / clip / epsilon");
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    cudaFree(h->roll_obs); cudaFree(h->roll_rew); cudaFree(h->roll_starts); cudaFree(h->roll_adv); cudaFree(h->roll_ret);
-    cudaFree(h->roll_stat); cudaFree(h->roll_partial); cudaFree(h->roll_norm); cudaFree(h->roll_acc);
-    h->roll_obs = h->roll_rew = h->roll_starts = h->roll_adv = h->roll_ret = nullptr;
-    h->roll_stat = h->roll_partial = h->roll_norm = h->roll_acc = nullptr;
-    h->have_roll = false;
+    glg_rollout *r = new (std::nothrow) glg_rollout();
+    if (!r) return fail(h, GLG_ERR_ALLOC, "glg_rollout_create: out of host memory");
+    r->h = h; r->device = h->cfg.device; r->n_steps = cfg->n_steps; r->gae_lambda = cfg->gae_lambda;
     const size_t B = (size_t)h->B, T = (size_t)cfg->n_steps, D = (size_t)h->obs_dim;
-    h->roll_blocks = (int)((B + GLG_ROLL_ROWS - 1) / GLG_ROLL_ROWS);
-    GLG_CUDA(h, dev_alloc(&h->roll_obs, (T + 1) * B * D));
-    GLG_CUDA(h, dev_alloc(&h->roll_rew, T * B));
-    GLG_CUDA(h, dev_alloc(&h->roll_starts, (T + 1) * B));
-    GLG_CUDA(h, dev_alloc(&h->roll_adv, T * B));
-    GLG_CUDA(h, dev_alloc(&h->roll_ret, T * B));
-    GLG_CUDA(h, dev_alloc(&h->roll_stat, (D + 1) * 3));
-    GLG_CUDA(h, dev_alloc(&h->roll_partial, (size_t)h->roll_blocks * (D + 1) * 2));
-    GLG_CUDA(h, dev_alloc(&h->roll_norm, (D + 1) * 2));
-    GLG_CUDA(h, dev_alloc(&h->roll_acc, B));
-    std::vector<double> st((D + 1) * 3);
-    for (size_t c = 0; c <= D; ++c) {  // RunningMeanStd: mean 0, var 1, count 1e-4
-        st[3 * c] = 0.0;
-        st[3 * c + 1] = 1.0;
-        st[3 * c + 2] = 1e-4;
+    cudaError_t e = dev_alloc(&r->obs, (T + 1) * B * D);
+    if (e == cudaSuccess) e = dev_alloc(&r->rew, T * B);
+    if (e == cudaSuccess) e = dev_alloc(&r->starts, (T + 1) * B);
+    if (e == cudaSuccess) e = dev_alloc(&r->adv, T * B);
+    if (e == cudaSuccess) e = dev_alloc(&r->ret, T * B);
+    if (e == cudaSuccess) e = norm_create(&r->norm, h, *cfg);
+    if (e != cudaSuccess) {
+        glg_rollout_destroy(r);
+        return fail(h, GLG_ERR_CUDA, (std::string("glg_rollout_create: ") + cudaGetErrorString(e)).c_str());
     }
-    GLG_CUDA(h, cudaMemcpy(h->roll_stat, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice));
-    h->roll = *cfg;
-    h->have_roll = true;
+    *out = r;
     return GLG_OK;
 }
-extern "C" int glg_rollout_store(glg_handle *h, int32_t t, void *stream) {
-    if (!h) return GLG_ERR_ARG;
-    if (!h->have_roll) return fail(h, GLG_ERR_STATE, "glg_rollout_store: no rollout buffer (glg_rollout_create)");
-    if (t < -1 || t >= h->roll.n_steps) return fail(h, GLG_ERR_ARG, "glg_rollout_store: t outside [-1, n_steps)");
-    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+extern "C" int glg_rollout_store(glg_rollout *r, int32_t t, void *stream) {
+    if (!r) return GLG_ERR_ARG;
+    glg_handle *h = r->h;
+    if (t < -1 || t >= r->n_steps) return fail(h, GLG_ERR_ARG, "glg_rollout_store: t outside [-1, n_steps)");
+    GLG_CUDA(h, cudaSetDevice(r->device));
     const size_t B = (size_t)h->B, D = (size_t)h->obs_dim;
-    GlgRollArgs a;
-    memset(&a, 0, sizeof a);
-    a.B = h->B; a.obs_dim = h->obs_dim; a.n_blocks = h->roll_blocks;
-    a.training = h->roll.training; a.norm_obs = h->roll.norm_obs; a.norm_reward = h->roll.norm_reward;
-    a.gamma = h->roll.gamma; a.clip_obs = h->roll.clip_obs; a.clip_reward = h->roll.clip_reward; a.epsilon = h->roll.epsilon;
-    a.obs = h->obs;
-    a.reward = t >= 0 ? h->reward : nullptr;
-    a.done = t >= 0 ? h->done : nullptr;
-    a.ret = h->roll_acc; a.stat = h->roll_stat; a.partial = h->roll_partial; a.norm64 = h->roll_norm;
-    a.obs_out = h->roll_obs + (size_t)(t + 1) * B * D;
-    a.reward_out = t >= 0 ? h->roll_rew + (size_t)t * B : nullptr;
-    a.starts_out = h->roll_starts + (size_t)(t + 1) * B;
-    cudaStream_t s = (cudaStream_t)stream;
-    glg_roll_moments_kernel<<<h->roll_blocks, GLG_ROLL_NT, 0, s>>>(a);
-    glg_roll_finish_kernel<<<(h->obs_dim + 1 + GLG_ROLL_NT / 32 - 1) / (GLG_ROLL_NT / 32), GLG_ROLL_NT, 0, s>>>(a);
-    glg_roll_apply_kernel<<<h->roll_blocks, GLG_ROLL_NT, 0, s>>>(a);
-    h->launches += 3;
+    norm_update(r->norm, h, t >= 0, r->obs + (size_t)(t + 1) * B * D, t >= 0 ? r->rew + (size_t)t * B : nullptr,
+                r->starts + (size_t)(t + 1) * B, (cudaStream_t)stream);
     GLG_CUDA(h, cudaGetLastError());
     return GLG_OK;
 }
-extern "C" int glg_rollout_carry(glg_handle *h, void *stream) {
-    if (!h) return GLG_ERR_ARG;
-    if (!h->have_roll) return fail(h, GLG_ERR_STATE, "glg_rollout_carry: no rollout buffer (glg_rollout_create)");
-    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim, T = (size_t)h->roll.n_steps;
-    GLG_CUDA(h, cudaMemcpyAsync(h->roll_obs, h->roll_obs + T * B * D, B * D * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
-    GLG_CUDA(h, cudaMemcpyAsync(h->roll_starts, h->roll_starts + T * B, B * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+extern "C" int glg_rollout_carry(glg_rollout *r, void *stream) {
+    if (!r) return GLG_ERR_ARG;
+    glg_handle *h = r->h;
+    GLG_CUDA(h, cudaSetDevice(r->device));
+    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim, T = (size_t)r->n_steps;
+    GLG_CUDA(h, cudaMemcpyAsync(r->obs, r->obs + T * B * D, B * D * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    GLG_CUDA(h, cudaMemcpyAsync(r->starts, r->starts + T * B, B * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return GLG_OK;
 }
-extern "C" int glg_rollout_gae(glg_handle *h, const float *values_dev, void *stream) {
-    if (!h || !values_dev) return GLG_ERR_ARG;
-    if (!h->have_roll) return fail(h, GLG_ERR_STATE, "glg_rollout_gae: no rollout buffer (glg_rollout_create)");
-    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    glg_roll_gae_kernel<<<(h->B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->roll.n_steps, h->B, h->roll.gamma, h->roll.gae_lambda, h->roll_rew,
-                                                                              values_dev, h->roll_starts, h->roll_adv, h->roll_ret);
+extern "C" int glg_rollout_gae(glg_rollout *r, const float *values_dev, void *stream) {
+    if (!r || !values_dev) return GLG_ERR_ARG;
+    glg_handle *h = r->h;
+    GLG_CUDA(h, cudaSetDevice(r->device));
+    glg_roll_gae_kernel<<<(h->B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(r->n_steps, h->B, r->norm.gamma, r->gae_lambda, r->rew,
+                                                                              values_dev, r->starts, r->adv, r->ret);
     h->launches += 1;
     GLG_CUDA(h, cudaGetLastError());
     return GLG_OK;
 }
-extern "C" float *glg_rollout_obs_dev(glg_handle *h) { return h ? h->roll_obs : nullptr; }
-extern "C" float *glg_rollout_rewards_dev(glg_handle *h) { return h ? h->roll_rew : nullptr; }
-extern "C" float *glg_rollout_starts_dev(glg_handle *h) { return h ? h->roll_starts : nullptr; }
-extern "C" float *glg_rollout_advantages_dev(glg_handle *h) { return h ? h->roll_adv : nullptr; }
-extern "C" float *glg_rollout_returns_dev(glg_handle *h) { return h ? h->roll_ret : nullptr; }
-extern "C" double *glg_rollout_stats_dev(glg_handle *h) { return h ? h->roll_stat : nullptr; }
+extern "C" float *glg_rollout_obs_dev(glg_rollout *r) { return r ? r->obs : nullptr; }
+extern "C" float *glg_rollout_rewards_dev(glg_rollout *r) { return r ? r->rew : nullptr; }
+extern "C" float *glg_rollout_starts_dev(glg_rollout *r) { return r ? r->starts : nullptr; }
+extern "C" float *glg_rollout_advantages_dev(glg_rollout *r) { return r ? r->adv : nullptr; }
+extern "C" float *glg_rollout_returns_dev(glg_rollout *r) { return r ? r->ret : nullptr; }
+extern "C" double *glg_rollout_stats_dev(glg_rollout *r) { return r ? r->norm.stat : nullptr; }
 
 // ---- device replay buffer (glg_replay.cuh): its own object, so several can share an env and none dangles from the handle ----
 struct glg_replay {
     glg_handle *h = nullptr;
     int device = 0;
-    glg_replay_config cfg = {};
+    uint64_t seed = 0;                   // Philox key of the sample indices
     unsigned long long weather_gen = 0;  // bank generation the keys refer to
     long long cap = 0, pos = 0;
     bool full = false, is_reset = false;
     uint32_t calls = 0;  // sample calls so far (Philox counter)
-    int blocks = 0, n_head = 0, nf = 0;
-    size_t bytes = 0;
+    int n_head = 0, nf = 0;
+    size_t bytes = 0;  // device bytes of the arrays below; glg_replay_bytes adds the normaliser's
+    GlgNorm norm;
     float *obs_norm = nullptr, *last_head = nullptr, *head_obs = nullptr, *head_next = nullptr, *act = nullptr, *rew = nullptr;
     int *key_obs = nullptr, *key_next = nullptr, *anchor_t = nullptr, *anchor_tbl = nullptr;
     unsigned char *dn = nullptr;
-    double *stat = nullptr, *partial = nullptr, *norm64 = nullptr, *ret = nullptr;
 };
 
 extern "C" void glg_replay_destroy(glg_replay *r) {
@@ -1013,14 +1050,8 @@ extern "C" void glg_replay_destroy(glg_replay *r) {
     cudaSetDevice(r->device);  // the handle may already be gone: nothing here reads it
     cudaFree(r->obs_norm); cudaFree(r->last_head); cudaFree(r->head_obs); cudaFree(r->head_next); cudaFree(r->act); cudaFree(r->rew);
     cudaFree(r->key_obs); cudaFree(r->key_next); cudaFree(r->anchor_t); cudaFree(r->anchor_tbl); cudaFree(r->dn);
-    cudaFree(r->stat); cudaFree(r->partial); cudaFree(r->norm64); cudaFree(r->ret);
+    norm_free(&r->norm);
     delete r;
-}
-
-template <typename T>
-static cudaError_t replay_alloc(glg_replay *r, T **p, size_t n) {
-    r->bytes += n * sizeof(T);
-    return dev_alloc(p, n);
 }
 
 extern "C" int glg_replay_create(glg_handle *h, const glg_replay_config *cfg, glg_replay **out) {
@@ -1041,37 +1072,24 @@ extern "C" int glg_replay_create(glg_handle *h, const glg_replay_config *cfg, gl
     if (!r) return fail(h, GLG_ERR_ALLOC, "glg_replay_create: out of host memory");
     r->h = h;
     r->device = h->cfg.device;
-    r->cfg = *cfg;
+    r->seed = cfg->seed;
     r->weather_gen = h->weather_gen;
     r->cap = cap;
-    r->blocks = (int)((B + GLG_ROLL_ROWS - 1) / GLG_ROLL_ROWS);
     r->nf = h->fc_off >= 0 ? 5 * h->cfg.Np : 0;
     r->n_head = h->obs_dim - r->nf;
     const size_t CB = (size_t)cap * B, H = (size_t)r->n_head;
-    cudaError_t e = replay_alloc(r, &r->head_obs, CB * H);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->head_next, CB * H);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->key_obs, CB);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->key_next, CB);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->act, CB * GLG_NU);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->rew, CB);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->dn, CB);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->obs_norm, B * D);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->last_head, B * H);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->anchor_t, B);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->anchor_tbl, B);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->ret, B);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->stat, (D + 1) * 3);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->partial, (size_t)r->blocks * (D + 1) * 2);
-    if (e == cudaSuccess) e = replay_alloc(r, &r->norm64, (D + 1) * 2);
-    if (e == cudaSuccess) {
-        std::vector<double> st((D + 1) * 3);
-        for (size_t c = 0; c <= D; ++c) {  // RunningMeanStd: mean 0, var 1, count 1e-4
-            st[3 * c] = 0.0;
-            st[3 * c + 1] = 1.0;
-            st[3 * c + 2] = 1e-4;
-        }
-        e = cudaMemcpy(r->stat, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice);
-    }
+    cudaError_t e = counted_alloc(&r->bytes, &r->head_obs, CB * H);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->head_next, CB * H);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->key_obs, CB);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->key_next, CB);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->act, CB * GLG_NU);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->rew, CB);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->dn, CB);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->obs_norm, B * D);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->last_head, B * H);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->anchor_t, B);
+    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->anchor_tbl, B);
+    if (e == cudaSuccess) e = norm_create(&r->norm, h, *cfg);
     if (e != cudaSuccess) {
         glg_replay_destroy(r);
         return fail(h, GLG_ERR_CUDA, (std::string("glg_replay_create: ") + cudaGetErrorString(e)).c_str());
@@ -1088,25 +1106,6 @@ static int replay_check(glg_replay *r, const char *what) {
         return GLG_ERR_STATE;
     }
     return GLG_OK;
-}
-
-// the VecNormalize part of a store / reset: glg_rollout.cuh's kernels on the buffer's own statistics
-static void replay_normalize(glg_replay *r, bool after_step, cudaStream_t s) {
-    glg_handle *h = r->h;
-    GlgRollArgs a;
-    memset(&a, 0, sizeof a);
-    a.B = h->B; a.obs_dim = h->obs_dim; a.n_blocks = r->blocks;
-    a.training = r->cfg.training; a.norm_obs = r->cfg.norm_obs; a.norm_reward = r->cfg.norm_reward;
-    a.gamma = r->cfg.gamma; a.clip_obs = r->cfg.clip_obs; a.clip_reward = r->cfg.clip_reward; a.epsilon = r->cfg.epsilon;
-    a.obs = h->obs;
-    a.reward = after_step ? h->reward : nullptr;
-    a.done = after_step ? h->done : nullptr;
-    a.ret = r->ret; a.stat = r->stat; a.partial = r->partial; a.norm64 = r->norm64;
-    a.obs_out = r->obs_norm;
-    glg_roll_moments_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(a);
-    glg_roll_finish_kernel<<<(h->obs_dim + 1 + GLG_ROLL_NT / 32 - 1) / (GLG_ROLL_NT / 32), GLG_ROLL_NT, 0, s>>>(a);
-    glg_roll_apply_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(a);
-    h->launches += 3;
 }
 
 static void replay_write_args(const glg_replay *r, GlgReplayArgs *w) {
@@ -1128,11 +1127,11 @@ extern "C" int glg_replay_reset(glg_replay *r, void *stream) {
     if (!h->is_reset) return fail(h, GLG_ERR_STATE, "glg_replay_reset: the env has not been reset (glg_reset)");
     GLG_CUDA(h, cudaSetDevice(r->device));
     cudaStream_t s = (cudaStream_t)stream;
-    replay_normalize(r, false, s);
+    norm_update(r->norm, h, false, r->obs_norm, nullptr, nullptr, s);
     GlgReplayArgs w;
     replay_write_args(r, &w);
     w.store = 0;
-    glg_replay_write_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(w);
+    glg_replay_write_kernel<<<r->norm.blocks, GLG_ROLL_NT, 0, s>>>(w);
     h->launches += 1;
     GLG_CUDA(h, cudaGetLastError());
     r->is_reset = true;
@@ -1148,13 +1147,13 @@ extern "C" int glg_replay_store(glg_replay *r, const float *actions_dev, void *s
     if (!r->is_reset) return fail(h, GLG_ERR_STATE, "glg_replay_store: store before glg_replay_reset");
     GLG_CUDA(h, cudaSetDevice(r->device));
     cudaStream_t s = (cudaStream_t)stream;
-    replay_normalize(r, true, s);
+    norm_update(r->norm, h, true, r->obs_norm, nullptr, nullptr, s);
     GlgReplayArgs w;
     replay_write_args(r, &w);
     w.store = 1;
     w.slot = (size_t)r->pos;
     w.actions = actions_dev;
-    glg_replay_write_kernel<<<r->blocks, GLG_ROLL_NT, 0, s>>>(w);
+    glg_replay_write_kernel<<<r->norm.blocks, GLG_ROLL_NT, 0, s>>>(w);
     h->launches += 1;
     GLG_CUDA(h, cudaGetLastError());
     if (++r->pos == r->cap) {
@@ -1178,10 +1177,10 @@ extern "C" int glg_replay_sample(glg_replay *r, int32_t n, float *obs_dev, float
     GlgReplaySampleArgs S;
     memset(&S, 0, sizeof S);
     S.n = n; S.B = h->B; S.obs_dim = h->obs_dim; S.n_head = r->n_head; S.nf = r->nf; S.fc_off = h->fc_off;
-    S.norm_obs = r->cfg.norm_obs; S.norm_reward = r->cfg.norm_reward;
-    S.upper = (uint32_t)upper; S.call = r->calls; S.seed = r->cfg.seed;
-    S.clip_obs = r->cfg.clip_obs; S.clip_reward = r->cfg.clip_reward;
-    S.norm64 = r->norm64;
+    S.norm_obs = r->norm.norm_obs; S.norm_reward = r->norm.norm_reward;
+    S.upper = (uint32_t)upper; S.call = r->calls; S.seed = r->seed;
+    S.clip_obs = r->norm.clip_obs; S.clip_reward = r->norm.clip_reward;
+    S.norm64 = r->norm.norm64;
     S.weather = h->weather;  // read on every call: glg_set_weather reallocates the bank
     S.head_obs = r->head_obs; S.head_next = r->head_next; S.key_obs = r->key_obs; S.key_next = r->key_next;
     S.act = r->act; S.rew = r->rew; S.dn = r->dn;
@@ -1196,9 +1195,9 @@ extern "C" int glg_replay_sample(glg_replay *r, int32_t n, float *obs_dev, float
 }
 
 extern "C" int64_t glg_replay_size(const glg_replay *r) { return r ? (r->full ? r->cap : r->pos) : 0; }
-extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)r->bytes : 0; }
+extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)(r->bytes + r->norm.bytes) : 0; }
 extern "C" float *glg_replay_obs_dev(glg_replay *r) { return r ? r->obs_norm : nullptr; }
-extern "C" double *glg_replay_stats_dev(glg_replay *r) { return r ? r->stat : nullptr; }
+extern "C" double *glg_replay_stats_dev(glg_replay *r) { return r ? r->norm.stat : nullptr; }
 
 // ---- receding-horizon planner (glg_plan.cuh): its own object holding a second, internal handle of B K planning envs that the
 // unchanged step kernels advance; the env handle is only read ----

@@ -95,7 +95,8 @@ SIGNATURES = {
     "glg_set_seed": (C.c_int, [C.c_void_p, C.c_uint64]),
     "glg_get_state_ex": (C.c_int, [C.c_void_p, C.POINTER(GlgEnvState)]),
     "glg_set_state_ex": (C.c_int, [C.c_void_p, C.POINTER(GlgEnvState)]),
-    "glg_rollout_create": (C.c_int, [C.c_void_p, C.POINTER(GlgRolloutConfig)]),
+    "glg_rollout_create": (C.c_int, [C.c_void_p, C.POINTER(GlgRolloutConfig), C.POINTER(C.c_void_p)]),
+    "glg_rollout_destroy": (None, [C.c_void_p]),
     "glg_rollout_store": (C.c_int, [C.c_void_p, C.c_int32, _VP]),
     "glg_rollout_carry": (C.c_int, [C.c_void_p, _VP]),
     "glg_rollout_gae": (C.c_int, [C.c_void_p, _FP, _VP]),

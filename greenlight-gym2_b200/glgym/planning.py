@@ -13,38 +13,27 @@ times, on a second handle of B * n_candidates planning envs; the env itself is o
 The planner uses the nominal model (no parametric uncertainty) and the weather bank as perfect weather over the horizon, which is
 the forecast the env observes as long as horizon <= Np.  `evaluate(seq)` scores caller-supplied sequences the same way.
 """
-import ctypes as C
-
 import torch
 
 from . import _lib
-from .vec_env import _DevArray
+from .vec_env import _EnvCompanion
 
 
-class DevicePlanner:
+class DevicePlanner(_EnvCompanion):
+    _kind, _destroy = "planner", "glg_plan_destroy"
+    _p = property(lambda self: self._obj)  # the glg_plan object, for calling the C entry points directly
+
     def __init__(self, env, horizon, n_candidates, n_elites, n_iterations, gamma=1.0, init_std=0.5, seed=0):
-        self.env = env
-        self._lib = env._lib
         cfg = _lib.GlgPlanConfig(int(horizon), int(n_candidates), int(n_elites), int(n_iterations), float(gamma), float(init_std),
                                  int(seed) & (2**64 - 1))
-        self._p = C.c_void_p()
-        _lib.check(self._lib.glg_plan_create(env._h, C.byref(cfg), C.byref(self._p)), env._h, "glg_plan_create")
+        super().__init__(env, "glg_plan_create", cfg)
         self.horizon, self.n_candidates, self.n_elites, self.n_iterations = int(horizon), int(n_candidates), int(n_elites), int(n_iterations)
-        H, B, K, dev = self.horizon, env.num_envs, self.n_candidates, env.device
-        view = lambda ptr, shape, ts: torch.as_tensor(_DevArray(ptr, shape, ts), device=dev)
-        L = self._lib
-        self.mean = view(L.glg_plan_mean_dev(self._p), (H, B, 6), "<f4")               # writeable: re-initialise the distribution
-        self.std = view(L.glg_plan_std_dev(self._p), (H, B, 6), "<f4")
-        self.candidates = view(L.glg_plan_candidates_dev(self._p), (H, B, K, 6), "<f4")  # last iteration's samples
-        self.returns = view(L.glg_plan_returns_dev(self._p), (B, K), "<f8")              # last roll-out's discounted returns
-        self._actions = torch.empty((B, 6), dtype=torch.float32, device=dev)
-
-    def _live(self):
-        if not self._p:
-            raise RuntimeError("the planner is closed")
-        if not self.env._h:
-            raise RuntimeError("the env of this planner is closed")
-        return self._p
+        H, B, K, p, L = self.horizon, env.num_envs, self.n_candidates, self._obj, self._lib
+        self.mean = self._view(L.glg_plan_mean_dev(p), (H, B, 6), "<f4")               # writeable: re-initialise the distribution
+        self.std = self._view(L.glg_plan_std_dev(p), (H, B, 6), "<f4")
+        self.candidates = self._view(L.glg_plan_candidates_dev(p), (H, B, K, 6), "<f4")  # last iteration's samples
+        self.returns = self._view(L.glg_plan_returns_dev(p), (B, K), "<f8")              # last roll-out's discounted returns
+        self._actions = torch.empty((B, 6), dtype=torch.float32, device=env.device)
 
     def plan(self):
         """One decision from the env's current states: n_iterations CEM iterations; returns the new mean[0] as a float32 [B, 6]
@@ -68,14 +57,3 @@ class DevicePlanner:
         _lib.check(self._lib.glg_plan_evaluate(p, s.data_ptr(), self.returns.data_ptr(), self.env._stream()), self.env._h,
                    "glg_plan_evaluate")
         return self.returns
-
-    def close(self):
-        if getattr(self, "_p", None):
-            self._lib.glg_plan_destroy(self._p)
-            self._p = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass

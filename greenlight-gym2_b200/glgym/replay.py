@@ -17,39 +17,30 @@ rounding except in columns clipped at +-clip_obs), and the sample indices come f
 global generator.  Replacing the env's weather bank (glg_set_weather) invalidates the buffer.
 """
 import collections
-import ctypes as C
 
 import torch
 
 from . import _lib
-from .vec_env import _DevArray
+from .vec_env import _EnvCompanion
 
 # SB3 common/type_aliases.py ReplayBufferSamples: field names and order
 ReplayBufferSamples = collections.namedtuple("ReplayBufferSamples", ["observations", "actions", "next_observations", "dones", "rewards"])
 
 
-class DeviceReplayBuffer:
+class DeviceReplayBuffer(_EnvCompanion):
+    _kind, _destroy = "replay buffer", "glg_replay_destroy"
+    _r = property(lambda self: self._obj)  # the glg_replay object, for calling the C entry points directly
+
     def __init__(self, env, buffer_size, gamma=0.99, norm_obs=True, norm_reward=True, clip_obs=10.0, clip_reward=10.0, epsilon=1e-8,
                  training=True, seed=0):
-        self.env = env
-        self._lib = env._lib
         cfg = _lib.GlgReplayConfig(int(buffer_size), int(training), int(norm_obs), int(norm_reward), 0, float(gamma), float(clip_obs),
                                    float(clip_reward), float(epsilon), int(seed) & (2**64 - 1))
-        self._r = C.c_void_p()
-        _lib.check(self._lib.glg_replay_create(env._h, C.byref(cfg), C.byref(self._r)), env._h, "glg_replay_create")
-        B, D, dev = env.num_envs, env.obs_dim, env.device
+        super().__init__(env, "glg_replay_create", cfg)
+        B, D, r, L = env.num_envs, env.obs_dim, self._obj, self._lib
         self.capacity = max(int(buffer_size) // B, 1)
-        view = lambda ptr, shape, ts: torch.as_tensor(_DevArray(ptr, shape, ts), device=dev)
-        self.obs = view(self._lib.glg_replay_obs_dev(self._r), (B, D), "<f4")      # normalised current observation
-        self.stats = view(self._lib.glg_replay_stats_dev(self._r), (D + 1, 3), "<f8")  # running (mean, var, count); last row: returns
+        self.obs = self._view(L.glg_replay_obs_dev(r), (B, D), "<f4")          # normalised current observation
+        self.stats = self._view(L.glg_replay_stats_dev(r), (D + 1, 3), "<f8")  # running (mean, var, count); last row: returns
         self._out = {}  # n -> output tensors of sample(n), reused by the next sample(n)
-
-    def _live(self):
-        if not self._r:
-            raise RuntimeError("the replay buffer is closed")
-        if not self.env._h:
-            raise RuntimeError("the env of this replay buffer is closed")
-        return self._r
 
     def reset(self, reset_env=True):
         """Resets every env and starts each env's next transition from its new observation; stored transitions are kept.
@@ -113,13 +104,5 @@ class DeviceReplayBuffer:
         return int(self._lib.glg_replay_bytes(self._live()))
 
     def close(self):
-        if getattr(self, "_r", None):
-            self._lib.glg_replay_destroy(self._r)
-            self._r = None
-            self._out = {}
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+        super().close()
+        self._out = {}

@@ -11,48 +11,48 @@ clipping straight into the [T+1][B][obs_dim] rollout buffer, and generalised adv
     values[T] = policy.value(obs)
     adv, ret = roll.finish(values)                   # GAE
     roll.begin()                                     # next rollout continues from slot T
+    roll.close()                                     # frees the buffers; several rollouts may share one env
 
 `glgym.normalize` keeps the same arithmetic as eager torch ops (the round-1 implementation, 4.5 ms per step at 65 536 envs);
 the tests check both against a numpy restatement of SB3 2.6.0, which is pinned by the reference but not installed here
 ("unpinned against real SB3").
 """
-import ctypes as C
-
 import torch
 
 from . import _lib
-from .vec_env import _DevArray
+from .vec_env import _EnvCompanion
 
 
-class DeviceRollout:
+class DeviceRollout(_EnvCompanion):
+    _kind, _destroy = "rollout buffer", "glg_rollout_destroy"
+
     def __init__(self, env, n_steps, gamma=0.99, gae_lambda=0.95, norm_obs=True, norm_reward=True, clip_obs=10.0, clip_reward=10.0,
                  epsilon=1e-8, training=True):
-        self.env, self.n_steps = env, int(n_steps)
-        self._lib, self._h = env._lib, env._h
+        self.n_steps = int(n_steps)
         cfg = _lib.GlgRolloutConfig(self.n_steps, int(training), int(norm_obs), int(norm_reward), float(gamma), float(gae_lambda),
                                     float(clip_obs), float(clip_reward), float(epsilon))
-        _lib.check(self._lib.glg_rollout_create(self._h, C.byref(cfg)), self._h, "glg_rollout_create")
-        T, B, D, dev = self.n_steps, env.num_envs, env.obs_dim, env.device
-        view = lambda ptr, shape, ts: torch.as_tensor(_DevArray(ptr, shape, ts), device=dev)
-        L = self._lib
-        self.obs = view(L.glg_rollout_obs_dev(self._h), (T + 1, B, D), "<f4")
-        self.rewards = view(L.glg_rollout_rewards_dev(self._h), (T, B), "<f4")
-        self.episode_starts = view(L.glg_rollout_starts_dev(self._h), (T + 1, B), "<f4")
-        self.advantages = view(L.glg_rollout_advantages_dev(self._h), (T, B), "<f4")
-        self.returns = view(L.glg_rollout_returns_dev(self._h), (T, B), "<f4")
-        self.stats = view(L.glg_rollout_stats_dev(self._h), (D + 1, 3), "<f8")  # running (mean, var, count); last row: returns
+        super().__init__(env, "glg_rollout_create", cfg)
+        T, B, D, r, L = self.n_steps, env.num_envs, env.obs_dim, self._obj, self._lib
+        self.obs = self._view(L.glg_rollout_obs_dev(r), (T + 1, B, D), "<f4")
+        self.rewards = self._view(L.glg_rollout_rewards_dev(r), (T, B), "<f4")
+        self.episode_starts = self._view(L.glg_rollout_starts_dev(r), (T + 1, B), "<f4")
+        self.advantages = self._view(L.glg_rollout_advantages_dev(r), (T, B), "<f4")
+        self.returns = self._view(L.glg_rollout_returns_dev(r), (T, B), "<f4")
+        self.stats = self._view(L.glg_rollout_stats_dev(r), (D + 1, 3), "<f8")  # running (mean, var, count); last row: returns
         self.t = 0
 
     def _store(self, t):
-        _lib.check(self._lib.glg_rollout_store(self._h, t, self.env._stream()), self._h, "glg_rollout_store")
+        _lib.check(self._lib.glg_rollout_store(self._live(), t, self.env._stream()), self.env._h, "glg_rollout_store")
 
     def reset(self):
+        self._live()
         self.env.reset_tensor()
         self._store(-1)
         self.t = 0
         return self.obs[0]
 
     def step(self, actions, noise=None):
+        self._live()
         if self.t >= self.n_steps:
             raise RuntimeError("rollout buffer is full: call finish() / begin()")
         _, _, done = self.env.step_tensor(actions, noise)
@@ -61,6 +61,7 @@ class DeviceRollout:
         return self.obs[self.t], self.rewards[self.t - 1], done
 
     def step_rule_based(self, noise=None):
+        self._live()
         _, _, done = self.env.step_rule_based_tensor(noise)
         self._store(self.t)
         self.t += 1
@@ -68,14 +69,15 @@ class DeviceRollout:
 
     def finish(self, values):
         """values: CUDA float32 [T+1, B] (row T = value of obs[T]).  Returns (advantages, returns) [T, B]."""
+        r = self._live()
         v = values.to(device=self.env.device, dtype=torch.float32).contiguous()
         assert v.shape == (self.n_steps + 1, self.env.num_envs)
-        _lib.check(self._lib.glg_rollout_gae(self._h, v.data_ptr(), self.env._stream()), self._h, "glg_rollout_gae")
+        _lib.check(self._lib.glg_rollout_gae(r, v.data_ptr(), self.env._stream()), self.env._h, "glg_rollout_gae")
         return self.advantages, self.returns
 
     def begin(self):
         """Continue with the next rollout: slot T becomes slot 0 (SB3 keeps `_last_obs` / `_last_episode_starts`)."""
-        _lib.check(self._lib.glg_rollout_carry(self._h, self.env._stream()), self._h, "glg_rollout_carry")
+        _lib.check(self._lib.glg_rollout_carry(self._live(), self.env._stream()), self.env._h, "glg_rollout_carry")
         self.t = 0
         return self.obs[0]
 

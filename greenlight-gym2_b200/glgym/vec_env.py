@@ -68,6 +68,39 @@ class _DevArray:
                                          "version": 2}
 
 
+class _EnvCompanion:
+    """Base of the device objects created on an env (DeviceRollout, DeviceReplayBuffer, DevicePlanner).  Each owns one C object
+    (`create(env._h, &cfg, &obj)`), so several may share an env; close() frees it, before or after the env is closed."""
+    _kind = ""     # what the error messages call it
+    _destroy = ""  # name of the C destructor
+
+    def __init__(self, env, create, cfg):
+        self.env, self._lib = env, env._lib
+        self._obj = C.c_void_p()
+        _lib.check(getattr(self._lib, create)(env._h, C.byref(cfg), C.byref(self._obj)), env._h, create)
+
+    def _view(self, ptr, shape, typestr):
+        return torch.as_tensor(_DevArray(ptr, shape, typestr), device=self.env.device)
+
+    def _live(self):
+        if not self._obj:
+            raise RuntimeError(f"the {self._kind} is closed")
+        if not self.env._h:
+            raise RuntimeError(f"the env of this {self._kind} is closed")
+        return self._obj
+
+    def close(self):
+        if getattr(self, "_obj", None):
+            getattr(self._lib, self._destroy)(self._obj)
+            self._obj = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 # observation modules (observations.py:35-182): name -> (id in glg_config.obs_modules, names, (low, high) of its Box)
 _WEATHER_NAMES = ["glob_rad", "temp_out", "rh_out", "co2_out", "wind_speed"]
 OBSERVATION_MODULES = {

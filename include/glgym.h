@@ -201,9 +201,10 @@ int glg_set_state_ex(glg_handle *h, const glg_env_state *in_host);
  * What the reference's training loop puts between env.step and the PPO update -- SubprocVecEnv -> VecMonitor -> VecNormalize
  * (gl_gym/RL/utils.py:60-67; norm_obs / norm_reward / clip_obs / clip_reward / gamma from RL/experiment_manager.py:142-147) and
  * SB3's RolloutBuffer with generalised advantage estimation (configs/agents/ppo.yml: n_steps, gamma, gae_lambda) -- as kernels
- * on the handle's own outputs (csrc/glg_rollout.cuh), so a rollout never leaves the device.  Episode return / length
- * bookkeeping (VecMonitor) is part of the step kernel (glg_stats_dev).
- * Buffers (device, owned by the handle): obs float32 [T+1][B][obs_dim] (normalised, clipped; slot t = what the policy sees
+ * on the handle's own outputs (csrc/glg_rollout.cuh), so a rollout never leaves the device.  Its own object: several rollout
+ * buffers may share one env handle; destroy each before glg_destroy of the handle.  Errors are reported through glg_last_error of
+ * the handle.  Episode return / length bookkeeping (VecMonitor) is part of the step kernel (glg_stats_dev).
+ * Buffers (device, owned by the rollout): obs float32 [T+1][B][obs_dim] (normalised, clipped; slot t = what the policy sees
  * at step t, slot T = the observation after the last step), rewards float32 [T][B] (normalised), episode_starts float32
  * [T+1][B], advantages / returns float32 [T][B], statistics double [obs_dim + 1][3] = running (mean, var, count) per observation
  * column, last row = statistics of the discounted return. */
@@ -214,22 +215,24 @@ typedef struct glg_rollout_config {
     double gamma, gae_lambda;
     double clip_obs, clip_reward, epsilon; /* 10, 10, 1e-8 in the reference's setup */
 } glg_rollout_config;
-int glg_rollout_create(glg_handle *h, const glg_rollout_config *cfg);
+typedef struct glg_rollout glg_rollout;
+int glg_rollout_create(glg_handle *h, const glg_rollout_config *cfg, glg_rollout **out);
+void glg_rollout_destroy(glg_rollout *r);
 /* After glg_reset (t = -1): statistics fed with the first observations, normalised into slot 0, returns zeroed, every env
  * starts an episode.  After the glg_step* of rollout step t (0 <= t < T): observation statistics updated with the new raw
  * observations, which are normalised into slot t + 1; ret <- ret gamma + reward feeds the return statistics; the normalised
  * reward goes to slot t; episode_starts[t + 1] = done; ret[done] = 0.  Three launches on `stream`. */
-int glg_rollout_store(glg_handle *h, int32_t t, void *stream);
+int glg_rollout_store(glg_rollout *r, int32_t t, void *stream);
 /* Start the next rollout without a reset: slot T (observation, episode_starts) becomes slot 0. */
-int glg_rollout_carry(glg_handle *h, void *stream);
+int glg_rollout_carry(glg_rollout *r, void *stream);
 /* RolloutBuffer.compute_returns_and_advantage: values_dev float32 [T+1][B] (row T = value of the slot-T observation). */
-int glg_rollout_gae(glg_handle *h, const float *values_dev, void *stream);
-float *glg_rollout_obs_dev(glg_handle *h);
-float *glg_rollout_rewards_dev(glg_handle *h);
-float *glg_rollout_starts_dev(glg_handle *h);
-float *glg_rollout_advantages_dev(glg_handle *h);
-float *glg_rollout_returns_dev(glg_handle *h);
-double *glg_rollout_stats_dev(glg_handle *h);
+int glg_rollout_gae(glg_rollout *r, const float *values_dev, void *stream);
+float *glg_rollout_obs_dev(glg_rollout *r);
+float *glg_rollout_rewards_dev(glg_rollout *r);
+float *glg_rollout_starts_dev(glg_rollout *r);
+float *glg_rollout_advantages_dev(glg_rollout *r);
+float *glg_rollout_returns_dev(glg_rollout *r);
+double *glg_rollout_stats_dev(glg_rollout *r);
 
 /* ---- device replay buffer for off-policy agents (SAC) ------------------------------------------------------------------------
  * SB3 2.6.0's ReplayBuffer (optimize_memory_usage False, handle_timeout_termination True) filled the way
