@@ -402,58 +402,42 @@ extern "C" int glg_reset(glg_handle *h, const uint8_t *mask_dev, const int32_t *
     return GLG_OK;
 }
 
+// Opts kernel F into `smem` bytes of dynamic shared memory on `device` when a launch needs more than F has been allowed there
+// so far (the attribute is per kernel and per context).
+template <auto F>
+static cudaError_t opt_in_smem(int device, size_t smem) {
+    static size_t attr_smem_dev[64] = {};  // largest size opted into so far, per device
+    size_t &attr_smem = attr_smem_dev[device & 63];
+    if (smem > attr_smem) {
+        cudaError_t e = cudaFuncSetAttribute(F, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        attr_smem = smem;
+    }
+    return cudaSuccess;
+}
+
 template <bool GENERAL, bool NOISY>
 static cudaError_t launch_step(glg_handle *h, const GlgStepArgs &a, cudaStream_t s) {
     constexpr int NT = 64;
     const size_t smem = GlgStepSmem<NT, NOISY>::bytes(a.Np);
-    static size_t attr_smem_dev[64] = {};  // largest size opted into so far, per device (the attribute is per context)
-    size_t &attr_smem = attr_smem_dev[h->cfg.device & 63];
-    if (smem > attr_smem) {
-        cudaError_t e = cudaFuncSetAttribute(glg_step_kernel<GENERAL, NOISY, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        attr_smem = smem;
-    }
+    cudaError_t e = opt_in_smem<glg_step_kernel<GENERAL, NOISY, NT>>(h->cfg.device, smem);
+    if (e != cudaSuccess) return e;
     glg_step_kernel<GENERAL, NOISY, NT><<<(a.B + NT - 1) / NT, NT, smem, s>>>(h->uni, a);
     return cudaGetLastError();
 }
 
-// NG group warps for the fp64 / fp32 unit kernels; MINB = CTAs per SM the register budget is compiled for
-#ifndef GLG_NG
-#define GLG_NG 12
-#endif
-#ifndef GLG_MINB_LAT
-#define GLG_MINB_LAT 1   // CTAs per SM of the latency variant (role_warps = 2)
-#endif
-#ifndef GLG_MINB_TPUT
-#define GLG_MINB_TPUT 4  // CTAs per SM of the throughput variant (role_warps = 3)
-#endif
-#ifndef GLG_TPUT_FUSED
-#define GLG_TPUT_FUSED true  // throughput variant: fused layout (4 warps = group role + owner), else dedicated owner warps
-#endif
-template <class T, bool GENERAL, bool NOISY, int MINB, bool FUSED>
-static cudaError_t launch_step_units_t(glg_handle *h, const GlgStepArgs &a, cudaStream_t s) {
-    constexpr int NG = FUSED ? GLG_NO : GLG_NG;
-    const size_t smem = GlgRoleSmem<T, NG, GENERAL, NOISY>::bytes(a.Np);
-    static size_t attr_smem_dev[64] = {};  // largest size opted into so far, per device (the attribute is per context)
-    size_t &attr_smem = attr_smem_dev[h->cfg.device & 63];
-    if (smem > attr_smem) {
-        cudaError_t e = cudaFuncSetAttribute(glg_step_units_kernel<T, GENERAL, NOISY, NG, MINB, FUSED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        attr_smem = smem;
-    }
-    glg_step_units_kernel<T, GENERAL, NOISY, NG, MINB, FUSED><<<(a.B + a.role_lanes - 1) / a.role_lanes, 32 * (NG + (FUSED ? 0 : GLG_NO)), smem, s>>>(h->uni, a);
-    return cudaGetLastError();
-}
-template <bool GENERAL, bool NOISY, int MINB, bool FUSED>
+// precision 0: fp64 parity mode ; 1: flux units in fp32, RK4 state / stage sums / epilogue in fp64
+template <bool FUSED, bool GENERAL, bool NOISY>
 static cudaError_t launch_step_units(glg_handle *h, const GlgStepArgs &a, cudaStream_t s) {
-    // precision 0: fp64 parity mode ; 1: flux units in fp32, RK4 state / stage sums / epilogue in fp64
-#ifdef GLG_DEV_FAST  // experimental builds (tools/ubench): only the fp64 nominal variants are compiled
-    if (GENERAL || NOISY || h->cfg.precision == 1) return cudaErrorNotSupported;
-    return launch_step_units_t<double, false, false, MINB, FUSED>(h, a, s);
-#else
-    return h->cfg.precision == 1 ? launch_step_units_t<float, GENERAL, NOISY, MINB, FUSED>(h, a, s)
-                                 : launch_step_units_t<double, GENERAL, NOISY, MINB, FUSED>(h, a, s);
-#endif
+    const auto launch = [&](auto t) {
+        using T = decltype(t);
+        const size_t smem = GlgRoleSmem<T, GlgLayout<FUSED>::NG, GENERAL, NOISY>::bytes(a.Np);
+        cudaError_t e = opt_in_smem<glg_step_units_kernel<T, GENERAL, NOISY, FUSED>>(h->cfg.device, smem);
+        if (e != cudaSuccess) return e;
+        glg_step_units_kernel<T, GENERAL, NOISY, FUSED><<<(a.B + a.role_lanes - 1) / a.role_lanes, GlgLayout<FUSED>::NT, smem, s>>>(h->uni, a);
+        return cudaGetLastError();
+    };
+    return h->cfg.precision == 1 ? launch(0.0f) : launch(0.0);
 }
 
 // Kernel variant: 1 = kernel A (one thread per env), 2 = kernel C latency layout (4 owner + 12 group warps per 32 envs, one CTA
@@ -464,6 +448,13 @@ static int pick_role_warps(const glg_handle *h) {
     if (h->cfg.role_warps != 0) return h->cfg.role_warps;
     return h->B <= 2 * h->sms * GLG_ROLE_LANES ? 2 : 3;
 }
+typedef cudaError_t (*StepLauncher)(glg_handle *, const GlgStepArgs &, cudaStream_t);
+static const StepLauncher kStepLaunchers[3][2][2] = {  // [kernel variant - 1][general][noisy]
+    {{launch_step<false, false>, launch_step<false, true>}, {launch_step<true, false>, launch_step<true, true>}},
+    {{launch_step_units<false, false, false>, launch_step_units<false, false, true>},
+     {launch_step_units<false, true, false>, launch_step_units<false, true, true>}},
+    {{launch_step_units<true, false, false>, launch_step_units<true, false, true>},
+     {launch_step_units<true, true, false>, launch_step_units<true, true, true>}}};
 
 static int step_common(glg_handle *h, const float *actions_dev, const double *controls_dev, const double *noise_dev,
                        void *stream, bool rule_based = false) {
@@ -480,19 +471,7 @@ static int step_common(glg_handle *h, const float *actions_dev, const double *co
     for (int i = 0; i < GLG_NCTRL; ++i) a.ctrl[i] = h->ctrl[i];
     a.noise = noise_dev;
     const bool noisy = (h->cfg.uncertainty_scale != 0.0) || (noise_dev != nullptr);
-    cudaStream_t s = (cudaStream_t)stream;
-    cudaError_t e;
-    const int rw = pick_role_warps(h);
-    if (rw == 2) {
-        if (h->general) e = noisy ? launch_step_units<true, true, GLG_MINB_LAT, false>(h, a, s) : launch_step_units<true, false, GLG_MINB_LAT, false>(h, a, s);
-        else e = noisy ? launch_step_units<false, true, GLG_MINB_LAT, false>(h, a, s) : launch_step_units<false, false, GLG_MINB_LAT, false>(h, a, s);
-    } else if (rw == 3) {
-        if (h->general) e = noisy ? launch_step_units<true, true, GLG_MINB_TPUT, GLG_TPUT_FUSED>(h, a, s) : launch_step_units<true, false, GLG_MINB_TPUT, GLG_TPUT_FUSED>(h, a, s);
-        else e = noisy ? launch_step_units<false, true, GLG_MINB_TPUT, GLG_TPUT_FUSED>(h, a, s) : launch_step_units<false, false, GLG_MINB_TPUT, GLG_TPUT_FUSED>(h, a, s);
-    } else {
-        if (h->general) e = noisy ? launch_step<true, true>(h, a, s) : launch_step<true, false>(h, a, s);
-        else e = noisy ? launch_step<false, true>(h, a, s) : launch_step<false, false>(h, a, s);
-    }
+    const cudaError_t e = kStepLaunchers[pick_role_warps(h) - 1][h->general][noisy](h, a, (cudaStream_t)stream);
     h->launches += 1;
     GLG_CUDA(h, e);
     return GLG_OK;

@@ -77,19 +77,12 @@ GLG_COEF double glg_kExpT[5] = {0x1.71547652b82fep+7 /*128/ln2*/, -0x1.62e42fefa
     0x1.f50765b6e4540p+0, 0x1.f7bfdad9cbe14p+0, 0x1.fa7c1819e90d8p+0, 0x1.fd3c22b8f71f1p+0
 #if defined(__CUDACC__)
 __device__ const double glg_exp_tbl_dev[128] = {GLG_EXP_TABLE_VALUES};
-// GLG_EXP_SMEM: per-CTA copy of the table in shared memory (a 32-bit address and an LDS instead of a 64-bit address and an L1 load:
-// two integer instructions fewer per exp).  Every kernel that evaluates an exp calls glg_exp_tbl_fill() before its first use.
-#ifndef GLG_EXP_SMEM
-#define GLG_EXP_SMEM 1
-#endif
-#if GLG_EXP_SMEM
+// Per-CTA copy of the table in shared memory (a 32-bit address and an LDS instead of a 64-bit address and an L1 load: two integer
+// instructions fewer per exp).  Every kernel that evaluates an exp calls glg_exp_tbl_fill() before its first use.
 __shared__ double glg_exp_tbl_sh[128];
-#endif
 __device__ __forceinline__ void glg_exp_tbl_fill() {
-#if GLG_EXP_SMEM
     for (int i = threadIdx.x; i < 128; i += blockDim.x) glg_exp_tbl_sh[i] = glg_exp_tbl_dev[i];
     __syncthreads();
-#endif
 }
 #endif
 static const double glg_exp_tbl_host[128] = {GLG_EXP_TABLE_VALUES};
@@ -156,15 +149,13 @@ GLG_HD double glg_sqrt(double x) {
 // ---- exp (table-driven, see glg_kExpT).  2^m goes through the exponent field; m is clamped on the integer pipe so the
 //      result stays a normal number and the function saturates (~1e-308 / ~1e308) instead of wrapping for |x| > 708.
 GLG_HD double glg_exp_tbl(int j) {
-#if defined(__CUDA_ARCH__) && GLG_EXP_SMEM
+#if defined(__CUDA_ARCH__)
     // address = base + 8 j as ONE multiply-add (left to itself the compiler emits shift, mask and add), 32-bit shared-window load
     unsigned a;
     double T;
     asm("mad.lo.u32 %0, %1, 8, %2;" : "=r"(a) : "r"(j), "r"((unsigned)__cvta_generic_to_shared(glg_exp_tbl_sh)));
     asm("ld.shared.f64 %0, [%1];" : "=d"(T) : "r"(a));
     return T;
-#elif defined(__CUDA_ARCH__)
-    return __ldg(glg_exp_tbl_dev + j);
 #else
     return glg_exp_tbl_host[j];
 #endif

@@ -9,12 +9,10 @@
 //   owner warp o : owns 28/NO states: classical RK4 stage update from the partial sums, state and stage sum in fp64
 //                  registers, next stage value back to shared memory.  Also decides the micro-step count of every nominal
 //                  substep (harvest guard, graded integrator) and tells the group warps when to stop.
-// Synchronisation per RHS evaluation: three named barriers used producer/consumer style (PTX bar.arrive / bar.sync):
-//   BAR_PARTS : early group warps arrive (do not wait), owner warps wait -- "partial sums of the early warps are in shared memory"
-//   BAR_LATE  : late group warps arrive, owner warps wait                -- "... of the late warps (glg_late_mask) too"
-//   BAR_XS    : owner warps arrive (do not wait), group warps wait       -- "stage state of the next evaluation is in shared memory"
-// so a group warp blocks once per evaluation, on the data it needs, and the owners have everything but the late warps' few
-// contributions added up by the time the slowest group warp arrives.
+// Synchronisation per RHS evaluation: two named barriers used producer/consumer style (PTX bar.arrive / bar.sync):
+//   BAR_PARTS : group warps arrive (do not wait), owner warps wait -- "partial sums are in shared memory"
+//   BAR_XS    : owner warps arrive (do not wait), group warps wait -- "stage state of the next evaluation is in shared memory"
+// so a group warp blocks once per evaluation, on the data it needs.
 // Every role has its own loop (no per-evaluation dispatch).  The loop bodies together must stay below the SM's 32 KB
 // instruction cache (tools/ubench/icache2.cu), which is why the three "condensing surface" warps (thermal screen, blackout
 // screen, cover) share ONE copy of their code with all addresses in registers (glg_surface_loop).
@@ -32,21 +30,10 @@
 
 #define GLG_ROLE_LANES 32
 constexpr int GLG_NO = 4;  // owner warps: warps 0..3, one per SM sub-partition
-constexpr int GLG_BAR_PARTS = 1, GLG_BAR_XS = 2, GLG_BAR_LATE = 3;
-// Layout switches, all measured at B = 4096 (DESIGN.md "Round-2 kernel experiments").  The role loops of the latency layout
-// together span ~32 KB of code, the SM's instruction-cache capacity (tools/ubench/icache2.cu): a variant whose loops span more
-// is 3-20 % slower whatever it was meant to gain, so every switch is judged with tools/sass_loop_size.py beside the timer.
-//   GLG_HREG        per-env-step constants of a group role in registers instead of re-read from shared memory per evaluation
-//                   (removes ~60 of the group warps' 139 shared-memory loads per evaluation): 1.447 -> 1.428 ms.  On.
-//   GLG_ORDER_TOKEN make the owners' barrier wait data-dependent on the work meant to precede it (ptxas sinks it behind the
-//                   barrier otherwise): the extra instructions push the loops over 32 KB, 1.524 ms.  Off.
-//   GLG_LATE_MASK   (glg_units.h) early / late split of the owners' reduction behind a third named barrier: 1.69 ms.  Off.
-#ifndef GLG_HREG
-#define GLG_HREG 1
-#endif
-#ifndef GLG_ORDER_TOKEN
-#define GLG_ORDER_TOKEN 0
-#endif
+constexpr int GLG_BAR_PARTS = 1, GLG_BAR_XS = 2;
+// The role loops of the latency layout together span ~32 KB of code, the SM's instruction-cache capacity
+// (tools/ubench/icache2.cu): a variant whose loops span more is 3-20 % slower at B = 4096 whatever it was meant to gain, so every
+// change to them is judged with tools/sass_loop_size.py beside the timer (DESIGN.md "Round-2 kernel experiments").
 constexpr int GLG_MAXCONTRIB = 8;
 constexpr int GLG_MAXROWS = 8;
 
@@ -61,23 +48,13 @@ __device__ long long glg_trace[32][16][2];
 #else
 #define GLG_TRACE_MARK(warp_, slot_, ev_) do {} while (0)
 #endif
-__device__ __forceinline__ void glg_bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
+// The barrier id is an immediate: with a register id the whole kernel reserves all 16 named barriers.
+template <int ID>
+__device__ __forceinline__ void glg_bar_sync(int nthreads) { asm volatile("bar.sync %1, %0;" ::"r"(nthreads), "n"(ID) : "memory"); }
 // Scheduling fences: the value must be in a register at this point of the instruction stream (ptxas otherwise sinks work that
 // was meant to overlap a barrier wait behind the barrier, and re-reads kernel parameters from the constant bank inside loops).
 __device__ __forceinline__ void glg_pin(double &v) { asm volatile("" : "+d"(v)); }
 __device__ __forceinline__ void glg_pin(int &v) { asm volatile("" : "+r"(v)); }
-// Register re-balancing between warpgroups (sm_90+ setmaxnreg): in the throughput variants (64 registers per thread at launch)
-// the three group warpgroups give registers up and the owner warpgroup (RK4 state of 7 states per thread) takes them.
-template <int N>
-__device__ __forceinline__ void glg_reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
-template <int N>
-__device__ __forceinline__ void glg_reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
-// bar.sync that ptxas cannot hoist above the computation of `token` (always 0 at run time, opaque at compile time): the barrier
-// is predicated on it.  Keeps the barrier id an immediate (a register id costs: the whole kernel then reserves 16 barriers).
-template <int ID>
-__device__ __forceinline__ void glg_bar_sync_after(int nthreads, int token) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.eq.s32 p, %1, 0;\n\t@p bar.sync %2, %0;\n\t}" ::"r"(nthreads), "r"(token), "n"(ID) : "memory");
-}
 __device__ __forceinline__ void glg_bar_arrive(int id, int nthreads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 
 // ---- owner plan and slot layout (see the header comment)
@@ -86,33 +63,20 @@ struct GlgOwnerPlan {
     int nj;                               // rows per owner warp
     int order[GLG_MAXROWS * GLG_NO];      // state of plan entry n, -1 pads
     int rank[GLG_NX];                     // plan entry of state i (states without contribution come after the active ones)
-    int row_early[GLG_MAXROWS];           // slots of early group warps row j loads (behind the first barrier)
-    int row_late[GLG_MAXROWS];            // slots of late group warps row j loads (behind the second barrier)
-    int row_base[GLG_MAXROWS + 1];        // prefix sum of row_early + row_late
+    int row_slots[GLG_MAXROWS];           // slots row j loads
+    int row_base[GLG_MAXROWS + 1];        // prefix sum of row_slots
     int slot[16][GLG_NX];                 // part slot of (group warp, state), -1 if none
     int scale_k[GLG_MAXROWS * GLG_NO];    // glg_state_scale_index of the entry's state (-1: 1.0, -2: canopy scale slot)
     int n_slots;                          // NO * row_base[nj]
-    int n_early_warps, n_late_warps;
 };
-constexpr GlgOwnerPlan glg_make_plan(const GlgWarpTable &wt, int ng, unsigned late_mask) {
+constexpr GlgOwnerPlan glg_make_plan(const GlgWarpTable &wt, int ng) {
     GlgOwnerPlan t{};
-    int ne[GLG_NX] = {}, nl[GLG_NX] = {};
-    for (int i = 0; i < GLG_NX; ++i)
-        for (int w = 0; w < ng; ++w)
-            if (wt.states[w] >> i & 1u) {
-                if (late_mask >> w & 1u) ++nl[i];
-                else ++ne[i];
-            }
-    for (int w = 0; w < ng; ++w) {
-        if (late_mask >> w & 1u) ++t.n_late_warps;
-        else ++t.n_early_warps;
-    }
-    // states sorted by (late, early) contribution counts, descending, and dealt round-robin to the owners: a row loads as many
-    // slots as its hungriest state
+    // states sorted by their contribution counts, descending, and dealt round-robin to the owners: a row loads as many slots as
+    // its hungriest state
     int n = 0;
-    for (int key = GLG_MAXCONTRIB * 16 + GLG_MAXCONTRIB; key >= 0; --key)
+    for (int key = GLG_MAXCONTRIB; key >= 0; --key)
         for (int i = 0; i < GLG_NX; ++i)
-            if (nl[i] * 16 + ne[i] == key) {
+            if (wt.contribs[i] == key) {
                 t.order[n] = i;
                 t.rank[i] = n;
                 t.scale_k[n] = glg_state_scale_index(i);
@@ -126,36 +90,30 @@ constexpr GlgOwnerPlan glg_make_plan(const GlgWarpTable &wt, int ng, unsigned la
     }
     t.row_base[0] = 0;
     for (int j = 0; j < GLG_MAXROWS; ++j) {
-        int e = 0, l = 0;
+        int e = 0;
         for (int o = 0; o < GLG_NO; ++o) {
             const int st = j * GLG_NO + o < GLG_NX ? t.order[j * GLG_NO + o] : -1;
-            if (st >= 0) {
-                e = ne[st] > e ? ne[st] : e;
-                l = nl[st] > l ? nl[st] : l;
-            }
+            if (st >= 0) e = wt.contribs[st] > e ? wt.contribs[st] : e;
         }
-        t.row_early[j] = e;
-        t.row_late[j] = l;
-        t.row_base[j + 1] = t.row_base[j] + e + l;
+        t.row_slots[j] = e;
+        t.row_base[j + 1] = t.row_base[j] + e;
     }
     t.n_slots = GLG_NO * t.row_base[t.nj];
     for (int w = 0; w < 16; ++w)
         for (int i = 0; i < GLG_NX; ++i) {
             t.slot[w][i] = -1;
             if (w < ng && (wt.states[w] >> i & 1u)) {
-                const bool late = late_mask >> w & 1u;
-                int c = 0;  // contributing warps of the same class in front of w
-                for (int ww = 0; ww < w; ++ww) c += (int)((wt.states[ww] >> i & 1u) && ((late_mask >> ww & 1u) != 0) == late);
+                int c = 0;  // contributing warps in front of w
+                for (int ww = 0; ww < w; ++ww) c += (int)(wt.states[ww] >> i & 1u);
                 const int r = t.rank[i], j = r / GLG_NO;
-                t.slot[w][i] = (t.row_base[j] + (late ? t.row_early[j] : 0) + c) * GLG_NO + r % GLG_NO;
+                t.slot[w][i] = (t.row_base[j] + c) * GLG_NO + r % GLG_NO;
             }
         }
     return t;
 }
 template <int NG, bool GENERAL>
 struct GlgPlan {
-    static constexpr GlgOwnerPlan plan = glg_make_plan(GlgWT<NG, GENERAL>::t, NG, glg_late_mask(NG));
-    static constexpr unsigned late_mask = glg_late_mask(NG);
+    static constexpr GlgOwnerPlan plan = glg_make_plan(GlgWT<NG, GENERAL>::t, NG);
     static constexpr int NJ = plan.nj;
     static constexpr int NPART = plan.n_slots;
     static constexpr int CANSCALE = NPART;  // GlgSpecial fields
@@ -276,29 +234,18 @@ __device__ __forceinline__ void glg_group_eval_dispatch(int gw, const GlgUniform
 // ---- group role: the evaluation loop of group warp W (generic: any unit list).  The per-env-step constants are loop
 // invariants: they are read from shared memory once, in front of the loop (the barriers' memory clobber would otherwise force a
 // reload per evaluation: ~60 of the group warps' 139 shared-memory loads per evaluation, tools/sasssim).
-template <int NG, int W, bool GENERAL>
-struct GlgArrive {  // barrier a group warp reports to, and that barrier's thread count
-    using PL = GlgPlan<NG, GENERAL>;
-    static constexpr bool late = (PL::late_mask >> W & 1u) != 0;
-    static constexpr int id = late ? GLG_BAR_LATE : GLG_BAR_PARTS;
-    static constexpr int count = 32 * (GLG_NO + (late ? PL::plan.n_late_warps : PL::plan.n_early_warps));
-};
 template <int NG, int W, bool GENERAL, bool NOISY, class T>
 __device__ __forceinline__ void glg_group_loop(const GlgUniform &U, const T *xs_col, T *part_col, T *h_col, T *c_col, const double *u,
                                                const volatile int *s_stop, int nthreads) {
-#if GLG_HREG
     GlgRegCol<T, H_COUNT> Hr;
     Hr.load(h_col);
     GlgRegCol<T, NOISY ? C_COUNT : 1> Cr;
     if (NOISY) Cr.load(c_col);
-#else
-    const GlgColT<T, GLG_ROLE_LANES> Hr{h_col}, Cr{c_col};
-#endif
     int last_eval;
     [[maybe_unused]] int ev = 0;
 #pragma unroll 1
     do {
-        glg_bar_sync(GLG_BAR_XS, nthreads);
+        glg_bar_sync<GLG_BAR_XS>(nthreads);
         GLG_TRACE_MARK(GLG_NO + W, 0, ev);
         // one flag per group warp (the load's immediate offset identifies the role in the SASS, tools/sasssim); read with the
         // stage state, consumed after the arrive: off the critical path
@@ -306,7 +253,7 @@ __device__ __forceinline__ void glg_group_loop(const GlgUniform &U, const T *xs_
         glg_group_eval_v<NG, W, GENERAL, NOISY, T>(U, xs_col, part_col, Hr, Cr, u);
         GLG_TRACE_MARK(GLG_NO + W, 1, ev);
         ++ev;
-        glg_bar_arrive(GlgArrive<NG, W, GENERAL>::id, GlgArrive<NG, W, GENERAL>::count);
+        glg_bar_arrive(GLG_BAR_PARTS, nthreads);
     } while (!last_eval);
 }
 
@@ -352,14 +299,12 @@ __device__ __forceinline__ void glg_surface_loop(int gw, const GlgUniform &U, co
     const T invvp = is_cv ? Kv[K_INVVPTOP] : Kv[K_INVVPAIR];
     const T L = Kv[K_L];
     const volatile int *stop = s_stop + gw;
-    static_assert(!SW::shared || ((PL::late_mask >> w_th | PL::late_mask >> w_bl | PL::late_mask >> w_cv) & 1u) == 0, "surface warps are early warps");
-    constexpr int n_arrive = 32 * (GLG_NO + PL::plan.n_early_warps);
     const T coef_a = h_col[ha], coef_b = h_col[hb];  // loop invariants
     int last_eval;
     [[maybe_unused]] int ev = 0;
 #pragma unroll 1
     do {
-        glg_bar_sync(GLG_BAR_XS, nthreads);
+        glg_bar_sync<GLG_BAR_XS>(nthreads);
         GLG_TRACE_MARK(GLG_NO + gw, 0, ev);
         T surf, air, far, vp;
         last_eval = *stop;
@@ -370,7 +315,7 @@ __device__ __forceinline__ void glg_surface_loop(int gw, const GlgUniform &U, co
         part_col[pv] = vp;
         GLG_TRACE_MARK(GLG_NO + gw, 1, ev);
         ++ev;
-        glg_bar_arrive(GLG_BAR_PARTS, n_arrive);
+        glg_bar_arrive(GLG_BAR_PARTS, nthreads);
     } while (!last_eval);
 }
 
@@ -397,19 +342,17 @@ __constant__ double glg_kStageW[4] = {1.0, 2.0, 2.0, 1.0};
 // its CTA mates.
 // Stage update in unscaled units: s = sum of the partial sums, k = scale * s.
 //   stage 0..2: acc = (stage ? acc : 0) + w s ; xs = x + (c h scale) s        stage 3: x += (h/6 scale) (acc + s) ; xs = x
-// One evaluation, in program order (the order matters: everything in front of the last barrier wait is off the critical path,
+// One evaluation, in program order (the order matters: everything in front of the barrier wait is off the critical path,
 // what follows it is the CTA's serial section behind its slowest group warp):
-//   book()       : stage-sum / state / counter updates of the PREVIOUS evaluation
-//   pre()        : (c h scale), the acc term of stage 3, the end-of-interval tests
-//   post_early() : partial sums of the early group warps -> pairwise tree -> pre-accumulated into the stage state
-//   order_token(): data dependence of the late barrier on all of the above (ptxas otherwise sinks it behind the barrier)
-//   post_late()  : partial sums of the late group warps -> one add + one FMA per affected row -> next stage state to shared memory
+//   book()   : stage-sum / state / counter updates of the PREVIOUS evaluation
+//   pre()    : (c h scale), the acc term of stage 3, the end-of-interval tests
+//   reduce() : partial sums of the group warps -> pairwise tree per row, harvest guard
+//   update() : micro-step count of a first evaluation, next stage state to shared memory
 template <class T, int NG, bool GENERAL>
 struct GlgOwner {
     using PL = GlgPlan<NG, GENERAL>;
     static constexpr int NJ = PL::NJ, NL = GLG_ROLE_LANES;
     static constexpr int can_row = PL::canopy_entry / GLG_NO;
-    static constexpr bool kHasLate = PL::late_mask != 0u;
     double xo[NJ], acc[NJ], scale[NJ];  // the RK4 state and stage sum stay fp64 in both precisions
     double hc[NJ], base[NJ], sum[NJ], xn[NJ];
     double h_nom, h_lane, cs, w, can_cs;
@@ -472,7 +415,7 @@ struct GlgOwner {
         }
     }
     __device__ __forceinline__ void pre(int lane) {
-        first = stage == 0 && q == 0;  // first evaluation of a nominal substep: the micro-step count is decided in post_late()
+        first = stage == 0 && q == 0;  // first evaluation of a nominal substep: the micro-step count is decided in update()
         last = stage == 3;
         cs = glg_kStageC[stage];  // 1/2, 1/2, 1, 1/6 : constant-bank lookups instead of select chains (loop code size)
         w = glg_kStageW[stage];   // 1, 2, 2, 1
@@ -504,56 +447,23 @@ struct GlgOwner {
             for (int c = 0; c + s < N; c += 2 * s) v[c] += v[c + s];
         return v[0];
     }
-    __device__ __forceinline__ void post_early(const T *part_col) {
+    __device__ __forceinline__ void reduce(const T *part_col) {
         const T *pbase = part_col + o * NL;  // row j, contribution c at pbase[(row_base[j] + c) * NO * NL]
         glg_static_for<0, NJ>([&](auto jc) {
             constexpr int j = decltype(jc)::value;
-            constexpr int n = PL::plan.row_early[j];
+            constexpr int n = PL::plan.row_slots[j];
             constexpr int rb = PL::plan.row_base[j];
             if constexpr (n == 0) sum[j] = 0.0;
             else sum[j] = tree<n>(pbase + rb * GLG_NO * NL);
         });
-        // the canopy's capacity scale K_INVCAPLEAF / LAI changes with the stage (its scale[] entry is 1); U_PIPES is an early unit
+        // the canopy's capacity scale K_INVCAPLEAF / LAI changes with the stage (its scale[] entry is 1)
         can_cs = can_owner ? (double)part_col[PL::CANSCALE * NL] : 1.0;
         sum[can_row] *= can_cs;
-        // harvest guard: m = 1 unless an organ is inside its harvest window (2 h lambda >= 1); U_MAINT is an early unit
+        // harvest guard: m = 1 unless an organ is inside its harvest window (2 h lambda >= 1)
         split_h = first && (2.0 * h_nom * (double)part_col[PL::LAMBDA * NL] >= 1.0);
-        if (kHasLate) {
-#pragma unroll
-            for (int j = 0; j < NJ; ++j) base[j] = glg_fma(hc[j], sum[j], base[j]);
-        }
     }
-    // 0 for the caller as far as ptxas can tell (zero is an opaque 0): added to the id of the barrier that follows, it makes the
-    // barrier wait data-dependent on everything computed so far
-    __device__ __forceinline__ int order_token(int zero) const {
-        int t = 0;
-#pragma unroll
-        for (int j = 0; j < NJ; ++j) t ^= __double2loint(hc[j]) ^ __double2loint(base[j]) ^ __double2loint(acc[j]) ^ __double2loint(sum[j]);
-        t ^= (int)split_h ^ final_eval ^ flag_next;
-#if GLG_ORDER_TOKEN
-        return t & zero;
-#else
-        return 0;
-#endif
-    }
-    __device__ __forceinline__ void post_late(const GlgUniform &U, const T *part_col, T *xs_col) {
-        const T *pbase = part_col + o * NL;
+    __device__ __forceinline__ void update(const GlgUniform &U, const T *part_col, T *xs_col) {
         T *xbase = xs_col + o * NL;  // row j at xbase[j * NO * NL]
-        if (kHasLate) {
-            glg_static_for<0, NJ>([&](auto jc) {
-                constexpr int j = decltype(jc)::value;
-                constexpr int n = PL::plan.row_late[j];
-                if constexpr (n == 0) {
-                    xn[j] = base[j];
-                } else {
-                    constexpr int rb = PL::plan.row_base[j] + PL::plan.row_early[j];
-                    double l = tree<n>(pbase + rb * GLG_NO * NL);
-                    if constexpr (j == can_row) l *= can_cs;
-                    xn[j] = glg_fma(hc[j], l, base[j]);
-                    sum[j] += l;
-                }
-            });
-        }
         if (first) {
             // m = 1 for every env of the CTA unless a harvest window is active, the graded integrator is at the start of the
             // interval or its stiffness rule asks for a split: one vote on the common path
@@ -577,21 +487,17 @@ struct GlgOwner {
                 // redo the stage update with the right step (first evaluation: stage 0, base = x)
                 const double hcs = cs * h_lane;
 #pragma unroll
-                for (int j = 0; j < NJ; ++j) {
-                    hc[j] = hcs * scale[j];
-                    if (kHasLate) xn[j] = glg_fma(hc[j], sum[j], xo[j]);
-                }
+                for (int j = 0; j < NJ; ++j) hc[j] = hcs * scale[j];
             }
             n_micro += m_lane;
         }
-        if (!kHasLate) {  // one copy of the stage update for all paths (the loop code must stay below the instruction cache)
+        // one copy of the stage update for all paths (the loop code must stay below the instruction cache)
 #pragma unroll
-            for (int j = 0; j < NJ; ++j) xn[j] = glg_fma(hc[j], sum[j], base[j]);
-        }
+        for (int j = 0; j < NJ; ++j) xn[j] = glg_fma(hc[j], sum[j], base[j]);
 #pragma unroll
         for (int j = 0; j < NJ; ++j) xbase[j * GLG_NO * NL] = (T)xn[j];
     }
-    // final state (xn of the last evaluation: the caller leaves its loop right behind that post_late()) -> s_xfin; returns 1 if
+    // final state (xn of the last evaluation: the caller leaves its loop right behind that update()) -> s_xfin; returns 1 if
     // any of this owner's states is not finite
     __device__ __forceinline__ int finish(double *s_xfin, int lane) const {
         int bad = 0;
@@ -599,7 +505,7 @@ struct GlgOwner {
             constexpr int j = decltype(jc)::value;
             const int st = row_state<j>();
             bad |= !(fabs(xn[j]) <= 1.79769313486231570e308);
-            if (!kStateInXs && st >= 0) s_xfin[st * NL + lane] = xn[j];  // fp64 units: post_late() left it in the stage-state block
+            if (!kStateInXs && st >= 0) s_xfin[st * NL + lane] = xn[j];  // fp64 units: update() left it in the stage-state block
         });
         return bad;
     }
@@ -615,15 +521,19 @@ struct GlgOwner {
 //           registers); one loop, two CTA barriers per evaluation, 4 CTAs per SM so that every SM sub-partition runs ONE role's
 //           code for four CTAs.  Compared with the round-1 kernel the owner side keeps only the RK4 state in registers (all
 //           addresses are immediates of the rank-ordered layout), so the unit code has ~95 registers for interleaving.
-// MINB = CTAs per SM the register budget is sized for.
-template <class T, bool GENERAL, bool NOISY, int NG, int MINB, bool FUSED>
-__global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_step_units_kernel(const __grid_constant__ GlgUniform U,
-                                                                                                 const __grid_constant__ GlgStepArgs A) {
+template <bool FUSED>
+struct GlgLayout {
+    static constexpr int NG = FUSED ? GLG_NO : 12;           // group warps per 32 envs
+    static constexpr int MINB = FUSED ? 4 : 1;               // CTAs per SM the register budget is sized for
+    static constexpr int NT = 32 * (NG + (FUSED ? 0 : GLG_NO));  // threads per CTA
+};
+template <class T, bool GENERAL, bool NOISY, bool FUSED>
+__global__ void __launch_bounds__(GlgLayout<FUSED>::NT, GlgLayout<FUSED>::MINB) glg_step_units_kernel(const __grid_constant__ GlgUniform U,
+                                                                                                       const __grid_constant__ GlgStepArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    static_assert(!FUSED || NG == GLG_NO, "fused layout: one group role per owner");
     glg_exp_tbl_fill();
     constexpr int NL = GLG_ROLE_LANES;
-    constexpr int NT = 32 * (NG + (FUSED ? 0 : GLG_NO));
+    constexpr int NG = GlgLayout<FUSED>::NG, NT = GlgLayout<FUSED>::NT;
     using PL = GlgPlan<NG, GENERAL>;
     using SW = GlgSurfaceWarps<NG, GENERAL>;
     constexpr int NJ = PL::NJ;
@@ -643,7 +553,7 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
     int *s_tbl_t = s_k + NL;
     int *s_k_t = s_tbl_t + NL;
     int *s_bad = s_k_t + NL;
-    int *s_misc = s_bad + NL;            // [0..1] weather staging
+    int *s_misc = s_bad + NL;            // [0..1] weather staging, [2] uniform weather, [3] 0
     volatile int *s_stop = s_misc + 4;   // [16] stop flag, one copy per group warp
 
     const int tid = threadIdx.x;
@@ -710,7 +620,7 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
         }
         if (lane == 0) {
             s_misc[2] = uniform;
-            s_misc[3] = 0;
+            s_misc[3] = 0;  // read by nothing; without this store ptxas allocates the registers of every variant differently
         }
     } else {
         for (int i = tid - 32; i < PL::NSLOTS * NL; i += NT - 32) s_part[i] = (T)0;
@@ -720,11 +630,6 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
     T *xs_col = s_xs + lane;
     T *part_col = s_part + lane;
     int n_micro = 0;  // RK4 micro-steps this env executed (owner warp 0 counts)
-    // register budget per thread at launch, and after re-balancing (throughput variants only)
-    constexpr int kLaunchRegs = (65536 / (MINB * NT)) / 8 * 8 > 255 ? 248 : (65536 / (MINB * NT)) / 8 * 8;
-    constexpr int kGroupRegs = kLaunchRegs >= 80 ? 64 : kLaunchRegs >= 64 ? 56 : 48;
-    constexpr int kOwnerRegs = (kLaunchRegs + (kLaunchRegs - kGroupRegs) * NG / GLG_NO) / 8 * 8;
-    constexpr bool kRebalance = !FUSED && MINB > 1 && kLaunchRegs > kGroupRegs && kLaunchRegs <= 80 && NG % 4 == 0;
     if (FUSED) {
         // ---- fused layout: every warp is group warp `warp` and owner `warp`
         if (GENERAL && active && warp == GlgWT<NG, GENERAL>::unit_warp(U_FIR)) {
@@ -738,8 +643,8 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
             glg_group_eval_dispatch<NG, 0, GENERAL, NOISY, T>(warp, U, xs_col, part_col, s_H + lane, s_C + lane, u);
             own.pre(lane);
             __syncthreads();
-            own.post_early(part_col);
-            own.post_late(U, part_col, xs_col);
+            own.reduce(part_col);
+            own.update(U, part_col, xs_col);
             if (own.final_eval) break;
             own.book();  // in front of the barrier: measured 13 % faster at B = 262 144 than at the top of the loop (more spills there)
             __syncthreads();
@@ -748,7 +653,6 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
         if (own.finish(s_xfin, lane)) s_bad[lane] = 1;  // benign race: every writer stores 1
     } else if (warp >= GLG_NO) {
         // ---- group warps
-        if (kRebalance) glg_reg_dec<kGroupRegs>();
         const int gw = warp - GLG_NO;
         if (GENERAL && active && gw == GlgWT<NG, GENERAL>::unit_warp(U_FIR)) {
             // U_FIR's general terms read the raw screen controls; warp 0's prologue stored the updated controls before the barrier
@@ -757,30 +661,20 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
         }
         if (SW::shared && (gw == SW::th || gw == SW::bl || gw == SW::cv)) glg_surface_loop<NG, GENERAL, T>(gw, U, xs_col, part_col, s_H + lane, s_stop, NT);
         else glg_group_dispatch<NG, 0, GENERAL, NOISY, T>(gw, U, xs_col, part_col, s_H + lane, s_C + lane, u, s_stop, NT);
-        if (kRebalance) glg_reg_inc<kLaunchRegs>();
     } else {
         // ---- owner warps (GlgOwner)
-        if (kRebalance) glg_reg_inc<kOwnerRegs>();
         GlgOwner<T, NG, GENERAL> own;
         own.init(warp, A, s_xfin, s_scale, xs_col, lane, true);
-        const int zero = *reinterpret_cast<const volatile int *>(s_misc + 3);  // 0, but not as far as ptxas knows (order_token)
-        constexpr int n_early = 32 * (GLG_NO + PL::plan.n_early_warps), n_late = 32 * (GLG_NO + PL::plan.n_late_warps);
         glg_bar_arrive(GLG_BAR_XS, NT);  // the prologue's stage state is in shared memory: release the group warps' first evaluation
         [[maybe_unused]] int ev = 0;
 #pragma unroll 1
         for (;;) {
             own.book();
             own.pre(lane);
-            if (PL::late_mask != 0u) {
-                glg_bar_sync(GLG_BAR_PARTS, n_early);
-                own.post_early(part_col);
-                glg_bar_sync_after<GLG_BAR_LATE>(n_late, own.order_token(zero));
-            } else {
-                glg_bar_sync_after<GLG_BAR_PARTS>(n_early, own.order_token(zero));
-                own.post_early(part_col);
-            }
+            glg_bar_sync<GLG_BAR_PARTS>(NT);
+            own.reduce(part_col);
             GLG_TRACE_MARK(warp, 0, ev);
-            own.post_late(U, part_col, xs_col);
+            own.update(U, part_col, xs_col);
             if (own.final_eval) break;
             if (own.flag_next) s_stop[lane] = 1;
             GLG_TRACE_MARK(warp, 1, ev);
@@ -790,7 +684,6 @@ __global__ void __launch_bounds__(32 * (NG + (FUSED ? 0 : GLG_NO)), MINB) glg_st
         n_micro = own.n_micro;
         const int bad = own.finish(s_xfin, lane);
         if (bad) s_bad[lane] = 1;  // benign race: every writer stores 1
-        if (kRebalance) glg_reg_dec<kLaunchRegs>();
     }
     __syncthreads();
 

@@ -527,43 +527,21 @@ GLG_HD constexpr GlgAssign glg_assign(int ng) {
     if (ng == 12) {
         // sub-partition of group warp w is (w + NO) % 4 with NO = 4 owner warps in front => w % 4
         // the heaviest unit of each sub-partition sits on the LOWEST warp id (measured: 1.73 ms vs 1.91 ms per step at B = 4096 with
-        // the order reversed)
-#ifndef GLG_ASSIGN12
-#define GLG_ASSIGN12 0
-#endif
-#if GLG_ASSIGN12 == 0
+        // the order reversed); moving floor convection to the maintenance unit's warp was measured and dropped (DESIGN.md item 4)
         const int t[12][2] = {{U_FIR, -1},    {U_PHOTO, -1}, {U_FLOWS, -1}, {U_SCR, -1},
                               {U_TRANSP, -1}, {U_OPT, -1},   {U_PIPES, -1}, {U_VENT, U_FLOOR},
                               {U_COVER, -1},  {U_THSCR, -1}, {U_MAINT, -1}, {U_BLSCR, -1}};
-#else  // floor convection with the maintenance unit: lightens the sub-partition of the slowest warp (screen air flux)
-        const int t[12][2] = {{U_FIR, -1},    {U_PHOTO, -1}, {U_FLOWS, -1}, {U_SCR, -1},
-                              {U_TRANSP, -1}, {U_OPT, -1},   {U_PIPES, -1}, {U_VENT, -1},
-                              {U_COVER, -1},  {U_THSCR, -1}, {U_MAINT, U_FLOOR}, {U_BLSCR, -1}};
-#endif
         for (int w = 0; w < 12; ++w)
             for (int k = 0; k < 2; ++k) a.unit[w][k] = t[w][k];
     } else if (ng == 4) {  // one fat warp per sub-partition (throughput layouts: all warps of a sub-partition run the same code)
-#ifndef GLG_ASSIGN4
-#define GLG_ASSIGN4 0
-#endif
-#if GLG_ASSIGN4 == 0
         const int t[4][5] = {{U_FIR, U_TRANSP, U_COVER, -1, -1}, {U_PHOTO, U_OPT, U_THSCR, -1, -1}, {U_FLOWS, U_PIPES, U_MAINT, -1, -1},
                              {U_SCR, U_VENT, U_FLOOR, U_BLSCR, -1}};
-        // measured at B = 262 144 (graded, 300 RK4 steps): 0 = 30.46 ms per step; 1 = 33.31; 2 = 33.98; 3 = 30.48 -- equal FP64
-        // instruction counts per warp do not balance the roles, the dependency chains inside the units do
-#elif GLG_ASSIGN4 == 1  // FP64 instructions per warp 225 / 234 / 227 / 232 instead of 255 / 234 / 232 / 197
-        const int t[4][5] = {{U_PHOTO, U_TRANSP, -1, -1, -1}, {U_FIR, U_PIPES, U_MAINT, -1, -1}, {U_FLOWS, U_THSCR, U_BLSCR, -1, -1},
-                             {U_SCR, U_VENT, U_FLOOR, U_COVER, U_OPT}};
-#elif GLG_ASSIGN4 == 2
-        const int t[4][5] = {{U_PHOTO, U_TRANSP, -1, -1, -1}, {U_FIR, U_PIPES, U_OPT, -1, -1}, {U_FLOWS, U_THSCR, U_BLSCR, -1, -1},
-                             {U_SCR, U_VENT, U_FLOOR, U_COVER, U_MAINT}};
-#else
-        const int t[4][5] = {{U_FIR, U_TRANSP, U_OPT, -1, -1}, {U_PHOTO, U_COVER, U_THSCR, -1, -1}, {U_FLOWS, U_PIPES, U_MAINT, -1, -1},
-                             {U_SCR, U_VENT, U_FLOOR, U_BLSCR, -1}};
-#endif
+        // measured at B = 262 144 (graded, 300 RK4 steps): this table 30.46 ms per step; three re-deals 33.31 (FP64 instructions
+        // per warp 225 / 234 / 227 / 232 instead of 255 / 234 / 232 / 197), 33.98 and 30.48 -- equal FP64 instruction counts per
+        // warp do not balance the roles, the dependency chains inside the units do
         for (int w = 0; w < 4; ++w)
             for (int k = 0; k < 5; ++k) a.unit[w][k] = t[w][k];
-    } else if (ng == 8) {
+    } else if (ng == 8) {  // the kernels do not use these two: the host build of the unit split checks them against the oracle
         const int t[8][3] = {{U_FIR, -1, -1},          {U_PHOTO, U_FLOOR, -1}, {U_FLOWS, U_MAINT, -1}, {U_SCR, U_VENT, -1},
                              {U_THSCR, U_TRANSP, -1},  {U_OPT, U_COVER, -1},   {U_PIPES, -1, -1},      {U_BLSCR, -1, -1}};
         for (int w = 0; w < 8; ++w)
@@ -573,14 +551,6 @@ GLG_HD constexpr GlgAssign glg_assign(int ng) {
     }
     return a;
 }
-// Group warps whose partial sums the owners add LAST (bit w = group warp w).  The owners wait for the other ("early") warps on
-// one named barrier, pre-add their partial sums, and only the few contributions of the late warps are loaded and added after
-// the second barrier -- the owners' critical section behind the slowest group warp shrinks from ~18 shared-memory loads per owner
-// to the late slots of its rows.  Pick the warps that finish last (the heaviest unit of every sub-partition, tools/sasssim).
-#ifndef GLG_LATE_MASK
-#define GLG_LATE_MASK 0x0u  // off; 0xE = photosynthesis, carbohydrate flows, screen air flux (NG = 12) measured 20 % slower
-#endif
-GLG_HD constexpr unsigned glg_late_mask(int ng) { return ng == 12 ? GLG_LATE_MASK : 0u; }
 // everything the kernel needs to know about the assignment, computed in one pass (cheap for the constexpr evaluator)
 struct GlgWarpTable {
     unsigned states[16];                         // states warp w contributes to

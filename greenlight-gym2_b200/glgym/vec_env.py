@@ -285,7 +285,7 @@ class GreenLightVecEnv(_VecEnvBase):
         cfg.role_lanes = int(role_lanes)  # kernel C envs-per-CTA override (0 = auto)
         for i, m in enumerate(mods):
             cfg.obs_modules[i] = OBSERVATION_MODULES[m][0]
-        cfg.role_warps = int(role_warps)  # 0 auto, 1 = one thread per env, 2 / 3 = warp-specialised kernel (1 / 2 CTAs per SM)
+        cfg.role_warps = int(role_warps)  # 0 auto, 1 = one thread per env, 2 / 3 = warp-specialised kernel (latency layout, 1 CTA per SM / throughput layout, 4 CTAs per SM)
         self.reward_params = rp
         self._seed = int(seed)
         self._h = C.c_void_p()

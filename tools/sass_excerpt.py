@@ -11,7 +11,7 @@ from parse import functions, parse  # noqa: E402
 import sim2  # noqa: E402
 
 lib = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "greenlight-gym2_b200", "glgym", "libglgym.so")
-fn = sys.argv[2] if len(sys.argv) > 2 else "glg_step_units_kernelIdLb0ELb0ELi12ELi1ELb0"
+fn = sys.argv[2] if len(sys.argv) > 2 else "glg_step_units_kernelIdLb0ELb0ELb0E"
 dump = "/tmp/_sass_excerpt.sass"
 open(dump, "w").write(subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True).stdout)
 arch = re.search(r"arch = (sm_\w+)", open(dump).read())

@@ -1,7 +1,7 @@
 """Byte size of kernel C's evaluation loops (all roles) in a SASS dump: python tools/sass_loop_size.py <dump.sass> [function substring]
 The loops must fit the SM's ~32 KB instruction cache together (tools/ubench/icache2.cu)."""
 import re, sys
-fn = sys.argv[2] if len(sys.argv) > 2 else "glg_step_units_kernelIdLb0ELb0ELi12ELi1ELb0"
+fn = sys.argv[2] if len(sys.argv) > 2 else "glg_step_units_kernelIdLb0ELb0ELb0E"
 cur, lo, hi, n64 = None, None, None, 0
 for line in open(sys.argv[1]):
     if "Function :" in line:
