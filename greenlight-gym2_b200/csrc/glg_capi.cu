@@ -9,6 +9,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <memory>
 #include <new>
 #include <string>
 #include <thread>
@@ -27,31 +28,69 @@
 #include "glg_plan.cuh"
 
 
-static thread_local std::string g_create_error = "";
+static thread_local std::string g_error = "";  // glg_last_error(NULL): the last failure of an entry point without a handle
+
+// The CUDA allocations of one object: device memory (zero-filled) and page-locked host memory, freed together by the
+// destructor, which runs with the object's device current.  Nothing else in this file frees CUDA memory.
+class CudaMem {
+  public:
+    CudaMem() = default;
+    CudaMem(const CudaMem &) = delete;
+    CudaMem &operator=(const CudaMem &) = delete;
+    ~CudaMem() {
+        for (const Block &b : blocks_) b.host ? cudaFreeHost(b.p) : cudaFree(b.p);
+    }
+    template <typename T>
+    cudaError_t dev(T **p, size_t n) {
+        cudaError_t e = cudaMalloc((void **)p, n * sizeof(T));
+        if (e != cudaSuccess) return e;
+        blocks_.push_back({*p, n * sizeof(T), false});
+        return cudaMemset(*p, 0, n * sizeof(T));
+    }
+    template <typename T>
+    cudaError_t host(T **p, size_t n) {
+        cudaError_t e = cudaMallocHost((void **)p, n * sizeof(T));
+        if (e == cudaSuccess) blocks_.push_back({*p, n * sizeof(T), true});
+        return e;
+    }
+    size_t bytes() const {
+        size_t n = 0;
+        for (const Block &b : blocks_) n += b.bytes;
+        return n;
+    }
+    void swap(CudaMem &o) { blocks_.swap(o.blocks_); }
+
+  private:
+    struct Block {
+        void *p;
+        size_t bytes;
+        bool host;
+    };
+    std::vector<Block> blocks_;
+};
 
 struct glg_handle {
-    glg_config cfg;
-    int B = 0, obs_dim = 0, nt = 64, role_lanes = 32, sms = 148;
-    bool have_params = false, have_weather = false, general = false, is_reset = false;
+    ~glg_handle();
+    glg_config cfg;  // as created; what the setters change since lives in `a`
+    // The env's launch state, kept current by the setters: sizes, config scalars, observation layout, ctrl, the bank and the
+    // state / output buffers.  Its per-call fields (actions, controls, noise, raw_control) stay 0 here; each launch sets them
+    // on a copy.
+    GlgStepArgs a = {};
+    int n_head = 0;  // obs_dim - 5 Np with a forecast block, else obs_dim: the packed row (obs_head) the host paths copy
+    int sms = 148;
+    bool have_params = false, general = false, is_reset = false;
     GlgUniform uni;
-    // device buffers
-    double *x = nullptr, *u = nullptr, *time = nullptr, *ep_return = nullptr, *ep_info = nullptr;
-    int *timestep = nullptr, *table = nullptr, *ep_len = nullptr;
-    unsigned int *step_ctr = nullptr;
-    float *obs = nullptr, *term_obs = nullptr, *actions = nullptr, *obs_head = nullptr;
-    double *reward = nullptr, *info = nullptr, *stats = nullptr;
-    unsigned char *done = nullptr, *res_block = nullptr;
-    double *weather = nullptr, *start_day = nullptr;
-    int *reset_tables = nullptr;
-    int n_tables = 0, rows = 0, n_reset_tables = 0;
+    CudaMem mem;                   // the state / output buffers `a` points into, `actions` and the pinned host staging
+    CudaMem bank, reset_list;      // what a.weather, a.start_day (glg_set_weather) and a.reset_tables point into
+    std::vector<float> fc_bank;    // [n_tables][rows][5] float32: the weather columns a forecast block shows, as the kernels cast them
     unsigned long long weather_gen = 0;  // bumped by every glg_set_weather: replay buffers hold keys into the bank
+    float *actions = nullptr;      // [B][6] device: the host step paths' actions
     // pinned host staging for glg_step_host
     float *h_actions = nullptr, *h_obs = nullptr;
     double *h_reward = nullptr;
     unsigned char *h_done = nullptr;
     // host side of glg_step_host's overlapped observation path (see there)
-    std::vector<float> fc_bank;  // [n_tables][rows][5] float32: the weather columns a forecast block shows, as the kernels cast them
-    float *h_head = nullptr;     // pinned [B][obs_dim - 5 Np]: staging of the packed columns for a pageable destination
+    float *h_head = nullptr;     // pinned [B][n_head]: staging of the packed columns for a pageable destination
     unsigned char *h_res = nullptr;  // pinned [2 buffers][17 B]: reward | timestep | table | done of every env after a glg_step_host
     int kt_cur = 0;              // buffer the last glg_step_host filled
     bool kt_valid = false;       // h_res[kt_cur] holds this handle's last host step (a prediction source, verified after every step)
@@ -60,11 +99,10 @@ struct glg_handle {
     cudaStream_t own_stream = nullptr;
     cudaEvent_t order_event = nullptr;  // glg_host_path_after
     long long launches = 0;
-    double ctrl[GLG_NCTRL];  // rule-based controller settings (defaults: configs/agents/rule_based.yml)
-    int obs_nmod = 0, obs_mod[GLG_MAXOBSMOD] = {}, obs_off[GLG_MAXOBSMOD] = {}, fc_off = -1;
     void *nccl_comm = nullptr;  // ncclComm_t (glg_nccl_init)
     std::string err;
 };
+// rule-based controller settings: configs/agents/rule_based.yml
 static const double kDefaultCtrl[GLG_NCTRL] = {0, 18, -1, 366, 400, 10, 19.5, 16.5, 0, 5, 800, 4, 85, 2, 5, 1, -1, 5, 10, -1, 4, -2,
                                                2, 2, 100, 85, -1, -100, 1};
 
@@ -111,15 +149,9 @@ extern "C" void glg_default_config(glg_config *c) {
     for (int i = 0; i < 8; ++i) c->obs_modules[i] = 0;  // empty = the default stack of TomatoEnv.yml
 }
 
-extern "C" const char *glg_last_error(const glg_handle *h) { return h ? h->err.c_str() : g_create_error.c_str(); }
+extern "C" const char *glg_last_error(const glg_handle *h) { return h ? h->err.c_str() : g_error.c_str(); }
 
 static size_t res_block_bytes(size_t B) { return 17 * B; }  // double reward[B] | int32 timestep[B] | int32 table[B] | uint8 done[B]
-template <typename T>
-static cudaError_t dev_alloc(T **p, size_t n) {
-    cudaError_t e = cudaMalloc((void **)p, n * sizeof(T));
-    if (e == cudaSuccess) e = cudaMemset(*p, 0, n * sizeof(T));
-    return e;
-}
 
 // ---- episode-statistics all-reduce over NCCL, bound at run time ---------------------------------------------
 struct NcclId {  // ncclUniqueId: 128 opaque bytes, passed by value
@@ -161,33 +193,25 @@ static NcclApi *nccl_api(std::string *err) {
     return &api;
 }
 
+glg_handle::~glg_handle() {  // memory goes with the CudaMem members
+    if (order_event) cudaEventDestroy(order_event);
+    if (own_stream) cudaStreamDestroy(own_stream);
+    if (nccl_comm) {
+        std::string e;
+        NcclApi *n = nccl_api(&e);
+        if (n) n->CommDestroy(nccl_comm);
+    }
+}
+
 extern "C" void glg_destroy(glg_handle *h) {
     if (!h) return;
     cudaSetDevice(h->cfg.device);
-    cudaFree(h->x); cudaFree(h->u); cudaFree(h->time); cudaFree(h->ep_return); cudaFree(h->ep_info);
-    cudaFree(h->res_block); cudaFree(h->ep_len); cudaFree(h->step_ctr);
-    cudaFree(h->obs_head);
-    cudaFree(h->obs); cudaFree(h->term_obs); cudaFree(h->actions); cudaFree(h->info);
-    cudaFree(h->stats); cudaFree(h->weather); cudaFree(h->start_day); cudaFree(h->reset_tables);
-    if (h->h_actions) cudaFreeHost(h->h_actions);
-    if (h->h_obs) cudaFreeHost(h->h_obs);
-    if (h->h_reward) cudaFreeHost(h->h_reward);
-    if (h->h_done) cudaFreeHost(h->h_done);
-    if (h->h_head) cudaFreeHost(h->h_head);
-    if (h->h_res) cudaFreeHost(h->h_res);
-    if (h->order_event) cudaEventDestroy(h->order_event);
-    if (h->own_stream) cudaStreamDestroy(h->own_stream);
-    if (h->nccl_comm) {
-        std::string e;
-        NcclApi *n = nccl_api(&e);
-        if (n) n->CommDestroy(h->nccl_comm);
-    }
     delete h;
 }
 
 extern "C" int glg_create(const glg_config *cfg, glg_handle **out) {
     if (!cfg || !out) {
-        g_create_error = "glg_create: null argument";
+        g_error = "glg_create: null argument";
         return GLG_ERR_ARG;
     }
     *out = nullptr;
@@ -195,23 +219,38 @@ extern "C" int glg_create(const glg_config *cfg, glg_handle **out) {
         (cfg->precision != 0 && cfg->precision != 1) ||
         (cfg->role_warps < 0 || cfg->role_warps > 3) ||
         (cfg->integrator != 0 && cfg->integrator != 1) || (cfg->precision == 1 && cfg->role_warps == 1)) {
-        g_create_error = (cfg->precision == 1 && cfg->role_warps == 1)
-                             ? "glg_create: the fp32 throughput mode runs on kernel C only (role_warps 0, 2 or 3)"
-                             : "glg_create: invalid num_envs / n_sub / N / Np / dt / precision / role_warps / integrator";
+        g_error = (cfg->precision == 1 && cfg->role_warps == 1)
+                      ? "glg_create: the fp32 throughput mode runs on kernel C only (role_warps 0, 2 or 3)"
+                      : "glg_create: invalid num_envs / n_sub / N / Np / dt / precision / role_warps / integrator";
         return GLG_ERR_ARG;
     }
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
     if (ce != cudaSuccess || ndev == 0 || cfg->device < 0 || cfg->device >= ndev) {
-        g_create_error = std::string("glg_create: no usable CUDA device (") + cudaGetErrorString(ce) +
-                         "); this library has no CPU fallback";
+        g_error = std::string("glg_create: no usable CUDA device (") + cudaGetErrorString(ce) + "); this library has no CPU fallback";
         return GLG_ERR_CUDA;
     }
     glg_handle *h = new (std::nothrow) glg_handle();
     if (!h) return GLG_ERR_ALLOC;
     h->cfg = *cfg;
-    for (int i = 0; i < GLG_NCTRL; ++i) h->ctrl[i] = kDefaultCtrl[i];
-    h->B = cfg->num_envs;
+    GlgStepArgs &a = h->a;
+    a.B = cfg->num_envs; a.n_sub = cfg->n_sub; a.N = cfg->N; a.Np = cfg->Np; a.auto_reset = cfg->auto_reset;
+    a.integrator = cfg->integrator;
+    a.dt = cfg->dt;
+    for (int i = 0; i < GLG_NU; ++i) {
+        a.u_min[i] = cfg->u_min[i];
+        a.u_max[i] = cfg->u_max[i];
+    }
+    a.delta_u_max_f32 = (float)cfg->delta_u_max;
+    for (int i = 0; i < 3; ++i) {
+        a.con_low[i] = cfg->con_low[i];
+        a.con_high[i] = cfg->con_high[i];
+    }
+    a.elec_price = cfg->elec_price; a.heating_price = cfg->heating_price; a.co2_price = cfg->co2_price;
+    a.fruit_price = cfg->fruit_price; a.dmfm = cfg->dmfm; a.fixed_costs = cfg->fixed_costs;
+    a.uncertainty_scale = cfg->uncertainty_scale;
+    a.seed = cfg->seed; a.env_id_offset = cfg->env_id_offset;
+    for (int i = 0; i < GLG_NCTRL; ++i) a.ctrl[i] = kDefaultCtrl[i];
     {
         // observation row layout from the module list (tomato_env.py:77-96)
         static const int kDefault[6] = {GLG_OBS_CLIMATE, GLG_OBS_CROP, GLG_OBS_CONTROL, GLG_OBS_WEATHER, GLG_OBS_TIME, GLG_OBS_FORECAST};
@@ -220,6 +259,7 @@ extern "C" int glg_create(const glg_config *cfg, glg_handle **out) {
         int off = 0;
         bool ok = true;
         const bool use_default = cfg->obs_modules[0] == 0;
+        a.fc_off = -1;
         for (int m = 0; m < GLG_MAXOBSMOD; ++m) {
             const int id = use_default ? (m < 6 ? kDefault[m] : 0) : cfg->obs_modules[m];
             if (id == 0) break;
@@ -228,53 +268,55 @@ extern "C" int glg_create(const glg_config *cfg, glg_handle **out) {
                 break;
             }
             seen |= 1u << id;
-            h->obs_mod[h->obs_nmod] = id;
-            h->obs_off[h->obs_nmod] = off;
-            if (id == GLG_OBS_FORECAST) h->fc_off = off;
+            a.obs_mod[a.obs_nmod] = id;
+            a.obs_off[a.obs_nmod] = off;
+            if (id == GLG_OBS_FORECAST) a.fc_off = off;
             off += sizes[id];
-            ++h->obs_nmod;
+            ++a.obs_nmod;
         }
         if (!ok || off < 3) {
-            g_create_error = "glg_create: obs_modules must list distinct module ids 1..7 with at least 3 observation entries in total";
+            g_error = "glg_create: obs_modules must list distinct module ids 1..7 with at least 3 observation entries in total";
             delete h;
             return GLG_ERR_ARG;
         }
-        h->obs_dim = off;
+        a.obs_dim = off;
+        h->n_head = off - (a.fc_off >= 0 ? 5 * cfg->Np : 0);
     }
-    h->nt = 64;
     // kernel B: envs per CTA.  32 (full warps) is fastest at every batch size measured: a CTA's step time grows with the
     // number of co-resident CTAs faster than under-filled warps could win back (profiles/r1_lane_sweep.txt).
-    h->role_lanes = (cfg->role_lanes >= 1 && cfg->role_lanes <= 32) ? cfg->role_lanes : 32;
+    a.role_lanes = (cfg->role_lanes >= 1 && cfg->role_lanes <= 32) ? cfg->role_lanes : 32;
     {
         cudaDeviceProp prop;
         if (cudaGetDeviceProperties(&prop, cfg->device) == cudaSuccess) h->sms = prop.multiProcessorCount;
     }
-    const size_t B = (size_t)h->B;
+    const size_t B = (size_t)a.B, D = (size_t)a.obs_dim;
+    CudaMem &m = h->mem;
+    unsigned char *res_block = nullptr;
     cudaError_t e = cudaSetDevice(cfg->device);
-    if (e == cudaSuccess) e = dev_alloc(&h->x, GLG_NX * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->u, GLG_NU * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->time, 2 * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->ep_return, B);
-    if (e == cudaSuccess) e = dev_alloc(&h->ep_info, GLG_NINFO * B);
+    if (e == cudaSuccess) e = m.dev(&a.x, GLG_NX * B);
+    if (e == cudaSuccess) e = m.dev(&a.u, GLG_NU * B);
+    if (e == cudaSuccess) e = m.dev(&a.time, 2 * B);
+    if (e == cudaSuccess) e = m.dev(&a.ep_return, B);
+    if (e == cudaSuccess) e = m.dev(&a.ep_info, GLG_NINFO * B);
     // reward | timestep | table | done share one allocation: glg_step_host fetches them with one device->host copy
-    if (e == cudaSuccess) e = dev_alloc(&h->res_block, res_block_bytes(B));
+    if (e == cudaSuccess) e = m.dev(&res_block, res_block_bytes(B));
     if (e == cudaSuccess) {
-        h->reward = reinterpret_cast<double *>(h->res_block);
-        h->timestep = reinterpret_cast<int *>(h->res_block + 8 * B);
-        h->table = h->timestep + B;
-        h->done = h->res_block + 16 * B;
+        a.reward = reinterpret_cast<double *>(res_block);
+        a.timestep = reinterpret_cast<int *>(res_block + 8 * B);
+        a.table = a.timestep + B;
+        a.done = res_block + 16 * B;
     }
-    if (e == cudaSuccess) e = dev_alloc(&h->ep_len, B);
-    if (e == cudaSuccess) e = dev_alloc(&h->step_ctr, B);
-    if (e == cudaSuccess) e = dev_alloc(&h->obs, (size_t)h->obs_dim * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->term_obs, (size_t)h->obs_dim * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->obs_head, (size_t)(h->obs_dim - (h->fc_off >= 0 ? 5 * cfg->Np : 0)) * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->actions, GLG_NU * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->info, GLG_NINFO * B);
-    if (e == cudaSuccess) e = dev_alloc(&h->stats, (size_t)GLG_NSTATS);
+    if (e == cudaSuccess) e = m.dev(&a.ep_len, B);
+    if (e == cudaSuccess) e = m.dev(&a.step_ctr, B);
+    if (e == cudaSuccess) e = m.dev(&a.obs, D * B);
+    if (e == cudaSuccess) e = m.dev(&a.term_obs, D * B);
+    if (e == cudaSuccess) e = m.dev(&a.obs_head, (size_t)h->n_head * B);
+    if (e == cudaSuccess) e = m.dev(&h->actions, GLG_NU * B);
+    if (e == cudaSuccess) e = m.dev(&a.info, GLG_NINFO * B);
+    if (e == cudaSuccess) e = m.dev(&a.stats, (size_t)GLG_NSTATS);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
-        g_create_error = std::string("glg_create: ") + cudaGetErrorString(e);
+        g_error = std::string("glg_create: ") + cudaGetErrorString(e);
         glg_destroy(h);
         return GLG_ERR_CUDA;
     }
@@ -284,7 +326,7 @@ extern "C" int glg_create(const glg_config *cfg, glg_handle **out) {
 
 extern "C" int glg_set_seed(glg_handle *h, uint64_t seed) {
     if (!h) return GLG_ERR_ARG;
-    h->cfg.seed = seed;
+    h->a.seed = seed;
     return GLG_OK;
 }
 
@@ -303,87 +345,58 @@ extern "C" int glg_set_params(glg_handle *h, const double *p_host) {
 extern "C" int glg_set_weather(glg_handle *h, const double *tables_host, int32_t n_tables, int32_t rows,
                                const double *start_day_host) {
     if (!h || !tables_host || n_tables < 1) return GLG_ERR_ARG;
-    if (rows < h->cfg.N + h->cfg.Np + 1) return fail(h, GLG_ERR_ARG, "glg_set_weather: rows < N + Np + 1");
+    if (rows < h->a.N + h->a.Np + 1) return fail(h, GLG_ERR_ARG, "glg_set_weather: rows < N + Np + 1");
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    cudaFree(h->weather); cudaFree(h->start_day); cudaFree(h->reset_tables);
-    h->weather = nullptr; h->start_day = nullptr; h->reset_tables = nullptr;
-    ++h->weather_gen;
+    // The new bank and its identity reset-table list are complete before the old ones are released (when `bank` and
+    // `reset_list` go out of scope after the swap): a failure leaves the handle as it was.
+    CudaMem bank, reset_list;
+    double *weather = nullptr, *start_day = nullptr;
+    int *reset_tables = nullptr;
     const size_t n = (size_t)n_tables * rows * GLG_ND;
-    GLG_CUDA(h, cudaMalloc((void **)&h->weather, n * sizeof(double)));
-    GLG_CUDA(h, cudaMemcpy(h->weather, tables_host, n * sizeof(double), cudaMemcpyHostToDevice));
+    GLG_CUDA(h, bank.dev(&weather, n));
+    GLG_CUDA(h, cudaMemcpy(weather, tables_host, n * sizeof(double), cudaMemcpyHostToDevice));
     std::vector<double> sd(n_tables, 0.0);
     if (start_day_host) sd.assign(start_day_host, start_day_host + n_tables);
-    GLG_CUDA(h, cudaMalloc((void **)&h->start_day, n_tables * sizeof(double)));
-    GLG_CUDA(h, cudaMemcpy(h->start_day, sd.data(), n_tables * sizeof(double), cudaMemcpyHostToDevice));
+    GLG_CUDA(h, bank.dev(&start_day, n_tables));
+    GLG_CUDA(h, cudaMemcpy(start_day, sd.data(), n_tables * sizeof(double), cudaMemcpyHostToDevice));
     std::vector<int> ids(n_tables);
     for (int i = 0; i < n_tables; ++i) ids[i] = i;
-    GLG_CUDA(h, cudaMalloc((void **)&h->reset_tables, n_tables * sizeof(int)));
-    GLG_CUDA(h, cudaMemcpy(h->reset_tables, ids.data(), n_tables * sizeof(int), cudaMemcpyHostToDevice));
-    h->n_tables = n_tables;
-    h->rows = rows;
-    h->n_reset_tables = n_tables;
-    h->have_weather = true;
+    GLG_CUDA(h, reset_list.dev(&reset_tables, n_tables));
+    GLG_CUDA(h, cudaMemcpy(reset_tables, ids.data(), n_tables * sizeof(int), cudaMemcpyHostToDevice));
     // host copy of what glg_write_forecast shows of the bank (columns 0..4, double -> float), for glg_step_host
-    h->fc_bank.resize((size_t)n_tables * rows * 5);
+    std::vector<float> fc_bank((size_t)n_tables * rows * 5);
     for (size_t r = 0; r < (size_t)n_tables * rows; ++r)
-        for (int c = 0; c < 5; ++c) h->fc_bank[r * 5 + c] = (float)tables_host[r * GLG_ND + c];
+        for (int c = 0; c < 5; ++c) fc_bank[r * 5 + c] = (float)tables_host[r * GLG_ND + c];
+    h->bank.swap(bank);
+    h->reset_list.swap(reset_list);
+    h->fc_bank.swap(fc_bank);
+    h->a.weather = weather; h->a.start_day = start_day; h->a.reset_tables = reset_tables;
+    h->a.n_tables = n_tables; h->a.rows = rows; h->a.n_reset_tables = n_tables;
+    ++h->weather_gen;
     h->kt_valid = false;
     return GLG_OK;
 }
 
 extern "C" int glg_set_reset_tables(glg_handle *h, const int32_t *ids, int32_t n) {
     if (!h || !ids || n < 1) return GLG_ERR_ARG;
-    if (!h->have_weather) return fail(h, GLG_ERR_STATE, "glg_set_reset_tables: set the weather bank first");
+    if (!h->a.weather) return fail(h, GLG_ERR_STATE, "glg_set_reset_tables: set the weather bank first");
     for (int i = 0; i < n; ++i)
-        if (ids[i] < 0 || ids[i] >= h->n_tables) return fail(h, GLG_ERR_ARG, "glg_set_reset_tables: id out of range");
+        if (ids[i] < 0 || ids[i] >= h->a.n_tables) return fail(h, GLG_ERR_ARG, "glg_set_reset_tables: id out of range");
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    cudaFree(h->reset_tables);
-    h->reset_tables = nullptr;
-    GLG_CUDA(h, cudaMalloc((void **)&h->reset_tables, n * sizeof(int)));
-    GLG_CUDA(h, cudaMemcpy(h->reset_tables, ids, n * sizeof(int), cudaMemcpyHostToDevice));
-    h->n_reset_tables = n;
+    CudaMem list;  // complete before the old list is released, as in glg_set_weather
+    int *reset_tables = nullptr;
+    GLG_CUDA(h, list.dev(&reset_tables, n));
+    GLG_CUDA(h, cudaMemcpy(reset_tables, ids, n * sizeof(int), cudaMemcpyHostToDevice));
+    h->reset_list.swap(list);
+    h->a.reset_tables = reset_tables;
+    h->a.n_reset_tables = n;
     return GLG_OK;
-}
-
-static void fill_args(const glg_handle *h, GlgStepArgs *a) {
-    memset(a, 0, sizeof *a);
-    const glg_config &c = h->cfg;
-    a->B = h->B; a->n_sub = c.n_sub; a->N = c.N; a->Np = c.Np; a->rows = h->rows; a->n_tables = h->n_tables;
-    a->obs_dim = h->obs_dim; a->auto_reset = c.auto_reset; a->n_reset_tables = h->n_reset_tables;
-    a->dt = c.dt;
-    for (int i = 0; i < GLG_NU; ++i) {
-        a->u_min[i] = c.u_min[i];
-        a->u_max[i] = c.u_max[i];
-    }
-    a->delta_u_max_f32 = (float)c.delta_u_max;
-    for (int i = 0; i < 3; ++i) {
-        a->con_low[i] = c.con_low[i];
-        a->con_high[i] = c.con_high[i];
-    }
-    a->elec_price = c.elec_price; a->heating_price = c.heating_price; a->co2_price = c.co2_price;
-    a->fruit_price = c.fruit_price; a->dmfm = c.dmfm; a->fixed_costs = c.fixed_costs;
-    a->uncertainty_scale = c.uncertainty_scale;
-    a->seed = c.seed; a->env_id_offset = c.env_id_offset;
-    a->role_lanes = h->role_lanes;
-    a->integrator = c.integrator;
-    a->obs_nmod = h->obs_nmod;
-    for (int i = 0; i < GLG_MAXOBSMOD; ++i) {
-        a->obs_mod[i] = h->obs_mod[i];
-        a->obs_off[i] = h->obs_off[i];
-    }
-    a->fc_off = h->fc_off;
-    a->weather = h->weather; a->start_day = h->start_day; a->reset_tables = h->reset_tables;
-    a->x = h->x; a->u = h->u; a->time = h->time; a->ep_return = h->ep_return; a->ep_info = h->ep_info;
-    a->timestep = h->timestep; a->table = h->table; a->ep_len = h->ep_len; a->step_ctr = h->step_ctr;
-    a->obs_head = h->obs_head;
-    a->obs = h->obs; a->term_obs = h->term_obs; a->reward = h->reward; a->info = h->info; a->stats = h->stats;
-    a->done = h->done;
 }
 
 static int check_ready(glg_handle *h) {
     if (!h) return GLG_ERR_ARG;
     if (!h->have_params) return fail(h, GLG_ERR_STATE, "parameters not set (glg_set_params)");
-    if (!h->have_weather) return fail(h, GLG_ERR_STATE, "weather bank not set (glg_set_weather)");
+    if (!h->a.weather) return fail(h, GLG_ERR_STATE, "weather bank not set (glg_set_weather)");
     return GLG_OK;
 }
 
@@ -391,10 +404,8 @@ extern "C" int glg_reset(glg_handle *h, const uint8_t *mask_dev, const int32_t *
     int rc = check_ready(h);
     if (rc) return rc;
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    GlgStepArgs a;
-    fill_args(h, &a);
     const int NT = 128;
-    glg_reset_kernel<NT><<<(h->B + NT - 1) / NT, NT, 0, (cudaStream_t)stream>>>(a, mask_dev, table_ids_dev);
+    glg_reset_kernel<NT><<<(h->a.B + NT - 1) / NT, NT, 0, (cudaStream_t)stream>>>(h->a, mask_dev, table_ids_dev);
     h->launches += 1;
     GLG_CUDA(h, cudaGetLastError());
     h->is_reset = true;
@@ -446,7 +457,7 @@ static cudaError_t launch_step_units(glg_handle *h, const GlgStepArgs &a, cudaSt
 // waves of CTAs (B = 9472 on 148 SMs: 1.735 vs 1.814 ms), the throughput layout beyond (B = 12 288: 2.60 vs 2.18 ms).
 static int pick_role_warps(const glg_handle *h) {
     if (h->cfg.role_warps != 0) return h->cfg.role_warps;
-    return h->B <= 2 * h->sms * GLG_ROLE_LANES ? 2 : 3;
+    return h->a.B <= 2 * h->sms * GLG_ROLE_LANES ? 2 : 3;
 }
 typedef cudaError_t (*StepLauncher)(glg_handle *, const GlgStepArgs &, cudaStream_t);
 static const StepLauncher kStepLaunchers[3][2][2] = {  // [kernel variant - 1][general][noisy]
@@ -463,14 +474,12 @@ static int step_common(glg_handle *h, const float *actions_dev, const double *co
     if (!h->is_reset) return fail(h, GLG_ERR_STATE, "step before reset");
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
     h->kt_valid = false;
-    GlgStepArgs a;
-    fill_args(h, &a);
+    GlgStepArgs a = h->a;
     a.actions = actions_dev;
     a.controls = controls_dev;
     a.raw_control = rule_based ? 2 : (controls_dev ? 1 : 0);
-    for (int i = 0; i < GLG_NCTRL; ++i) a.ctrl[i] = h->ctrl[i];
     a.noise = noise_dev;
-    const bool noisy = (h->cfg.uncertainty_scale != 0.0) || (noise_dev != nullptr);
+    const bool noisy = (a.uncertainty_scale != 0.0) || (noise_dev != nullptr);
     const cudaError_t e = kStepLaunchers[pick_role_warps(h) - 1][h->general][noisy](h, a, (cudaStream_t)stream);
     h->launches += 1;
     GLG_CUDA(h, e);
@@ -489,7 +498,7 @@ extern "C" int glg_step_raw_control(glg_handle *h, const double *controls_dev, c
 
 extern "C" int glg_set_rule_controller(glg_handle *h, const double *settings29) {
     if (!h) return GLG_ERR_ARG;
-    for (int i = 0; i < GLG_NCTRL; ++i) h->ctrl[i] = settings29 ? settings29[i] : kDefaultCtrl[i];
+    for (int i = 0; i < GLG_NCTRL; ++i) h->a.ctrl[i] = settings29 ? settings29[i] : kDefaultCtrl[i];
     return GLG_OK;
 }
 
@@ -513,7 +522,7 @@ __global__ void glg_rule_control_kernel(GlgStepArgs A, const double *x, const do
 extern "C" int glg_rule_control_batch(const double *settings29, const double *x_dev, const double *d_dev, const double *hod_dev,
                                       const double *doy_dev, double *u_dev, int32_t n, int32_t device, void *stream) {
     if (!x_dev || !d_dev || !hod_dev || !doy_dev || !u_dev || n < 1) {
-        g_create_error = "glg_rule_control_batch: invalid argument";
+        g_error = "glg_rule_control_batch: invalid argument";
         return GLG_ERR_ARG;
     }
     GlgStepArgs a;
@@ -525,7 +534,7 @@ extern "C" int glg_rule_control_batch(const double *settings29, const double *x_
         e = cudaGetLastError();
     }
     if (e != cudaSuccess) {
-        g_create_error = std::string("glg_rule_control_batch: ") + cudaGetErrorString(e);
+        g_error = std::string("glg_rule_control_batch: ") + cudaGetErrorString(e);
         return GLG_ERR_CUDA;
     }
     return GLG_OK;
@@ -590,6 +599,13 @@ extern "C" int glg_set_host_obs_mode(glg_handle *h, int32_t mode) {
     return GLG_OK;
 }
 
+// Every host step path: the actions into the handle's device buffer, then the step, both on the handle's own stream.  The
+// caller's actions may be pageable (the runtime stages them); page-locked ones make the copy asynchronous.
+static int step_from_host(glg_handle *h, const float *actions_host) {
+    GLG_CUDA(h, cudaMemcpyAsync(h->actions, actions_host, GLG_NU * (size_t)h->a.B * sizeof(float), cudaMemcpyHostToDevice, h->own_stream));
+    return step_common(h, h->actions, nullptr, nullptr, h->own_stream);
+}
+
 // Overlapped observation path (host_obs_mode 0, the default, for stacks with a WeatherForecastObservations block): 5 Np of the
 // row's floats (240 of 263 in the default stack) are weather rows kw+1 .. kw+Np of the env's table, kw = min(timestep before the
 // step, rows - Np - 1) -- known before the kernel runs.  So only the rest of the row (glg_write_obs_row's packed copy, obs_head)
@@ -600,14 +616,14 @@ extern "C" int glg_set_host_obs_mode(glg_handle *h, int32_t mode) {
 // between (reset, tensor steps, set_state), are filled again from the verified values.  The result is the same [B][obs_dim]
 // array the full device->host copy (mode 1) delivers, bit for bit (tests/test_gpu_features.py).
 static int step_host_overlapped(glg_handle *h, const float *a_src, float *obs_host, double *reward_host, uint8_t *done_host, bool o_pin) {
-    const size_t B = (size_t)h->B;
-    const int Np = h->cfg.Np, nf = 5 * Np, D = h->obs_dim, n_head = D - nf, fc = h->fc_off, rows = h->rows;
+    const size_t B = (size_t)h->a.B;
+    const int Np = h->a.Np, nf = 5 * Np, D = h->a.obs_dim, n_head = h->n_head, fc = h->a.fc_off, rows = h->a.rows;
     if (!h->h_res) {
-        GLG_CUDA(h, cudaMallocHost((void **)&h->h_res, 2 * res_block_bytes(B)));
+        GLG_CUDA(h, h->mem.host(&h->h_res, 2 * res_block_bytes(B)));
         h->fc_pred.assign(2 * B, -1);
         h->kt_valid = false;
     }
-    if (!o_pin && !h->h_head) GLG_CUDA(h, cudaMallocHost((void **)&h->h_head, (size_t)n_head * B * sizeof(float)));
+    if (!o_pin && !h->h_head) GLG_CUDA(h, h->mem.host(&h->h_head, (size_t)n_head * B));
     cudaStream_t s = h->own_stream;
     // result block of the previous host step (prediction source) / of this one
     const unsigned char *res_cur = h->h_res + (size_t)h->kt_cur * res_block_bytes(B);
@@ -615,25 +631,26 @@ static int step_host_overlapped(glg_handle *h, const float *a_src, float *obs_ho
     const int *cur = reinterpret_cast<const int *>(res_cur + 8 * B);
     const int *nxt = reinterpret_cast<const int *>(res_nxt + 8 * B);
     const bool valid = h->kt_valid;  // every entry that moves the envs clears it (step_common included: set again below)
-    GLG_CUDA(h, cudaMemcpyAsync(h->actions, a_src, GLG_NU * B * sizeof(float), cudaMemcpyHostToDevice, s));
-    int rc = step_common(h, h->actions, nullptr, nullptr, s);
+    int rc = step_from_host(h, a_src);
     if (rc) return rc;
+    const float *obs_head = h->a.obs_head;
     if (o_pin) {
         // page-locked destination: the copy engine puts the packed columns straight into the rows (strided 2-D copy)
         if (fc > 0)
-            GLG_CUDA(h, cudaMemcpy2DAsync(obs_host, (size_t)D * sizeof(float), h->obs_head, (size_t)n_head * sizeof(float), (size_t)fc * sizeof(float), B,
+            GLG_CUDA(h, cudaMemcpy2DAsync(obs_host, (size_t)D * sizeof(float), obs_head, (size_t)n_head * sizeof(float), (size_t)fc * sizeof(float), B,
                                           cudaMemcpyDeviceToHost, s));
         if (n_head > fc)
-            GLG_CUDA(h, cudaMemcpy2DAsync(obs_host + fc + nf, (size_t)D * sizeof(float), h->obs_head + fc, (size_t)n_head * sizeof(float),
+            GLG_CUDA(h, cudaMemcpy2DAsync(obs_host + fc + nf, (size_t)D * sizeof(float), obs_head + fc, (size_t)n_head * sizeof(float),
                                           (size_t)(n_head - fc) * sizeof(float), B, cudaMemcpyDeviceToHost, s));
     } else {
-        GLG_CUDA(h, cudaMemcpyAsync(h->h_head, h->obs_head, (size_t)n_head * B * sizeof(float), cudaMemcpyDeviceToHost, s));
+        GLG_CUDA(h, cudaMemcpyAsync(h->h_head, obs_head, (size_t)n_head * B * sizeof(float), cudaMemcpyDeviceToHost, s));
     }
-    GLG_CUDA(h, cudaMemcpyAsync(res_nxt, h->res_block, res_block_bytes(B), cudaMemcpyDeviceToHost, s));  // reward | timestep | table | done
+    // reward | timestep | table | done: one block that starts at a.reward
+    GLG_CUDA(h, cudaMemcpyAsync(res_nxt, h->a.reward, res_block_bytes(B), cudaMemcpyDeviceToHost, s));
     // ---- while the GPU works: forecast blocks from the predicted (table, row)
     const float *bank = h->fc_bank.data();
     int *pred_t = h->fc_pred.data(), *pred_r = pred_t + B;
-    const int n_tables = h->n_tables, kmax = rows - Np - 1;
+    const int n_tables = h->a.n_tables, kmax = rows - Np - 1;
     host_rows(B, (size_t)nf * sizeof(float), [=](size_t lo, size_t hi) {
         for (size_t i = lo; i < hi; ++i) {
             const int k = valid ? cur[i] : -1, t = valid ? cur[B + i] : -1;
@@ -676,11 +693,11 @@ extern "C" int glg_step_host(glg_handle *h, const float *actions_host, float *ob
                              uint8_t *done_host) {
     if (!h || !actions_host) return GLG_ERR_ARG;
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    const size_t B = (size_t)h->B;
+    const size_t B = (size_t)h->a.B, D = (size_t)h->a.obs_dim;
     if (!h->h_actions) {
-        GLG_CUDA(h, cudaMallocHost((void **)&h->h_actions, GLG_NU * B * sizeof(float)));
-        GLG_CUDA(h, cudaMallocHost((void **)&h->h_reward, B * sizeof(double)));
-        GLG_CUDA(h, cudaMallocHost((void **)&h->h_done, B));
+        GLG_CUDA(h, h->mem.host(&h->h_actions, GLG_NU * B));
+        GLG_CUDA(h, h->mem.host(&h->h_reward, B));
+        GLG_CUDA(h, h->mem.host(&h->h_done, B));
     }
     cudaStream_t s = h->own_stream;
     // caller buffers that are page-locked are used directly; pageable ones are staged through the handle's pinned buffers
@@ -692,20 +709,18 @@ extern "C" int glg_step_host(glg_handle *h, const float *actions_host, float *ob
         memcpy(h->h_actions, actions_host, GLG_NU * B * sizeof(float));
         a_src = h->h_actions;
     }
-    if (obs_host && h->host_obs_mode == 0 && h->fc_off >= 0 && !h->fc_bank.empty()) {
+    if (obs_host && h->host_obs_mode == 0 && h->a.fc_off >= 0 && !h->fc_bank.empty()) {
         return step_host_overlapped(h, a_src, obs_host, reward_host, done_host, o_pin);
     } else {
         h->kt_valid = false;
-        if (obs_host && !o_pin && !h->h_obs) GLG_CUDA(h, cudaMallocHost((void **)&h->h_obs, (size_t)h->obs_dim * B * sizeof(float)));
-        GLG_CUDA(h, cudaMemcpyAsync(h->actions, a_src, GLG_NU * B * sizeof(float), cudaMemcpyHostToDevice, s));
-        int rc = step_common(h, h->actions, nullptr, nullptr, s);
+        if (obs_host && !o_pin && !h->h_obs) GLG_CUDA(h, h->mem.host(&h->h_obs, D * B));
+        int rc = step_from_host(h, a_src);
         if (rc) return rc;
-        if (obs_host)
-            GLG_CUDA(h, cudaMemcpyAsync(o_pin ? obs_host : h->h_obs, h->obs, (size_t)h->obs_dim * B * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (reward_host) GLG_CUDA(h, cudaMemcpyAsync(r_pin ? reward_host : h->h_reward, h->reward, B * sizeof(double), cudaMemcpyDeviceToHost, s));
-        if (done_host) GLG_CUDA(h, cudaMemcpyAsync(d_pin ? done_host : h->h_done, h->done, B, cudaMemcpyDeviceToHost, s));
+        if (obs_host) GLG_CUDA(h, cudaMemcpyAsync(o_pin ? obs_host : h->h_obs, h->a.obs, D * B * sizeof(float), cudaMemcpyDeviceToHost, s));
+        if (reward_host) GLG_CUDA(h, cudaMemcpyAsync(r_pin ? reward_host : h->h_reward, h->a.reward, B * sizeof(double), cudaMemcpyDeviceToHost, s));
+        if (done_host) GLG_CUDA(h, cudaMemcpyAsync(d_pin ? done_host : h->h_done, h->a.done, B, cudaMemcpyDeviceToHost, s));
         GLG_CUDA(h, cudaStreamSynchronize(s));
-        if (obs_host && !o_pin) memcpy(obs_host, h->h_obs, (size_t)h->obs_dim * B * sizeof(float));
+        if (obs_host && !o_pin) memcpy(obs_host, h->h_obs, D * B * sizeof(float));
     }
     if (reward_host && !r_pin) memcpy(reward_host, h->h_reward, B * sizeof(double));
     if (done_host && !d_pin) memcpy(done_host, h->h_done, B);
@@ -716,119 +731,43 @@ extern "C" int glg_step_host_split(glg_handle *h, const float *actions_host, flo
                                    int32_t *table_host, double *reward_host, uint8_t *done_host) {
     if (!h || !actions_host) return GLG_ERR_ARG;
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    const size_t B = (size_t)h->B;
+    const size_t B = (size_t)h->a.B;
     cudaStream_t s = h->own_stream;
     // pageable buffers work too (the runtime stages them); page-locked ones (the Python wrapper's) make the copies asynchronous
-    GLG_CUDA(h, cudaMemcpyAsync(h->actions, actions_host, GLG_NU * B * sizeof(float), cudaMemcpyHostToDevice, s));
-    int rc = step_common(h, h->actions, nullptr, nullptr, s);
+    int rc = step_from_host(h, actions_host);
     if (rc) return rc;
-    if (head_host) {  // the kernels write the row without its forecast block a second time, packed: one contiguous copy
-        const size_t n_head = (size_t)(h->obs_dim - (h->fc_off >= 0 ? 5 * h->cfg.Np : 0));
-        GLG_CUDA(h, cudaMemcpyAsync(head_host, h->obs_head, n_head * B * sizeof(float), cudaMemcpyDeviceToHost, s));
-    }
-    if (timestep_host) GLG_CUDA(h, cudaMemcpyAsync(timestep_host, h->timestep, B * sizeof(int), cudaMemcpyDeviceToHost, s));
-    if (table_host) GLG_CUDA(h, cudaMemcpyAsync(table_host, h->table, B * sizeof(int), cudaMemcpyDeviceToHost, s));
-    if (reward_host) GLG_CUDA(h, cudaMemcpyAsync(reward_host, h->reward, B * sizeof(double), cudaMemcpyDeviceToHost, s));
-    if (done_host) GLG_CUDA(h, cudaMemcpyAsync(done_host, h->done, B, cudaMemcpyDeviceToHost, s));
+    // the kernels write the row without its forecast block a second time, packed: one contiguous copy
+    if (head_host) GLG_CUDA(h, cudaMemcpyAsync(head_host, h->a.obs_head, (size_t)h->n_head * B * sizeof(float), cudaMemcpyDeviceToHost, s));
+    if (timestep_host) GLG_CUDA(h, cudaMemcpyAsync(timestep_host, h->a.timestep, B * sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (table_host) GLG_CUDA(h, cudaMemcpyAsync(table_host, h->a.table, B * sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (reward_host) GLG_CUDA(h, cudaMemcpyAsync(reward_host, h->a.reward, B * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (done_host) GLG_CUDA(h, cudaMemcpyAsync(done_host, h->a.done, B, cudaMemcpyDeviceToHost, s));
     GLG_CUDA(h, cudaStreamSynchronize(s));
     return GLG_OK;
 }
 
-extern "C" int32_t glg_obs_dim(const glg_handle *h) { return h ? h->obs_dim : 0; }
-extern "C" float *glg_obs_dev(glg_handle *h) { return h ? h->obs : nullptr; }
-extern "C" float *glg_terminal_obs_dev(glg_handle *h) { return h ? h->term_obs : nullptr; }
-extern "C" double *glg_reward_dev(glg_handle *h) { return h ? h->reward : nullptr; }
-extern "C" uint8_t *glg_done_dev(glg_handle *h) { return h ? h->done : nullptr; }
-extern "C" double *glg_info_dev(glg_handle *h) { return h ? h->info : nullptr; }
-extern "C" double *glg_state_dev(glg_handle *h) { return h ? h->x : nullptr; }
-extern "C" double *glg_controls_dev(glg_handle *h) { return h ? h->u : nullptr; }
-extern "C" int32_t *glg_timestep_dev(glg_handle *h) { return h ? h->timestep : nullptr; }
-extern "C" int32_t *glg_table_dev(glg_handle *h) { return h ? h->table : nullptr; }
-extern "C" double *glg_time_dev(glg_handle *h) { return h ? h->time : nullptr; }
-extern "C" double *glg_stats_dev(glg_handle *h) { return h ? h->stats : nullptr; }
+extern "C" int32_t glg_obs_dim(const glg_handle *h) { return h ? h->a.obs_dim : 0; }
+extern "C" float *glg_obs_dev(glg_handle *h) { return h ? h->a.obs : nullptr; }
+extern "C" float *glg_terminal_obs_dev(glg_handle *h) { return h ? h->a.term_obs : nullptr; }
+extern "C" double *glg_reward_dev(glg_handle *h) { return h ? h->a.reward : nullptr; }
+extern "C" uint8_t *glg_done_dev(glg_handle *h) { return h ? h->a.done : nullptr; }
+extern "C" double *glg_info_dev(glg_handle *h) { return h ? h->a.info : nullptr; }
+extern "C" double *glg_state_dev(glg_handle *h) { return h ? h->a.x : nullptr; }
+extern "C" double *glg_controls_dev(glg_handle *h) { return h ? h->a.u : nullptr; }
+extern "C" int32_t *glg_timestep_dev(glg_handle *h) { return h ? h->a.timestep : nullptr; }
+extern "C" int32_t *glg_table_dev(glg_handle *h) { return h ? h->a.table : nullptr; }
+extern "C" double *glg_time_dev(glg_handle *h) { return h ? h->a.time : nullptr; }
+extern "C" double *glg_stats_dev(glg_handle *h) { return h ? h->a.stats : nullptr; }
 extern "C" int64_t glg_launch_count(const glg_handle *h) { return h ? h->launches : 0; }
 
 extern "C" int glg_clear_stats(glg_handle *h, void *stream) {
     if (!h) return GLG_ERR_ARG;
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    GLG_CUDA(h, cudaMemsetAsync(h->stats, 0, GLG_NSTATS * sizeof(double), (cudaStream_t)stream));
+    GLG_CUDA(h, cudaMemsetAsync(h->a.stats, 0, GLG_NSTATS * sizeof(double), (cudaStream_t)stream));
     return GLG_OK;
 }
 
-// [B][n] row-major host  <->  [n][B] device SoA
-static void to_soa(const double *aos, double *soa, int B, int n) {
-    for (int b = 0; b < B; ++b)
-        for (int i = 0; i < n; ++i) soa[(size_t)i * B + b] = aos[(size_t)b * n + i];
-}
-static void to_aos(const double *soa, double *aos, int B, int n) {
-    for (int b = 0; b < B; ++b)
-        for (int i = 0; i < n; ++i) aos[(size_t)b * n + i] = soa[(size_t)i * B + b];
-}
-
-extern "C" int glg_set_state(glg_handle *h, const double *x_host, const double *u_host, const int32_t *timestep_host) {
-    if (!h) return GLG_ERR_ARG;
-    h->kt_valid = false;
-    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    GLG_CUDA(h, cudaDeviceSynchronize());
-    const int B = h->B;
-    std::vector<double> tmp;
-    if (x_host) {
-        tmp.resize((size_t)GLG_NX * B);
-        to_soa(x_host, tmp.data(), B, GLG_NX);
-        GLG_CUDA(h, cudaMemcpy(h->x, tmp.data(), tmp.size() * sizeof(double), cudaMemcpyHostToDevice));
-    }
-    if (u_host) {
-        tmp.resize((size_t)GLG_NU * B);
-        to_soa(u_host, tmp.data(), B, GLG_NU);
-        GLG_CUDA(h, cudaMemcpy(h->u, tmp.data(), tmp.size() * sizeof(double), cudaMemcpyHostToDevice));
-    }
-    if (timestep_host) {
-        // the env clock follows the timestep (tomato_env.py:126-128, :246-247): doy = start_day(table) + k dt/86400 (summed the way
-        // the step does, one increment per step), hod = (k dt/3600) mod 24
-        if (!h->have_weather) return fail(h, GLG_ERR_STATE, "glg_set_state: set the weather bank first");
-        for (int b = 0; b < B; ++b)
-            if (timestep_host[b] < 0 || timestep_host[b] > h->cfg.N) return fail(h, GLG_ERR_ARG, "glg_set_state: timestep outside [0, N]");
-        std::vector<int> tb(B);
-        std::vector<double> sd(h->n_tables), tm((size_t)2 * B);
-        GLG_CUDA(h, cudaMemcpy(tb.data(), h->table, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost));
-        GLG_CUDA(h, cudaMemcpy(sd.data(), h->start_day, (size_t)h->n_tables * sizeof(double), cudaMemcpyDeviceToHost));
-        const double ddoy = fmod(h->cfg.dt / 86400.0, 365.0), dhod = h->cfg.dt / 3600.0;
-        for (int b = 0; b < B; ++b) {
-            double doy = sd[tb[b]], hod = 0.0;
-            for (int k = 0; k < timestep_host[b]; ++k) {
-                doy += ddoy;
-                hod = fmod(hod + dhod, 24.0);
-            }
-            tm[b] = doy;
-            tm[(size_t)B + b] = hod;
-        }
-        GLG_CUDA(h, cudaMemcpy(h->time, tm.data(), tm.size() * sizeof(double), cudaMemcpyHostToDevice));
-        GLG_CUDA(h, cudaMemcpy(h->timestep, timestep_host, (size_t)B * sizeof(int), cudaMemcpyHostToDevice));
-    }
-    return GLG_OK;
-}
-
-extern "C" int glg_get_state(glg_handle *h, double *x_host, double *u_host, int32_t *timestep_host) {
-    if (!h) return GLG_ERR_ARG;
-    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    GLG_CUDA(h, cudaDeviceSynchronize());
-    const int B = h->B;
-    std::vector<double> tmp;
-    if (x_host) {
-        tmp.resize((size_t)GLG_NX * B);
-        GLG_CUDA(h, cudaMemcpy(tmp.data(), h->x, tmp.size() * sizeof(double), cudaMemcpyDeviceToHost));
-        to_aos(tmp.data(), x_host, B, GLG_NX);
-    }
-    if (u_host) {
-        tmp.resize((size_t)GLG_NU * B);
-        GLG_CUDA(h, cudaMemcpy(tmp.data(), h->u, tmp.size() * sizeof(double), cudaMemcpyDeviceToHost));
-        to_aos(tmp.data(), u_host, B, GLG_NU);
-    }
-    if (timestep_host) GLG_CUDA(h, cudaMemcpy(timestep_host, h->timestep, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost));
-    return GLG_OK;
-}
-
-// full per-env state: checkpoint / restore
+// full per-env state (checkpoint / restore): [B][n] row-major host <-> [n][B] device SoA when `soa`
 template <class T>
 static cudaError_t copy_field(bool to_dev, T *dev, T *host, size_t n_per_env, int B, bool soa) {
     if (!host) return cudaSuccess;
@@ -845,104 +784,139 @@ static cudaError_t copy_field(bool to_dev, T *dev, T *host, size_t n_per_env, in
         for (size_t i = 0; i < n_per_env; ++i) host[(size_t)b * n_per_env + i] = tmp[i * B + b];
     return e;
 }
+
+extern "C" int glg_set_state(glg_handle *h, const double *x_host, const double *u_host, const int32_t *timestep_host) {
+    if (!h) return GLG_ERR_ARG;
+    h->kt_valid = false;
+    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+    GLG_CUDA(h, cudaDeviceSynchronize());
+    const int B = h->a.B;
+    // copy_field only reads the host side on its way to the device
+    GLG_CUDA(h, copy_field(true, h->a.x, const_cast<double *>(x_host), GLG_NX, B, true));
+    GLG_CUDA(h, copy_field(true, h->a.u, const_cast<double *>(u_host), GLG_NU, B, true));
+    if (timestep_host) {
+        // the env clock follows the timestep (tomato_env.py:126-128, :246-247): doy = start_day(table) + k dt/86400 (summed the way
+        // the step does, one increment per step), hod = (k dt/3600) mod 24
+        if (!h->a.weather) return fail(h, GLG_ERR_STATE, "glg_set_state: set the weather bank first");
+        for (int b = 0; b < B; ++b)
+            if (timestep_host[b] < 0 || timestep_host[b] > h->a.N) return fail(h, GLG_ERR_ARG, "glg_set_state: timestep outside [0, N]");
+        std::vector<int> tb(B);
+        std::vector<double> sd(h->a.n_tables), tm((size_t)2 * B);
+        GLG_CUDA(h, cudaMemcpy(tb.data(), h->a.table, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost));
+        GLG_CUDA(h, cudaMemcpy(sd.data(), h->a.start_day, (size_t)h->a.n_tables * sizeof(double), cudaMemcpyDeviceToHost));
+        const double ddoy = fmod(h->a.dt / 86400.0, 365.0), dhod = h->a.dt / 3600.0;
+        for (int b = 0; b < B; ++b) {
+            double doy = sd[tb[b]], hod = 0.0;
+            for (int k = 0; k < timestep_host[b]; ++k) {
+                doy += ddoy;
+                hod = fmod(hod + dhod, 24.0);
+            }
+            tm[b] = doy;
+            tm[(size_t)B + b] = hod;
+        }
+        GLG_CUDA(h, cudaMemcpy(h->a.time, tm.data(), tm.size() * sizeof(double), cudaMemcpyHostToDevice));
+        GLG_CUDA(h, cudaMemcpy(h->a.timestep, timestep_host, (size_t)B * sizeof(int), cudaMemcpyHostToDevice));
+    }
+    return GLG_OK;
+}
+
 static int state_ex(glg_handle *h, const glg_env_state *s, bool to_dev) {
     if (!h || !s) return GLG_ERR_ARG;
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
     GLG_CUDA(h, cudaDeviceSynchronize());
-    const int B = h->B;
+    const GlgStepArgs &a = h->a;
+    const int B = a.B;
     if (to_dev) h->kt_valid = false;
     if (to_dev) {
         if (s->table) {
-            if (!h->have_weather) return fail(h, GLG_ERR_STATE, "glg_set_state_ex: set the weather bank first");
+            if (!a.weather) return fail(h, GLG_ERR_STATE, "glg_set_state_ex: set the weather bank first");
             for (int b = 0; b < B; ++b)
-                if (s->table[b] < 0 || s->table[b] >= h->n_tables) return fail(h, GLG_ERR_ARG, "glg_set_state_ex: table id out of range");
+                if (s->table[b] < 0 || s->table[b] >= a.n_tables) return fail(h, GLG_ERR_ARG, "glg_set_state_ex: table id out of range");
         }
         if (s->timestep)
             for (int b = 0; b < B; ++b)
-                if (s->timestep[b] < 0 || s->timestep[b] > h->cfg.N + 1) return fail(h, GLG_ERR_ARG, "glg_set_state_ex: timestep outside [0, N + 1]");
+                if (s->timestep[b] < 0 || s->timestep[b] > a.N + 1) return fail(h, GLG_ERR_ARG, "glg_set_state_ex: timestep outside [0, N + 1]");
     }
-    GLG_CUDA(h, copy_field(to_dev, h->x, s->x, GLG_NX, B, true));
-    GLG_CUDA(h, copy_field(to_dev, h->u, s->u, GLG_NU, B, true));
-    GLG_CUDA(h, copy_field(to_dev, h->timestep, s->timestep, 1, B, false));
-    GLG_CUDA(h, copy_field(to_dev, h->table, s->table, 1, B, false));
-    GLG_CUDA(h, copy_field(to_dev, h->time, s->time, 2, B, true));
-    GLG_CUDA(h, copy_field(to_dev, h->step_ctr, s->step_ctr, 1, B, false));
-    GLG_CUDA(h, copy_field(to_dev, h->ep_return, s->ep_return, 1, B, false));
-    GLG_CUDA(h, copy_field(to_dev, h->ep_len, s->ep_len, 1, B, false));
-    GLG_CUDA(h, copy_field(to_dev, h->ep_info, s->ep_info, GLG_NINFO, B, true));
+    GLG_CUDA(h, copy_field(to_dev, a.x, s->x, GLG_NX, B, true));
+    GLG_CUDA(h, copy_field(to_dev, a.u, s->u, GLG_NU, B, true));
+    GLG_CUDA(h, copy_field(to_dev, a.timestep, s->timestep, 1, B, false));
+    GLG_CUDA(h, copy_field(to_dev, a.table, s->table, 1, B, false));
+    GLG_CUDA(h, copy_field(to_dev, a.time, s->time, 2, B, true));
+    GLG_CUDA(h, copy_field(to_dev, a.step_ctr, s->step_ctr, 1, B, false));
+    GLG_CUDA(h, copy_field(to_dev, a.ep_return, s->ep_return, 1, B, false));
+    GLG_CUDA(h, copy_field(to_dev, a.ep_len, s->ep_len, 1, B, false));
+    GLG_CUDA(h, copy_field(to_dev, a.ep_info, s->ep_info, GLG_NINFO, B, true));
     if (to_dev) h->is_reset = true;
     return GLG_OK;
 }
 extern "C" int glg_get_state_ex(glg_handle *h, const glg_env_state *out_host) { return state_ex(h, out_host, false); }
 extern "C" int glg_set_state_ex(glg_handle *h, const glg_env_state *in_host) { return state_ex(h, in_host, true); }
 
+extern "C" int glg_get_state(glg_handle *h, double *x_host, double *u_host, int32_t *timestep_host) {
+    glg_env_state s = {};
+    s.x = x_host; s.u = u_host; s.timestep = timestep_host;
+    return state_ex(h, &s, false);
+}
+
 // ---- VecNormalize state of a rollout or replay buffer, updated by the glg_roll_* kernels (glg_rollout.cuh) ----
 struct GlgNorm {
     int training = 0, norm_obs = 0, norm_reward = 0, blocks = 0;
     double gamma = 0.0, clip_obs = 0.0, clip_reward = 0.0, epsilon = 0.0;
-    size_t bytes = 0;  // device bytes of the arrays below
     double *ret = nullptr, *stat = nullptr, *partial = nullptr, *norm64 = nullptr;
 };
 
-template <typename T>
-static cudaError_t counted_alloc(size_t *bytes, T **p, size_t n) {
-    *bytes += n * sizeof(T);
-    return dev_alloc(p, n);
-}
-
-// c: glg_rollout_config or glg_replay_config, which share the VecNormalize fields.  Arrays for the handle's batch.
+// c: glg_rollout_config or glg_replay_config, which share the VecNormalize fields.  Arrays for the handle's batch, owned by `mem`
+// (the rollout's or replay buffer's).
 template <class Cfg>
-static cudaError_t norm_create(GlgNorm *n, const glg_handle *h, const Cfg &c) {
+static cudaError_t norm_create(GlgNorm *n, CudaMem &mem, const glg_handle *h, const Cfg &c) {
     n->training = c.training; n->norm_obs = c.norm_obs; n->norm_reward = c.norm_reward;
     n->gamma = c.gamma; n->clip_obs = c.clip_obs; n->clip_reward = c.clip_reward; n->epsilon = c.epsilon;
-    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim;
+    const size_t B = (size_t)h->a.B, D = (size_t)h->a.obs_dim;
     n->blocks = (int)((B + GLG_ROLL_ROWS - 1) / GLG_ROLL_ROWS);
-    cudaError_t e = counted_alloc(&n->bytes, &n->ret, B);
-    if (e == cudaSuccess) e = counted_alloc(&n->bytes, &n->stat, (D + 1) * 3);
-    if (e == cudaSuccess) e = counted_alloc(&n->bytes, &n->partial, (size_t)n->blocks * (D + 1) * 2);
-    if (e == cudaSuccess) e = counted_alloc(&n->bytes, &n->norm64, (D + 1) * 2);
+    cudaError_t e = mem.dev(&n->ret, B);
+    if (e == cudaSuccess) e = mem.dev(&n->stat, (D + 1) * 3);
+    if (e == cudaSuccess) e = mem.dev(&n->partial, (size_t)n->blocks * (D + 1) * 2);
+    if (e == cudaSuccess) e = mem.dev(&n->norm64, (D + 1) * 2);
     if (e != cudaSuccess) return e;
     std::vector<double> st;
     for (size_t c = 0; c <= D; ++c) st.insert(st.end(), {0.0, 1.0, 1e-4});  // RunningMeanStd: mean 0, var 1, count 1e-4
     return cudaMemcpy(n->stat, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice);
 }
 
-static void norm_free(GlgNorm *n) { cudaFree(n->ret); cudaFree(n->stat); cudaFree(n->partial); cudaFree(n->norm64); }
-
 // VecNormalize.step_wait (after_step) or .reset on the handle's current outputs: statistics updated, normalised observations into
 // obs_out, normalised rewards into reward_out and episode starts into starts_out (either may be NULL).  Three launches on s.
 static void norm_update(const GlgNorm &n, glg_handle *h, bool after_step, float *obs_out, float *reward_out, float *starts_out,
                         cudaStream_t s) {
+    const GlgStepArgs &e = h->a;
     GlgRollArgs a;
     memset(&a, 0, sizeof a);
-    a.B = h->B; a.obs_dim = h->obs_dim; a.n_blocks = n.blocks;
+    a.B = e.B; a.obs_dim = e.obs_dim; a.n_blocks = n.blocks;
     a.training = n.training; a.norm_obs = n.norm_obs; a.norm_reward = n.norm_reward;
     a.gamma = n.gamma; a.clip_obs = n.clip_obs; a.clip_reward = n.clip_reward; a.epsilon = n.epsilon;
-    a.obs = h->obs;
-    a.reward = after_step ? h->reward : nullptr;
-    a.done = after_step ? h->done : nullptr;
+    a.obs = e.obs;
+    a.reward = after_step ? e.reward : nullptr;
+    a.done = after_step ? e.done : nullptr;
     a.ret = n.ret; a.stat = n.stat; a.partial = n.partial; a.norm64 = n.norm64;
     a.obs_out = obs_out; a.reward_out = reward_out; a.starts_out = starts_out;
     glg_roll_moments_kernel<<<n.blocks, GLG_ROLL_NT, 0, s>>>(a);
-    glg_roll_finish_kernel<<<(h->obs_dim + 1 + GLG_ROLL_NT / 32 - 1) / (GLG_ROLL_NT / 32), GLG_ROLL_NT, 0, s>>>(a);
+    glg_roll_finish_kernel<<<(e.obs_dim + 1 + GLG_ROLL_NT / 32 - 1) / (GLG_ROLL_NT / 32), GLG_ROLL_NT, 0, s>>>(a);
     glg_roll_apply_kernel<<<n.blocks, GLG_ROLL_NT, 0, s>>>(a);
     h->launches += 3;
 }
 
 // ---- device rollout: VecNormalize + rollout buffer + GAE (glg_rollout.cuh); its own object, like the replay buffer ----------
 struct glg_rollout {
-    glg_handle *h = nullptr;
+    glg_handle *h = nullptr;  // not read on destruction: the env may already be gone
     int device = 0, n_steps = 0;
     double gae_lambda = 0.0;
+    CudaMem mem;
     GlgNorm norm;
     float *obs = nullptr, *rew = nullptr, *starts = nullptr, *adv = nullptr, *ret = nullptr;
 };
 
 extern "C" void glg_rollout_destroy(glg_rollout *r) {
     if (!r) return;
-    cudaSetDevice(r->device);  // the handle may already be gone: nothing here reads it
-    cudaFree(r->obs); cudaFree(r->rew); cudaFree(r->starts); cudaFree(r->adv); cudaFree(r->ret);
-    norm_free(&r->norm);
+    cudaSetDevice(r->device);
     delete r;
 }
 
@@ -956,13 +930,13 @@ extern "C" int glg_rollout_create(glg_handle *h, const glg_rollout_config *cfg, 
     glg_rollout *r = new (std::nothrow) glg_rollout();
     if (!r) return fail(h, GLG_ERR_ALLOC, "glg_rollout_create: out of host memory");
     r->h = h; r->device = h->cfg.device; r->n_steps = cfg->n_steps; r->gae_lambda = cfg->gae_lambda;
-    const size_t B = (size_t)h->B, T = (size_t)cfg->n_steps, D = (size_t)h->obs_dim;
-    cudaError_t e = dev_alloc(&r->obs, (T + 1) * B * D);
-    if (e == cudaSuccess) e = dev_alloc(&r->rew, T * B);
-    if (e == cudaSuccess) e = dev_alloc(&r->starts, (T + 1) * B);
-    if (e == cudaSuccess) e = dev_alloc(&r->adv, T * B);
-    if (e == cudaSuccess) e = dev_alloc(&r->ret, T * B);
-    if (e == cudaSuccess) e = norm_create(&r->norm, h, *cfg);
+    const size_t B = (size_t)h->a.B, T = (size_t)cfg->n_steps, D = (size_t)h->a.obs_dim;
+    cudaError_t e = r->mem.dev(&r->obs, (T + 1) * B * D);
+    if (e == cudaSuccess) e = r->mem.dev(&r->rew, T * B);
+    if (e == cudaSuccess) e = r->mem.dev(&r->starts, (T + 1) * B);
+    if (e == cudaSuccess) e = r->mem.dev(&r->adv, T * B);
+    if (e == cudaSuccess) e = r->mem.dev(&r->ret, T * B);
+    if (e == cudaSuccess) e = norm_create(&r->norm, r->mem, h, *cfg);
     if (e != cudaSuccess) {
         glg_rollout_destroy(r);
         return fail(h, GLG_ERR_CUDA, (std::string("glg_rollout_create: ") + cudaGetErrorString(e)).c_str());
@@ -975,7 +949,7 @@ extern "C" int glg_rollout_store(glg_rollout *r, int32_t t, void *stream) {
     glg_handle *h = r->h;
     if (t < -1 || t >= r->n_steps) return fail(h, GLG_ERR_ARG, "glg_rollout_store: t outside [-1, n_steps)");
     GLG_CUDA(h, cudaSetDevice(r->device));
-    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim;
+    const size_t B = (size_t)h->a.B, D = (size_t)h->a.obs_dim;
     norm_update(r->norm, h, t >= 0, r->obs + (size_t)(t + 1) * B * D, t >= 0 ? r->rew + (size_t)t * B : nullptr,
                 r->starts + (size_t)(t + 1) * B, (cudaStream_t)stream);
     GLG_CUDA(h, cudaGetLastError());
@@ -985,7 +959,7 @@ extern "C" int glg_rollout_carry(glg_rollout *r, void *stream) {
     if (!r) return GLG_ERR_ARG;
     glg_handle *h = r->h;
     GLG_CUDA(h, cudaSetDevice(r->device));
-    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim, T = (size_t)r->n_steps;
+    const size_t B = (size_t)h->a.B, D = (size_t)h->a.obs_dim, T = (size_t)r->n_steps;
     GLG_CUDA(h, cudaMemcpyAsync(r->obs, r->obs + T * B * D, B * D * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     GLG_CUDA(h, cudaMemcpyAsync(r->starts, r->starts + T * B, B * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return GLG_OK;
@@ -994,8 +968,8 @@ extern "C" int glg_rollout_gae(glg_rollout *r, const float *values_dev, void *st
     if (!r || !values_dev) return GLG_ERR_ARG;
     glg_handle *h = r->h;
     GLG_CUDA(h, cudaSetDevice(r->device));
-    glg_roll_gae_kernel<<<(h->B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(r->n_steps, h->B, r->norm.gamma, r->gae_lambda, r->rew,
-                                                                              values_dev, r->starts, r->adv, r->ret);
+    glg_roll_gae_kernel<<<(h->a.B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(r->n_steps, h->a.B, r->norm.gamma, r->gae_lambda,
+                                                                                r->rew, values_dev, r->starts, r->adv, r->ret);
     h->launches += 1;
     GLG_CUDA(h, cudaGetLastError());
     return GLG_OK;
@@ -1009,15 +983,14 @@ extern "C" double *glg_rollout_stats_dev(glg_rollout *r) { return r ? r->norm.st
 
 // ---- device replay buffer (glg_replay.cuh): its own object, so several can share an env and none dangles from the handle ----
 struct glg_replay {
-    glg_handle *h = nullptr;
+    glg_handle *h = nullptr;  // not read on destruction: the env may already be gone
     int device = 0;
     uint64_t seed = 0;                   // Philox key of the sample indices
     unsigned long long weather_gen = 0;  // bank generation the keys refer to
     long long cap = 0, pos = 0;
     bool full = false, is_reset = false;
     uint32_t calls = 0;  // sample calls so far (Philox counter)
-    int n_head = 0, nf = 0;
-    size_t bytes = 0;  // device bytes of the arrays below; glg_replay_bytes adds the normaliser's
+    CudaMem mem;         // every device array below and the normaliser's: glg_replay_bytes
     GlgNorm norm;
     float *obs_norm = nullptr, *last_head = nullptr, *head_obs = nullptr, *head_next = nullptr, *act = nullptr, *rew = nullptr;
     int *key_obs = nullptr, *key_next = nullptr, *anchor_t = nullptr, *anchor_tbl = nullptr;
@@ -1026,25 +999,22 @@ struct glg_replay {
 
 extern "C" void glg_replay_destroy(glg_replay *r) {
     if (!r) return;
-    cudaSetDevice(r->device);  // the handle may already be gone: nothing here reads it
-    cudaFree(r->obs_norm); cudaFree(r->last_head); cudaFree(r->head_obs); cudaFree(r->head_next); cudaFree(r->act); cudaFree(r->rew);
-    cudaFree(r->key_obs); cudaFree(r->key_next); cudaFree(r->anchor_t); cudaFree(r->anchor_tbl); cudaFree(r->dn);
-    norm_free(&r->norm);
+    cudaSetDevice(r->device);
     delete r;
 }
 
 extern "C" int glg_replay_create(glg_handle *h, const glg_replay_config *cfg, glg_replay **out) {
     if (!h || !cfg || !out) {
-        g_create_error = "glg_replay_create: null argument";
+        g_error = "glg_replay_create: null argument";
         return GLG_ERR_ARG;
     }
     *out = nullptr;
     if (cfg->buffer_size < 1 || !(cfg->gamma >= 0.0 && cfg->gamma <= 1.0) || !(cfg->clip_obs > 0) || !(cfg->clip_reward > 0) ||
         !(cfg->epsilon > 0))
         return fail(h, GLG_ERR_ARG, "glg_replay_create: invalid buffer_size / gamma / clip / epsilon");
-    if (!h->have_weather) return fail(h, GLG_ERR_STATE, "glg_replay_create: weather bank not set (glg_set_weather)");
-    const size_t B = (size_t)h->B, D = (size_t)h->obs_dim;
-    const long long cap = cfg->buffer_size / h->B > 1 ? cfg->buffer_size / h->B : 1;  // ReplayBuffer: max(buffer_size // n_envs, 1)
+    if (!h->a.weather) return fail(h, GLG_ERR_STATE, "glg_replay_create: weather bank not set (glg_set_weather)");
+    const size_t B = (size_t)h->a.B, D = (size_t)h->a.obs_dim;
+    const long long cap = cfg->buffer_size / h->a.B > 1 ? cfg->buffer_size / h->a.B : 1;  // ReplayBuffer: max(buffer_size // n_envs, 1)
     if (cap > INT32_MAX) return fail(h, GLG_ERR_ARG, "glg_replay_create: more than 2^31 - 1 slots per env");
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
     glg_replay *r = new (std::nothrow) glg_replay();
@@ -1054,21 +1024,20 @@ extern "C" int glg_replay_create(glg_handle *h, const glg_replay_config *cfg, gl
     r->seed = cfg->seed;
     r->weather_gen = h->weather_gen;
     r->cap = cap;
-    r->nf = h->fc_off >= 0 ? 5 * h->cfg.Np : 0;
-    r->n_head = h->obs_dim - r->nf;
-    const size_t CB = (size_t)cap * B, H = (size_t)r->n_head;
-    cudaError_t e = counted_alloc(&r->bytes, &r->head_obs, CB * H);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->head_next, CB * H);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->key_obs, CB);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->key_next, CB);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->act, CB * GLG_NU);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->rew, CB);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->dn, CB);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->obs_norm, B * D);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->last_head, B * H);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->anchor_t, B);
-    if (e == cudaSuccess) e = counted_alloc(&r->bytes, &r->anchor_tbl, B);
-    if (e == cudaSuccess) e = norm_create(&r->norm, h, *cfg);
+    const size_t CB = (size_t)cap * B, H = (size_t)h->n_head;
+    CudaMem &m = r->mem;
+    cudaError_t e = m.dev(&r->head_obs, CB * H);
+    if (e == cudaSuccess) e = m.dev(&r->head_next, CB * H);
+    if (e == cudaSuccess) e = m.dev(&r->key_obs, CB);
+    if (e == cudaSuccess) e = m.dev(&r->key_next, CB);
+    if (e == cudaSuccess) e = m.dev(&r->act, CB * GLG_NU);
+    if (e == cudaSuccess) e = m.dev(&r->rew, CB);
+    if (e == cudaSuccess) e = m.dev(&r->dn, CB);
+    if (e == cudaSuccess) e = m.dev(&r->obs_norm, B * D);
+    if (e == cudaSuccess) e = m.dev(&r->last_head, B * H);
+    if (e == cudaSuccess) e = m.dev(&r->anchor_t, B);
+    if (e == cudaSuccess) e = m.dev(&r->anchor_tbl, B);
+    if (e == cudaSuccess) e = norm_create(&r->norm, m, h, *cfg);
     if (e != cudaSuccess) {
         glg_replay_destroy(r);
         return fail(h, GLG_ERR_CUDA, (std::string("glg_replay_create: ") + cudaGetErrorString(e)).c_str());
@@ -1088,11 +1057,11 @@ static int replay_check(glg_replay *r, const char *what) {
 }
 
 static void replay_write_args(const glg_replay *r, GlgReplayArgs *w) {
-    const glg_handle *h = r->h;
+    const GlgStepArgs &a = r->h->a;
     memset(w, 0, sizeof *w);
-    w->B = h->B; w->obs_dim = h->obs_dim; w->n_head = r->n_head; w->nf = r->nf; w->fc_off = h->fc_off; w->Np = h->cfg.Np;
-    w->rows = h->rows; w->auto_reset = h->cfg.auto_reset;
-    w->obs = h->obs; w->term_obs = h->term_obs; w->reward = h->reward; w->done = h->done; w->timestep = h->timestep; w->table = h->table;
+    w->B = a.B; w->obs_dim = a.obs_dim; w->n_head = r->h->n_head; w->nf = a.obs_dim - r->h->n_head; w->fc_off = a.fc_off; w->Np = a.Np;
+    w->rows = a.rows; w->auto_reset = a.auto_reset;
+    w->obs = a.obs; w->term_obs = a.term_obs; w->reward = a.reward; w->done = a.done; w->timestep = a.timestep; w->table = a.table;
     w->last_head = r->last_head; w->anchor_t = r->anchor_t; w->anchor_tbl = r->anchor_tbl;
     w->head_obs = r->head_obs; w->head_next = r->head_next; w->key_obs = r->key_obs; w->key_next = r->key_next;
     w->act = r->act; w->rew = r->rew; w->dn = r->dn;
@@ -1155,12 +1124,12 @@ extern "C" int glg_replay_sample(glg_replay *r, int32_t n, float *obs_dev, float
     GLG_CUDA(h, cudaSetDevice(r->device));
     GlgReplaySampleArgs S;
     memset(&S, 0, sizeof S);
-    S.n = n; S.B = h->B; S.obs_dim = h->obs_dim; S.n_head = r->n_head; S.nf = r->nf; S.fc_off = h->fc_off;
+    S.n = n; S.B = h->a.B; S.obs_dim = h->a.obs_dim; S.n_head = h->n_head; S.nf = h->a.obs_dim - h->n_head; S.fc_off = h->a.fc_off;
     S.norm_obs = r->norm.norm_obs; S.norm_reward = r->norm.norm_reward;
     S.upper = (uint32_t)upper; S.call = r->calls; S.seed = r->seed;
     S.clip_obs = r->norm.clip_obs; S.clip_reward = r->norm.clip_reward;
     S.norm64 = r->norm.norm64;
-    S.weather = h->weather;  // read on every call: glg_set_weather reallocates the bank
+    S.weather = h->a.weather;  // read on every call: glg_set_weather reallocates the bank
     S.head_obs = r->head_obs; S.head_next = r->head_next; S.key_obs = r->key_obs; S.key_next = r->key_next;
     S.act = r->act; S.rew = r->rew; S.dn = r->dn;
     S.obs_out = obs_dev; S.next_out = next_obs_dev; S.act_out = actions_dev; S.rew_out = rewards_dev; S.done_out = dones_dev;
@@ -1174,19 +1143,21 @@ extern "C" int glg_replay_sample(glg_replay *r, int32_t n, float *obs_dev, float
 }
 
 extern "C" int64_t glg_replay_size(const glg_replay *r) { return r ? (r->full ? r->cap : r->pos) : 0; }
-extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)(r->bytes + r->norm.bytes) : 0; }
+extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)r->mem.bytes() : 0; }
 extern "C" float *glg_replay_obs_dev(glg_replay *r) { return r ? r->obs_norm : nullptr; }
 extern "C" double *glg_replay_stats_dev(glg_replay *r) { return r ? r->norm.stat : nullptr; }
 
 // ---- receding-horizon planner (glg_plan.cuh): its own object holding a second, internal handle of B K planning envs that the
 // unchanged step kernels advance; the env handle is only read ----
 struct glg_plan {
-    glg_handle *h = nullptr;   // the env whose states are planned from (read only)
-    glg_handle *hp = nullptr;  // planning envs: B K, no auto-reset, nominal model; shares h's weather bank (see plan_sync)
+    glg_handle *h = nullptr;  // the env whose states are planned from (read only; not on destruction: it may already be gone)
+    // planning envs: B K, no auto-reset, nominal model; points at h's weather bank and owns none (see plan_sync)
+    std::unique_ptr<glg_handle> hp;
     int device = 0, B = 0, BK = 0;
     glg_plan_config cfg = {};
     unsigned long long weather_gen = 0;  // bank generation hp's pointers refer to
     uint32_t calls = 0;                  // glg_plan_run calls so far (Philox counter word 1)
+    CudaMem mem;
     float *mean = nullptr, *std = nullptr, *cand = nullptr;
     double *ret = nullptr;
     unsigned char *alive = nullptr;
@@ -1196,18 +1167,13 @@ static constexpr long long kPlanMaxBatch = 4194304;  // B K: the largest batch t
 
 extern "C" void glg_plan_destroy(glg_plan *p) {
     if (!p) return;
-    cudaSetDevice(p->device);  // the env handle may already be gone: nothing here reads it
-    if (p->hp) {
-        p->hp->weather = nullptr; p->hp->start_day = nullptr; p->hp->reset_tables = nullptr;  // the env's, not hp's
-        glg_destroy(p->hp);
-    }
-    cudaFree(p->mean); cudaFree(p->std); cudaFree(p->cand); cudaFree(p->ret); cudaFree(p->alive);
+    cudaSetDevice(p->device);
     delete p;
 }
 
 extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_plan **out) {
     if (!h || !cfg || !out) {
-        g_create_error = "glg_plan_create: null argument";
+        g_error = "glg_plan_create: null argument";
         return GLG_ERR_ARG;
     }
     *out = nullptr;
@@ -1217,11 +1183,11 @@ extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_pl
         return fail(h, GLG_ERR_ARG, "glg_plan_create: need horizon >= 1, 1 <= n_elites <= n_candidates <= 4096, n_iterations >= 1");
     if (!(c.gamma > 0.0 && c.gamma <= 1.0) || !(c.init_std > 0.0 && c.init_std < 3.4e38))  // std is stored as float
         return fail(h, GLG_ERR_ARG, "glg_plan_create: need 0 < gamma <= 1 and a finite init_std > 0");
-    if ((long long)h->B * c.n_candidates > kPlanMaxBatch)
+    if ((long long)h->a.B * c.n_candidates > kPlanMaxBatch)
         return fail(h, GLG_ERR_ARG, "glg_plan_create: num_envs * n_candidates > 4194304 planning envs");
     if ((uint64_t)c.n_iterations * (uint64_t)c.horizon * 3u > UINT32_MAX)
         return fail(h, GLG_ERR_ARG, "glg_plan_create: n_iterations * horizon * 3 must fit the 32-bit Philox counter word");
-    if (!h->have_params || !h->have_weather)
+    if (!h->have_params || !h->a.weather)
         return fail(h, GLG_ERR_STATE, "glg_plan_create: set the env's parameters and weather bank first");
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
     glg_plan *p = new (std::nothrow) glg_plan();
@@ -1229,28 +1195,31 @@ extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_pl
     p->h = h;
     p->device = h->cfg.device;
     p->cfg = c;
-    p->B = h->B;
-    p->BK = h->B * c.n_candidates;
+    p->B = h->a.B;
+    p->BK = h->a.B * c.n_candidates;
     glg_config pc = h->cfg;  // precision, integrator, n_sub, N, Np, prices, constraints and the observation stack stay the env's
     pc.num_envs = p->BK;
     pc.auto_reset = 0;
     pc.uncertainty_scale = 0.0;
+    pc.seed = h->a.seed;  // the env's current seed (glg_set_seed): StateObservations entries are keyed by it
     pc.env_id_offset = 0;
     pc.role_warps = 0;
     pc.role_lanes = 0;
-    int rc = glg_create(&pc, &p->hp);
+    glg_handle *hp = nullptr;
+    int rc = glg_create(&pc, &hp);
+    p->hp.reset(hp);
     if (rc != GLG_OK) {
-        h->err = std::string("glg_plan_create: planning handle: ") + g_create_error;
+        h->err = std::string("glg_plan_create: planning handle: ") + g_error;
         glg_plan_destroy(p);
         return rc;
     }
-    p->hp->is_reset = true;  // every run / evaluate loads its states (fan-out) before stepping
+    hp->is_reset = true;  // every run / evaluate loads its states (fan-out) before stepping
     const size_t HB6 = (size_t)c.horizon * p->B * GLG_NU, HBK6 = (size_t)c.horizon * p->BK * GLG_NU;
-    cudaError_t e = dev_alloc(&p->mean, HB6);
-    if (e == cudaSuccess) e = dev_alloc(&p->std, HB6);
-    if (e == cudaSuccess) e = dev_alloc(&p->cand, HBK6);
-    if (e == cudaSuccess) e = dev_alloc(&p->ret, (size_t)p->BK);
-    if (e == cudaSuccess) e = dev_alloc(&p->alive, (size_t)p->BK);
+    cudaError_t e = p->mem.dev(&p->mean, HB6);
+    if (e == cudaSuccess) e = p->mem.dev(&p->std, HB6);
+    if (e == cudaSuccess) e = p->mem.dev(&p->cand, HBK6);
+    if (e == cudaSuccess) e = p->mem.dev(&p->ret, (size_t)p->BK);
+    if (e == cudaSuccess) e = p->mem.dev(&p->alive, (size_t)p->BK);
     if (e == cudaSuccess) {
         std::vector<float> s0(HB6, (float)c.init_std);
         e = cudaMemcpy(p->std, s0.data(), HB6 * sizeof(float), cudaMemcpyHostToDevice);
@@ -1267,7 +1236,7 @@ extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_pl
 // Before every run / evaluate: the env must be reset and still hold the bank the planner was created under; its parameters
 // (glg_set_params may have been called since) and bank pointers are copied into the planning handle.  Host fields only.
 static int plan_sync(glg_plan *p, const char *what) {
-    glg_handle *h = p->h, *hp = p->hp;
+    glg_handle *h = p->h, *hp = p->hp.get();
     if (p->weather_gen != h->weather_gen) {
         h->err = std::string(what) + ": the weather bank was replaced (glg_set_weather) after this planner was created";
         return GLG_ERR_STATE;
@@ -1279,29 +1248,28 @@ static int plan_sync(glg_plan *p, const char *what) {
     hp->uni = h->uni;
     hp->general = h->general;
     hp->have_params = true;
-    hp->weather = h->weather; hp->start_day = h->start_day; hp->reset_tables = h->reset_tables;
-    hp->n_tables = h->n_tables; hp->rows = h->rows; hp->n_reset_tables = h->n_reset_tables;
-    hp->have_weather = true;
+    hp->a.weather = h->a.weather; hp->a.start_day = h->a.start_day; hp->a.reset_tables = h->a.reset_tables;
+    hp->a.n_tables = h->a.n_tables; hp->a.rows = h->a.rows; hp->a.n_reset_tables = h->a.n_reset_tables;
     return GLG_OK;
 }
 
 static int plan_fanout(glg_plan *p, cudaStream_t s) {
-    glg_handle *h = p->h, *hp = p->hp;
+    const GlgStepArgs &e = p->h->a, &pe = p->hp->a;
     GlgPlanFanArgs A;
     memset(&A, 0, sizeof A);
     A.B = p->B; A.K = p->cfg.n_candidates;
-    A.x = h->x; A.u = h->u; A.time = h->time; A.timestep = h->timestep; A.table = h->table; A.step_ctr = h->step_ctr;
-    A.px = hp->x; A.pu = hp->u; A.ptime = hp->time; A.pep_return = hp->ep_return; A.pep_info = hp->ep_info;
-    A.ptimestep = hp->timestep; A.ptable = hp->table; A.pep_len = hp->ep_len; A.pstep_ctr = hp->step_ctr; A.pdone = hp->done;
+    A.x = e.x; A.u = e.u; A.time = e.time; A.timestep = e.timestep; A.table = e.table; A.step_ctr = e.step_ctr;
+    A.px = pe.x; A.pu = pe.u; A.ptime = pe.time; A.pep_return = pe.ep_return; A.pep_info = pe.ep_info;
+    A.ptimestep = pe.timestep; A.ptable = pe.table; A.pep_len = pe.ep_len; A.pstep_ctr = pe.step_ctr; A.pdone = pe.done;
     A.ret = p->ret; A.alive = p->alive;
     glg_plan_fanout_kernel<<<(p->BK + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, s>>>(A);
-    GLG_CUDA(h, cudaGetLastError());
+    GLG_CUDA(p->h, cudaGetLastError());
     return GLG_OK;
 }
 
 // H steps of the planning envs with the actions seq[t] ([B K][6] each), discounted returns accumulated into p->ret
 static int plan_rollout(glg_plan *p, const float *seq, cudaStream_t s) {
-    glg_handle *h = p->h, *hp = p->hp;
+    glg_handle *h = p->h, *hp = p->hp.get();
     const size_t step_stride = (size_t)p->BK * GLG_NU;
     double d = 1.0;
     for (int t = 0; t < p->cfg.horizon; ++t) {
@@ -1310,8 +1278,8 @@ static int plan_rollout(glg_plan *p, const float *seq, cudaStream_t s) {
             h->err = "planning step: " + hp->err;
             return rc;
         }
-        glg_plan_accum_kernel<<<(p->BK + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, s>>>(p->BK, d, hp->reward, hp->done, p->ret,
-                                                                                            p->alive);
+        glg_plan_accum_kernel<<<(p->BK + GLG_PLAN_NT - 1) / GLG_PLAN_NT, GLG_PLAN_NT, 0, s>>>(p->BK, d, hp->a.reward, hp->a.done,
+                                                                                            p->ret, p->alive);
         GLG_CUDA(h, cudaGetLastError());
         d *= p->cfg.gamma;
     }
@@ -1384,13 +1352,13 @@ extern "C" int glg_nccl_unique_id(uint8_t id_out[128]) {
     std::string err;
     NcclApi *n = nccl_api(&err);
     if (!n) {
-        g_create_error = err;
+        g_error = err;
         return GLG_ERR_STATE;
     }
     NcclId id;
     const int rc = n->GetUniqueId(&id);
     if (rc != 0) {
-        g_create_error = std::string("ncclGetUniqueId: ") + (n->GetErrorString ? n->GetErrorString(rc) : "error");
+        g_error = std::string("ncclGetUniqueId: ") + (n->GetErrorString ? n->GetErrorString(rc) : "error");
         return GLG_ERR_CUDA;
     }
     memcpy(id_out, id.internal, 128);
@@ -1420,13 +1388,12 @@ extern "C" int glg_allreduce_stats(glg_handle *h, void *stream) {
     NcclApi *n = nccl_api(&h->err);
     if (!n) return GLG_ERR_STATE;
     GLG_CUDA(h, cudaSetDevice(h->cfg.device));
-    const int rc = n->AllReduce(h->stats, h->stats, GLG_NSTATS, /*ncclDouble*/ 8, /*ncclSum*/ 0, h->nccl_comm, (cudaStream_t)stream);
+    const int rc = n->AllReduce(h->a.stats, h->a.stats, GLG_NSTATS, /*ncclDouble*/ 8, /*ncclSum*/ 0, h->nccl_comm, (cudaStream_t)stream);
     if (rc != 0) return fail(h, GLG_ERR_CUDA, (std::string("ncclAllReduce: ") + (n->GetErrorString ? n->GetErrorString(rc) : "error")).c_str());
     return GLG_OK;
 }
 
 // ---- batched evalF (handle-free) ------------------------------------------------------------------------
-static thread_local std::string g_evalf_error;
 
 template <bool GENERAL, bool PER_ENV_P>
 static cudaError_t launch_evalf(const GlgUniform &uni, const double *x, const double *u, const double *d, const double *p,
@@ -1450,7 +1417,7 @@ extern "C" int glg_evalf_batch_ex(const double *x_dev, const double *u_dev, cons
                                   int32_t integrator, int32_t device, void *stream) {
     if (!x_dev || !u_dev || !d_dev || !p_dev || !x_next_dev || B < 1 || n_sub < 1 || (p_stride != 0 && p_stride != GLG_NP) ||
         (integrator != 0 && integrator != 1)) {
-        g_create_error = "glg_evalf_batch: invalid argument";
+        g_error = "glg_evalf_batch: invalid argument";
         return GLG_ERR_ARG;
     }
     cudaError_t e = cudaSetDevice(device);
@@ -1474,7 +1441,7 @@ extern "C" int glg_evalf_batch_ex(const double *x_dev, const double *u_dev, cons
         }
     }
     if (e != cudaSuccess) {
-        g_create_error = std::string("glg_evalf_batch: ") + cudaGetErrorString(e);
+        g_error = std::string("glg_evalf_batch: ") + cudaGetErrorString(e);
         return GLG_ERR_CUDA;
     }
     return GLG_OK;
@@ -1488,12 +1455,13 @@ static int measure_peak(int device, double *out) {
     cudaDeviceProp prop;
     if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, device);
     if (e != cudaSuccess) {
-        g_create_error = std::string("glg_measure_peak: ") + cudaGetErrorString(e);
+        g_error = std::string("glg_measure_peak: ") + cudaGetErrorString(e);
         return GLG_ERR_CUDA;
     }
     const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 4096;
+    CudaMem mem;
     T *buf = nullptr;
-    cudaMalloc((void **)&buf, (size_t)blocks * threads * sizeof(T));
+    mem.dev(&buf, (size_t)blocks * threads);
     cudaEvent_t a, b;
     cudaEventCreate(&a);
     cudaEventCreate(&b);
@@ -1511,9 +1479,8 @@ static int measure_peak(int device, double *out) {
     e = cudaGetLastError();
     cudaEventDestroy(a);
     cudaEventDestroy(b);
-    cudaFree(buf);
     if (e != cudaSuccess) {
-        g_create_error = std::string("glg_measure_peak: ") + cudaGetErrorString(e);
+        g_error = std::string("glg_measure_peak: ") + cudaGetErrorString(e);
         return GLG_ERR_CUDA;
     }
     *out = best;
@@ -1533,7 +1500,7 @@ extern "C" int glg_debug_math(int32_t op, const double *in_dev, double *out_dev,
     glg_math_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(op, in_dev, out_dev, n);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
-        g_create_error = std::string("glg_debug_math: ") + cudaGetErrorString(e);
+        g_error = std::string("glg_debug_math: ") + cudaGetErrorString(e);
         return GLG_ERR_CUDA;
     }
     return GLG_OK;
