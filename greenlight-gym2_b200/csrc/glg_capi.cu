@@ -540,6 +540,36 @@ extern "C" int glg_rule_control_batch(const double *settings29, const double *x_
     return GLG_OK;
 }
 
+// the controls glg_step_rule_based computes in its prologue, for every env of a handle: one thread per env, from the same
+// inputs (x[0], x[2], x[15] of the SoA state, the weather row the step reads, the clock) and the same glg_rule_control, with
+// row e of `settings` (double [B][29]) or, when it is NULL, the handle's settings
+__global__ void glg_rule_controls_kernel(const __grid_constant__ GlgStepArgs A, const double *settings, double *controls) {
+    glg_exp_tbl_fill();
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= A.B) return;
+    const int B = A.B;
+    const int kw = min(A.timestep[e], A.rows - A.Np - 1);  // the step kernels' clamp
+    const double *wrow = A.weather + ((size_t)A.table[e] * A.rows + (size_t)kw) * GLG_ND;
+    double xc[GLG_NX], dc[GLG_ND], u[GLG_NU];
+    for (int i = 0; i < GLG_NX; ++i) xc[i] = (i == 0 || i == 2 || i == 15) ? A.x[(size_t)i * B + e] : 0.0;
+    for (int i = 0; i < GLG_ND; ++i) dc[i] = wrow[i];
+    const double *s = settings ? settings + (size_t)e * GLG_NCTRL : A.ctrl;
+    glg_rule_control(s, xc, dc, A.time[(size_t)B + e], A.time[e], u);
+    for (int i = 0; i < GLG_NU; ++i) controls[(size_t)e * GLG_NU + i] = u[i];
+}
+extern "C" int glg_rule_controls(glg_handle *h, const double *settings_dev, double *controls_dev, void *stream) {
+    if (!h || !controls_dev) return GLG_ERR_ARG;
+    int rc = check_ready(h);
+    if (rc) return rc;
+    if (!h->is_reset) return fail(h, GLG_ERR_STATE, "rule controls before reset");
+    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+    const int NT = 128;
+    glg_rule_controls_kernel<<<(h->a.B + NT - 1) / NT, NT, 0, (cudaStream_t)stream>>>(h->a, settings_dev, controls_dev);
+    h->launches += 1;
+    GLG_CUDA(h, cudaGetLastError());
+    return GLG_OK;
+}
+
 static bool is_pinned(const void *p) {
     // small per-thread cache: the callers pass the same few buffers every step, and a stale answer is harmless (a pageable
     // buffer taken for page-locked makes cudaMemcpyAsync stage it itself; the reverse costs one staging copy)

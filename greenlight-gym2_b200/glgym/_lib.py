@@ -73,6 +73,7 @@ SIGNATURES = {
     "glg_set_rule_controller": (C.c_int, [C.c_void_p, _DP]),
     "glg_step_rule_based": (C.c_int, [C.c_void_p, _DP, _VP]),
     "glg_rule_control_batch": (C.c_int, [_DP, _DP, _DP, _DP, _DP, _DP, C.c_int32, C.c_int32, _VP]),
+    "glg_rule_controls": (C.c_int, [C.c_void_p, _DP, _DP, _VP]),
     "glg_step_host": (C.c_int, [C.c_void_p, _FP, _FP, _DP, _U8P]),
     "glg_step_host_split": (C.c_int, [C.c_void_p, _FP, _FP, _IP, _IP, _DP, _U8P]),
     "glg_set_host_obs_mode": (C.c_int, [C.c_void_p, C.c_int32]),

@@ -17,6 +17,7 @@ DEFAULT_SETTINGS = dict(  # configs/agents/rule_based.yml
     thScrPband=-1, thScrDeadZone=4, thScrRh=-2, thScrRhPband=2, lampExtraHeat=2, blScrExtraRh=100, rhMax=85, tHeatBand=-1,
     co2Band=-100, useBlScr=1,
 )
+SETTING_NAMES = tuple(DEFAULT_SETTINGS)  # the 29 keys in rule_based.yml order: the columns of a settings vector
 
 
 def proportional_control(process_var, set_pt, p_band, min_val, max_val):
@@ -29,6 +30,14 @@ class RuleBasedController:
         cfg = dict(DEFAULT_SETTINGS)
         cfg.update(settings)
         self.__dict__.update(cfg)
+
+    @classmethod
+    def from_vector(cls, v):
+        """The controller of a settings vector: 29 numbers in the order of SETTING_NAMES (the inverse of settings_vector)."""
+        v = np.asarray(v, dtype=np.float64).reshape(-1)
+        if v.shape != (len(SETTING_NAMES),):
+            raise ValueError(f"a settings vector has {len(SETTING_NAMES)} entries; got {v.shape[0]}")
+        return cls(**{k: float(x) for k, x in zip(SETTING_NAMES, v)})
 
     def settings_vector(self):
         """float64[29] in the order of rule_based.yml -- what `glg_set_rule_controller` / `glg_rule_control_batch` take."""

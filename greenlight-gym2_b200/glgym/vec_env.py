@@ -383,6 +383,22 @@ class GreenLightVecEnv(_VecEnvBase):
         _lib.check(self._lib.glg_step_rule_based(self._h, n, self._stream()), self._h, "glg_step_rule_based")
         return self.obs_t, self.reward_t, self.done_t
 
+    def rule_controls_tensor(self, settings=None):
+        """RuleBasedController.predict for every env on its current state, weather row and clock: the controls
+        `step_rule_based_tensor` would apply.  settings: CUDA float64 [B, 29] in rule_based.yml order, one row per env, or None
+        for the env's own settings (`set_rule_controller`).  Returns a float64 [B, 6] view of a buffer the env owns, overwritten
+        by the next call; `step_raw_control_tensor` with it steps exactly as `step_rule_based_tensor` would."""
+        s = 0
+        if settings is not None:
+            if tuple(settings.shape) != (self.num_envs, 29):
+                raise ValueError(f"settings must have shape ({self.num_envs}, 29); got {tuple(settings.shape)}")
+            settings = settings.to(device=self.device, dtype=torch.float64).contiguous()
+            s = settings.data_ptr()
+        if getattr(self, "_rule_u", None) is None:
+            self._rule_u = torch.empty((self.num_envs, self.nu), dtype=torch.float64, device=self.device)
+        _lib.check(self._lib.glg_rule_controls(self._h, s, self._rule_u.data_ptr(), self._stream()), self._h, "glg_rule_controls")
+        return self._rule_u
+
     def step_rule_based(self):
         self.step_rule_based_tensor()
         torch.cuda.synchronize(self.device)

@@ -127,6 +127,12 @@ int glg_step_rule_based(glg_handle *h, const double *noise_dev, void *stream);
  * -> u_dev double [n][6]. */
 int glg_rule_control_batch(const double *settings29, const double *x_dev, const double *d_dev, const double *hod_dev,
                            const double *doy_dev, double *u_dev, int32_t n, int32_t device, void *stream);
+/* RuleBasedController.predict for every env of the handle, on its CURRENT state, the weather row of its current timestep and
+ * its clock -- the controls glg_step_rule_based computes in its prologue.  settings_dev: NULL (the handle's settings,
+ * glg_set_rule_controller) or double [B][29] in rule_based.yml order, one row per env.  controls_dev: double [B][6].
+ * glg_step_raw_control(h, controls_dev, noise_dev, stream) then steps exactly as glg_step_rule_based would.  One launch.
+ * GLG_ERR_ARG on a NULL handle or NULL controls_dev, GLG_ERR_STATE before the first glg_reset. */
+int glg_rule_controls(glg_handle *h, const double *settings_dev, double *controls_dev, void *stream);
 
 /* End-to-end convenience for host callers (the SB3 VecEnv numpy path; replaces SubprocVecEnv.step_async / step_wait over
  * TomatoEnv.step, RL/utils.py:44-58): copies actions host->device, runs glg_step on the handle's own stream, delivers
