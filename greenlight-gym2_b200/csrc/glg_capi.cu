@@ -26,6 +26,7 @@
 #include "glg_rollout.cuh"
 #include "glg_replay.cuh"
 #include "glg_plan.cuh"
+#include "glg_tangent.cuh"
 
 
 static thread_local std::string g_error = "";  // glg_last_error(NULL): the last failure of an entry point without a handle
@@ -1474,6 +1475,85 @@ extern "C" int glg_evalf_batch_ex(const double *x_dev, const double *u_dev, cons
         g_error = std::string("glg_evalf_batch: ") + cudaGetErrorString(e);
         return GLG_ERR_CUDA;
     }
+    return GLG_OK;
+}
+
+// ---- linearisation (glg_tangent.cuh) -----------------------------------------------------------------------
+
+// the pure entry points: arguments validated like glg_evalf_batch_ex, the variant selected the same way
+template <bool STEP>
+static int tangent_batch(const char *name, const double *x, const double *u, const double *d, const double *p, int p_stride,
+                         double *f, double *jx, double *ju, uint8_t *bad, int B, double dt, int n_sub, int integrator, int device,
+                         void *stream) {
+    if (!x || !u || !d || !p || !jx || B < 1 || n_sub < 1 || (p_stride != 0 && p_stride != GLG_NP) || (integrator != 0 && integrator != 1)) {
+        g_error = std::string(name) + ": invalid argument";
+        return GLG_ERR_ARG;
+    }
+    GlgTanArgs a{};
+    a.x = x; a.xe = GLG_NX; a.xi = 1;
+    a.u = u; a.ue = GLG_NU; a.ui = 1;
+    a.d = d; a.p = p;
+    a.f = f; a.jx = jx; a.ju = ju; a.bad = bad;
+    a.B = B; a.dt = dt; a.n_sub = n_sub; a.integrator = integrator;
+    cudaError_t e = cudaSetDevice(device);
+    cudaStream_t s = (cudaStream_t)stream;
+    GlgUniform uni{};
+    if (e == cudaSuccess) {
+        if (p_stride == 0) {
+            double ph[GLG_NP];
+            e = cudaMemcpyAsync(ph, p, sizeof ph, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+            if (e == cudaSuccess) {
+                for (int i = 0; i < GLG_NP; ++i) uni.P[i] = ph[i];
+                glg_make_k(ph, uni.K);
+                glg_make_c(ph, uni.C);
+                e = glg_launch_tangent_any<STEP>(uni, !glg_params_nominal_structure(ph), false, a, s);
+            }
+        } else {
+            e = glg_launch_tangent_any<STEP>(uni, true, true, a, s);
+        }
+    }
+    if (e != cudaSuccess) {
+        g_error = std::string(name) + ": " + cudaGetErrorString(e);
+        return GLG_ERR_CUDA;
+    }
+    return GLG_OK;
+}
+extern "C" int glg_rhs_jacobian_batch(const double *x_dev, const double *u_dev, const double *d_dev, const double *p_dev,
+                                      int32_t p_stride, double *f_dev, double *jx_dev, double *ju_dev, int32_t B, int32_t device,
+                                      void *stream) {
+    return tangent_batch<false>("glg_rhs_jacobian_batch", x_dev, u_dev, d_dev, p_dev, p_stride, f_dev, jx_dev, ju_dev, nullptr, B,
+                                900.0, 1, 0, device, stream);
+}
+extern "C" int glg_evalf_jacobian_batch(const double *x_dev, const double *u_dev, const double *d_dev, const double *p_dev,
+                                        int32_t p_stride, double *x_next_dev, double *jx_dev, double *ju_dev, uint8_t *bad_dev,
+                                        int32_t B, double dt, int32_t n_sub, int32_t integrator, int32_t device, void *stream) {
+    return tangent_batch<true>("glg_evalf_jacobian_batch", x_dev, u_dev, d_dev, p_dev, p_stride, x_next_dev, jx_dev, ju_dev, bad_dev,
+                               B, dt, n_sub, integrator, device, stream);
+}
+// the handle's envs: state and u straight from the SoA buffers, the weather row through the step kernels' clamp, the nominal
+// parameters in h->uni (fp64 whatever the handle's precision; noise never enters)
+extern "C" int glg_linearize(glg_handle *h, const double *controls_dev, double *x_next_dev, double *jx_dev, double *ju_dev, void *stream) {
+    if (!h || !jx_dev) return GLG_ERR_ARG;
+    int rc = check_ready(h);
+    if (rc) return rc;
+    if (!h->is_reset) return fail(h, GLG_ERR_STATE, "linearize before reset");
+    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+    const int B = h->a.B;
+    GlgTanArgs a{};
+    a.x = h->a.x; a.xe = 1; a.xi = B;
+    if (controls_dev) {
+        a.u = controls_dev; a.ue = GLG_NU; a.ui = 1;
+    } else {
+        a.u = h->a.u; a.ue = 1; a.ui = B;
+    }
+    a.d = nullptr;
+    a.weather = h->a.weather; a.timestep = h->a.timestep; a.table = h->a.table; a.rows = h->a.rows; a.Np = h->a.Np;
+    a.f = x_next_dev; a.jx = jx_dev; a.ju = ju_dev; a.bad = nullptr;
+    a.B = B; a.dt = h->a.dt; a.n_sub = h->a.n_sub; a.integrator = h->a.integrator;
+    const cudaError_t e = glg_launch_tangent_any<true>(h->uni, h->general, false, a, (cudaStream_t)stream);
+    h->launches += 1;
+    GLG_CUDA(h, e);
     return GLG_OK;
 }
 

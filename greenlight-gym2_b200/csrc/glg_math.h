@@ -20,6 +20,8 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <type_traits>
+
 #if defined(__CUDACC__)
 #define GLG_HD __host__ __device__ __forceinline__
 #else
@@ -498,3 +500,226 @@ GLG_HD void glg_cbrt_n(const float (&x)[N], float (&y)[N]) {
 #pragma unroll
     for (int i = 0; i < N; ++i) y[i] = glg_cbrt(x[i]);
 }
+
+// =========================================================================================================
+// Forward-mode tangents (glg_tangent.cuh): GlgDual<N> is an fp64 value and N fp64 tangent directions.  The flux units, the hoist
+// and the RK4 tangent are templates over their scalar type, so instantiating them with GlgDual<N> gives the exact derivative of
+// the same arithmetic: every value part goes through exactly the double function above, so it is what the double code computes.
+// Derivatives are formed from the primal result where possible (exp' = y, rcp' = -y^2, sqrt' = 0.5/y, cbrt' = y/(3x),
+// pow(b, e)' = e y / b, inv1pexp' = -y (1 - y)).
+// Conventions at non-smooth points:
+//   fabs'(0) = 0 (CasADi's sign(0) = 0);
+//   fmin / fmax / ?: carry the derivative of the branch the primal takes (the first argument on a tie);
+//   exponents of glg_pow / pow are constants: their tangent is not propagated (every call site passes a literal);
+//   step-count decisions (harvest micro-steps, the graded integrator's splits) are taken on value parts only, so a tangent is
+//   the exact derivative of the discrete map on the grid that was executed.
+// Operators with a plain double exist so constants (K, C, p) cost no tangent arithmetic: 0 * x cannot be folded under IEEE rules.
+// =========================================================================================================
+template <int N>
+struct GlgDual {
+    double v;
+    double t[N];
+    GlgDual() = default;
+    GLG_HD GlgDual(double a) : v(a) {
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+        for (int i = 0; i < N; ++i) t[i] = 0.0;
+    }
+    GLG_HD GlgDual &operator+=(const GlgDual &b) { return *this = *this + b; }
+    GLG_HD GlgDual &operator-=(const GlgDual &b) { return *this = *this - b; }
+    GLG_HD GlgDual &operator*=(const GlgDual &b) { return *this = *this * b; }
+    GLG_HD GlgDual &operator+=(double b) { v += b; return *this; }
+    GLG_HD GlgDual &operator-=(double b) { v -= b; return *this; }
+};
+template <class T>
+struct glg_is_dual : std::false_type {};
+template <int N>
+struct glg_is_dual<GlgDual<N>> : std::true_type {};
+
+GLG_HD double glg_value(double a) { return a; }
+GLG_HD float glg_value(float a) { return a; }
+template <int N>
+GLG_HD double glg_value(const GlgDual<N> &a) { return a.v; }
+
+// y with tangent s * a.t: the chain rule of a unary function whose derivative at a.v is s
+template <int N>
+GLG_HD GlgDual<N> glg_chain(double y, double s, const GlgDual<N> &a) {
+    GlgDual<N> r;
+    r.v = y;
+#pragma unroll
+    for (int i = 0; i < N; ++i) r.t[i] = s * a.t[i];
+    return r;
+}
+
+template <int N>
+GLG_HD GlgDual<N> operator-(const GlgDual<N> &a) { return glg_chain(-a.v, -1.0, a); }
+template <int N>
+GLG_HD GlgDual<N> operator+(const GlgDual<N> &a, const GlgDual<N> &b) {
+    GlgDual<N> r;
+    r.v = a.v + b.v;
+#pragma unroll
+    for (int i = 0; i < N; ++i) r.t[i] = a.t[i] + b.t[i];
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator-(const GlgDual<N> &a, const GlgDual<N> &b) {
+    GlgDual<N> r;
+    r.v = a.v - b.v;
+#pragma unroll
+    for (int i = 0; i < N; ++i) r.t[i] = a.t[i] - b.t[i];
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator*(const GlgDual<N> &a, const GlgDual<N> &b) {
+    GlgDual<N> r;
+    r.v = a.v * b.v;
+#pragma unroll
+    for (int i = 0; i < N; ++i) r.t[i] = a.t[i] * b.v + a.v * b.t[i];
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator/(const GlgDual<N> &a, const GlgDual<N> &b) {
+    GlgDual<N> r;
+    r.v = a.v / b.v;
+    const double ib = 1.0 / b.v;
+#pragma unroll
+    for (int i = 0; i < N; ++i) r.t[i] = (a.t[i] - r.v * b.t[i]) * ib;
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator+(const GlgDual<N> &a, double b) {
+    GlgDual<N> r = a;
+    r.v = a.v + b;
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator+(double a, const GlgDual<N> &b) {
+    GlgDual<N> r = b;
+    r.v = a + b.v;
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator-(const GlgDual<N> &a, double b) {
+    GlgDual<N> r = a;
+    r.v = a.v - b;
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> operator-(double a, const GlgDual<N> &b) { return glg_chain(a - b.v, -1.0, b); }
+template <int N>
+GLG_HD GlgDual<N> operator*(const GlgDual<N> &a, double b) { return glg_chain(a.v * b, b, a); }
+template <int N>
+GLG_HD GlgDual<N> operator*(double a, const GlgDual<N> &b) { return glg_chain(a * b.v, a, b); }
+template <int N>
+GLG_HD GlgDual<N> operator/(const GlgDual<N> &a, double b) { return glg_chain(a.v / b, 1.0 / b, a); }
+template <int N>
+GLG_HD GlgDual<N> operator/(double a, const GlgDual<N> &b) {
+    const double y = a / b.v;
+    return glg_chain(y, -y / b.v, b);
+}
+#define GLG_DUAL_CMP(OP)                                                                                   \
+    template <int N>                                                                                       \
+    GLG_HD bool operator OP(const GlgDual<N> &a, const GlgDual<N> &b) { return a.v OP b.v; }             \
+    template <int N>                                                                                       \
+    GLG_HD bool operator OP(const GlgDual<N> &a, double b) { return a.v OP b; }                           \
+    template <int N>                                                                                       \
+    GLG_HD bool operator OP(double a, const GlgDual<N> &b) { return a OP b.v; }
+GLG_DUAL_CMP(<)
+GLG_DUAL_CMP(>)
+GLG_DUAL_CMP(<=)
+GLG_DUAL_CMP(>=)
+GLG_DUAL_CMP(==)
+GLG_DUAL_CMP(!=)
+#undef GLG_DUAL_CMP
+
+template <int N>
+GLG_HD GlgDual<N> fabs(const GlgDual<N> &a) { return glg_chain(fabs(a.v), a.v > 0.0 ? 1.0 : (a.v < 0.0 ? -1.0 : 0.0), a); }
+template <int N>
+GLG_HD GlgDual<N> fmin(const GlgDual<N> &a, const GlgDual<N> &b) {
+    GlgDual<N> r = b.v < a.v ? b : a;
+    r.v = fmin(a.v, b.v);
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> fmax(const GlgDual<N> &a, const GlgDual<N> &b) {
+    GlgDual<N> r = b.v > a.v ? b : a;
+    r.v = fmax(a.v, b.v);
+    return r;
+}
+template <int N>
+GLG_HD GlgDual<N> sqrt(const GlgDual<N> &a) {
+    const double y = sqrt(a.v);
+    return glg_chain(y, 0.5 / y, a);
+}
+template <int N>
+GLG_HD GlgDual<N> exp(const GlgDual<N> &a) {
+    const double y = exp(a.v);
+    return glg_chain(y, y, a);
+}
+template <int N>
+GLG_HD GlgDual<N> pow(const GlgDual<N> &b, double e) {
+    const double y = pow(b.v, e);
+    return glg_chain(y, e * y / b.v, b);
+}
+
+template <int N>
+GLG_HD GlgDual<N> glg_exp(const GlgDual<N> &a) {
+    const double y = glg_exp(a.v);
+    return glg_chain(y, y, a);
+}
+template <int N>
+GLG_HD GlgDual<N> glg_rcp(const GlgDual<N> &a) {
+    const double y = glg_rcp(a.v);
+    return glg_chain(y, -(y * y), a);
+}
+template <int N>
+GLG_HD GlgDual<N> glg_sqrt(const GlgDual<N> &a) {
+    const double y = glg_sqrt(a.v);
+    return glg_chain(y, 0.5 / y, a);
+}
+template <int N>
+GLG_HD GlgDual<N> glg_cbrt(const GlgDual<N> &a) {
+    const double y = glg_cbrt(a.v);
+    return glg_chain(y, y / (3.0 * a.v), a);
+}
+template <int N>
+GLG_HD GlgDual<N> glg_pow(const GlgDual<N> &b, double e) {
+    const double y = glg_pow(b.v, e);
+    return glg_chain(y, e * y / b.v, b);
+}
+template <int N>
+GLG_HD GlgDual<N> glg_pow(const GlgDual<N> &b, const GlgDual<N> &e) { return glg_pow(b, e.v); }  // constant exponent
+template <int N>
+GLG_HD GlgDual<N> glg_root34(const GlgDual<N> &a, bool cube) {
+    const double y = glg_root34(a.v, cube);
+    return glg_chain(y, y * (cube ? 0x1.5555555555555p-2 : 0.25) / a.v, a);
+}
+template <int N>
+GLG_HD GlgDual<N> glg_inv1pexp(const GlgDual<N> &z) {
+    const double y = glg_inv1pexp(z.v);
+    return glg_chain(y, -(y * (1.0 - y)), z);
+}
+#if defined(__CUDA_ARCH__)
+#define GLG_UNROLL _Pragma("unroll")
+#else
+#define GLG_UNROLL
+#endif
+// interleaved batches: the value parts go through the double batch functions, so they are bit-identical to them
+#define GLG_DUAL_BATCH(NAME, DERIV)                                                      \
+    template <int M, int N>                                                              \
+    GLG_HD void NAME(const GlgDual<N>(&x)[M], GlgDual<N>(&y)[M]) {                       \
+        double xv[M], yv[M];                                                             \
+        GLG_UNROLL for (int i = 0; i < M; ++i) xv[i] = x[i].v;                           \
+        NAME<M>(xv, yv);                                                                 \
+        GLG_UNROLL for (int i = 0; i < M; ++i) {                                         \
+            const double yy = yv[i], xx = xv[i];                                         \
+            (void)xx;                                                                    \
+            y[i] = glg_chain(yy, DERIV, x[i]);                                           \
+        }                                                                                \
+    }
+GLG_DUAL_BATCH(glg_exp_n, yy)
+GLG_DUAL_BATCH(glg_rcp_n, -(yy * yy))
+GLG_DUAL_BATCH(glg_sqrt_n, 0.5 / yy)
+GLG_DUAL_BATCH(glg_cbrt_n, yy / (3.0 * xx))
+#undef GLG_DUAL_BATCH

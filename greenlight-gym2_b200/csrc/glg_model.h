@@ -112,9 +112,12 @@ GLG_HD T glg_cond(T hec, T vp1, T vp2) {
 }
 
 // two-layer optics (aux_states.hpp:25-41)
-GLG_HD double glg_tau12(double t1, double t2, double r1d, double r2u) { return t1 * t2 / (1. - r1d * r2u); }
-GLG_HD double glg_rhoup(double t1, double r1u, double r1d, double r2u) { return r1u + (t1 * t1 * r2u) / (1. - r1d * r2u); }
-GLG_HD double glg_rhodn(double t2, double r1d, double r2u, double r2d) { return r2d + (t2 * t2 * r1d) / (1. - r1d * r2u); }
+template <class T>
+GLG_HD T glg_tau12(T t1, T t2, T r1d, T r2u) { return t1 * t2 / (1. - r1d * r2u); }
+template <class T>
+GLG_HD T glg_rhoup(T t1, T r1u, T r1d, T r2u) { return r1u + (t1 * t1 * r2u) / (1. - r1d * r2u); }
+template <class T>
+GLG_HD T glg_rhodn(T t2, T r1d, T r2u, T r2d) { return r2d + (t2 * t2 * r1d) / (1. - r1d * r2u); }
 
 // ---------------------------------------------------------------------------------------------------------
 // K: parameter-only constants.  P is anything indexable as p[i] -> double.
@@ -207,40 +210,41 @@ GLG_HD void glg_make_c(const P &p, double *C) {
 // H: everything that depends on (u, d, p) but not on the state.  Executed once per env-step.
 //   u[6]: boil, co2, thScr, vent, lamp, blScr (aux_states.hpp:97-105)   d[>=7]: iGlob,tOut,vpOut,co2Out,wind,tSky,tSoOut
 // ---------------------------------------------------------------------------------------------------------
-template <class P, class HOUT>
-GLG_HD void glg_hoist(const P &p, const double *u, const double *d, HOUT &H) {
+// Generic in u's scalar type T (double in the step kernels; GlgDual for the derivative with respect to the controls).
+template <class P, class T, class HOUT>
+GLG_HD void glg_hoist(const P &p, const T *u, const double *d, HOUT &H) {
     const double pi = 3.14159265358979323846;
-    const double thScr = u[2], blScr = u[5];
+    const T thScr = u[2], blScr = u[5];
     // cover optics: roof+thermal screen -> +blackout screen -> +lamp layer, PAR and NIR (:111-194)
-    const double tauThPar = 1 - thScr * (1 - p[80]), rhoThPar = thScr * p[77];
-    const double tauA = glg_tau12(p[69], tauThPar, p[66], rhoThPar);
-    const double rupA = glg_rhoup(p[69], p[66], p[66], rhoThPar);
-    const double rdnA = glg_rhodn(tauThPar, p[66], rhoThPar, rhoThPar);
-    const double tauThNir = 1 - thScr * (1 - p[79]), rhoThNir = thScr * p[76];
-    const double tauB = glg_tau12(p[68], tauThNir, p[65], rhoThNir);
-    const double rupB = glg_rhoup(p[68], p[65], p[65], rhoThNir);
-    const double rdnB = glg_rhodn(tauThNir, p[65], rhoThNir, rhoThNir);
-    const double tauBlPar = 1 - blScr * (1 - p[90]), rhoBlPar = blScr * p[88];
-    const double tauA2 = glg_tau12(tauA, tauBlPar, rdnA, rhoBlPar);
-    const double rupA2 = glg_rhoup(tauA, rupA, rdnA, rhoBlPar);
-    const double rdnA2 = glg_rhodn(tauBlPar, rdnA, rhoBlPar, rhoBlPar);
-    const double tauBlNir = 1 - blScr * (1 - p[89]), rhoBlNir = blScr * p[87];
-    const double tauB2 = glg_tau12(tauB, tauBlNir, rdnB, rhoBlNir);
-    const double rupB2 = glg_rhoup(tauB, rupB, rdnB, rhoBlNir);
-    const double rdnB2 = glg_rhodn(tauBlNir, rdnB, rhoBlNir, rhoBlNir);
-    const double tauCovPar = glg_tau12(tauA2, p[176], rdnA2, p[179]);
-    const double rhoCovPar = glg_rhoup(tauA2, rupA2, rdnA2, p[179]);
-    const double tauCovNir = glg_tau12(tauB2, p[177], rdnB2, p[180]);
-    const double rhoCovNir = glg_rhoup(tauB2, rupB2, rdnB2, p[180]);
-    const double aCovPar = 1 - tauCovPar - rhoCovPar, aCovNir = 1 - tauCovNir - rhoCovNir;
+    const T tauThPar = 1 - thScr * (1 - p[80]), rhoThPar = thScr * p[77];
+    const T tauA = glg_tau12<T>(p[69], tauThPar, p[66], rhoThPar);
+    const T rupA = glg_rhoup<T>(p[69], p[66], p[66], rhoThPar);
+    const T rdnA = glg_rhodn<T>(tauThPar, p[66], rhoThPar, rhoThPar);
+    const T tauThNir = 1 - thScr * (1 - p[79]), rhoThNir = thScr * p[76];
+    const T tauB = glg_tau12<T>(p[68], tauThNir, p[65], rhoThNir);
+    const T rupB = glg_rhoup<T>(p[68], p[65], p[65], rhoThNir);
+    const T rdnB = glg_rhodn<T>(tauThNir, p[65], rhoThNir, rhoThNir);
+    const T tauBlPar = 1 - blScr * (1 - p[90]), rhoBlPar = blScr * p[88];
+    const T tauA2 = glg_tau12<T>(tauA, tauBlPar, rdnA, rhoBlPar);
+    const T rupA2 = glg_rhoup<T>(tauA, rupA, rdnA, rhoBlPar);
+    const T rdnA2 = glg_rhodn<T>(tauBlPar, rdnA, rhoBlPar, rhoBlPar);
+    const T tauBlNir = 1 - blScr * (1 - p[89]), rhoBlNir = blScr * p[87];
+    const T tauB2 = glg_tau12<T>(tauB, tauBlNir, rdnB, rhoBlNir);
+    const T rupB2 = glg_rhoup<T>(tauB, rupB, rdnB, rhoBlNir);
+    const T rdnB2 = glg_rhodn<T>(tauBlNir, rdnB, rhoBlNir, rhoBlNir);
+    const T tauCovPar = glg_tau12<T>(tauA2, p[176], rdnA2, p[179]);
+    const T rhoCovPar = glg_rhoup<T>(tauA2, rupA2, rdnA2, p[179]);
+    const T tauCovNir = glg_tau12<T>(tauB2, p[177], rdnB2, p[180]);
+    const T rhoCovNir = glg_rhoup<T>(tauB2, rupB2, rdnB2, p[180]);
+    const T aCovPar = 1 - tauCovPar - rhoCovPar, aCovNir = 1 - tauCovNir - rhoCovNir;
     const double epsCovFir = 1 - p[70] - p[67];
 
     // radiation above the canopy (:256-295)
     const double iGlob = d[0];
-    const double qLamp = p[172] * u[4];                          // a37
-    const double parSun = (1 - p[44]) * tauCovPar * p[6] * iGlob;  // a39
-    const double parLamp = p[174] * qLamp;                        // a40
-    const double rCan = (1 - p[44]) * iGlob * (p[6] * tauCovPar + p[5] * tauCovNir) + (p[174] + p[175]) * qLamp;  // a45
+    const T qLamp = p[172] * u[4];                          // a37
+    const T parSun = (1 - p[44]) * tauCovPar * p[6] * iGlob;  // a39
+    const T parLamp = p[174] * qLamp;                        // a40
+    const T rCan = (1 - p[44]) * iGlob * (p[6] * tauCovPar + p[5] * tauCovNir) + (p[174] + p[175]) * qLamp;  // a45
     H[H_PARCAN_W] = (parSun + parLamp) * (1 - p[10]);
     H[H_PARLAMP_W] = parLamp * (1 - p[10]);
     H[H_PARFLR_W] = (1 - p[98]) * (parSun + parLamp);
@@ -259,8 +263,8 @@ GLG_HD void glg_hoist(const P &p, const double *u, const double *d, HOUT &H) {
 
     // FIR pair coefficients area*eps1*eps2*F12*sigma that depend on the screens (:476-632)
     const double sigma = p[2];
-    const double tauThFir = 1 - thScr * (1 - p[81]);  // a81
-    const double tauBlFir = 1 - blScr * (1 - p[91]);  // a82
+    const T tauThFir = 1 - thScr * (1 - p[81]);  // a81
+    const T tauBlFir = 1 - blScr * (1 - p[91]);  // a82
     const double fPipe = 0.49 * pi * p[107] * p[105];
     const double t178 = p[178], t199 = p[199];
     H[H_C84] = p[3] * epsCovFir * (t178 * tauThFir * tauBlFir) * sigma;                          // can-covIn  x aCan
@@ -283,12 +287,12 @@ GLG_HD void glg_hoist(const P &p, const double *u, const double *d, HOUT &H) {
     // ventilation (:698-779).  a126 (side vents) is hard-wired to 0 in the reference, so a134=0 and
     // a137=(1-cLeakTop)*fLeakage for both if_else branches; a133 reduces to its wind term.
     const double tOut = d[1], wind = d[4];
-    const double aRoofU = u[3] * p[55];
+    const T aRoofU = u[3] * p[55];
     const double cD = p[59], cW = p[61];
-    const double v132a = u[3] * p[55] * cD / (2. * p[46]);
-    const double a133 = cD / p[46] * sqrt(1e-8 + (glg_sq(aRoofU) * cW * (wind * wind)));
+    const T v132a = u[3] * p[55] * cD / (2. * p[46]);
+    const T a133 = cD / p[46] * sqrt(1e-8 + (glg_sq(aRoofU) * cW * (wind * wind)));
     const double fLeak = (wind < p[205]) ? p[205] * p[60] : p[60] * wind;
-    const double scrMax = fmax(thScr, blScr);
+    const T scrMax = fmax(thScr, blScr);
     const bool roofOnly = (1.0 >= p[8]);  // a127 = 1
     H[H_TOUT] = tOut;
     H[H_TOUT_2K] = tOut + 2 * GLG_C2K;
@@ -312,7 +316,7 @@ GLG_HD void glg_hoist(const P &p, const double *u, const double *d, HOUT &H) {
     H[H_TSOOUT] = d[6];
 
     // stomata (:940-954)
-    const double sRs = 1. / (1. + exp(p[43] * (rCan - p[40])));
+    const T sRs = 1. / (1. + exp(p[43] * (rCan - p[40])));
     H[H_CEVAP3] = p[20] * (1. - sRs) + p[19] * sRs;
     H[H_CEVAP4] = p[22] * (1. - sRs) + p[21] * sRs;
     H[H_RS] = p[42] * ((rCan + p[17]) / (rCan + p[18]));

@@ -26,6 +26,13 @@
 #pragma once
 #include "glg_model.h"
 
+// Scalar type of the units: the stage state's type when it is a tangent type (GlgDual: K, C and p stay plain doubles, so
+// constants cost no tangent arithmetic), else the constant sets' type (double in parity mode, float in throughput mode).
+template <class XV>
+using glg_x_scalar_t = typename std::decay<decltype(std::declval<const XV &>().template at<0>())>::type;
+template <class KV, class XV>
+using glg_unit_t = typename std::conditional<glg_is_dual<glg_x_scalar_t<XV>>::value, glg_x_scalar_t<XV>, glg_scalar_t<KV>>::type;
+
 enum GlgUnitId { U_OPT, U_PIPES, U_FIR, U_VENT, U_SCR, U_FLOOR, U_THSCR, U_BLSCR, U_COVER, U_TRANSP, U_PHOTO, U_FLOWS, U_MAINT, U_COUNT };
 
 // states unit u contributes to (bit i = state i).  GENERAL adds the interlight node 18 and the grow-pipe FIR term.
@@ -85,7 +92,7 @@ struct GlgArrayX {  // plain array in state order (host tests, kernel A style ca
 
 template <bool GENERAL, class KV, class CV, class HV, class XV, class PT>
 GLG_HD void glg_unit_opt(const KV &K, const CV &C, const HV &H, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     const T lai = C[C_SLA] * GLG_X(x, 23);
     const T ea[3] = {-K[K_K1PAR] * lai, -K[K_KNIR] * lai, -K[K_K2PAR] * lai};
     T ey[3];
@@ -119,8 +126,8 @@ GLG_HD void glg_unit_opt(const KV &K, const CV &C, const HV &H, const XV &x, con
 }
 
 template <class KV, class CV, class XV, class PT>
-GLG_HD void glg_unit_pipes(const KV &K, const CV &C, const XV &x, const PT &pt, GlgSpecial<glg_scalar_t<KV>> &sp) {
-    typedef glg_scalar_t<KV> T;
+GLG_HD void glg_unit_pipes(const KV &K, const CV &C, const XV &x, const PT &pt, GlgSpecial<glg_unit_t<KV, XV>> &sp) {
+    typedef glg_unit_t<KV, XV> T;
     const T tAir = GLG_X(x, 2), tCan = GLG_X(x, 4), tPipe = GLG_X(x, 9), tGroPipe = GLG_X(x, 19);
     pt.template put<21>((T(1.) / T(86400.)) * (tCan - GLG_X(x, 21)));
     pt.template put<26>((T(1.) / T(86400.)) * tCan);
@@ -135,9 +142,9 @@ GLG_HD void glg_unit_pipes(const KV &K, const CV &C, const XV &x, const PT &pt, 
     sp.canscale = K[K_INVCAPLEAF] * glg_rcp(C[C_SLA] * GLG_X(x, 23));
 }
 
-template <bool GENERAL, class KV, class CV, class HV, class P, class XV, class PT>
-GLG_HD void glg_unit_fir(const KV &K, const CV &C, const HV &H, const P &p, const double *u, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+template <bool GENERAL, class KV, class CV, class HV, class P, class UT, class XV, class PT>
+GLG_HD void glg_unit_fir(const KV &K, const CV &C, const HV &H, const P &p, const UT *u, const XV &x, const PT &pt) {
+    typedef glg_unit_t<KV, XV> T;
     const T tCan = GLG_X(x, 4), tCovIn = GLG_X(x, 5), tCovE = GLG_X(x, 6), tThScr = GLG_X(x, 7), tFlr = GLG_X(x, 8), tPipe = GLG_X(x, 9);
     const T tLamp = GLG_X(x, 17), tBlScr = GLG_X(x, 20);
     const T lai = C[C_SLA] * GLG_X(x, 23);
@@ -237,8 +244,8 @@ GLG_HD void glg_unit_fir(const KV &K, const CV &C, const HV &H, const P &p, cons
 
 // roof ventilation and leakage: exchange with the outside air
 template <class KV, class HV, class XV, class PT>
-GLG_HD void glg_unit_vent(const KV &K, const HV &H, const XV &x, const PT &pt, GlgSpecial<glg_scalar_t<KV>> &sp) {
-    typedef glg_scalar_t<KV> T;
+GLG_HD void glg_unit_vent(const KV &K, const HV &H, const XV &x, const PT &pt, GlgSpecial<glg_unit_t<KV, XV>> &sp) {
+    typedef glg_unit_t<KV, XV> T;
     const T co2Air = GLG_X(x, 0), co2Top = GLG_X(x, 1), tAir = GLG_X(x, 2), tTop = GLG_X(x, 3), vpAir = GLG_X(x, 15), vpTop = GLG_X(x, 16);
     const T tOut = H[H_TOUT];
     const T tkAir = tAir + T(GLG_C2K), tkTop = tTop + T(GLG_C2K);
@@ -262,8 +269,8 @@ GLG_HD void glg_unit_vent(const KV &K, const HV &H, const XV &x, const PT &pt, G
 
 // air flux through the screens: exchange main air <-> top compartment
 template <class KV, class HV, class XV, class PT>
-GLG_HD void glg_unit_scr(const KV &K, const HV &H, const XV &x, const PT &pt, GlgSpecial<glg_scalar_t<KV>> &sp) {
-    typedef glg_scalar_t<KV> T;
+GLG_HD void glg_unit_scr(const KV &K, const HV &H, const XV &x, const PT &pt, GlgSpecial<glg_unit_t<KV, XV>> &sp) {
+    typedef glg_unit_t<KV, XV> T;
     const T co2Air = GLG_X(x, 0), co2Top = GLG_X(x, 1), tAir = GLG_X(x, 2), tTop = GLG_X(x, 3), vpAir = GLG_X(x, 15), vpTop = GLG_X(x, 16);
     const T tkAir = tAir + T(GLG_C2K), tkTop = tTop + T(GLG_C2K);
     const T ra[2] = {tkAir, tkTop};
@@ -307,7 +314,7 @@ GLG_HD double glg_stiffness(const KV &K, double aScr, double aVentRoof) {
 
 template <bool GENERAL, class KV, class CV, class P, class XV, class PT>
 GLG_HD void glg_unit_floor(const KV &K, const CV &C, const P &p, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     const T tAir = GLG_X(x, 2), tCan = GLG_X(x, 4), tFlr = GLG_X(x, 8), tLamp = GLG_X(x, 17);
     const T hLampAir = K[K_HLAMPAIR] * (tLamp - tAir);
     const T hCanAir = fabs(K[K_2ALFA] * (C[C_SLA] * GLG_X(x, 23))) * (tCan - tAir);
@@ -357,7 +364,7 @@ GLG_HD void glg_surface_core(T tA, T tS, T tB, T vpA, T coefA, T coefB, T invvp,
 // one screen (thermal: I_SCR = 7, blackout: I_SCR = 20): convection main air -> screen -> top compartment, condensation
 template <int I_SCR, class KV, class HV, class XV, class PT>
 GLG_HD void glg_unit_screen(const KV &K, const HV &H, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     T surf, air, far, vp;
     glg_surface_core<true, T>(GLG_X(x, 2), GLG_X(x, I_SCR), GLG_X(x, 3), GLG_X(x, 15), I_SCR == 7 ? H[H_17TH] : H[H_17BL],
                               I_SCR == 7 ? H[H_17TH] : H[H_17BL], K[K_INVVPAIR], K[K_L], surf, air, far, vp);
@@ -369,7 +376,7 @@ GLG_HD void glg_unit_screen(const KV &K, const HV &H, const XV &x, const PT &pt)
 
 template <class KV, class HV, class XV, class PT>
 GLG_HD void glg_unit_cover(const KV &K, const HV &H, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     T surf, air, far, vp;
     glg_surface_core<false, T>(GLG_X(x, 3), GLG_X(x, 5), T(0), GLG_X(x, 16), H[H_HECIN], T(0), K[K_INVVPTOP], K[K_L], surf, air, far, vp);
     pt.template put<5>(surf);
@@ -379,7 +386,7 @@ GLG_HD void glg_unit_cover(const KV &K, const HV &H, const XV &x, const PT &pt) 
 
 template <class KV, class CV, class HV, class XV, class PT>
 GLG_HD void glg_unit_transp(const KV &K, const CV &C, const HV &H, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     const T co2Air = GLG_X(x, 0), tAir = GLG_X(x, 2), tCan = GLG_X(x, 4), vpAir = GLG_X(x, 15);
     const T vpd = glg_satvp_f(tCan) - vpAir;
     const T lai = C[C_SLA] * GLG_X(x, 23);
@@ -393,7 +400,7 @@ GLG_HD void glg_unit_transp(const KV &K, const CV &C, const HV &H, const XV &x, 
 
 template <bool GENERAL, class KV, class CV, class HV, class XV, class PT>
 GLG_HD void glg_unit_photo(const KV &K, const CV &C, const HV &H, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     const T co2Air = GLG_X(x, 0), tAir = GLG_X(x, 2), tCan = GLG_X(x, 4), cBuf = GLG_X(x, 22);
     const T lai = C[C_SLA] * GLG_X(x, 23);
     const T j25 = lai * C[C_J25];
@@ -440,7 +447,7 @@ GLG_HD void glg_unit_photo(const KV &K, const CV &C, const HV &H, const XV &x, c
 
 template <class KV, class CV, class XV, class PT>
 GLG_HD void glg_unit_flows(const KV &K, const CV &C, const XV &x, const PT &pt) {
-    typedef glg_scalar_t<KV> T;
+    typedef glg_unit_t<KV, XV> T;
     const T tCan = GLG_X(x, 4), tCan24 = GLG_X(x, 21), cBuf = GLG_X(x, 22);
     const T gT24 = T(0.047) * tCan24 + T(0.06);
     const T ea[5] = {-T(1.1587) * (tCan24 - C[C_T24MIN]), T(1.3904) * (tCan24 - C[C_T24MAX]), -T(0.869) * (tCan - C[C_TCANMIN]),
@@ -470,8 +477,8 @@ GLG_HD void glg_unit_flows(const KV &K, const CV &C, const XV &x, const PT &pt) 
 }
 
 template <class KV, class CV, class XV, class PT>
-GLG_HD void glg_unit_maint(const KV &K, const CV &C, const XV &x, const PT &pt, GlgSpecial<glg_scalar_t<KV>> &sp) {
-    typedef glg_scalar_t<KV> T;
+GLG_HD void glg_unit_maint(const KV &K, const CV &C, const XV &x, const PT &pt, GlgSpecial<glg_unit_t<KV, XV>> &sp) {
+    typedef glg_unit_t<KV, XV> T;
     const T tCan24 = GLG_X(x, 21), cLeaf = GLG_X(x, 23), cStem = GLG_X(x, 24), cFruit = GLG_X(x, 25);
     const T kHar = T(2.0) * T(4.6052) / T(1e4);  // smoothHar(v, cutoff, 1e4, 5e4) = 5e4/(1+exp(-kHar (v-cutoff)))  (:75-79)
     const T ea[3] = {C[C_LNQ10X] * (tCan24 - 25), -kHar * (cLeaf - C[C_CLEAFMAX]), -kHar * (cFruit - C[C_CFRUITMAX])};
@@ -492,9 +499,9 @@ GLG_HD void glg_unit_maint(const KV &K, const CV &C, const XV &x, const PT &pt, 
 }
 
 // dispatcher: unit U with the argument set every unit can pick from
-template <int U, bool GENERAL, class KV, class CV, class HV, class P, class XV, class PT>
-GLG_HD void glg_unit(const KV &K, const CV &C, const HV &H, const P &p, const double *u, const XV &x, const PT &pt,
-                     GlgSpecial<glg_scalar_t<KV>> &sp) {
+template <int U, bool GENERAL, class KV, class CV, class HV, class P, class UT, class XV, class PT>
+GLG_HD void glg_unit(const KV &K, const CV &C, const HV &H, const P &p, const UT *u, const XV &x, const PT &pt,
+                     GlgSpecial<glg_unit_t<KV, XV>> &sp) {
     if (U == U_OPT) glg_unit_opt<GENERAL>(K, C, H, x, pt);
     else if (U == U_PIPES) glg_unit_pipes(K, C, x, pt, sp);
     else if (U == U_FIR) glg_unit_fir<GENERAL>(K, C, H, p, u, x, pt);
@@ -600,8 +607,8 @@ struct GlgWT {
 };
 
 // evaluates the units of group warp W in order, accumulating into v[28]; specials into sp
-template <int NG, int W, int Kk, bool GENERAL, class KV, class CV, class HV, class P, class XV, class T>
-GLG_HD void glg_run_warp_units(const KV &K, const CV &C, const HV &H, const P &p, const double *u, const XV &x, T *v,
+template <int NG, int W, int Kk, bool GENERAL, class KV, class CV, class HV, class P, class UT, class XV, class T>
+GLG_HD void glg_run_warp_units(const KV &K, const CV &C, const HV &H, const P &p, const UT *u, const XV &x, T *v,
                                GlgSpecial<T> &sp) {
     constexpr int U = glg_assign(NG).unit[W][Kk < GLG_MAXUNITS_PER_WARP ? Kk : 0];
     if constexpr (Kk < GLG_MAXUNITS_PER_WARP && U >= 0) {
@@ -610,4 +617,52 @@ GLG_HD void glg_run_warp_units(const KV &K, const CV &C, const HV &H, const P &p
         glg_unit<U, GENERAL>(K, C, H, p, u, x, pt, sp);
         glg_run_warp_units<NG, W, Kk + 1, GENERAL>(K, C, H, p, u, x, v, sp);
     }
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// One-lane RHS assembled from the units: S[i] = dx_i/dt for one env, generic in the scalar type (double, float, GlgDual).  The
+// units of each group warp of the NG-warp assignment are accumulated into that warp's partial sums, the partial sums are added in
+// warp order and the owners' capacity scales (glg_state_scale_index) are applied -- the data flow of the warp-specialised kernel,
+// in one thread (the sum order of tests/hostmath's hm_rhs_units).  Returns the transient-stiffness estimate of the graded
+// integrator, from value parts: it only feeds step-count decisions.
+template <class T>
+struct GlgArrayXT {  // plain array of scalar type T in state order
+    const T *p;
+    template <int I>
+    GLG_HD T at() const { return p[I]; }
+};
+template <int NG, int W, bool GENERAL, class KV, class CV, class HV, class P, class UT, class XV, class ST, class T>
+GLG_HD void glg_rhs_units_warps(const KV &K, const CV &C, const HV &H, const P &p, const UT *u, const XV &x, ST *sum, GlgSpecial<T> &sp) {
+    if constexpr (W < NG) {
+        T v[GLG_NX] = {};
+        glg_run_warp_units<NG, W, 0, GENERAL>(K, C, H, p, u, x, v, sp);
+        constexpr unsigned mask = GlgWT<NG, GENERAL>::t.states[W];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+        for (int i = 0; i < GLG_NX; ++i)
+            if (mask >> i & 1u) sum[i] += static_cast<ST>(v[i]);
+        glg_rhs_units_warps<NG, W + 1, GENERAL>(K, C, H, p, u, x, sum, sp);
+    }
+}
+template <bool GENERAL, int NG = U_COUNT, class KV, class CV, class HV, class P, class UT, class XV, class ST>
+GLG_HD double glg_rhs_units(const KV &K, const CV &C, const HV &H, const P &p, const UT *u, const XV &x, ST *S) {
+    typedef glg_unit_t<KV, XV> T;
+    ST sum[GLG_NX];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int i = 0; i < GLG_NX; ++i) sum[i] = ST(0.0);
+    GlgSpecial<T> sp{};
+    glg_rhs_units_warps<NG, 0, GENERAL>(K, C, H, p, u, x, sum, sp);
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int i = 0; i < GLG_NX; ++i) {
+        const int sk = glg_state_scale_index(i);
+        if (sk >= 0) S[i] = K[sk] * sum[i];
+        else if (sk == -1) S[i] = sum[i];
+        else S[i] = static_cast<ST>(sp.canscale) * sum[i];
+    }
+    return glg_stiffness(K, (double)glg_value(sp.ascr), (double)glg_value(sp.avent));
 }

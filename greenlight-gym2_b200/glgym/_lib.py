@@ -132,6 +132,10 @@ SIGNATURES = {
                                   C.c_int32, _VP]),
     "glg_evalf_batch_ex": (C.c_int, [_DP, _DP, _DP, _DP, C.c_int32, _DP, _U8P, C.c_int32, C.c_double, C.c_int32,
                                      C.c_int32, C.c_int32, _VP]),
+    "glg_rhs_jacobian_batch": (C.c_int, [_DP, _DP, _DP, _DP, C.c_int32, _DP, _DP, _DP, C.c_int32, C.c_int32, _VP]),
+    "glg_evalf_jacobian_batch": (C.c_int, [_DP, _DP, _DP, _DP, C.c_int32, _DP, _DP, _DP, _U8P, C.c_int32, C.c_double,
+                                           C.c_int32, C.c_int32, C.c_int32, _VP]),
+    "glg_linearize": (C.c_int, [C.c_void_p, _DP, _DP, _DP, _DP, _VP]),
     "glg_launch_count": (C.c_int64, [C.c_void_p]),
     "glg_measure_fp64_peak": (C.c_int, [C.c_int32, C.POINTER(C.c_double)]),
     "glg_measure_fp32_peak": (C.c_int, [C.c_int32, C.POINTER(C.c_double)]),

@@ -27,9 +27,7 @@ class GreenLight:
         self.device = int(device)
         self._lib = _lib.load()
 
-    def evalF_batch(self, x, u, d, p, return_bad=False):
-        """x [B,28], u [B,6], d [B,10], p [208] or [B,208]; torch CUDA float64 tensors or array-likes.
-        Returns x_next [B,28] as a CUDA float64 tensor."""
+    def _inputs(self, x, u, d, p):
         dev = torch.device("cuda", self.device)
         as_t = lambda a: torch.as_tensor(np.asarray(a, dtype=np.float64) if not torch.is_tensor(a) else a,
                                          dtype=torch.float64, device=dev).contiguous()
@@ -38,6 +36,12 @@ class GreenLight:
         assert x.shape == (B, 28) and u.shape == (B, 6) and d.shape == (B, 10)
         p_stride = 0 if p.dim() == 1 else _lib.NP
         assert p.shape[-1] == _lib.NP and (p.dim() == 1 or p.shape[0] == B)
+        return dev, x, u, d, p, B, p_stride
+
+    def evalF_batch(self, x, u, d, p, return_bad=False):
+        """x [B,28], u [B,6], d [B,10], p [208] or [B,208]; torch CUDA float64 tensors or array-likes.
+        Returns x_next [B,28] as a CUDA float64 tensor."""
+        dev, x, u, d, p, B, p_stride = self._inputs(x, u, d, p)
         out = torch.empty_like(x)
         bad = torch.zeros(B, dtype=torch.uint8, device=dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
@@ -46,6 +50,35 @@ class GreenLight:
                                           self.device, stream)
         _lib.check(rc, None, "glg_evalf_batch_ex")
         return (out, bad) if return_bad else out
+
+    def rhs_jacobian_batch(self, x, u, d, p):
+        """Continuous-time right-hand side and its exact Jacobians (forward-mode differentiation of the model, fp64).
+        Inputs as evalF_batch.  Returns (f [B,28], df/dx [B,28,28], df/du [B,28,6]) as CUDA float64 tensors."""
+        dev, x, u, d, p, B, p_stride = self._inputs(x, u, d, p)
+        f = torch.empty_like(x)
+        jx = torch.empty((B, 28, 28), dtype=torch.float64, device=dev)
+        ju = torch.empty((B, 28, 6), dtype=torch.float64, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = self._lib.glg_rhs_jacobian_batch(x.data_ptr(), u.data_ptr(), d.data_ptr(), p.data_ptr(), p_stride, f.data_ptr(),
+                                              jx.data_ptr(), ju.data_ptr(), B, self.device, stream)
+        _lib.check(rc, None, "glg_rhs_jacobian_batch")
+        return f, jx, ju
+
+    def jacobian_batch(self, x, u, d, p, return_bad=False):
+        """One control interval (evalF_batch) and its exact Jacobians on the executed integration grid.  Inputs as evalF_batch.
+        Returns (x_next [B,28], dx_next/dx [B,28,28], dx_next/du [B,28,6]) as CUDA float64 tensors, plus the uint8 [B]
+        non-finite flags when return_bad is set."""
+        dev, x, u, d, p, B, p_stride = self._inputs(x, u, d, p)
+        xn = torch.empty_like(x)
+        jx = torch.empty((B, 28, 28), dtype=torch.float64, device=dev)
+        ju = torch.empty((B, 28, 6), dtype=torch.float64, device=dev)
+        bad = torch.zeros(B, dtype=torch.uint8, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = self._lib.glg_evalf_jacobian_batch(x.data_ptr(), u.data_ptr(), d.data_ptr(), p.data_ptr(), p_stride, xn.data_ptr(),
+                                                jx.data_ptr(), ju.data_ptr(), bad.data_ptr(), B, self.dt, self.n_sub,
+                                                0 if self.integrator == "fixed" else 1, self.device, stream)
+        _lib.check(rc, None, "glg_evalf_jacobian_batch")
+        return (xn, jx, ju, bad) if return_bad else (xn, jx, ju)
 
     def evalF(self, x, u, d, p):
         """Single-env call with the reference's signature; returns a list of 28 floats. Raises RuntimeError if the

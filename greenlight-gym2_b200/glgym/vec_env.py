@@ -399,6 +399,25 @@ class GreenLightVecEnv(_VecEnvBase):
         _lib.check(self._lib.glg_rule_controls(self._h, s, self._rule_u.data_ptr(), self._stream()), self._h, "glg_rule_controls")
         return self._rule_u
 
+    def linearize_tensor(self, controls=None):
+        """Linearise the step `step_raw_control_tensor(controls)` would take from every env's current state, without taking it:
+        returns (x_next [B,28], A [B,28,28], Bu [B,28,6]) with A = dx_next/dx and Bu = dx_next/du, exact derivatives of the
+        integration on its executed grid.  controls: CUDA float64 [B, 6], or None for the envs' current u.  Always fp64 and the
+        nominal model (also for precision=1 and under parametric uncertainty); the env's state is not touched."""
+        c = 0
+        if controls is not None:
+            if tuple(controls.shape) != (self.num_envs, self.nu):
+                raise ValueError(f"controls must have shape ({self.num_envs}, {self.nu}); got {tuple(controls.shape)}")
+            controls = controls.to(device=self.device, dtype=torch.float64).contiguous()
+            c = controls.data_ptr()
+        B = self.num_envs
+        xn = torch.empty((B, 28), dtype=torch.float64, device=self.device)
+        A = torch.empty((B, 28, 28), dtype=torch.float64, device=self.device)
+        Bu = torch.empty((B, 28, self.nu), dtype=torch.float64, device=self.device)
+        _lib.check(self._lib.glg_linearize(self._h, c, xn.data_ptr(), A.data_ptr(), Bu.data_ptr(), self._stream()), self._h,
+                   "glg_linearize")
+        return xn, A, Bu
+
     def step_rule_based(self):
         self.step_rule_based_tensor()
         torch.cuda.synchronize(self.device)

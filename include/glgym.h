@@ -344,6 +344,25 @@ int glg_evalf_batch_ex(const double *x_dev, const double *u_dev, const double *d
                        double *x_next_dev, uint8_t *bad_dev, int32_t B, double dt, int32_t n_sub, int32_t integrator,
                        int32_t device, void *stream);
 
+/* Linearisation by forward-mode differentiation of the model (exact up to rounding, fp64).  All matrices are row-major float64,
+ * J[b][i][j] = d out_i / d in_j; inputs as glg_evalf_batch_ex (x[B][28], u[B][6], d[B][10], p shared (p_stride = 0) or [B][208]).
+ * Non-smooth points: fabs'(0) = 0; fmin / fmax / branches take the derivative of the branch the value takes; step-count decisions
+ * (harvest micro-steps, graded splits) are frozen at the values, so the result is the Jacobian of the map on the executed grid.
+ * Continuous-time RHS and its Jacobians: f_dev [B][28], jx_dev [B][28][28], ju_dev [B][28][6]; f_dev and ju_dev may be NULL. */
+int glg_rhs_jacobian_batch(const double *x_dev, const double *u_dev, const double *d_dev, const double *p_dev, int32_t p_stride,
+                           double *f_dev, double *jx_dev, double *ju_dev, int32_t B, int32_t device, void *stream);
+/* Derivative of glg_evalf_batch_ex: x_next_dev [B][28], jx_dev [B][28][28], ju_dev [B][28][6], bad_dev uint8 [B];
+ * x_next_dev, ju_dev and bad_dev may be NULL. */
+int glg_evalf_jacobian_batch(const double *x_dev, const double *u_dev, const double *d_dev, const double *p_dev, int32_t p_stride,
+                             double *x_next_dev, double *jx_dev, double *ju_dev, uint8_t *bad_dev, int32_t B, double dt,
+                             int32_t n_sub, int32_t integrator, int32_t device, void *stream);
+/* Linearise the step glg_step_raw_control(h, controls, NULL) would take, for every env of the handle, from its current state:
+ * controls_dev double [B][6] (NULL: the env's current u), the weather row the step reads, the handle's nominal parameters,
+ * dt, n_sub and integrator.  Always fp64 and the nominal model (also on a precision = 1 handle and under uncertainty_scale > 0).
+ * x_next_dev [B][28] and ju_dev [B][28][6] may be NULL.  Writes nothing of the handle's; one launch.  GLG_ERR_ARG on a NULL
+ * handle or NULL jx_dev, GLG_ERR_STATE before the first glg_reset. */
+int glg_linearize(glg_handle *h, const double *controls_dev, double *x_next_dev, double *jx_dev, double *ju_dev, void *stream);
+
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t glg_launch_count(const glg_handle *h);
 /* Measured FP64 FMA throughput of the device [FLOP/s] (dependent-chain-free DFMA loop, all SMs); the roofline
