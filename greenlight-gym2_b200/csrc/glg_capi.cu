@@ -27,6 +27,7 @@
 #include "glg_replay.cuh"
 #include "glg_plan.cuh"
 #include "glg_tangent.cuh"
+#include "glg_est.cuh"
 
 
 static thread_local std::string g_error = "";  // glg_last_error(NULL): the last failure of an entry point without a handle
@@ -1178,6 +1179,51 @@ extern "C" int64_t glg_replay_bytes(const glg_replay *r) { return r ? (int64_t)r
 extern "C" float *glg_replay_obs_dev(glg_replay *r) { return r ? r->obs_norm : nullptr; }
 extern "C" double *glg_replay_stats_dev(glg_replay *r) { return r ? r->norm.stat : nullptr; }
 
+// ---- the internal handle of a planner or an estimator ------------------------------------------------------
+// n envs that the unchanged step kernels advance from states their owner loads: the env's configuration except auto_reset 0,
+// uncertainty_scale 0 (nominal model), env_id_offset 0 and automatic kernel selection; obs_modules (NULL: the env's stack)
+// replaces the observation stack.  It counts as reset, since its owner loads every state before stepping, and it owns no
+// weather bank: companion_sync points it at the env's before every use.
+static int companion_create(glg_handle *h, int n, const int32_t *obs_modules, const char *what, std::unique_ptr<glg_handle> *out) {
+    glg_config pc = h->cfg;  // precision, integrator, n_sub, N, Np, prices and constraints stay the env's
+    pc.num_envs = n;
+    pc.auto_reset = 0;
+    pc.uncertainty_scale = 0.0;
+    pc.seed = h->a.seed;  // the env's current seed (glg_set_seed): StateObservations entries are keyed by it
+    pc.env_id_offset = 0;
+    pc.role_warps = 0;
+    pc.role_lanes = 0;
+    if (obs_modules) memcpy(pc.obs_modules, obs_modules, sizeof pc.obs_modules);
+    glg_handle *hs = nullptr;
+    const int rc = glg_create(&pc, &hs);
+    out->reset(hs);
+    if (rc != GLG_OK) {
+        h->err = std::string(what) + g_error;
+        return rc;
+    }
+    hs->is_reset = true;
+    return GLG_OK;
+}
+
+// Before every use: the env must be reset and still hold the bank generation `gen` the owner was created under; its parameters
+// (glg_set_params may have been called since) and bank pointers are copied into the internal handle.  Host fields only.
+static int companion_sync(glg_handle *h, glg_handle *hs, unsigned long long gen, const char *what, const char *kind) {
+    if (gen != h->weather_gen) {
+        h->err = std::string(what) + ": the weather bank was replaced (glg_set_weather) after this " + kind + " was created";
+        return GLG_ERR_STATE;
+    }
+    if (!h->is_reset) {
+        h->err = std::string(what) + ": the env has not been reset (glg_reset)";
+        return GLG_ERR_STATE;
+    }
+    hs->uni = h->uni;
+    hs->general = h->general;
+    hs->have_params = true;
+    hs->a.weather = h->a.weather; hs->a.start_day = h->a.start_day; hs->a.reset_tables = h->a.reset_tables;
+    hs->a.n_tables = h->a.n_tables; hs->a.rows = h->a.rows; hs->a.n_reset_tables = h->a.n_reset_tables;
+    return GLG_OK;
+}
+
 // ---- receding-horizon planner (glg_plan.cuh): its own object holding a second, internal handle of B K planning envs that the
 // unchanged step kernels advance; the env handle is only read ----
 struct glg_plan {
@@ -1228,23 +1274,11 @@ extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_pl
     p->cfg = c;
     p->B = h->a.B;
     p->BK = h->a.B * c.n_candidates;
-    glg_config pc = h->cfg;  // precision, integrator, n_sub, N, Np, prices, constraints and the observation stack stay the env's
-    pc.num_envs = p->BK;
-    pc.auto_reset = 0;
-    pc.uncertainty_scale = 0.0;
-    pc.seed = h->a.seed;  // the env's current seed (glg_set_seed): StateObservations entries are keyed by it
-    pc.env_id_offset = 0;
-    pc.role_warps = 0;
-    pc.role_lanes = 0;
-    glg_handle *hp = nullptr;
-    int rc = glg_create(&pc, &hp);
-    p->hp.reset(hp);
+    const int rc = companion_create(h, p->BK, nullptr, "glg_plan_create: planning handle: ", &p->hp);
     if (rc != GLG_OK) {
-        h->err = std::string("glg_plan_create: planning handle: ") + g_error;
         glg_plan_destroy(p);
         return rc;
     }
-    hp->is_reset = true;  // every run / evaluate loads its states (fan-out) before stepping
     const size_t HB6 = (size_t)c.horizon * p->B * GLG_NU, HBK6 = (size_t)c.horizon * p->BK * GLG_NU;
     cudaError_t e = p->mem.dev(&p->mean, HB6);
     if (e == cudaSuccess) e = p->mem.dev(&p->std, HB6);
@@ -1264,32 +1298,14 @@ extern "C" int glg_plan_create(glg_handle *h, const glg_plan_config *cfg, glg_pl
     return GLG_OK;
 }
 
-// Before every run / evaluate: the env must be reset and still hold the bank the planner was created under; its parameters
-// (glg_set_params may have been called since) and bank pointers are copied into the planning handle.  Host fields only.
-static int plan_sync(glg_plan *p, const char *what) {
-    glg_handle *h = p->h, *hp = p->hp.get();
-    if (p->weather_gen != h->weather_gen) {
-        h->err = std::string(what) + ": the weather bank was replaced (glg_set_weather) after this planner was created";
-        return GLG_ERR_STATE;
-    }
-    if (!h->is_reset) {
-        h->err = std::string(what) + ": the env has not been reset (glg_reset)";
-        return GLG_ERR_STATE;
-    }
-    hp->uni = h->uni;
-    hp->general = h->general;
-    hp->have_params = true;
-    hp->a.weather = h->a.weather; hp->a.start_day = h->a.start_day; hp->a.reset_tables = h->a.reset_tables;
-    hp->a.n_tables = h->a.n_tables; hp->a.rows = h->a.rows; hp->a.n_reset_tables = h->a.n_reset_tables;
-    return GLG_OK;
-}
+static int plan_sync(glg_plan *p, const char *what) { return companion_sync(p->h, p->hp.get(), p->weather_gen, what, "planner"); }
 
-static int plan_fanout(glg_plan *p, cudaStream_t s) {
+static int plan_fanout(glg_plan *p, const double *x, cudaStream_t s) {
     const GlgStepArgs &e = p->h->a, &pe = p->hp->a;
     GlgPlanFanArgs A;
     memset(&A, 0, sizeof A);
     A.B = p->B; A.K = p->cfg.n_candidates;
-    A.x = e.x; A.u = e.u; A.time = e.time; A.timestep = e.timestep; A.table = e.table; A.step_ctr = e.step_ctr;
+    A.x = x; A.u = e.u; A.time = e.time; A.timestep = e.timestep; A.table = e.table; A.step_ctr = e.step_ctr;
     A.px = pe.x; A.pu = pe.u; A.ptime = pe.time; A.pep_return = pe.ep_return; A.pep_info = pe.ep_info;
     A.ptimestep = pe.timestep; A.ptable = pe.table; A.pep_len = pe.ep_len; A.pstep_ctr = pe.step_ctr; A.pdone = pe.done;
     A.ret = p->ret; A.alive = p->alive;
@@ -1317,17 +1333,17 @@ static int plan_rollout(glg_plan *p, const float *seq, cudaStream_t s) {
     return GLG_OK;
 }
 
-extern "C" int glg_plan_run(glg_plan *p, float *actions_dev, void *stream) {
-    if (!p) return GLG_ERR_ARG;
+// glg_plan_run from the states x ([28][B] SoA); everything else of the planning envs' start comes from the env
+static int plan_run(glg_plan *p, const double *x, float *actions_dev, cudaStream_t s, const char *what) {
     glg_handle *h = p->h;
-    if (!actions_dev) return fail(h, GLG_ERR_ARG, "glg_plan_run: actions_dev is NULL");
-    int rc = plan_sync(p, "glg_plan_run");
+    if (!actions_dev) return fail(h, GLG_ERR_ARG, (std::string(what) + ": actions_dev is NULL").c_str());
+    if (!x) return fail(h, GLG_ERR_ARG, (std::string(what) + ": x_dev is NULL").c_str());
+    int rc = plan_sync(p, what);
     if (rc) return rc;
     GLG_CUDA(h, cudaSetDevice(p->device));
-    cudaStream_t s = (cudaStream_t)stream;
     const glg_plan_config &c = p->cfg;
     for (int it = 0; it < c.n_iterations; ++it) {
-        if ((rc = plan_fanout(p, s))) return rc;
+        if ((rc = plan_fanout(p, x, s))) return rc;
         GlgPlanSampleArgs S;
         memset(&S, 0, sizeof S);
         S.B = p->B; S.K = c.n_candidates; S.H = c.horizon; S.it = (uint32_t)it; S.call = p->calls; S.seed = c.seed;
@@ -1347,6 +1363,16 @@ extern "C" int glg_plan_run(glg_plan *p, float *actions_dev, void *stream) {
     return GLG_OK;
 }
 
+extern "C" int glg_plan_run(glg_plan *p, float *actions_dev, void *stream) {
+    if (!p) return GLG_ERR_ARG;
+    return plan_run(p, p->h->a.x, actions_dev, (cudaStream_t)stream, "glg_plan_run");
+}
+
+extern "C" int glg_plan_run_from(glg_plan *p, const double *x_dev, float *actions_dev, void *stream) {
+    if (!p) return GLG_ERR_ARG;
+    return plan_run(p, x_dev, actions_dev, (cudaStream_t)stream, "glg_plan_run_from");
+}
+
 extern "C" int glg_plan_evaluate(glg_plan *p, const float *seq_dev, double *returns_dev, void *stream) {
     if (!p) return GLG_ERR_ARG;
     glg_handle *h = p->h;
@@ -1355,7 +1381,7 @@ extern "C" int glg_plan_evaluate(glg_plan *p, const float *seq_dev, double *retu
     if (rc) return rc;
     GLG_CUDA(h, cudaSetDevice(p->device));
     cudaStream_t s = (cudaStream_t)stream;
-    if ((rc = plan_fanout(p, s))) return rc;
+    if ((rc = plan_fanout(p, h->a.x, s))) return rc;
     if ((rc = plan_rollout(p, seq_dev, s))) return rc;
     if (returns_dev != p->ret)
         GLG_CUDA(h, cudaMemcpyAsync(returns_dev, p->ret, (size_t)p->BK * sizeof(double), cudaMemcpyDeviceToDevice, s));
@@ -1376,6 +1402,141 @@ extern "C" float *glg_plan_mean_dev(glg_plan *p) { return p ? p->mean : nullptr;
 extern "C" float *glg_plan_std_dev(glg_plan *p) { return p ? p->std : nullptr; }
 extern "C" float *glg_plan_candidates_dev(glg_plan *p) { return p ? p->cand : nullptr; }
 extern "C" double *glg_plan_returns_dev(glg_plan *p) { return p ? p->ret : nullptr; }
+
+// ---- state estimation (glg_est.cuh): an unscented Kalman filter whose sigma points are the envs of an internal handle of B S
+// shadow envs (S = 57); the env handle is only read ----
+struct glg_est {
+    glg_handle *h = nullptr;  // the env whose states are estimated (read only; not on destruction: it may already be gone)
+    std::unique_ptr<glg_handle> hs;  // B S shadow envs: shadow env b S + i steps sigma point i of env b
+    int device = 0, B = 0;
+    unsigned long long weather_gen = 0;
+    bool is_reset = false;  // glg_est_reset has run
+    GlgEstArgs a = {};      // weights, variances and the estimator's buffers; the handles' pointers are set per call
+    CudaMem mem;
+};
+
+extern "C" void glg_est_destroy(glg_est *e) {
+    if (!e) return;
+    cudaSetDevice(e->device);
+    delete e;
+}
+
+extern "C" int glg_est_create(glg_handle *h, const glg_est_config *cfg, glg_est **out) {
+    if (!h || !cfg || !out) {
+        g_error = "glg_est_create: null argument";
+        return GLG_ERR_ARG;
+    }
+    *out = nullptr;
+    const glg_est_config &c = *cfg;
+    const int mask = c.meas_mask == 0 ? 0x7f : c.meas_mask;
+    if (mask < 0 || mask > 0x7f) return fail(h, GLG_ERR_ARG, "glg_est_create: meas_mask must be 0 (all 7) or a subset of bits 0..6");
+    const double n = GLG_NX, npl = c.alpha * c.alpha * (n + c.kappa);  // n + lambda
+    if (!(c.alpha > 0.0) || !isfinite(c.alpha) || !(c.beta >= 0.0) || !isfinite(c.beta) || !isfinite(c.kappa) || !(npl > 0.0) ||
+        !isfinite(npl))
+        return fail(h, GLG_ERR_ARG, "glg_est_create: need alpha > 0, beta >= 0, a finite kappa and n + lambda = alpha^2 (n + kappa) > 0");
+    for (int i = 0; i < GLG_NX; ++i)
+        if (!(c.p0_std[i] >= 0.0) || !isfinite(c.p0_std[i]) || !(c.q_std[i] >= 0.0) || !isfinite(c.q_std[i]))
+            return fail(h, GLG_ERR_ARG, "glg_est_create: p0_std and q_std must be finite and >= 0");
+    for (int r = 0; r < GLG_EST_NM; ++r)
+        if (!(c.r_std[r] >= 0.0) || !isfinite(c.r_std[r]) || ((mask >> r & 1) && !(c.r_std[r] > 0.0)))
+            return fail(h, GLG_ERR_ARG, "glg_est_create: r_std must be finite, >= 0, and > 0 for every measured entry");
+    if ((long long)h->a.B * GLG_EST_S > kPlanMaxBatch)
+        return fail(h, GLG_ERR_ARG, "glg_est_create: num_envs * 57 > 4194304 sigma points");
+    if (!h->have_params || !h->a.weather)
+        return fail(h, GLG_ERR_STATE, "glg_est_create: set the env's parameters and weather bank first");
+    GLG_CUDA(h, cudaSetDevice(h->cfg.device));
+    glg_est *e = new (std::nothrow) glg_est();
+    if (!e) return fail(h, GLG_ERR_ALLOC, "glg_est_create: out of host memory");
+    e->h = h;
+    e->device = h->cfg.device;
+    e->B = h->a.B;
+    GlgEstArgs &a = e->a;
+    a.B = e->B;
+    for (int r = 0; r < GLG_EST_NM; ++r)
+        if (mask >> r & 1) a.midx[a.m++] = r;
+    const double lambda = npl - n;
+    a.gamma = sqrt(npl);
+    a.wm0 = lambda / npl;
+    a.wc0 = a.wm0 + 1.0 - c.alpha * c.alpha + c.beta;
+    a.wi = 1.0 / (2.0 * npl);
+    for (int i = 0; i < GLG_NX; ++i) {
+        a.p0var[i] = c.p0_std[i] * c.p0_std[i];
+        a.qvar[i] = c.q_std[i] * c.q_std[i];
+    }
+    for (int r = 0; r < GLG_EST_NM; ++r) a.rvar[r] = c.r_std[r] * c.r_std[r];
+    // the smallest observation stack: nothing reads the shadow envs' rows
+    const int32_t climate_only[8] = {GLG_OBS_CLIMATE, 0, 0, 0, 0, 0, 0, 0};
+    int rc = companion_create(h, e->B * GLG_EST_S, climate_only, "glg_est_create: shadow handle: ", &e->hs);
+    if (rc != GLG_OK) {
+        glg_est_destroy(e);
+        return rc;
+    }
+    const size_t B = (size_t)e->B;
+    cudaError_t ce = e->mem.dev(&a.mean, GLG_NX * B);
+    if (ce == cudaSuccess) ce = e->mem.dev(&a.cov, GLG_EST_NX2 * B);
+    if (ce == cudaSuccess) ce = e->mem.dev(&a.innov, GLG_EST_NM * B);
+    if (ce == cudaSuccess) ce = e->mem.dev(&a.ctr, B);
+    if (ce == cudaSuccess) ce = e->mem.dev(&a.status, B);
+    if (ce == cudaSuccess) ce = e->mem.dev(&a.sctrl, GLG_NU * B * GLG_EST_S);
+    if (ce != cudaSuccess) {
+        glg_est_destroy(e);
+        return fail(h, GLG_ERR_CUDA, (std::string("glg_est_create: ") + cudaGetErrorString(ce)).c_str());
+    }
+    e->weather_gen = h->weather_gen;
+    *out = e;
+    return GLG_OK;
+}
+
+// the per-call fields of the kernels' arguments: env and shadow buffers, the env's season length and auto-reset mode
+static GlgEstArgs est_args(const glg_est *e) {
+    GlgEstArgs a = e->a;
+    const GlgStepArgs &h = e->h->a, &s = e->hs->a;
+    a.N = h.N; a.auto_reset = h.auto_reset; a.dt = h.dt;
+    a.x = h.x; a.u = h.u; a.time = h.time; a.timestep = h.timestep; a.table = h.table; a.step_ctr = h.step_ctr; a.done = h.done;
+    a.sx = s.x; a.stime = s.time; a.stimestep = s.timestep; a.stable = s.table; a.sdone = s.done;
+    return a;
+}
+
+extern "C" int glg_est_reset(glg_est *e, const double *x0_dev, void *stream) {
+    if (!e) return GLG_ERR_ARG;
+    glg_handle *h = e->h;
+    int rc = companion_sync(h, e->hs.get(), e->weather_gen, "glg_est_reset", "estimator");
+    if (rc) return rc;
+    GLG_CUDA(h, cudaSetDevice(e->device));
+    GlgEstArgs a = est_args(e);
+    a.x0 = x0_dev ? x0_dev : h->a.x;
+    glg_est_init_kernel<<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+    GLG_CUDA(h, cudaGetLastError());
+    e->is_reset = true;
+    return GLG_OK;
+}
+
+extern "C" int glg_est_update(glg_est *e, const double *y_dev, void *stream) {
+    if (!e) return GLG_ERR_ARG;
+    glg_handle *h = e->h, *hs = e->hs.get();
+    int rc = companion_sync(h, hs, e->weather_gen, "glg_est_update", "estimator");
+    if (rc) return rc;
+    if (!e->is_reset) return fail(h, GLG_ERR_STATE, "glg_est_update: the estimator has not been reset (glg_est_reset)");
+    GLG_CUDA(h, cudaSetDevice(e->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    GlgEstArgs a = est_args(e);
+    a.y = y_dev;
+    glg_est_sigma_kernel<<<e->B, GLG_EST_NT, 0, s>>>(a);
+    GLG_CUDA(h, cudaGetLastError());
+    if ((rc = glg_step_raw_control(hs, a.sctrl, nullptr, s))) {
+        h->err = "glg_est_update: shadow step: " + hs->err;
+        return rc;
+    }
+    glg_est_ut_kernel<<<e->B, GLG_EST_NT, 0, s>>>(a);
+    GLG_CUDA(h, cudaGetLastError());
+    return GLG_OK;
+}
+
+extern "C" double *glg_est_mean_dev(glg_est *e) { return e ? e->a.mean : nullptr; }
+extern "C" double *glg_est_cov_dev(glg_est *e) { return e ? e->a.cov : nullptr; }
+extern "C" double *glg_est_innovation_dev(glg_est *e) { return e ? e->a.innov : nullptr; }
+extern "C" double *glg_est_sigma_dev(glg_est *e) { return e ? e->hs->a.x : nullptr; }
+extern "C" uint8_t *glg_est_status_dev(glg_est *e) { return e ? e->a.status : nullptr; }
 
 // ---- episode-statistics all-reduce over NCCL (run-time binding: nccl_api above)
 extern "C" int glg_nccl_unique_id(uint8_t id_out[128]) {

@@ -172,11 +172,9 @@ __device__ __forceinline__ void glg_init_state(const double *w0, double *x) {
     x[27] = 0.;
 }
 
-// The 23 entries of the five per-env modules (observations.py:59-161) for state x, controls u, weather row w, timestep k
-// (pre-increment), day_of_year, hour_of_day, in the canonical order climate(4) crop(3) control(6) weather(5) time(5), fp64.
-__device__ __forceinline__ void glg_obs_head(const double *x, const double *u, const double *w, int k, double doy,
-                                             double hod, double *hd) {
-    const double two_pi = 2 * 3.14159265358979323846;
+// The 7 state-dependent observation entries: co2_air [ppm], temp_air, rh_air, pipe_temp (IndoorClimateObservations), 24CanTemp,
+// cFruit, tSum (BasicCropObservations).  Also the state estimator's measurement function h(x) (glg_est.cuh).
+__device__ __forceinline__ void glg_obs_state7(const double *x, double *hd) {
     hd[0] = glg_dens2ppm(x[2], x[0] * 1e-6);
     hd[1] = x[2];
     hd[2] = glg_rh(x[2], x[15]);
@@ -184,6 +182,14 @@ __device__ __forceinline__ void glg_obs_head(const double *x, const double *u, c
     hd[4] = x[21];
     hd[5] = x[25];
     hd[6] = x[26];
+}
+
+// The 23 entries of the five per-env modules (observations.py:59-161) for state x, controls u, weather row w, timestep k
+// (pre-increment), day_of_year, hour_of_day, in the canonical order climate(4) crop(3) control(6) weather(5) time(5), fp64.
+__device__ __forceinline__ void glg_obs_head(const double *x, const double *u, const double *w, int k, double doy,
+                                             double hod, double *hd) {
+    const double two_pi = 2 * 3.14159265358979323846;
+    glg_obs_state7(x, hd);
 #pragma unroll
     for (int i = 0; i < GLG_NU; ++i) hd[7 + i] = u[i];
     hd[13] = w[0];

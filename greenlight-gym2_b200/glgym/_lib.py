@@ -51,6 +51,12 @@ class GlgPlanConfig(C.Structure):
                 ("gamma", C.c_double), ("init_std", C.c_double), ("seed", C.c_uint64)]
 
 
+class GlgEstConfig(C.Structure):
+    """struct glg_est_config (include/glgym.h)."""
+    _fields_ = [("alpha", C.c_double), ("beta", C.c_double), ("kappa", C.c_double), ("meas_mask", C.c_int32), ("reserved", C.c_int32),
+                ("p0_std", C.c_double * NX), ("q_std", C.c_double * NX), ("r_std", C.c_double * 7)]
+
+
 class GlgEnvState(C.Structure):
     """struct glg_env_state (include/glgym.h): host pointers, NULL = skip."""
     _fields_ = [("x", C.c_void_p), ("u", C.c_void_p), ("timestep", C.c_void_p), ("table", C.c_void_p), ("time", C.c_void_p),
@@ -121,10 +127,20 @@ SIGNATURES = {
     "glg_plan_run": (C.c_int, [C.c_void_p, _FP, _VP]),
     "glg_plan_evaluate": (C.c_int, [C.c_void_p, _FP, _DP, _VP]),
     "glg_plan_shift": (C.c_int, [C.c_void_p, _VP]),
+    "glg_plan_run_from": (C.c_int, [C.c_void_p, _DP, _FP, _VP]),
     "glg_plan_mean_dev": (C.c_void_p, [C.c_void_p]),
     "glg_plan_std_dev": (C.c_void_p, [C.c_void_p]),
     "glg_plan_candidates_dev": (C.c_void_p, [C.c_void_p]),
     "glg_plan_returns_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_est_create": (C.c_int, [C.c_void_p, C.POINTER(GlgEstConfig), C.POINTER(C.c_void_p)]),
+    "glg_est_destroy": (None, [C.c_void_p]),
+    "glg_est_reset": (C.c_int, [C.c_void_p, _DP, _VP]),
+    "glg_est_update": (C.c_int, [C.c_void_p, _DP, _VP]),
+    "glg_est_mean_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_est_cov_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_est_innovation_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_est_sigma_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_est_status_dev": (C.c_void_p, [C.c_void_p]),
     "glg_nccl_unique_id": (C.c_int, [C.c_void_p]),
     "glg_nccl_init": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "glg_allreduce_stats": (C.c_int, [C.c_void_p, _VP]),

@@ -12,6 +12,7 @@ times, on a second handle of B * n_candidates planning envs; the env itself is o
 
 The planner uses the nominal model (no parametric uncertainty) and the weather bank as perfect weather over the horizon, which is
 the forecast the env observes as long as horizon <= Np.  `evaluate(seq)` scores caller-supplied sequences the same way.
+`plan(x)` plans from given states instead of the env's, e.g. a DeviceStateEstimator's estimate (output-feedback MPC).
 """
 import torch
 
@@ -35,11 +36,22 @@ class DevicePlanner(_EnvCompanion):
         self.returns = self._view(L.glg_plan_returns_dev(p), (B, K), "<f8")              # last roll-out's discounted returns
         self._actions = torch.empty((B, 6), dtype=torch.float32, device=env.device)
 
-    def plan(self):
-        """One decision from the env's current states: n_iterations CEM iterations; returns the new mean[0] as a float32 [B, 6]
-        tensor (overwritten by the next plan())."""
+    def plan(self, x=None):
+        """One decision: n_iterations CEM iterations from the env's current states, or from the states x (a float64 CUDA [B, 28]
+        tensor, e.g. a DeviceStateEstimator's `mean`, which is used without a copy; the env's controls, clock and timestep still
+        apply).  Returns the new mean[0] as a float32 [B, 6] tensor (overwritten by the next plan())."""
         p = self._live()
-        _lib.check(self._lib.glg_plan_run(p, self._actions.data_ptr(), self.env._stream()), self.env._h, "glg_plan_run")
+        if x is None:
+            _lib.check(self._lib.glg_plan_run(p, self._actions.data_ptr(), self.env._stream()), self.env._h, "glg_plan_run")
+            return self._actions
+        B = self.env.num_envs
+        if not (isinstance(x, torch.Tensor) and x.dtype == torch.float64 and x.device == self.env.device and tuple(x.shape) == (B, 28)):
+            raise ValueError(f"x must be a float64 tensor of shape [{B}, 28] on {self.env.device}")
+        xs = x.t()  # the C side reads [28][B]
+        if not xs.is_contiguous():
+            xs = xs.contiguous()
+        _lib.check(self._lib.glg_plan_run_from(p, xs.data_ptr(), self._actions.data_ptr(), self.env._stream()), self.env._h,
+                   "glg_plan_run_from")
         return self._actions
 
     def shift(self):

@@ -319,10 +319,71 @@ int glg_plan_run(glg_plan *p, float *actions_dev, void *stream);
 int glg_plan_evaluate(glg_plan *p, const float *seq_dev, double *returns_dev, void *stream);
 /* Receding horizon: mean[t] <- mean[t + 1], mean[H - 1] <- 0 (hold the current controls), std <- init_std. */
 int glg_plan_shift(glg_plan *p, void *stream);
+/* glg_plan_run from caller-given states x_dev double [28][B] (SoA, the layout of glg_state_dev; e.g. glg_est_mean_dev) instead of
+ * the env's x: output feedback.  u, timestep, table, clock and step_ctr still come from the env.  glg_plan_run(p, a, s) is
+ * glg_plan_run_from(p, glg_state_dev(env), a, s). */
+int glg_plan_run_from(glg_plan *p, const double *x_dev, float *actions_dev, void *stream);
 float *glg_plan_mean_dev(glg_plan *p);        /* float32 [H][B][6]; writeable (re-initialise the distribution) */
 float *glg_plan_std_dev(glg_plan *p);         /* float32 [H][B][6]; writeable */
 float *glg_plan_candidates_dev(glg_plan *p);  /* float32 [H][B K][6]: the last iteration's samples */
 double *glg_plan_returns_dev(glg_plan *p);    /* double [B K]: the last roll-out's returns */
+
+/* ---- state estimation: an unscented Kalman filter (UKF) over the envs' observations -------------------------------------------
+ * An estimator belongs to one env handle of B envs and keeps, per env, a state estimate x^ (double [28][B], the layout of
+ * glg_state_dev) and its covariance P (double [B][28][28]).  It owns a second, internal handle of B S shadow envs (S = 57; sigma
+ * point c = b S + i belongs to env b) created with the env's configuration except auto_reset 0, uncertainty_scale 0 (nominal
+ * model), env_id_offset 0, automatic kernel selection and the IndoorClimateObservations stack alone.  The env handle is only read.
+ * Filter contract (n = 28, S = 2n + 1 = 57):
+ *   Weights: scaled unscented transform with alpha > 0, beta >= 0, kappa and n + lambda > 0: lambda = alpha^2 (n + kappa) - n,
+ *     gamma = sqrt(n + lambda); Wm0 = lambda / (n + lambda), Wc0 = Wm0 + 1 - alpha^2 + beta; Wi = 1 / (2 (n + lambda)) for i >= 1.
+ *     Defaults: alpha = 1, beta = 2, kappa = 0.
+ *   Cholesky rule: P = L L^T column by column, summing over k in ascending order.  For column j, d = P[j][j] - sum_k L[j][k]^2; if
+ *     d <= 1e-12 P[j][j] (which includes P[j][j] = 0), column j of L is zero; otherwise L[j][j] = sqrt(d) and
+ *     L[i][j] = (P[i][j] - sum_k L[i][k] L[j][k]) / L[j][j].  (x27, the day counter, is deterministic: with p0_std[27] =
+ *     q_std[27] = 0 its variance is exactly 0.)
+ *   Sigma points: chi_0 = x^, chi_i = x^ + gamma L[:, i-1], chi_{n+i} = x^ - gamma L[:, i-1].
+ *   Predict: chi'_i is one control interval of the env's nominal model (the env's precision, integrator and n_sub) from chi_i, with
+ *     the controls the env just applied and the weather row the env's step just read.  xbar = sum Wm_i chi'_i,
+ *     P- = sum Wc_i (chi'_i - xbar)(chi'_i - xbar)^T + diag(q_std^2); sums over i in ascending order.
+ *   Measurement: h(x) = the 7 state-dependent observation entries in glg_obs_head order (co2_air ppm = dens2ppm(x2, 1e-6 x0), x2,
+ *     rh(x2, x15), x9, x21, x25, x26: co2_air, temp_air, rh_air, pipe_temp, 24CanTemp, cFruit, tSum); meas_mask selects the measured
+ *     subset M (bit r = entry r; 0 = all 7).  Additive-noise UKF on the propagated points, no redraw after adding Q:
+ *     Y_i = h_M(chi'_i), ybar = sum Wm_i Y_i, S = sum Wc_i (Y_i - ybar)(Y_i - ybar)^T + diag(r_std_M^2),
+ *     C = sum Wc_i (chi'_i - xbar)(Y_i - ybar)^T, K = C S^-1 (through the Cholesky of S), x^ = xbar + K (y - ybar),
+ *     P = sym(P- - K S K^T), sym(A) = (A + A^T) / 2.  Without a measurement (y_dev NULL): x^ = xbar, P = P-.
+ *   Episodes, read from the env handle after its step: the interval is the one at the env's pre-step timestep (timestep - 1; weather
+ *     row min(k, rows - Np - 1) as in the step kernels) with the env's u and table.  An env that finished under auto_reset
+ *     restarts: x^ <- the env's new state, P <- diag(p0_std^2).  The reset state is init_state(d0), a known function of the
+ *     weather table, so the restart uses no privileged information.
+ *   Status (uint8 bit flags per env, rewritten by every glg_est_update):
+ *     1  a sigma point's step was non-finite (its shadow env is done while the pre-step timestep is < N): x^ and P unchanged;
+ *     2  S is not positive definite: the prediction is kept, the update skipped;
+ *     4  re-initialised by an auto-reset;
+ *     8  the env's step_ctr is not the recorded value + 1 (the env was stepped or reset other than once since the last
+ *        glg_est_update / glg_est_reset; the new value is recorded): x^ and P unchanged.
+ * glg_set_weather on the env invalidates the estimator (GLG_ERR_STATE).  Errors are reported through glg_last_error of the env
+ * handle.  The estimator may be destroyed before or after its env handle. */
+typedef struct glg_est_config {
+    double alpha, beta, kappa;
+    int32_t meas_mask, reserved;
+    double p0_std[28], q_std[28], r_std[7]; /* >= 0, finite; r_std > 0 for every measured entry */
+} glg_est_config;
+typedef struct glg_est glg_est;
+/* GLG_ERR_ARG for NULLs, a bad configuration or num_envs * 57 > 4194304; GLG_ERR_STATE before the env has params and weather. */
+int glg_est_create(glg_handle *h, const glg_est_config *cfg, glg_est **out);
+void glg_est_destroy(glg_est *e);
+/* x^ <- x0_dev (double [28][B] SoA; NULL = the env's x), P <- diag(p0_std^2), innovation 0, status 0, and the env's step_ctr
+ * recorded.  GLG_ERR_STATE before the env's first glg_reset.  One launch. */
+int glg_est_reset(glg_est *e, const double *x0_dev, void *stream);
+/* After each step of the env: predict over the interval the env just took, then update with y_dev double [B][7] (entries in h
+ * order; unmeasured ones are not read) or, when y_dev is NULL, predict only.  GLG_ERR_STATE before glg_est_reset.  Three launches:
+ * the sigma kernel, glg_step_raw_control of the shadow handle, the UT kernel. */
+int glg_est_update(glg_est *e, const double *y_dev, void *stream);
+double *glg_est_mean_dev(glg_est *e);        /* [28][B], same layout as glg_state_dev */
+double *glg_est_cov_dev(glg_est *e);         /* [B][28][28] */
+double *glg_est_innovation_dev(glg_est *e);  /* [B][7]: y - ybar, 0 where not measured or not updated */
+double *glg_est_sigma_dev(glg_est *e);       /* [28][B*57]: the propagated sigma points (the shadow handle's x) */
+uint8_t *glg_est_status_dev(glg_est *e);     /* [B] */
 
 /* Multi-GPU episode statistics (SURVEY 8e): the step path has no collective; the one exchange is a sum of the 16-entry
  * statistics vector over the ranks' handles, once per logging interval -- ncclAllReduce on the handle's device buffer.
