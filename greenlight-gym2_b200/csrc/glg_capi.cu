@@ -28,6 +28,7 @@
 #include "glg_plan.cuh"
 #include "glg_tangent.cuh"
 #include "glg_est.cuh"
+#include "glg_smooth.cuh"
 
 
 static thread_local std::string g_error = "";  // glg_last_error(NULL): the last failure of an entry point without a handle
@@ -1413,10 +1414,29 @@ struct glg_est {
     bool is_reset = false;  // glg_est_reset has run
     GlgEstArgs a = {};      // weights, variances and the estimator's buffers; the handles' pointers are set per call
     CudaMem mem;
+    glg_smooth *sm = nullptr;  // the smoother recording this estimator's estimates, if any
+};
+
+// ---- state smoothing (glg_smooth.cuh): an unscented RTS smoother over a ring of the estimator's last W estimates, recorded by
+// the RECORD instantiations of the estimator's kernels ----
+struct glg_smooth {
+    glg_est *e = nullptr;  // the estimator recorded; cleared when the estimator is destroyed first
+    int device = 0, B = 0, W = 0;
+    long long count = 0;   // slots written since the estimator's last glg_est_reset; 0 = nothing recorded yet
+    unsigned int active = 0;  // bit j: state j is not deterministic (p0_std[j] or q_std[j] > 0)
+    // the record, ring order: [W][28][B] means, [W][B][28][28] matrices, [W][B] status and timestep
+    double *mean = nullptr, *xbar = nullptr, *cov = nullptr, *pm = nullptr, *d = nullptr;
+    unsigned char *status = nullptr;
+    int *timestep = nullptr;
+    double *lfac = nullptr;  // [B][28][28] the sigma kernel's factor, read by the UT kernel
+    // glg_smooth_run's output, oldest first
+    double *s_mean = nullptr, *s_cov = nullptr, *gain = nullptr;
+    CudaMem mem;
 };
 
 extern "C" void glg_est_destroy(glg_est *e) {
     if (!e) return;
+    if (e->sm) e->sm->e = nullptr;
     cudaSetDevice(e->device);
     delete e;
 }
@@ -1497,6 +1517,19 @@ static GlgEstArgs est_args(const glg_est *e) {
     return a;
 }
 
+// The record fields of the kernels' arguments: ring slot `slot` of the smoother's record
+static void smooth_slot(const glg_smooth *m, long long slot, GlgEstArgs *a) {
+    const size_t r = (size_t)slot, B = (size_t)m->B;
+    a->lfac = m->lfac;
+    a->r_mean = m->mean + r * GLG_NX * B;
+    a->r_xbar = m->xbar + r * GLG_NX * B;
+    a->r_cov = m->cov + r * GLG_EST_NX2 * B;
+    a->r_pm = m->pm + r * GLG_EST_NX2 * B;
+    a->r_d = m->d + r * GLG_EST_NX2 * B;
+    a->r_status = m->status + r * B;
+    a->r_timestep = m->timestep + r * B;
+}
+
 extern "C" int glg_est_reset(glg_est *e, const double *x0_dev, void *stream) {
     if (!e) return GLG_ERR_ARG;
     glg_handle *h = e->h;
@@ -1505,9 +1538,15 @@ extern "C" int glg_est_reset(glg_est *e, const double *x0_dev, void *stream) {
     GLG_CUDA(h, cudaSetDevice(e->device));
     GlgEstArgs a = est_args(e);
     a.x0 = x0_dev ? x0_dev : h->a.x;
-    glg_est_init_kernel<<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+    if (e->sm) {  // a reset starts the smoother's record over: it writes slot 0
+        smooth_slot(e->sm, 0, &a);
+        glg_est_init_kernel<true><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+    } else {
+        glg_est_init_kernel<false><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+    }
     GLG_CUDA(h, cudaGetLastError());
     e->is_reset = true;
+    if (e->sm) e->sm->count = 1;
     return GLG_OK;
 }
 
@@ -1521,14 +1560,19 @@ extern "C" int glg_est_update(glg_est *e, const double *y_dev, void *stream) {
     cudaStream_t s = (cudaStream_t)stream;
     GlgEstArgs a = est_args(e);
     a.y = y_dev;
-    glg_est_sigma_kernel<<<e->B, GLG_EST_NT, 0, s>>>(a);
+    glg_smooth *m = e->sm && e->sm->count > 0 ? e->sm : nullptr;  // a smoother records from the first reset after its creation
+    if (m) smooth_slot(m, m->count % m->W, &a);
+    if (m) glg_est_sigma_kernel<true><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    else glg_est_sigma_kernel<false><<<e->B, GLG_EST_NT, 0, s>>>(a);
     GLG_CUDA(h, cudaGetLastError());
     if ((rc = glg_step_raw_control(hs, a.sctrl, nullptr, s))) {
         h->err = "glg_est_update: shadow step: " + hs->err;
         return rc;
     }
-    glg_est_ut_kernel<<<e->B, GLG_EST_NT, 0, s>>>(a);
+    if (m) glg_est_ut_kernel<true><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    else glg_est_ut_kernel<false><<<e->B, GLG_EST_NT, 0, s>>>(a);
     GLG_CUDA(h, cudaGetLastError());
+    if (m) ++m->count;
     return GLG_OK;
 }
 
@@ -1537,6 +1581,86 @@ extern "C" double *glg_est_cov_dev(glg_est *e) { return e ? e->a.cov : nullptr; 
 extern "C" double *glg_est_innovation_dev(glg_est *e) { return e ? e->a.innov : nullptr; }
 extern "C" double *glg_est_sigma_dev(glg_est *e) { return e ? e->hs->a.x : nullptr; }
 extern "C" uint8_t *glg_est_status_dev(glg_est *e) { return e ? e->a.status : nullptr; }
+
+extern "C" void glg_smooth_destroy(glg_smooth *m) {
+    if (!m) return;
+    if (m->e) m->e->sm = nullptr;
+    cudaSetDevice(m->device);
+    delete m;
+}
+
+extern "C" int glg_smooth_create(glg_est *e, int32_t window, glg_smooth **out) {
+    if (!e || !out) {
+        g_error = "glg_smooth_create: null argument";
+        return GLG_ERR_ARG;
+    }
+    *out = nullptr;
+    glg_handle *h = e->h;
+    if (window < 2) return fail(h, GLG_ERR_ARG, "glg_smooth_create: window must be >= 2");
+    if (e->sm) return fail(h, GLG_ERR_STATE, "glg_smooth_create: the estimator already has a smoother");
+    GLG_CUDA(h, cudaSetDevice(e->device));
+    glg_smooth *m = new (std::nothrow) glg_smooth();
+    if (!m) return fail(h, GLG_ERR_ALLOC, "glg_smooth_create: out of host memory");
+    m->device = e->device;
+    m->B = e->B;
+    m->W = window;
+    for (int j = 0; j < GLG_NX; ++j)
+        if (e->a.p0var[j] > 0.0 || e->a.qvar[j] > 0.0) m->active |= 1u << j;
+    const size_t B = (size_t)m->B, WB = (size_t)window * B;
+    cudaError_t ce = m->mem.dev(&m->mean, GLG_NX * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->xbar, GLG_NX * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->cov, GLG_EST_NX2 * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->pm, GLG_EST_NX2 * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->d, GLG_EST_NX2 * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->status, WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->timestep, WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->lfac, GLG_EST_NX2 * B);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->s_mean, GLG_NX * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->s_cov, GLG_EST_NX2 * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->gain, GLG_EST_NX2 * WB);
+    if (ce != cudaSuccess) {
+        glg_smooth_destroy(m);
+        return fail(h, GLG_ERR_CUDA, (std::string("glg_smooth_create: ") + cudaGetErrorString(ce)).c_str());
+    }
+    m->e = e;
+    e->sm = m;
+    *out = m;
+    return GLG_OK;
+}
+
+extern "C" int32_t glg_smooth_length(const glg_smooth *m) { return m ? (int32_t)(m->count < m->W ? m->count : m->W) : 0; }
+extern "C" int32_t glg_smooth_first(const glg_smooth *m) { return m && m->count > m->W ? (int32_t)(m->count % m->W) : 0; }
+
+extern "C" int glg_smooth_run(glg_smooth *m, void *stream) {
+    if (!m) return GLG_ERR_ARG;
+    if (!m->e) {
+        g_error = "glg_smooth_run: the smoother's estimator was destroyed";
+        return GLG_ERR_STATE;
+    }
+    glg_handle *h = m->e->h;
+    if (m->count == 0)
+        return fail(h, GLG_ERR_STATE, "glg_smooth_run: nothing recorded yet (glg_est_reset after glg_smooth_create starts the record)");
+    GLG_CUDA(h, cudaSetDevice(m->device));
+    GlgSmoothArgs a = {};
+    a.B = m->B; a.W = m->W; a.len = glg_smooth_length(m); a.first = glg_smooth_first(m); a.active = m->active;
+    a.mean = m->mean; a.xbar = m->xbar; a.cov = m->cov; a.pm = m->pm; a.d = m->d; a.status = m->status;
+    a.s_mean = m->s_mean; a.s_cov = m->s_cov; a.gain = m->gain;
+    glg_smooth_kernel<<<m->B, GLG_SMOOTH_NT, 0, (cudaStream_t)stream>>>(a);
+    GLG_CUDA(h, cudaGetLastError());
+    return GLG_OK;
+}
+
+extern "C" int64_t glg_smooth_bytes(const glg_smooth *m) { return m ? (int64_t)m->mem.bytes() : 0; }
+extern "C" double *glg_smooth_mean_dev(glg_smooth *m) { return m ? m->s_mean : nullptr; }
+extern "C" double *glg_smooth_cov_dev(glg_smooth *m) { return m ? m->s_cov : nullptr; }
+extern "C" double *glg_smooth_gain_dev(glg_smooth *m) { return m ? m->gain : nullptr; }
+extern "C" double *glg_smooth_filtered_mean_dev(glg_smooth *m) { return m ? m->mean : nullptr; }
+extern "C" double *glg_smooth_filtered_cov_dev(glg_smooth *m) { return m ? m->cov : nullptr; }
+extern "C" double *glg_smooth_prior_mean_dev(glg_smooth *m) { return m ? m->xbar : nullptr; }
+extern "C" double *glg_smooth_prior_cov_dev(glg_smooth *m) { return m ? m->pm : nullptr; }
+extern "C" double *glg_smooth_cross_dev(glg_smooth *m) { return m ? m->d : nullptr; }
+extern "C" uint8_t *glg_smooth_status_dev(glg_smooth *m) { return m ? m->status : nullptr; }
+extern "C" int32_t *glg_smooth_timestep_dev(glg_smooth *m) { return m ? m->timestep : nullptr; }
 
 // ---- episode-statistics all-reduce over NCCL (run-time binding: nccl_api above)
 extern "C" int glg_nccl_unique_id(uint8_t id_out[128]) {

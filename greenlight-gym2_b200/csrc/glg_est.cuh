@@ -8,6 +8,8 @@
 //                          controls array [B S][6], and the pre-step timestep, table and clock of the env into its shadow envs.
 //   glg_est_ut_kernel    : one CTA per env.  Mean and covariance of the propagated points, measurement points h(chi'), S, C, the
 //                          m x m Cholesky solve and the posterior.  All sums run in ascending index order; no atomics.
+// Each kernel takes RECORD: the <true> instantiations also write one slot of a smoother's forward record (glg_smooth.cuh) and are
+// launched only for an estimator with a smoother; the <false> ones are the filter alone.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -45,7 +47,45 @@ struct GlgEstArgs {
     double *innov;       // [B][7]
     unsigned int *ctr;   // [B] the env's step counter at the last reset / update
     unsigned char *status;
+    // RECORD kernels only: the sigma kernel's factor, and the slot of the smoother's record this reset / update writes.  Kept
+    // last, so the fields above sit at the same parameter offsets in every instantiation.
+    double *lfac;                          // [B][28][28] L of the last sigma kernel, zero above the diagonal
+    double *r_mean, *r_xbar;               // [28][B] filtered mean, xbar
+    double *r_cov, *r_pm, *r_d;            // [B][28][28] filtered P, P-, D
+    unsigned char *r_status;               // [B]
+    int *r_timestep;                       // [B]
 };
+
+// A slot without a one-interval prediction behind it (a reset, status 1, 4 or 8): the filtered mean and covariance as they stand
+// after this kernel, xbar = P- = D = 0, and the status and timestep.  Each thread copies entries it alone wrote, if any.
+__device__ __forceinline__ void glg_est_record_start(const GlgEstArgs &A, int b, unsigned char status) {
+    const int B = A.B;
+    const size_t pb = (size_t)b * GLG_EST_NX2;
+    for (int o = threadIdx.x; o < GLG_EST_NX2; o += blockDim.x) {
+        A.r_cov[pb + o] = A.cov[pb + o];
+        A.r_pm[pb + o] = 0.0;
+        A.r_d[pb + o] = 0.0;
+    }
+    for (int i = threadIdx.x; i < GLG_NX; i += blockDim.x) {
+        A.r_mean[(size_t)i * B + b] = A.mean[(size_t)i * B + b];
+        A.r_xbar[(size_t)i * B + b] = 0.0;
+    }
+    if (threadIdx.x == 0) {
+        A.r_status[b] = status;
+        A.r_timestep[b] = A.timestep[b];
+    }
+}
+
+// A slot whose estimate is the prediction (predict only, or status 2): mean xbar and covariance P-, and the status and timestep
+__device__ __forceinline__ void glg_est_record_posterior(const GlgEstArgs &A, int b, const double *xbar,
+                                                        const double (*Pm)[GLG_NX + 1]) {
+    if (threadIdx.x < GLG_NX) A.r_mean[(size_t)threadIdx.x * A.B + b] = xbar[threadIdx.x];
+    for (int o = threadIdx.x; o < GLG_EST_NX2; o += blockDim.x) A.r_cov[(size_t)b * GLG_EST_NX2 + o] = Pm[o / GLG_NX][o % GLG_NX];
+    if (threadIdx.x == 0) {
+        A.r_status[b] = A.status[b];
+        A.r_timestep[b] = A.timestep[b];
+    }
+}
 
 // mean <- src, P <- diag(p0var), innovation 0, for env b; the block's threads share the 784 entries of P
 __device__ __forceinline__ void glg_est_restart(const GlgEstArgs &A, int b, const double *src) {
@@ -59,6 +99,7 @@ __device__ __forceinline__ void glg_est_restart(const GlgEstArgs &A, int b, cons
     for (int r = threadIdx.x; r < GLG_EST_NM; r += blockDim.x) A.innov[(size_t)b * GLG_EST_NM + r] = 0.0;
 }
 
+template <bool RECORD>
 __global__ void __launch_bounds__(GLG_EST_NT) glg_est_init_kernel(const __grid_constant__ GlgEstArgs A) {
     const int b = blockIdx.x;
     glg_est_restart(A, b, A.x0);
@@ -66,8 +107,10 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_init_kernel(const __grid_c
         A.ctr[b] = A.step_ctr[b];
         A.status[b] = 0;
     }
+    if constexpr (RECORD) glg_est_record_start(A, b, 0);
 }
 
+template <bool RECORD>
 __global__ void __launch_bounds__(GLG_EST_NT) glg_est_sigma_kernel(const __grid_constant__ GlgEstArgs A) {
     __shared__ double L[GLG_NX][GLG_NX + 1];  // P's lower triangle, factored in place
     __shared__ double xh[GLG_NX];
@@ -130,8 +173,15 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_sigma_kernel(const __grid_
         A.stime[BS + c0 + t] = fmod(A.time[(size_t)B + b] - fmod(A.dt / 3600.0, 24.0) + 24.0, 24.0);
     }
     for (int o = t; o < GLG_EST_S * GLG_NU; o += GLG_EST_NT) A.sctrl[c0 * GLG_NU + o] = A.u[(size_t)(o % GLG_NU) * B + b];
+    if constexpr (RECORD) {  // L for the UT kernel's D; both branches above end in a barrier
+        for (int o = t; o < GLG_EST_NX2; o += GLG_EST_NT) {
+            const int i = o / GLG_NX, j = o - i * GLG_NX;
+            A.lfac[(size_t)b * GLG_EST_NX2 + o] = j <= i ? L[i][j] : 0.0;
+        }
+    }
 }
 
+template <bool RECORD>
 __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_constant__ GlgEstArgs A) {
     __shared__ double X[GLG_EST_S][GLG_NX + 1];      // propagated points, then their deviations from the mean
     __shared__ double Y[GLG_EST_S][GLG_EST_NM + 1];  // measurement points, then their deviations
@@ -143,13 +193,17 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
     __shared__ int s_pd;
     const int b = blockIdx.x, t = threadIdx.x, B = A.B, m = A.m;
     const size_t BS = (size_t)B * GLG_EST_S, c0 = (size_t)b * GLG_EST_S;
-    if (A.status[b] & (GLG_EST_REINIT | GLG_EST_OUT_OF_STEP)) return;  // uniform over the CTA
+    if (A.status[b] & (GLG_EST_REINIT | GLG_EST_OUT_OF_STEP)) {  // uniform over the CTA
+        if constexpr (RECORD) glg_est_record_start(A, b, A.status[b]);
+        return;
+    }
     double *innov = A.innov + (size_t)b * GLG_EST_NM;
     // a sigma point's step failed: the shadow env ended before the season did
     const int bad = __syncthreads_or(t < GLG_EST_S && A.sdone[c0 + t] && A.timestep[b] - 1 < A.N);
     if (bad) {
         if (t == 0) A.status[b] |= GLG_EST_NONFINITE;
         if (t < GLG_EST_NM) innov[t] = 0.0;
+        if constexpr (RECORD) glg_est_record_start(A, b, A.status[b] | GLG_EST_NONFINITE);
         return;
     }
     for (int o = t; o < GLG_EST_S * GLG_NX; o += GLG_EST_NT) {
@@ -172,6 +226,7 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
         double s = A.wm0 * X[0][t];
         for (int k = 1; k < GLG_EST_S; ++k) s += A.wi * X[k][t];
         xbar[t] = s;
+        if constexpr (RECORD) A.r_xbar[(size_t)t * B + b] = s;
     } else if (t >= 32 && t < 32 + m) {
         const int r = t - 32;
         double s = A.wm0 * Y[0][r];
@@ -197,6 +252,24 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
         if (i == j) s += A.qvar[i];
         Pm[i][j] = s;
         Pm[j][i] = s;
+        if constexpr (RECORD) {
+            A.r_pm[(size_t)b * GLG_EST_NX2 + o] = s;
+            A.r_pm[(size_t)b * GLG_EST_NX2 + j * GLG_NX + i] = s;
+        }
+    }
+    if constexpr (RECORD) {
+        // D = sum_{i >= 1} Wc_i (chi_i - x^)(chi'_i - xbar)^T with chi_i - x^ = +-gamma L[:, i-1], the product the sigma kernel
+        // added (the i = 0 term is zero); written to the slot as formed
+        const double *Lb = A.lfac + (size_t)b * GLG_EST_NX2;
+        for (int o = t; o < GLG_EST_NX2; o += GLG_EST_NT) {
+            const int i = o / GLG_NX, j = o - i * GLG_NX;
+            double s = 0.0;
+            for (int k = 1; k < GLG_EST_S; ++k) {
+                const double off = __dmul_rn(k <= GLG_NX ? A.gamma : -A.gamma, Lb[i * GLG_NX + (k - 1) % GLG_NX]);
+                s += A.wi * (off * X[k][j]);
+            }
+            A.r_d[(size_t)b * GLG_EST_NX2 + o] = s;
+        }
     }
     for (int o = t; o < m * m + GLG_NX * m; o += GLG_EST_NT) {
         if (o < m * m) {
@@ -220,6 +293,7 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
         if (t < GLG_NX) A.mean[(size_t)t * B + b] = xbar[t];
         if (t < GLG_EST_NM) innov[t] = 0.0;
         for (int o = t; o < GLG_EST_NX2; o += GLG_EST_NT) P[o] = Pm[o / GLG_NX][o % GLG_NX];
+        if constexpr (RECORD) glg_est_record_posterior(A, b, xbar, Pm);
         return;
     }
     if (t == 0) {  // S = Ls Ls^T (plain Cholesky: d <= 0 or non-finite means S is not positive definite); innovation y - ybar
@@ -248,6 +322,7 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
     if (!s_pd) {  // keep the prediction
         if (t < GLG_NX) A.mean[(size_t)t * B + b] = xbar[t];
         for (int o = t; o < GLG_EST_NX2; o += GLG_EST_NT) P[o] = Pm[o / GLG_NX][o % GLG_NX];
+        if constexpr (RECORD) glg_est_record_posterior(A, b, xbar, Pm);
         return;
     }
     if (t < GLG_NX) {
@@ -266,6 +341,7 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
         double xn = xbar[t];
         for (int r = 0; r < m; ++r) xn += z[r] * v[r];
         A.mean[(size_t)t * B + b] = xn;
+        if constexpr (RECORD) A.r_mean[(size_t)t * B + b] = xn;
         for (int a = 0; a < m; ++a) {
             double s = 0.0;
             for (int q = 0; q < m; ++q) s += Sm[a][q] * z[q];
@@ -281,6 +357,14 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
             kij += Km[i][a] * Cm[j][a];
             kji += Km[j][a] * Cm[i][a];
         }
-        P[o] = 0.5 * ((Pm[i][j] - kij) + (Pm[j][i] - kji));
+        const double p = 0.5 * ((Pm[i][j] - kij) + (Pm[j][i] - kji));
+        P[o] = p;
+        if constexpr (RECORD) A.r_cov[(size_t)b * GLG_EST_NX2 + o] = p;
+    }
+    if constexpr (RECORD) {
+        if (t == 0) {
+            A.r_status[b] = A.status[b];
+            A.r_timestep[b] = A.timestep[b];
+        }
     }
 }

@@ -141,6 +141,22 @@ SIGNATURES = {
     "glg_est_innovation_dev": (C.c_void_p, [C.c_void_p]),
     "glg_est_sigma_dev": (C.c_void_p, [C.c_void_p]),
     "glg_est_status_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_create": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_void_p)]),
+    "glg_smooth_destroy": (None, [C.c_void_p]),
+    "glg_smooth_run": (C.c_int, [C.c_void_p, _VP]),
+    "glg_smooth_length": (C.c_int32, [C.c_void_p]),
+    "glg_smooth_first": (C.c_int32, [C.c_void_p]),
+    "glg_smooth_bytes": (C.c_int64, [C.c_void_p]),
+    "glg_smooth_mean_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_cov_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_gain_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_filtered_mean_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_filtered_cov_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_prior_mean_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_prior_cov_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_cross_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_status_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_smooth_timestep_dev": (C.c_void_p, [C.c_void_p]),
     "glg_nccl_unique_id": (C.c_int, [C.c_void_p]),
     "glg_nccl_init": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "glg_allreduce_stats": (C.c_int, [C.c_void_p, _VP]),

@@ -25,7 +25,20 @@ Defaults (per state, in the model's units; x27 is the deterministic day counter 
   the rule-based controller, measured with tools/estimate_q.py (DESIGN.md, "State estimation").
 - r_std: sensor-like values: 20 ppm CO2, 0.2 K air temperature, 2 % RH, 0.5 K pipe and 24 h canopy temperature, 1 % of the reset
   fruit weight (553 mg m^-2) and 10 C d for the temperature sum.
+
+DeviceStateSmoother -- an unscented Rauch-Tung-Striebel smoother over the estimator's last `window` estimates
+(csrc/glg_smooth.cuh behind glg_smooth_* in include/glgym.h).  The filter's estimate at step k uses the observations up to k; the
+smoothed one uses every observation in the window, which is what analysing a logged season or an EM fit of the noise wants:
+
+    smoother = DeviceStateSmoother(est, window=192)   # records from the estimator's next reset on
+    est.reset()
+    for step in range(192):
+        env.step_rule_based_tensor()
+        est.update(est.measurements() + sensor_noise)
+    s = smoother.smooth()                             # s.mean [L, B, 28], s.cov and s.gain [L, B, 28, 28], oldest first
 """
+import collections
+import ctypes as C
 import math
 
 import numpy as np
@@ -162,3 +175,65 @@ class DeviceStateEstimator(_EnvCompanion):
             y[:, j] = o[:, int(offsets[mod]) + col].to(torch.float64)
         return y
 
+
+
+Smoothed = collections.namedtuple("Smoothed", "mean cov gain")
+
+
+class DeviceStateSmoother(_EnvCompanion):
+    """Records every glg_est_reset / glg_est_update of `est` into a ring of `window` slots per env and smooths the valid slots on
+    demand.  Recording does not change the estimator's outputs.  Keeps the estimator alive; close the smoother before closing the
+    estimator explicitly."""
+    _kind, _destroy = "smoother", "glg_smooth_destroy"
+
+    def __init__(self, est, window):
+        if isinstance(window, bool) or not isinstance(window, (int, np.integer)) or int(window) < 2:
+            raise ValueError("window must be an integer >= 2")
+        if not isinstance(est, DeviceStateEstimator):
+            raise TypeError("est must be a DeviceStateEstimator")
+        W, B = int(window), int(est.env.num_envs)
+        self.est, self.env, self._lib, self.window = est, est.env, est._lib, W
+        self._obj = C.c_void_p()
+        _lib.check(self._lib.glg_smooth_create(est._live(), W, C.byref(self._obj)), self.env._h, "glg_smooth_create")
+        s, L = self._obj, self._lib
+        mean = lambda ptr: self._view(ptr, (W, 28, B), "<f8").permute(0, 2, 1)  # [W, B, 28] view of [W][28][B]
+        mat = lambda ptr: self._view(ptr, (W, B, 28, 28), "<f8")
+        self._out = Smoothed(mean(L.glg_smooth_mean_dev(s)), mat(L.glg_smooth_cov_dev(s)), mat(L.glg_smooth_gain_dev(s)))
+        self._rec = {"filtered_mean": mean(L.glg_smooth_filtered_mean_dev(s)), "filtered_cov": mat(L.glg_smooth_filtered_cov_dev(s)),
+                     "prior_mean": mean(L.glg_smooth_prior_mean_dev(s)), "prior_cov": mat(L.glg_smooth_prior_cov_dev(s)),
+                     "cross_cov": mat(L.glg_smooth_cross_dev(s)),
+                     "status": self._view(L.glg_smooth_status_dev(s), (W, B), "|u1"),
+                     "timestep": self._view(L.glg_smooth_timestep_dev(s), (W, B), "<i4")}
+        self.bytes = int(L.glg_smooth_bytes(s))
+
+    def _live(self):
+        self.est._live()
+        return super()._live()
+
+    @property
+    def length(self):
+        """The number of valid slots: min(estimates recorded since the estimator's last reset, window)."""
+        return int(self._lib.glg_smooth_length(self._live()))
+
+    def smooth(self):
+        """Runs the backward pass and returns Smoothed(mean [L, B, 28], cov [L, B, 28, 28], gain [L, B, 28, 28]), float64 views
+        of the smoother's output, oldest first (L = length).  gain[k] is G_k; it is 0 at the last slot of a segment, and
+        cov[k + 1] @ gain[k].transpose(-1, -2) is the lag-one cross-covariance."""
+        s = self._live()
+        _lib.check(self._lib.glg_smooth_run(s, self.env._stream()), self.env._h, "glg_smooth_run")
+        n = self.length
+        return Smoothed(*(v[:n] for v in self._out))
+
+    def _rolled(self, name):
+        """A recorded quantity, oldest first (a copy: the record is a ring)."""
+        s = self._live()
+        n, first = self.length, int(self._lib.glg_smooth_first(s))
+        return torch.roll(self._rec[name], -first, 0)[:n]
+
+    filtered_mean = property(lambda self: self._rolled("filtered_mean"), doc="x^ [L, B, 28]: the estimator's means")
+    filtered_cov = property(lambda self: self._rolled("filtered_cov"), doc="P [L, B, 28, 28]: the estimator's covariances")
+    prior_mean = property(lambda self: self._rolled("prior_mean"), doc="xbar [L, B, 28]; 0 where no prediction leads to the slot")
+    prior_cov = property(lambda self: self._rolled("prior_cov"), doc="P- [L, B, 28, 28]; 0 where no prediction leads to the slot")
+    cross_cov = property(lambda self: self._rolled("cross_cov"), doc="D [L, B, 28, 28]: sum Wc (chi - x^)(chi' - xbar)^T")
+    status = property(lambda self: self._rolled("status"), doc="[L, B] the estimator's status bits of each slot")
+    timestep = property(lambda self: self._rolled("timestep"), doc="[L, B] the env's timestep of each slot")

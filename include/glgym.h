@@ -385,6 +385,55 @@ double *glg_est_innovation_dev(glg_est *e);  /* [B][7]: y - ybar, 0 where not me
 double *glg_est_sigma_dev(glg_est *e);       /* [28][B*57]: the propagated sigma points (the shadow handle's x) */
 uint8_t *glg_est_status_dev(glg_est *e);     /* [B] */
 
+/* ---- state smoothing: an unscented Rauch-Tung-Striebel smoother (URTS) over a recorded window of an estimator -----------------
+ * A smoother belongs to one estimator and keeps, per env, a ring of W slots of the filter's forward quantities.  Recording does not
+ * change a bit of the estimator's outputs (mean, cov, innovation, status).  Notation as in the filter contract above.
+ * Smoother contract:
+ *   Record: from the estimator's next glg_est_reset on.  Every glg_est_reset starts the record over and writes slot 0 (x^_0, P_0);
+ *     each glg_est_update appends slot k+1 holding
+ *       x^_{k+1}, P_{k+1}  the estimator's outputs after the update, bit for bit;
+ *       xbar_{k+1}, P-_{k+1}  as the filter forms them, diag(q_std^2) included;
+ *       D_{k+1} = sum_{i=1..2n} Wc_i (chi_i - x^_k)(chi'_i - xbar_{k+1})^T in ascending i, with chi_i - x^_k the offset
+ *         +-gamma L[:, i-1] (the product the sigma points were formed with) and L the factor of P_k the update used;
+ *       the env's status bits from this update and the env's timestep after its step.
+ *     A slot that no one-interval prediction leads to (the reset slot, status 1, 4 or 8) holds xbar = P- = D = 0.  The ring keeps
+ *     the last W estimates.
+ *   Segments: slot k+1 starts a new segment when its status has bit 1, 4 or 8.  Status 2 and predict-only updates link to the slot
+ *     before.  No gain crosses a segment start; the last slot of each segment is smoothed to its filtered value and its gain is 0.
+ *   Deterministic states: a state j with p0_std[j] = q_std[j] = 0 (x27, the day counter, with the defaults) is left out: row and
+ *     column j of G are 0, xs_j = x^_j, and row and column j of Ps are P's.  The rest of P- is factored by the filter's
+ *     zero-column Cholesky rule.
+ *   Backward pass, k from the newest slot down to the oldest in each segment:
+ *     G_k = D_{k+1} (P-_{k+1})^-1: row i solves P- g_i = d_i by forward substitution through the factor and back substitution
+ *       through its transpose; a component whose column of the factor is zero is 0.
+ *     xs_k = x^_k + G_k (xs_{k+1} - xbar_{k+1}),  Ps_k = sym(P_k + G_k (Ps_{k+1} - P-_{k+1}) G_k^T).
+ *     Sums run in ascending index order, without atomics: the result is deterministic.  The record is only read, so the smoother
+ *     can run again as the window moves (run after every update: fixed-lag smoothing).  The lag-one cross-covariance EM needs is
+ *     Ps_{k+1} G_k^T.
+ * The smoother's memory is its own.  Destroy the smoother before its estimator; a smoother whose estimator is gone can only be
+ * destroyed (glg_smooth_run returns GLG_ERR_STATE).  Errors are reported through glg_last_error of the env handle. */
+typedef struct glg_smooth glg_smooth;
+/* window >= 2 slots per env.  GLG_ERR_ARG for NULLs or a bad window, GLG_ERR_STATE if the estimator already has a smoother. */
+int glg_smooth_create(glg_est *e, int32_t window, glg_smooth **out);
+void glg_smooth_destroy(glg_smooth *s);
+/* The backward pass over the valid slots into the output views.  GLG_ERR_STATE before the first recorded reset.  One launch. */
+int glg_smooth_run(glg_smooth *s, void *stream);
+int32_t glg_smooth_length(const glg_smooth *s);  /* valid slots: min(recorded, window) */
+int32_t glg_smooth_first(const glg_smooth *s);   /* ring slot of the oldest valid estimate */
+int64_t glg_smooth_bytes(const glg_smooth *s);   /* device bytes the smoother owns */
+/* written by glg_smooth_run, oldest first (slot 0 is the oldest valid estimate) */
+double *glg_smooth_mean_dev(glg_smooth *s);           /* [W][28][B] smoothed means */
+double *glg_smooth_cov_dev(glg_smooth *s);            /* [W][B][28][28] smoothed covariances */
+double *glg_smooth_gain_dev(glg_smooth *s);           /* [W][B][28][28] G_k; 0 at a segment's last slot */
+/* the record, in ring order (glg_smooth_first names the oldest slot) */
+double *glg_smooth_filtered_mean_dev(glg_smooth *s);  /* [W][28][B] x^ */
+double *glg_smooth_filtered_cov_dev(glg_smooth *s);   /* [W][B][28][28] P */
+double *glg_smooth_prior_mean_dev(glg_smooth *s);     /* [W][28][B] xbar */
+double *glg_smooth_prior_cov_dev(glg_smooth *s);      /* [W][B][28][28] P- */
+double *glg_smooth_cross_dev(glg_smooth *s);          /* [W][B][28][28] D */
+uint8_t *glg_smooth_status_dev(glg_smooth *s);        /* [W][B] */
+int32_t *glg_smooth_timestep_dev(glg_smooth *s);      /* [W][B] */
+
 /* Multi-GPU episode statistics (SURVEY 8e): the step path has no collective; the one exchange is a sum of the 16-entry
  * statistics vector over the ranks' handles, once per logging interval -- ncclAllReduce on the handle's device buffer.
  * NCCL is bound at run time (dlopen of libnccl.so.2, the copy torch already loaded when there is one), so libglgym.so has no
