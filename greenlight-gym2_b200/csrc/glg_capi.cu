@@ -29,6 +29,7 @@
 #include "glg_tangent.cuh"
 #include "glg_est.cuh"
 #include "glg_smooth.cuh"
+#include "glg_em.cuh"
 
 
 static thread_local std::string g_error = "";  // glg_last_error(NULL): the last failure of an entry point without a handle
@@ -458,9 +459,9 @@ static cudaError_t launch_step_units(glg_handle *h, const GlgStepArgs &a, cudaSt
 // per SM: the step time of a batch that leaves SMs under-filled is the latency of one CTA), 3 = kernel C throughput layout
 // (4 fused warps per 32 envs, 4 CTAs per SM).  Auto-pick: measured with tools/layout_sweep.py the latency layout wins up to two
 // waves of CTAs (B = 9472 on 148 SMs: 1.735 vs 1.814 ms), the throughput layout beyond (B = 12 288: 2.60 vs 2.18 ms).
-static int pick_role_warps(const glg_handle *h) {
+static int pick_role_warps(const glg_handle *h, int B) {
     if (h->cfg.role_warps != 0) return h->cfg.role_warps;
-    return h->a.B <= 2 * h->sms * GLG_ROLE_LANES ? 2 : 3;
+    return B <= 2 * h->sms * GLG_ROLE_LANES ? 2 : 3;
 }
 typedef cudaError_t (*StepLauncher)(glg_handle *, const GlgStepArgs &, cudaStream_t);
 static const StepLauncher kStepLaunchers[3][2][2] = {  // [kernel variant - 1][general][noisy]
@@ -470,8 +471,10 @@ static const StepLauncher kStepLaunchers[3][2][2] = {  // [kernel variant - 1][g
     {{launch_step_units<true, false, false>, launch_step_units<true, false, true>},
      {launch_step_units<true, true, false>, launch_step_units<true, true, true>}}};
 
+// n_envs > 0 steps envs 0 .. n_envs - 1 only, laid out as a batch of n_envs (SoA strides n_envs), with the kernel picked for that
+// batch: an owner that fills a prefix of an internal handle steps no padding
 static int step_common(glg_handle *h, const float *actions_dev, const double *controls_dev, const double *noise_dev,
-                       void *stream, bool rule_based = false) {
+                       void *stream, bool rule_based = false, int n_envs = 0) {
     int rc = check_ready(h);
     if (rc) return rc;
     if (!h->is_reset) return fail(h, GLG_ERR_STATE, "step before reset");
@@ -482,8 +485,9 @@ static int step_common(glg_handle *h, const float *actions_dev, const double *co
     a.controls = controls_dev;
     a.raw_control = rule_based ? 2 : (controls_dev ? 1 : 0);
     a.noise = noise_dev;
+    if (n_envs > 0) a.B = n_envs;
     const bool noisy = (a.uncertainty_scale != 0.0) || (noise_dev != nullptr);
-    const cudaError_t e = kStepLaunchers[pick_role_warps(h) - 1][h->general][noisy](h, a, (cudaStream_t)stream);
+    const cudaError_t e = kStepLaunchers[pick_role_warps(h, a.B) - 1][h->general][noisy](h, a, (cudaStream_t)stream);
     h->launches += 1;
     GLG_CUDA(h, e);
     return GLG_OK;
@@ -1415,7 +1419,12 @@ struct glg_est {
     GlgEstArgs a = {};      // weights, variances and the estimator's buffers; the handles' pointers are set per call
     CudaMem mem;
     glg_smooth *sm = nullptr;  // the smoother recording this estimator's estimates, if any
+    // glg_est_set_noise's settings, applied by the next glg_est_reset so that no record mixes two noise models
+    bool staged = false;
+    double p0var[GLG_NX] = {}, qvar[GLG_NX] = {}, rvar[GLG_EST_NM] = {};
 };
+
+struct glg_em;
 
 // ---- state smoothing (glg_smooth.cuh): an unscented RTS smoother over a ring of the estimator's last W estimates, recorded by
 // the RECORD instantiations of the estimator's kernels ----
@@ -1432,7 +1441,46 @@ struct glg_smooth {
     // glg_smooth_run's output, oldest first
     double *s_mean = nullptr, *s_cov = nullptr, *gain = nullptr;
     CudaMem mem;
+    glg_em *em = nullptr;          // the EM object logging alongside this record, if any
+    unsigned long long writes = 0;  // slots written so far; run_writes: its value at the last glg_smooth_run (~0: none)
+    unsigned long long run_writes = ~0ull;
 };
+
+// ---- noise identification (glg_em.cuh): the data log a smoother's record keeps for an EM fit of Q and R, and the E-step over the
+// smoother's output, whose sigma points an internal handle (the EM handle) steps in chunks of at most max_points ----
+struct glg_em {
+    glg_smooth *sm = nullptr;  // cleared when the smoother is destroyed first
+    int device = 0, B = 0, W = 0, ncap = 0;  // at most ncap pairs per chunk: the EM handle holds ncap 57 envs
+    bool logging = false;      // the log has run since a glg_est_reset (it starts with the first reset after creation)
+    std::unique_ptr<glg_handle> hh;
+    unsigned long long weather_gen = 0;
+    // the log, ring order (the smoother's ring slots)
+    double *u = nullptr, *y = nullptr, *ll = nullptr;  // [W][6][B], [W][7][B], [W][B]
+    int *table = nullptr;                              // [W][B]
+    unsigned char *flags = nullptr;                    // [W][B]
+    // glg_em_estep's output: per pair oldest first, per env, pooled
+    double *ex = nullptr, *fbar = nullptr, *env_stats = nullptr, *total = nullptr;
+    unsigned char *used = nullptr;
+    double *ctrl = nullptr;  // [ncap 57][6] the EM envs' controls
+    CudaMem mem;
+};
+
+static void em_slot(const glg_em *m, long long slot, GlgEstArgs *a) {
+    const size_t r = (size_t)slot, B = (size_t)m->B;
+    a->l_u = m->u + r * GLG_NU * B;
+    a->l_table = m->table + r * B;
+    a->l_y = m->y + r * GLG_EST_NM * B;
+    a->l_flags = m->flags + r * B;
+    a->l_ll = m->ll + r * B;
+}
+
+// bit j: state j takes part in smoothing (p0_std[j] or q_std[j] > 0)
+static unsigned int active_states(const GlgEstArgs &a) {
+    unsigned int active = 0;
+    for (int j = 0; j < GLG_NX; ++j)
+        if (a.p0var[j] > 0.0 || a.qvar[j] > 0.0) active |= 1u << j;
+    return active;
+}
 
 extern "C" void glg_est_destroy(glg_est *e) {
     if (!e) return;
@@ -1536,17 +1584,33 @@ extern "C" int glg_est_reset(glg_est *e, const double *x0_dev, void *stream) {
     int rc = companion_sync(h, e->hs.get(), e->weather_gen, "glg_est_reset", "estimator");
     if (rc) return rc;
     GLG_CUDA(h, cudaSetDevice(e->device));
+    if (e->staged) {  // glg_est_set_noise's settings take effect here, with the smoother's deterministic-state mask
+        memcpy(e->a.p0var, e->p0var, sizeof e->p0var);
+        memcpy(e->a.qvar, e->qvar, sizeof e->qvar);
+        memcpy(e->a.rvar, e->rvar, sizeof e->rvar);
+        e->staged = false;
+        if (e->sm) e->sm->active = active_states(e->a);
+    }
     GlgEstArgs a = est_args(e);
     a.x0 = x0_dev ? x0_dev : h->a.x;
-    if (e->sm) {  // a reset starts the smoother's record over: it writes slot 0
+    glg_em *em = e->sm ? e->sm->em : nullptr;
+    if (em) {  // the reset starts the record and the log over: both write slot 0
         smooth_slot(e->sm, 0, &a);
-        glg_est_init_kernel<true><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+        em_slot(em, 0, &a);
+        glg_est_init_kernel<GLG_EST_LOG><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+    } else if (e->sm) {  // a reset starts the smoother's record over: it writes slot 0
+        smooth_slot(e->sm, 0, &a);
+        glg_est_init_kernel<GLG_EST_RECORD><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
     } else {
-        glg_est_init_kernel<false><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
+        glg_est_init_kernel<GLG_EST_FILTER><<<e->B, GLG_EST_NT, 0, (cudaStream_t)stream>>>(a);
     }
     GLG_CUDA(h, cudaGetLastError());
     e->is_reset = true;
-    if (e->sm) e->sm->count = 1;
+    if (e->sm) {
+        e->sm->count = 1;
+        ++e->sm->writes;
+    }
+    if (em) em->logging = true;
     return GLG_OK;
 }
 
@@ -1561,18 +1625,25 @@ extern "C" int glg_est_update(glg_est *e, const double *y_dev, void *stream) {
     GlgEstArgs a = est_args(e);
     a.y = y_dev;
     glg_smooth *m = e->sm && e->sm->count > 0 ? e->sm : nullptr;  // a smoother records from the first reset after its creation
+    glg_em *em = m && m->em && m->em->logging ? m->em : nullptr;  // and an EM object logs from the first reset after its creation
     if (m) smooth_slot(m, m->count % m->W, &a);
-    if (m) glg_est_sigma_kernel<true><<<e->B, GLG_EST_NT, 0, s>>>(a);
-    else glg_est_sigma_kernel<false><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    if (em) em_slot(em, m->count % m->W, &a);
+    if (em) glg_est_sigma_kernel<GLG_EST_LOG><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    else if (m) glg_est_sigma_kernel<GLG_EST_RECORD><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    else glg_est_sigma_kernel<GLG_EST_FILTER><<<e->B, GLG_EST_NT, 0, s>>>(a);
     GLG_CUDA(h, cudaGetLastError());
     if ((rc = glg_step_raw_control(hs, a.sctrl, nullptr, s))) {
         h->err = "glg_est_update: shadow step: " + hs->err;
         return rc;
     }
-    if (m) glg_est_ut_kernel<true><<<e->B, GLG_EST_NT, 0, s>>>(a);
-    else glg_est_ut_kernel<false><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    if (em) glg_est_ut_kernel<GLG_EST_LOG><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    else if (m) glg_est_ut_kernel<GLG_EST_RECORD><<<e->B, GLG_EST_NT, 0, s>>>(a);
+    else glg_est_ut_kernel<GLG_EST_FILTER><<<e->B, GLG_EST_NT, 0, s>>>(a);
     GLG_CUDA(h, cudaGetLastError());
-    if (m) ++m->count;
+    if (m) {
+        ++m->count;
+        ++m->writes;
+    }
     return GLG_OK;
 }
 
@@ -1582,9 +1653,38 @@ extern "C" double *glg_est_innovation_dev(glg_est *e) { return e ? e->a.innov : 
 extern "C" double *glg_est_sigma_dev(glg_est *e) { return e ? e->hs->a.x : nullptr; }
 extern "C" uint8_t *glg_est_status_dev(glg_est *e) { return e ? e->a.status : nullptr; }
 
+extern "C" int glg_est_set_noise(glg_est *e, const double *p0_std, const double *q_std, const double *r_std) {
+    if (!e) return GLG_ERR_ARG;
+    glg_handle *h = e->h;
+    for (int i = 0; i < GLG_NX; ++i)
+        if ((p0_std && (!(p0_std[i] >= 0.0) || !isfinite(p0_std[i]))) || (q_std && (!(q_std[i] >= 0.0) || !isfinite(q_std[i]))))
+            return fail(h, GLG_ERR_ARG, "glg_est_set_noise: p0_std and q_std must be finite and >= 0");
+    if (r_std) {
+        unsigned int mask = 0;
+        for (int q = 0; q < e->a.m; ++q) mask |= 1u << e->a.midx[q];
+        for (int r = 0; r < GLG_EST_NM; ++r)
+            if (!(r_std[r] >= 0.0) || !isfinite(r_std[r]) || ((mask >> r & 1u) && !(r_std[r] > 0.0)))
+                return fail(h, GLG_ERR_ARG, "glg_est_set_noise: r_std must be finite, >= 0, and > 0 for every measured entry");
+    }
+    if (!e->staged) {  // start from the settings in force
+        memcpy(e->p0var, e->a.p0var, sizeof e->p0var);
+        memcpy(e->qvar, e->a.qvar, sizeof e->qvar);
+        memcpy(e->rvar, e->a.rvar, sizeof e->rvar);
+    }
+    for (int i = 0; i < GLG_NX; ++i) {
+        if (p0_std) e->p0var[i] = p0_std[i] * p0_std[i];
+        if (q_std) e->qvar[i] = q_std[i] * q_std[i];
+    }
+    for (int r = 0; r < GLG_EST_NM; ++r)
+        if (r_std) e->rvar[r] = r_std[r] * r_std[r];
+    e->staged = true;
+    return GLG_OK;
+}
+
 extern "C" void glg_smooth_destroy(glg_smooth *m) {
     if (!m) return;
     if (m->e) m->e->sm = nullptr;
+    if (m->em) m->em->sm = nullptr;
     cudaSetDevice(m->device);
     delete m;
 }
@@ -1604,8 +1704,7 @@ extern "C" int glg_smooth_create(glg_est *e, int32_t window, glg_smooth **out) {
     m->device = e->device;
     m->B = e->B;
     m->W = window;
-    for (int j = 0; j < GLG_NX; ++j)
-        if (e->a.p0var[j] > 0.0 || e->a.qvar[j] > 0.0) m->active |= 1u << j;
+    m->active = active_states(e->a);
     const size_t B = (size_t)m->B, WB = (size_t)window * B;
     cudaError_t ce = m->mem.dev(&m->mean, GLG_NX * WB);
     if (ce == cudaSuccess) ce = m->mem.dev(&m->xbar, GLG_NX * WB);
@@ -1647,6 +1746,7 @@ extern "C" int glg_smooth_run(glg_smooth *m, void *stream) {
     a.s_mean = m->s_mean; a.s_cov = m->s_cov; a.gain = m->gain;
     glg_smooth_kernel<<<m->B, GLG_SMOOTH_NT, 0, (cudaStream_t)stream>>>(a);
     GLG_CUDA(h, cudaGetLastError());
+    m->run_writes = m->writes;
     return GLG_OK;
 }
 
@@ -1661,6 +1761,127 @@ extern "C" double *glg_smooth_prior_cov_dev(glg_smooth *m) { return m ? m->pm : 
 extern "C" double *glg_smooth_cross_dev(glg_smooth *m) { return m ? m->d : nullptr; }
 extern "C" uint8_t *glg_smooth_status_dev(glg_smooth *m) { return m ? m->status : nullptr; }
 extern "C" int32_t *glg_smooth_timestep_dev(glg_smooth *m) { return m ? m->timestep : nullptr; }
+
+extern "C" void glg_em_destroy(glg_em *m) {
+    if (!m) return;
+    if (m->sm) m->sm->em = nullptr;
+    cudaSetDevice(m->device);
+    delete m;
+}
+
+extern "C" int glg_em_create(glg_smooth *s, int64_t max_points, glg_em **out) {
+    if (!s || !out) {
+        g_error = "glg_em_create: null argument";
+        return GLG_ERR_ARG;
+    }
+    *out = nullptr;
+    if (!s->e) {
+        g_error = "glg_em_create: the smoother's estimator was destroyed";
+        return GLG_ERR_STATE;
+    }
+    glg_handle *h = s->e->h;
+    if (max_points == 0) max_points = kPlanMaxBatch;
+    if (max_points < GLG_EST_S || max_points > kPlanMaxBatch)
+        return fail(h, GLG_ERR_ARG, "glg_em_create: max_points must be 0 (4194304) or in 57 .. 4194304");
+    if (s->em) return fail(h, GLG_ERR_STATE, "glg_em_create: the smoother already has an EM object");
+    GLG_CUDA(h, cudaSetDevice(s->device));
+    glg_em *m = new (std::nothrow) glg_em();
+    if (!m) return fail(h, GLG_ERR_ALLOC, "glg_em_create: out of host memory");
+    m->device = s->device;
+    m->B = s->B;
+    m->W = s->W;
+    m->ncap = (int)std::min<long long>((long long)s->B * s->W, max_points / GLG_EST_S);
+    const int32_t climate_only[8] = {GLG_OBS_CLIMATE, 0, 0, 0, 0, 0, 0, 0};  // nothing reads the EM envs' rows
+    int rc = companion_create(h, m->ncap * GLG_EST_S, climate_only, "glg_em_create: EM handle: ", &m->hh);
+    if (rc != GLG_OK) {
+        glg_em_destroy(m);
+        return rc;
+    }
+    const size_t B = (size_t)m->B, WB = (size_t)m->W * B;
+    cudaError_t ce = m->mem.dev(&m->u, GLG_NU * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->y, GLG_EST_NM * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->ll, WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->table, WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->flags, WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->ex, GLG_EM_NE * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->fbar, GLG_NX * WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->used, WB);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->env_stats, GLG_EM_NS * B);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->total, (size_t)GLG_EM_NS);
+    if (ce == cudaSuccess) ce = m->mem.dev(&m->ctrl, (size_t)m->ncap * GLG_EST_S * GLG_NU);
+    if (ce != cudaSuccess) {
+        glg_em_destroy(m);
+        return fail(h, GLG_ERR_CUDA, (std::string("glg_em_create: ") + cudaGetErrorString(ce)).c_str());
+    }
+    m->weather_gen = h->weather_gen;
+    m->sm = s;
+    s->em = m;
+    *out = m;
+    return GLG_OK;
+}
+
+extern "C" int glg_em_estep(glg_em *m, void *stream) {
+    if (!m) return GLG_ERR_ARG;
+    if (!m->sm || !m->sm->e) {
+        g_error = "glg_em_estep: the EM object's smoother or its estimator was destroyed";
+        return GLG_ERR_STATE;
+    }
+    glg_smooth *sm = m->sm;
+    glg_est *e = sm->e;
+    glg_handle *h = e->h, *hh = m->hh.get();
+    int rc = companion_sync(h, hh, m->weather_gen, "glg_em_estep", "EM object");
+    if (rc) return rc;
+    if (!m->logging || sm->count == 0)
+        return fail(h, GLG_ERR_STATE, "glg_em_estep: nothing logged yet (glg_est_reset after glg_em_create starts the log)");
+    if (sm->run_writes != sm->writes)
+        return fail(h, GLG_ERR_STATE, "glg_em_estep: the record changed since the last glg_smooth_run; run the smoother first");
+    GLG_CUDA(h, cudaSetDevice(m->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    GlgEmArgs a;
+    memset(&a, 0, sizeof a);
+    a.B = m->B; a.W = m->W; a.len = glg_smooth_length(sm); a.first = glg_smooth_first(sm); a.N = h->a.N;
+    a.m = e->a.m;
+    for (int q = 0; q < GLG_EST_NM; ++q) a.midx[q] = e->a.midx[q];
+    a.gamma = e->a.gamma; a.wm0 = e->a.wm0; a.wc0 = e->a.wc0; a.wi = e->a.wi;
+    a.s_mean = sm->s_mean; a.s_cov = sm->s_cov; a.gain = sm->gain; a.status = sm->status; a.timestep = sm->timestep;
+    a.l_u = m->u; a.l_y = m->y; a.l_ll = m->ll; a.l_table = m->table; a.l_flags = m->flags;
+    const GlgStepArgs &ha = hh->a;
+    a.hx = ha.x; a.hctrl = m->ctrl; a.htime = ha.time; a.htimestep = ha.timestep; a.htable = ha.table; a.hdone = ha.done;
+    a.ex = m->ex; a.fbar = m->fbar; a.used = m->used; a.env_stats = m->env_stats; a.total = m->total;
+    // balanced chunks of at most ncap pairs; each steps exactly its own points: the first np 57 envs of the EM handle, laid out
+    // as a batch of that size
+    const int pairs = m->B * a.len, chunks = (pairs + m->ncap - 1) / m->ncap, per = (pairs + chunks - 1) / chunks;
+    for (a.p0 = 0; a.p0 < pairs; a.p0 += per) {
+        a.np = std::min(per, pairs - a.p0);
+        glg_em_sigma_kernel<<<a.np, GLG_EM_NT, 0, s>>>(a);
+        GLG_CUDA(h, cudaGetLastError());
+        if ((rc = step_common(hh, nullptr, m->ctrl, nullptr, s, false, a.np * GLG_EST_S))) {
+            h->err = "glg_em_estep: EM step: " + hh->err;
+            return rc;
+        }
+        glg_em_expect_kernel<<<a.np, GLG_EM_NT, 0, s>>>(a);
+        GLG_CUDA(h, cudaGetLastError());
+    }
+    glg_em_env_kernel<<<(m->B * GLG_EM_NS + 127) / 128, 128, 0, s>>>(a);
+    GLG_CUDA(h, cudaGetLastError());
+    glg_em_total_kernel<<<1, 64, 0, s>>>(a);
+    GLG_CUDA(h, cudaGetLastError());
+    return GLG_OK;
+}
+
+extern "C" int64_t glg_em_bytes(const glg_em *m) { return m ? (int64_t)m->mem.bytes() : 0; }
+extern "C" int64_t glg_em_logged(const glg_em *m) { return m && m->logging && m->sm ? m->sm->count : 0; }
+extern "C" int32_t glg_em_chunk_pairs(const glg_em *m) { return m ? m->ncap : 0; }
+extern "C" double *glg_em_controls_dev(glg_em *m) { return m ? m->u : nullptr; }
+extern "C" int32_t *glg_em_table_dev(glg_em *m) { return m ? m->table : nullptr; }
+extern "C" double *glg_em_measurements_dev(glg_em *m) { return m ? m->y : nullptr; }
+extern "C" uint8_t *glg_em_flags_dev(glg_em *m) { return m ? m->flags : nullptr; }
+extern "C" double *glg_em_loglik_dev(glg_em *m) { return m ? m->ll : nullptr; }
+extern "C" double *glg_em_expectation_dev(glg_em *m) { return m ? m->ex : nullptr; }
+extern "C" double *glg_em_prediction_dev(glg_em *m) { return m ? m->fbar : nullptr; }
+extern "C" uint8_t *glg_em_used_dev(glg_em *m) { return m ? m->used : nullptr; }
+extern "C" double *glg_em_env_stats_dev(glg_em *m) { return m ? m->env_stats : nullptr; }
+extern "C" double *glg_em_totals_dev(glg_em *m) { return m ? m->total : nullptr; }
 
 // ---- episode-statistics all-reduce over NCCL (run-time binding: nccl_api above)
 extern "C" int glg_nccl_unique_id(uint8_t id_out[128]) {

@@ -8,8 +8,10 @@
 //                          controls array [B S][6], and the pre-step timestep, table and clock of the env into its shadow envs.
 //   glg_est_ut_kernel    : one CTA per env.  Mean and covariance of the propagated points, measurement points h(chi'), S, C, the
 //                          m x m Cholesky solve and the posterior.  All sums run in ascending index order; no atomics.
-// Each kernel takes RECORD: the <true> instantiations also write one slot of a smoother's forward record (glg_smooth.cuh) and are
-// launched only for an estimator with a smoother; the <false> ones are the filter alone.
+// Each kernel takes a MODE: the GLG_EST_FILTER instantiations are the filter alone; the GLG_EST_RECORD ones also write one slot of
+// a smoother's forward record (glg_smooth.cuh) and are launched only for an estimator with a smoother; the GLG_EST_LOG ones also
+// write one slot of an EM object's data log (glg_em.cuh): the controls and table the step used, the measurement as given, the
+// update flags and the slot's log-likelihood term.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -24,6 +26,10 @@ constexpr int GLG_EST_NX2 = GLG_NX * GLG_NX;
 
 // status bits (per env, rewritten by every glg_est_update)
 constexpr unsigned char GLG_EST_NONFINITE = 1, GLG_EST_S_NOT_PD = 2, GLG_EST_REINIT = 4, GLG_EST_OUT_OF_STEP = 8;
+// log flags (per env and slot): y_dev was given; the update was applied (y_dev given and status 0)
+constexpr unsigned char GLG_EST_LOG_Y = 1, GLG_EST_LOG_APPLIED = 2;
+// kernel modes: the filter alone; also the smoother's record; also the record and the EM object's log
+constexpr int GLG_EST_FILTER = 0, GLG_EST_RECORD = 1, GLG_EST_LOG = 2;
 
 struct GlgEstArgs {
     int B, N, auto_reset, m;   // m measured entries, midx[0..m) their index in h(x)
@@ -54,7 +60,27 @@ struct GlgEstArgs {
     double *r_cov, *r_pm, *r_d;            // [B][28][28] filtered P, P-, D
     unsigned char *r_status;               // [B]
     int *r_timestep;                       // [B]
+    // LOG kernels only: the slot of the EM object's log this reset / update writes
+    double *l_u;                           // [6][B] the controls the env applied
+    int *l_table;                          // [B] its weather table
+    double *l_y;                           // [7][B] y as given; 0 where not measured or y is NULL
+    unsigned char *l_flags;                // [B] GLG_EST_LOG_Y | GLG_EST_LOG_APPLIED
+    double *l_ll;                          // [B] -(v^T S^-1 v + log det S + m log 2 pi) / 2; 0 where no update was applied
 };
+
+// The log's measurement and flags for a slot without an applied update; the UT kernel overwrites flags and ll where it applies one
+__device__ __forceinline__ void glg_est_log_start(const GlgEstArgs &A, int b) {
+    const int B = A.B;
+    for (int r = threadIdx.x; r < GLG_EST_NM; r += blockDim.x) {
+        bool meas = false;
+        for (int q = 0; q < A.m; ++q) meas |= A.midx[q] == r;
+        A.l_y[(size_t)r * B + b] = A.y && meas ? A.y[(size_t)b * GLG_EST_NM + r] : 0.0;
+    }
+    if (threadIdx.x == 0) {
+        A.l_flags[b] = A.y ? GLG_EST_LOG_Y : 0;
+        A.l_ll[b] = 0.0;
+    }
+}
 
 // A slot without a one-interval prediction behind it (a reset, status 1, 4 or 8): the filtered mean and covariance as they stand
 // after this kernel, xbar = P- = D = 0, and the status and timestep.  Each thread copies entries it alone wrote, if any.
@@ -99,7 +125,7 @@ __device__ __forceinline__ void glg_est_restart(const GlgEstArgs &A, int b, cons
     for (int r = threadIdx.x; r < GLG_EST_NM; r += blockDim.x) A.innov[(size_t)b * GLG_EST_NM + r] = 0.0;
 }
 
-template <bool RECORD>
+template <int MODE>
 __global__ void __launch_bounds__(GLG_EST_NT) glg_est_init_kernel(const __grid_constant__ GlgEstArgs A) {
     const int b = blockIdx.x;
     glg_est_restart(A, b, A.x0);
@@ -107,10 +133,15 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_init_kernel(const __grid_c
         A.ctr[b] = A.step_ctr[b];
         A.status[b] = 0;
     }
-    if constexpr (RECORD) glg_est_record_start(A, b, 0);
+    if constexpr (MODE >= GLG_EST_RECORD) glg_est_record_start(A, b, 0);
+    if constexpr (MODE == GLG_EST_LOG) {  // the reset slot: no controls, no measurement
+        glg_est_log_start(A, b);
+        if (threadIdx.x < GLG_NU) A.l_u[(size_t)threadIdx.x * A.B + b] = 0.0;
+        if (threadIdx.x == 0) A.l_table[b] = A.table[b];
+    }
 }
 
-template <bool RECORD>
+template <int MODE>
 __global__ void __launch_bounds__(GLG_EST_NT) glg_est_sigma_kernel(const __grid_constant__ GlgEstArgs A) {
     __shared__ double L[GLG_NX][GLG_NX + 1];  // P's lower triangle, factored in place
     __shared__ double xh[GLG_NX];
@@ -173,7 +204,11 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_sigma_kernel(const __grid_
         A.stime[BS + c0 + t] = fmod(A.time[(size_t)B + b] - fmod(A.dt / 3600.0, 24.0) + 24.0, 24.0);
     }
     for (int o = t; o < GLG_EST_S * GLG_NU; o += GLG_EST_NT) A.sctrl[c0 * GLG_NU + o] = A.u[(size_t)(o % GLG_NU) * B + b];
-    if constexpr (RECORD) {  // L for the UT kernel's D; both branches above end in a barrier
+    if constexpr (MODE == GLG_EST_LOG) {
+        if (t < GLG_NU) A.l_u[(size_t)t * B + b] = A.u[(size_t)t * B + b];
+        if (t == 0) A.l_table[b] = A.table[b];
+    }
+    if constexpr (MODE >= GLG_EST_RECORD) {  // L for the UT kernel's D; both branches above end in a barrier
         for (int o = t; o < GLG_EST_NX2; o += GLG_EST_NT) {
             const int i = o / GLG_NX, j = o - i * GLG_NX;
             A.lfac[(size_t)b * GLG_EST_NX2 + o] = j <= i ? L[i][j] : 0.0;
@@ -181,8 +216,9 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_sigma_kernel(const __grid_
     }
 }
 
-template <bool RECORD>
+template <int MODE>
 __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_constant__ GlgEstArgs A) {
+    constexpr bool RECORD = MODE >= GLG_EST_RECORD;
     __shared__ double X[GLG_EST_S][GLG_NX + 1];      // propagated points, then their deviations from the mean
     __shared__ double Y[GLG_EST_S][GLG_EST_NM + 1];  // measurement points, then their deviations
     __shared__ double Pm[GLG_NX][GLG_NX + 1];        // prior covariance P-
@@ -193,6 +229,7 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
     __shared__ int s_pd;
     const int b = blockIdx.x, t = threadIdx.x, B = A.B, m = A.m;
     const size_t BS = (size_t)B * GLG_EST_S, c0 = (size_t)b * GLG_EST_S;
+    if constexpr (MODE == GLG_EST_LOG) glg_est_log_start(A, b);
     if (A.status[b] & (GLG_EST_REINIT | GLG_EST_OUT_OF_STEP)) {  // uniform over the CTA
         if constexpr (RECORD) glg_est_record_start(A, b, A.status[b]);
         return;
@@ -317,6 +354,20 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
         }
         s_pd = pd;
         if (!pd) A.status[b] |= GLG_EST_S_NOT_PD;
+        if constexpr (MODE == GLG_EST_LOG) {
+            if (pd) {  // l = -(|z|^2 + 2 sum log Ls_rr + m log 2 pi) / 2 with Ls z = v
+                double z[GLG_EST_NM], q = 0.0, ld = 0.0;
+                for (int r = 0; r < m; ++r) {
+                    double s = v[r];
+                    for (int k = 0; k < r; ++k) s -= Ls[r][k] * z[k];
+                    z[r] = s / Ls[r][r];
+                    q += z[r] * z[r];
+                    ld += log(Ls[r][r]);
+                }
+                A.l_flags[b] = GLG_EST_LOG_Y | GLG_EST_LOG_APPLIED;
+                A.l_ll[b] = -0.5 * (q + 2.0 * ld + m * 1.8378770664093454836);  // log 2 pi
+            }
+        }
     }
     __syncthreads();
     if (!s_pd) {  // keep the prediction
@@ -368,3 +419,4 @@ __global__ void __launch_bounds__(GLG_EST_NT) glg_est_ut_kernel(const __grid_con
         }
     }
 }
+

@@ -157,6 +157,23 @@ SIGNATURES = {
     "glg_smooth_cross_dev": (C.c_void_p, [C.c_void_p]),
     "glg_smooth_status_dev": (C.c_void_p, [C.c_void_p]),
     "glg_smooth_timestep_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_est_set_noise": (C.c_int, [C.c_void_p, _DP, _DP, _DP]),
+    "glg_em_create": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
+    "glg_em_destroy": (None, [C.c_void_p]),
+    "glg_em_estep": (C.c_int, [C.c_void_p, _VP]),
+    "glg_em_bytes": (C.c_int64, [C.c_void_p]),
+    "glg_em_logged": (C.c_int64, [C.c_void_p]),
+    "glg_em_chunk_pairs": (C.c_int32, [C.c_void_p]),
+    "glg_em_controls_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_table_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_measurements_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_flags_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_loglik_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_expectation_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_prediction_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_used_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_env_stats_dev": (C.c_void_p, [C.c_void_p]),
+    "glg_em_totals_dev": (C.c_void_p, [C.c_void_p]),
     "glg_nccl_unique_id": (C.c_int, [C.c_void_p]),
     "glg_nccl_init": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "glg_allreduce_stats": (C.c_int, [C.c_void_p, _VP]),

@@ -36,6 +36,19 @@ smoothed one uses every observation in the window, which is what analysing a log
         env.step_rule_based_tensor()
         est.update(est.measurements() + sensor_noise)
     s = smoother.smooth()                             # s.mean [L, B, 28], s.cov and s.gain [L, B, 28, 28], oldest first
+
+DeviceNoiseEM -- an EM fit of the estimator's diagonal process and measurement noise (q_std, r_std) from the observations alone,
+over a smoother's window (csrc/glg_em.cuh behind glg_em_* in include/glgym.h).  It logs, beside the smoother's record, what a replay
+of the run needs (the controls, tables and measurements) and each update's log-likelihood term; its E-step steps the sigma points of
+every (env, slot) transition of the window in a few wide launches:
+
+    em = DeviceNoiseEM(smoother)                      # logs from the estimator's next reset on
+    start = env.state_dict()
+    est.reset()
+    for step in range(192):
+        env.step_rule_based_tensor()
+        est.update(est.measurements() + sensor_noise)
+    history = em.fit(start, iterations=10)            # estimate, set_noise, replay; history[-1].q_std / .r_std
 """
 import collections
 import ctypes as C
@@ -124,6 +137,7 @@ class DeviceStateEstimator(_EnvCompanion):
         super().__init__(env, "glg_est_create", cfg)
         self.measured = [MEASUREMENT_NAMES[i] for i in idx]
         self.p0_std, self.q_std, self.r_std = p0, q, r
+        self._staged = None  # set_noise's settings until the next reset
         e, L = self._obj, self._lib
         self.mean = self._view(L.glg_est_mean_dev(e), (28, B), "<f8").t()        # [B, 28] view of the [28][B] estimate
         self.cov = self._view(L.glg_est_cov_dev(e), (B, 28, 28), "<f8")
@@ -144,6 +158,7 @@ class DeviceStateEstimator(_EnvCompanion):
             keep = keep.t().contiguous()
             ptr = keep.data_ptr()
         _lib.check(self._lib.glg_est_reset(e, ptr, self.env._stream()), self.env._h, "glg_est_reset")
+        self._reset_noise()
 
     def update(self, y=None):
         """After each env step: predict over the interval the env just took, then update with y (float64 [B, 7] in
@@ -157,6 +172,25 @@ class DeviceStateEstimator(_EnvCompanion):
             self._y = yy.contiguous()  # kept alive until the next update: the kernels read it asynchronously
             ptr = self._y.data_ptr()
         _lib.check(self._lib.glg_est_update(e, ptr, self.env._stream()), self.env._h, "glg_est_update")
+
+    def set_noise(self, p0_std=None, q_std=None, r_std=None):
+        """Stages new noise settings (None keeps a setting); they take effect at the next reset(), so one smoother record never
+        mixes two noise models.  Validated as in the constructor."""
+        p0 = None if p0_std is None else _std_vector(p0_std, 28, "p0_std")
+        q = None if q_std is None else _std_vector(q_std, 28, "q_std")
+        r = None if r_std is None else _std_vector(r_std, 7, "r_std")
+        if r is not None and any(r[MEASUREMENT_NAMES.index(n)] <= 0 for n in self.measured):
+            raise ValueError("r_std must be > 0 for every measured entry")
+        e = self._live()
+        ptr = lambda a: 0 if a is None else a.ctypes.data
+        _lib.check(self._lib.glg_est_set_noise(e, ptr(p0), ptr(q), ptr(r)), self.env._h, "glg_est_set_noise")
+        cur = self._staged or (self.p0_std, self.q_std, self.r_std)
+        self._staged = tuple(old if new is None else new for new, old in zip((p0, q, r), cur))
+
+    def _reset_noise(self):
+        if self._staged is not None:
+            self.p0_std, self.q_std, self.r_std = self._staged
+            self._staged = None
 
     def measurements(self, obs=None):
         """The 7 measurement entries as float64 [B, 7] read from an observation batch (default: the env's current obs_t), zeros in
@@ -237,3 +271,143 @@ class DeviceStateSmoother(_EnvCompanion):
     cross_cov = property(lambda self: self._rolled("cross_cov"), doc="D [L, B, 28, 28]: sum Wc (chi - x^)(chi' - xbar)^T")
     status = property(lambda self: self._rolled("status"), doc="[L, B] the estimator's status bits of each slot")
     timestep = property(lambda self: self._rolled("timestep"), doc="[L, B] the env's timestep of each slot")
+
+
+EMStep = collections.namedtuple("EMStep", "q_std r_std loglik transitions measurements")
+
+
+def _mask(v, n, name, default):
+    if v is None:
+        return default.copy()
+    a = np.asarray(v)
+    if a.shape != (n,) or a.dtype != np.bool_:
+        raise ValueError(f"{name} must be a boolean mask of {n} entries")
+    return a.copy()
+
+
+class DeviceNoiseEM(_EnvCompanion):
+    """EM of the estimator's diagonal Q and R over `smoother`'s window.  Logs every reset / update of the estimator from its next
+    reset on; estimate() is one E-step and M-step over the logged window, replay() re-runs the logged window under the estimator's
+    current (staged) noise, fit() alternates them.  Keeps the smoother alive; close the EM object before closing the smoother.
+
+    fit_q / fit_r: boolean masks of the fitted entries (defaults: every state that takes part in smoothing, p0_std or q_std > 0,
+    except x27; every measured entry).  q_floor / r_floor: lower bounds of the fitted values (defaults: 1e-3 x the estimator
+    defaults).  max_points: sigma points per E-step launch (it bounds the memory of the internal handle that steps them)."""
+    _kind, _destroy = "EM object", "glg_em_destroy"
+
+    def __init__(self, smoother, fit_q=None, fit_r=None, q_floor=None, r_floor=None, max_points=MAX_SIGMA_POINTS):
+        if not isinstance(smoother, DeviceStateSmoother):
+            raise TypeError("smoother must be a DeviceStateSmoother")
+        if isinstance(max_points, bool) or not isinstance(max_points, (int, np.integer)) or not 57 <= int(max_points) <= MAX_SIGMA_POINTS:
+            raise ValueError(f"max_points must be an integer in 57 .. {MAX_SIGMA_POINTS}")
+        est = smoother.est
+        active = (np.asarray(est.p0_std) > 0) | (np.asarray(est.q_std) > 0)
+        active[27] = False
+        measured = np.zeros(7, dtype=bool)
+        measured[[MEASUREMENT_NAMES.index(n) for n in est.measured]] = True
+        self.fit_q = _mask(fit_q, 28, "fit_q", active)
+        self.fit_r = _mask(fit_r, 7, "fit_r", measured)
+        if self.fit_q[27]:
+            raise ValueError("fit_q: x27, the day counter, is deterministic and never fitted")
+        if np.any(self.fit_r & ~measured):
+            raise ValueError("fit_r may only select measured entries")
+        self.q_floor = _std_vector(1e-3 * np.asarray(DEFAULT_Q_STD) if q_floor is None else q_floor, 28, "q_floor")
+        self.r_floor = _std_vector(1e-3 * np.asarray(DEFAULT_R_STD) if r_floor is None else r_floor, 7, "r_floor")
+        W, B = smoother.window, int(est.env.num_envs)
+        self.smoother, self.est, self.env, self._lib, self.window = smoother, est, est.env, est._lib, W
+        self._obj = C.c_void_p()
+        _lib.check(self._lib.glg_em_create(smoother._live(), int(max_points), C.byref(self._obj)), self.env._h, "glg_em_create")
+        m, L = self._obj, self._lib
+        self._log = {"controls": self._view(L.glg_em_controls_dev(m), (W, 6, B), "<f8").permute(0, 2, 1),
+                     "table": self._view(L.glg_em_table_dev(m), (W, B), "<i4"),
+                     "measurements": self._view(L.glg_em_measurements_dev(m), (W, 7, B), "<f8").permute(0, 2, 1),
+                     "flags": self._view(L.glg_em_flags_dev(m), (W, B), "|u1"),
+                     "loglik": self._view(L.glg_em_loglik_dev(m), (W, B), "<f8")}
+        self._expectation = self._view(L.glg_em_expectation_dev(m), (W, B, 35), "<f8")
+        self._prediction = self._view(L.glg_em_prediction_dev(m), (W, 28, B), "<f8").permute(0, 2, 1)
+        self._used = self._view(L.glg_em_used_dev(m), (W, B), "|u1")
+        self.env_stats = self._view(L.glg_em_env_stats_dev(m), (B, 38), "<f8")  # 35 sums, transitions, measured slots, sum of l
+        self.totals = self._view(L.glg_em_totals_dev(m), (38,), "<f8")
+        self.bytes = int(L.glg_em_bytes(m))
+        self.chunk_pairs = int(L.glg_em_chunk_pairs(m))
+
+    def _live(self):
+        self.smoother._live()
+        return super()._live()
+
+    def _rolled(self, name):
+        """A logged quantity, oldest first (a copy: the log is a ring)."""
+        m = self._live()
+        n, first = self.smoother.length, int(self._lib.glg_smooth_first(self.smoother._obj))
+        return torch.roll(self._log[name], -first, 0)[:n]
+
+    controls = property(lambda self: self._rolled("controls"), doc="[L, B, 6] the controls each env applied; 0 at a reset slot")
+    tables = property(lambda self: self._rolled("table"), doc="[L, B] the weather table of each slot's step")
+    measurements = property(lambda self: self._rolled("measurements"), doc="[L, B, 7] y as given; 0 where not measured")
+    flags = property(lambda self: self._rolled("flags"), doc="[L, B] bit 0: y was given; bit 1: the update was applied")
+    loglik = property(lambda self: self._rolled("loglik"), doc="[L, B] each update's log-likelihood term; 0 where none applied")
+
+    @property
+    def prediction(self):
+        """[L, B, 28] fbar of the last estimate(): the smoothed one-step prediction (0 where no transition leads to the slot)."""
+        return self._prediction[:self.smoother.length]
+
+    @property
+    def expectation(self):
+        """[L, B, 35] of the last estimate(): the 28 Q terms E_k, then the 7 R terms; 0 where a slot does not enter a sum."""
+        return self._expectation[:self.smoother.length]
+
+    @property
+    def used(self):
+        """[L, B] of the last estimate(): bit 0: the slot's transition entered the Q sums; bit 1: its measurement the R sums."""
+        return self._used[:self.smoother.length]
+
+    def estep(self):
+        """Runs the smoother, then the E-step over its output (device views expectation, prediction, used, env_stats, totals)."""
+        self.smoother.smooth()
+        _lib.check(self._lib.glg_em_estep(self._live(), self.env._stream()), self.env._h, "glg_em_estep")
+
+    def estimate(self):
+        """One E-step and M-step: EMStep(q_std, r_std, loglik, transitions, measurements).  loglik is the log-likelihood of the
+        logged window under the noise it was filtered with; q_std and r_std are the maximisers for the fitted entries, floored, and
+        the estimator's current values elsewhere."""
+        self.estep()
+        tot = self.totals.cpu().numpy()
+        ntr, nme = int(round(tot[35])), int(round(tot[36]))
+        q, r = np.array(self.est.q_std, dtype=np.float64), np.array(self.est.r_std, dtype=np.float64)
+        if ntr > 0:
+            q[self.fit_q] = np.maximum(np.sqrt(np.maximum(tot[:28] / ntr, 0.0)), self.q_floor)[self.fit_q]
+        if nme > 0:
+            r[self.fit_r] = np.maximum(np.sqrt(np.maximum(tot[28:35] / nme, 0.0)), self.r_floor)[self.fit_r]
+        return EMStep(q, r, float(tot[37]), ntr, nme)
+
+    def replay(self, env_state, x0=None):
+        """Re-runs the logged window: restores the env from env_state (its state_dict() taken before the logged reset), resets the
+        estimator (x0 as given to that reset), then steps the env with the logged controls and updates the estimator with the
+        logged measurements (None where the logged update had none).  A run can be replayed when each update followed one env step
+        and the log holds the whole run (at most `window` slots since the reset)."""
+        m = self._live()
+        n = int(self._lib.glg_em_logged(m))
+        if n == 0:
+            raise RuntimeError("nothing logged yet: the log starts with the estimator's first reset after the EM object's creation")
+        if n > self.window:
+            raise RuntimeError(f"the run has {n} slots and the log keeps the last {self.window}: it cannot be replayed")
+        u, y, flags = self.controls.clone(), self.measurements.clone(), self.flags.cpu().numpy()
+        self.env.load_state_dict(env_state)
+        self.est.reset(x0)
+        for k in range(1, n):
+            self.env.step_raw_control_tensor(u[k])
+            self.est.update(y[k] if np.any(flags[k] & 1) else None)
+
+    def fit(self, env_state, iterations, x0=None):
+        """`iterations` rounds of estimate(), set_noise(q_std, r_std) and replay(); returns the list of EMSteps (the loglik of step
+        i is that of the noise the step started from)."""
+        if isinstance(iterations, bool) or not isinstance(iterations, (int, np.integer)) or int(iterations) < 1:
+            raise ValueError("iterations must be an integer >= 1")
+        history = []
+        for _ in range(int(iterations)):
+            step = self.estimate()
+            history.append(step)
+            self.est.set_noise(q_std=step.q_std, r_std=step.r_std)
+            self.replay(env_state, x0)
+        return history

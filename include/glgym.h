@@ -434,6 +434,64 @@ double *glg_smooth_cross_dev(glg_smooth *s);          /* [W][B][28][28] D */
 uint8_t *glg_smooth_status_dev(glg_smooth *s);        /* [W][B] */
 int32_t *glg_smooth_timestep_dev(glg_smooth *s);      /* [W][B] */
 
+/* Noise settings that can change: p0_std, q_std, r_std (host arrays of 28, 28 and 7 doubles; NULL keeps a setting), validated as
+ * in glg_est_create.  They are staged and take effect at the next glg_est_reset, so one record never mixes two noise models; that
+ * reset also recomputes the smoother's deterministic-state mask.  GLG_ERR_ARG for a NULL estimator or a bad setting. */
+int glg_est_set_noise(glg_est *e, const double *p0_std, const double *q_std, const double *r_std);
+
+/* ---- noise identification: the E-step of an EM fit of the estimator's diagonal Q and R over a smoother's window -----------------
+ * An EM object belongs to one smoother, as the smoother belongs to an estimator.  Notation as in the filter and smoother contracts.
+ *   Log: from the estimator's next glg_est_reset on, per ring slot of the smoother and env: the controls the env applied (double
+ *     [W][6][B]; 0 at a reset slot), the env's weather table ([W][B]), the measurement y_dev as given ([W][7][B]; 0 where not
+ *     measured or y_dev is NULL), flags ([W][B]: bit 0 y_dev was non-NULL, bit 1 the update was applied: y_dev non-NULL and status
+ *     0), and l = -(v^T S^-1 v + log det S + m log 2 pi) / 2 from the UT kernel's Cholesky of S and the innovation v (0 where no
+ *     update was applied).  Logging does not change a bit of the estimator's outputs or of the smoother's record.
+ *   E-step (glg_em_estep), over the smoother's output of its last glg_smooth_run (ms, Ps, G, oldest first); L is a factor by the
+ *     filter's zero-column rule, the weights and gamma are the estimator's.
+ *     Q term, for every slot k whose predecessor k-1 is in the window and linked to it (no status bit 1, 4 or 8 at k):
+ *       chi_i: the sigma points of (ms_{k-1}, Ps_{k-1}); f_i one interval of the env's nominal model from chi_i with slot k's
+ *       logged controls and table at pre-step timestep timestep_k - 1 (weather row min(k, rows - Np - 1)): the interval the
+ *       filter's update stepped.  fbar = sum Wm_i f_i, Phi = sum Wc_i (f_i - fbar)(f_i - fbar)^T in ascending i;
+ *       Delta_j = Wi gamma (f_{j+} - f_{j-}) (row j), Z = L^-T Delta by back substitution (a component whose column of L is zero is
+ *       0), C = (Ps_k G_{k-1}^T) Z;  E_k = diag[Ps_k + (ms_k - fbar)(ms_k - fbar)^T + Phi - C - C^T].
+ *       E_k is the expectation of (x_k - f(x_{k-1}))^2 under the smoothed joint of (x_{k-1}, x_k), with the cross term from the
+ *       Gaussian regression of x_k on x_{k-1}; for f(x) = A x it is Shumway-Stoffer's.  A transition whose stepped point is
+ *       non-finite (its EM env done before the season's end) is left out.
+ *     R term, for every slot with the applied flag: the sigma points of (ms_k, Ps_k) through h;
+ *       E_r = (y_r - hbar_r)^2 + sum Wc_i (h_ir - hbar_r)^2 for each measured entry r.
+ *     Sums: per env in ascending slot order, then pooled in ascending env order; no atomics, so the result is deterministic.
+ *   The points of all (env, slot) pairs are stepped by the unchanged step kernels of an internal handle (the EM handle, created
+ *   like the estimator's shadow handle) in balanced chunks of at most max_points points, each stepped as a batch of exactly its
+ *   own points (no padding, also while the window is not yet full): per chunk the sigma kernel, the step and the expectation
+ *   kernel; then two reduction kernels.  The M-step (q_j^2 = pooled E_j / transitions, r_r^2 = pooled R_r /
+ *   measured slots) is the caller's: glgym.estimation.DeviceNoiseEM.
+ * Destroy the EM object before its smoother; one whose smoother or estimator is gone can only be destroyed (glg_em_estep returns
+ * GLG_ERR_STATE).  glg_set_weather on the env makes glg_em_estep return GLG_ERR_STATE.  Errors are reported through glg_last_error
+ * of the env handle. */
+typedef struct glg_em glg_em;
+/* max_points: sigma points per launch, 0 = 4194304, else 57 .. 4194304 (it bounds the EM handle's memory).  GLG_ERR_ARG for NULLs
+ * or a bad max_points, GLG_ERR_STATE if the smoother already has an EM object or its estimator is gone. */
+int glg_em_create(glg_smooth *s, int64_t max_points, glg_em **out);
+void glg_em_destroy(glg_em *m);
+/* The E-step over the smoother's output.  GLG_ERR_STATE before the first logged reset, or when the record changed since the last
+ * glg_smooth_run.  Launches: 3 per chunk, then 2. */
+int glg_em_estep(glg_em *m, void *stream);
+int64_t glg_em_bytes(const glg_em *m);        /* device bytes of the log, the outputs and the EM envs' controls (not the EM handle) */
+int64_t glg_em_logged(const glg_em *m);       /* slots logged since the estimator's last reset (more than W: the oldest are gone) */
+int32_t glg_em_chunk_pairs(const glg_em *m);  /* most (env, slot) pairs per launch: min(B W, max_points / 57) */
+/* the log, in the smoother's ring order (glg_smooth_first names the oldest slot) */
+double *glg_em_controls_dev(glg_em *m);       /* [W][6][B] */
+int32_t *glg_em_table_dev(glg_em *m);         /* [W][B] */
+double *glg_em_measurements_dev(glg_em *m);   /* [W][7][B] */
+uint8_t *glg_em_flags_dev(glg_em *m);         /* [W][B] */
+double *glg_em_loglik_dev(glg_em *m);         /* [W][B] l */
+/* written by glg_em_estep, oldest first */
+double *glg_em_expectation_dev(glg_em *m);    /* [W][B][35]: E_k (28), then the R terms (7); 0 where a slot enters no sum */
+double *glg_em_prediction_dev(glg_em *m);     /* [W][28][B] fbar: the smoothed one-step prediction; 0 where no transition */
+uint8_t *glg_em_used_dev(glg_em *m);          /* [W][B] bit 0: the slot's transition entered the Q sums; bit 1: its R terms */
+double *glg_em_env_stats_dev(glg_em *m);      /* [B][38] per env: the 35 sums, transitions, measured slots, sum of l */
+double *glg_em_totals_dev(glg_em *m);         /* [38] pooled over the envs */
+
 /* Multi-GPU episode statistics (SURVEY 8e): the step path has no collective; the one exchange is a sum of the 16-entry
  * statistics vector over the ranks' handles, once per logging interval -- ncclAllReduce on the handle's device buffer.
  * NCCL is bound at run time (dlopen of libnccl.so.2, the copy torch already loaded when there is one), so libglgym.so has no
